@@ -10,16 +10,22 @@ envs are independent, sharded by index, no collective on the step path), uniform
 max_steps=100, auto-reset on.  A "step" is one ts_step launch advancing every env by one action.
 
 How a number is taken (DESIGN.md section 6):
-  * the K steps of a block are one CUDA graph of K ts_step launches (one launch per step); after
-    the W warm-up steps the graph is replayed until the GPU has been busy for >= 150 ms, so the
-    graph is resident and the SM clock has left its idle state before anything is timed (the
-    round-1 line timed 1.5 ms straight after start-up and read 2x slow on 8 GPUs);
-  * R blocks of exactly K steps are then timed back to back with CUDA events on the launching
-    stream; per block the job time is the MAX over ranks; `value` comes from the MEDIAN block,
-    and the line carries first / best / worst block and per-rank [min, median, max] so that a
-    straggler is visible instead of folded into the headline;
-  * NVML clocks / throttle reasons are read by the main thread while the GPU works through the
-    queued blocks (no polling thread competing with the launches).
+  * a block of K steps is replayed from CUDA graphs of up to 50 ts_step launches each (one
+    launch per step); after the W warm-up steps blocks are replayed until the GPU has been busy
+    for >= 150 ms, so the graphs are resident and the SM clock has left its idle state before
+    anything is timed (the round-1 line timed 1.5 ms straight after start-up and read 2x slow on
+    8 GPUs);
+  * the batch is then reset to its initial boards, whole blocks of at least 256 steps in all
+    run untimed back to back, and exactly K steps are timed right behind them with CUDA events
+    on the launching stream, so that they run under continuous load and are queued before the
+    GPU reaches them; the job time is the MAX over ranks, and the line carries first / best /
+    worst graph chunk and per-rank [min, median, max] so that a straggler is visible instead of
+    folded into the headline;
+  * what those K steps compute depends only on the arguments: the same puzzles, action rows and
+    start state on every run, so `--dump-outputs DIR` can store the last step's outputs for
+    comparing two builds;
+  * NVML clocks / throttle reasons are read by the main thread every 0.5 ms while the GPU works
+    through the untimed and the timed steps (no polling thread competing with the launches).
 `value` = total env-steps/s over all ranks with actions resident in HBM.  `e2e` = the same step
 driven from pinned HOST buffers through ts_step_host (actions uploaded, reward+done downloaded
 every step).  `roofline` = algorithmic bytes (3T + ceil(S^2/8) + 8 per env-step, SURVEY 8(d)) over
@@ -67,8 +73,10 @@ METRIC = "env-steps/sec at 1/2/4/8 B200 and % HBM roofline vs reference CPU step
 UNIT = "env-steps/s"
 N_ACTION_ROWS = 8                               # distinct pre-generated action vectors, cycled
 GRAPH_STEPS_MAX = 50                            # launches per captured graph
-RAMP_MS = 150.0                                 # GPU-busy time before the timed blocks
+RAMP_MS = 150.0                                 # GPU-busy time before the timed steps
+PREROLL_STEPS = 256                             # untimed steps right before the timed ones (whole blocks)
 L2_BYTES = 126e6
+DUMP_BYTES = 60_000_000                         # --dump-outputs: array bytes written, at most
 
 
 def bytes_moved(cfg: Config, ts) -> dict:
@@ -99,6 +107,23 @@ def workload_config(cfg: Config, n_gpus: int, envs_per_gpu: int, extra: dict | N
     if extra:
         out.update(extra)
     return out
+
+
+def dump_outputs(env, out_dir: str) -> None:
+    """What the last step returned to its caller -- state (as tile positions), reward, done -- as
+    float32 .npy files in out_dir, with the float64 indices of the envs they belong to.  Above
+    DUMP_BYTES the envs are a fixed, seeded sample, the same for every build and run."""
+    import numpy as np
+    import torch
+    n = env.n_envs
+    m = min(n, DUMP_BYTES // (4 * (2 * env.n_tiles + 2) + 8))
+    idx = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    sel = torch.from_numpy(idx).to(env.device)
+    arrays = {"env_index": idx.astype(np.float64), "positions": env.positions()[sel].float().cpu().numpy(),
+              "reward": env.reward[sel].cpu().numpy(), "done": env.done[sel].float().cpu().numpy()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -288,7 +313,7 @@ class Clocks:
         s = sorted(self.samples)
         return {"sm_mhz": s[len(s) // 2] if s else None, "sm_min_mhz": s[0] if s else None, "sm_max_mhz": self.max_mhz,
                 "samples": len(s), "reasons": sorted(self.reasons),
-                "how": "NVML, main thread, while the GPU executes the queued timed blocks"}
+                "how": "NVML, main thread, while the GPU executes the untimed steps before the timed ones and the timed ones"}
 
 
 # ------------------------------------------------------------------------------------------
@@ -333,8 +358,8 @@ class Runner:
         self.dist.all_gather_into_tensor(out, mine)
         return out.view(self.world, -1).tolist()
 
-    def measure(self, cfg: Config, n_local: int, steps: int, warmup: int, use_graph: bool = True, max_blocks: int = 30,
-                budget_s: float = 0.4, clocks: Clocks | None = None, ramp_ms: float = RAMP_MS) -> dict:
+    def measure(self, cfg: Config, n_local: int, steps: int, warmup: int, use_graph: bool = True,
+                clocks: Clocks | None = None, ramp_ms: float = RAMP_MS, dump_dir: str | None = None) -> dict:
         """Device-resident throughput of one config (see the module docstring)."""
         torch, ts = self.torch, self.ts
         env = ts.BatchedTilerSliderEnv.synthetic(n_local, cfg.size, cfg.tiles, cfg.walls, cfg.multi, seed=cfg.puzzle_seed,
@@ -344,75 +369,85 @@ class Runner:
         actions = torch.randint(0, 4, (N_ACTION_ROWS, env.capacity), dtype=torch.uint8, device=self.dev, generator=gen)
         for k in range(warmup):                                   # the W warm-up steps, launched one by one
             env.step(actions[k % N_ACTION_ROWS])
+        # a block is `steps` steps in chunks of at most GRAPH_STEPS_MAX; step k of a chunk takes action row k
         cs = min(steps, GRAPH_STEPS_MAX)
         n_rep, rem = divmod(steps, cs)
+        chunks = [cs] * n_rep + ([rem] if rem else [])
         if use_graph:
             rows = actions[torch.arange(cs, device=self.dev) % N_ACTION_ROWS] if cs > N_ACTION_ROWS else actions[:cs]
-            g_main = env.capture_steps(rows.contiguous())
-            g_rem = env.capture_steps(rows[:rem].contiguous()) if rem else None
+            graphs = {cs: env.capture_steps(rows.contiguous())}
+            if rem:
+                graphs[rem] = env.capture_steps(rows[:rem].contiguous())
 
-            def block():
-                for _ in range(n_rep):
-                    g_main.replay()
-                if g_rem is not None:
-                    g_rem.replay()
+            def chunk(n):
+                graphs[n].replay()
         else:
-            def block():
-                for k in range(steps):
+            def chunk(n):
+                for k in range(n):
                     env.step(actions[k % N_ACTION_ROWS])
+
+        def block():
+            for n in chunks:
+                chunk(n)
         # graph upload + clock ramp: keep the GPU busy for RAMP_MS before anything is timed
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         block()
         torch.cuda.synchronize()
-        ramp_blocks, busy_ms, est_ms = 1, 0.0, None
-        while busy_ms < ramp_ms or est_ms is None:
+        ramp_blocks, busy_ms = 1, 0.0
+        while ramp_blocks == 1 or busy_ms < ramp_ms:
             ev0.record()
             block()
             ev1.record()
             ev1.synchronize()
-            est_ms = ev0.elapsed_time(ev1)
-            busy_ms += est_ms
+            busy_ms += ev0.elapsed_time(ev1)
             ramp_blocks += 1
-        n_blocks = int(max(5, min(max_blocks, budget_s * 1e3 / max(est_ms, 1e-3))))
-        n_blocks = int(min(r[0] for r in self.gather([float(n_blocks)])))     # the same count on every rank
-        starts = [torch.cuda.Event(enable_timing=True) for _ in range(n_blocks)]
-        stops = [torch.cuda.Event(enable_timing=True) for _ in range(n_blocks)]
         self.barrier()
-        for b in range(n_blocks):                                 # R blocks of exactly `steps` launches, back to back
-            starts[b].record()
+        # back to the initial boards, so that what the timed steps compute does not depend on how long
+        # the ramp ran; then untimed blocks back to back, so that the timed steps run under continuous
+        # load as they would in a long run
+        env.reset()
+        pre_blocks = -(-PREROLL_STEPS // steps)
+        for _ in range(pre_blocks):
             block()
-            stops[b].record()
-        if clocks is not None:
-            clocks.sample_until(stops[-1])
+        marks = [torch.cuda.Event(enable_timing=True) for _ in range(len(chunks) + 1)]
+        marks[0].record()
+        for i, n in enumerate(chunks):                            # exactly `steps` timed launches, back to back
+            chunk(n)
+            marks[i + 1].record()
+        if clocks is not None:          # from the untimed steps on: a throttle they bring on shows too
+            clocks.sample_until(marks[-1])
         self.barrier()
-        mine = [starts[b].elapsed_time(stops[b]) for b in range(n_blocks)]
-        per_rank = self.gather(mine)                              # [world][blocks] ms
-        job = sorted(max(per_rank[r][b] for r in range(self.world)) for b in range(n_blocks))
-        first = max(per_rank[r][0] for r in range(self.world))
-        med = job[n_blocks // 2]
+        if dump_dir is not None and self.rank == 0:
+            dump_outputs(env, dump_dir)
+        mine = [marks[i].elapsed_time(marks[i + 1]) / n for i, n in enumerate(chunks)] + [marks[0].elapsed_time(marks[-1])]
+        per_rank = self.gather(mine)                              # [world][chunks + 1]: ms per step of each chunk, total ms
+        total = max(r[-1] for r in per_rank)
+        per_chunk = [max(r[i] for r in per_rank) for i in range(len(chunks))]
         total_envs = n_local * self.world
-        per_launch_s = med * 1e-3 / steps
+        per_launch_s = total * 1e-3 / steps
         achieved = cfg.algo_bytes * n_local / per_launch_s / 1e9
         moved = bytes_moved(cfg, ts)
         wins = int(self.gather([float(env.is_won().sum())])[0][0]) if self.world == 1 else \
             int(sum(r[0] for r in self.gather([float(env.is_won().sum())])))
         kernel = f"ts::step_kernel<{cfg.size},{cfg.tiles}>" if cfg.size <= 8 else f"ts::wide_step_kernel<{cfg.tiles}>"
-        out = {"value": total_envs * steps / (med * 1e-3), "ms_per_step": med / steps,
-               "blocks": {"n": n_blocks, "steps_per_block": steps, "statistic": "median over blocks of (max over ranks)",
-                          "first_ms_per_step": first / steps, "best_ms_per_step": job[0] / steps,
-                          "worst_ms_per_step": job[-1] / steps,
-                          "per_rank_ms_per_step_min_med_max": [[min(r) / steps, sorted(r)[len(r) // 2] / steps, max(r) / steps]
+        out = {"value": total_envs * steps / (total * 1e-3), "ms_per_step": total / steps,
+               "blocks": {"n": len(chunks), "steps_per_block": cs,
+                          "statistic": "value: all timed steps back to back (max over ranks); first / best / worst and "
+                                       "per rank: per graph chunk of up to 50 of them",
+                          "first_ms_per_step": per_chunk[0], "best_ms_per_step": min(per_chunk),
+                          "worst_ms_per_step": max(per_chunk),
+                          "per_rank_ms_per_step_min_med_max": [[min(r[:-1]), sorted(r[:-1])[len(chunks) // 2], max(r[:-1])]
                                                                for r in per_rank]},
-               "warmup_launches": warmup + ramp_blocks * steps,
+               "warmup_launches": warmup + (ramp_blocks + pre_blocks) * steps,
                "roofline": {"bound": "hbm", "achieved": achieved, "peak": self.peak, "unit": "GB/s", "frac": achieved / self.peak,
                             "traffic": None, "kernel": kernel,
                             "algorithmic_bytes_per_launch": cfg.algo_bytes * n_local, "avg_launch_ms": per_launch_s * 1e3,
                             "bytes_moved_per_env_step": moved,
                             "frac_on_bytes_moved": moved["total"] * n_local / per_launch_s / 1e9 / self.peak,
-                            "per_rank_frac": [cfg.algo_bytes * n_local / (sorted(r)[len(r) // 2] * 1e-3 / steps) / 1e9 / self.peak
+                            "per_rank_frac": [cfg.algo_bytes * n_local / (r[-1] * 1e-3 / steps) / 1e9 / self.peak
                                               for r in per_rank],
                             "peak_source": self.peak_source},
-               "gpu_launches": n_blocks * steps, "wins_in_last_step": wins, "cuda_graph": bool(use_graph),
+               "gpu_launches": steps, "wins_in_last_step": wins, "cuda_graph": bool(use_graph),
                "envs_per_gpu": n_local}
         traffic = ncu_traffic(cfg, n_local)
         if traffic:
@@ -567,7 +602,7 @@ def run_ours(args) -> int:
     n_local = args.envs
     clk = Clocks(R.local)
     head = R.measure(cfg, n_local, args.steps, args.warmup, use_graph=args.graph, clocks=clk, ramp_ms=args.ramp_ms,
-                     max_blocks=args.max_blocks)
+                     dump_dir=args.dump_outputs)
     clocks = clk.summary()
     e2e = R.e2e(cfg, n_local, max(3, min(args.steps, args.e2e_steps))) if args.e2e_steps > 0 else None
     line = {"metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": R.world, "steps": args.steps,
@@ -582,14 +617,14 @@ def run_ours(args) -> int:
         # BASELINE's literal "16M envs sharded over 1/2/4/8": the config's env count split over the ranks
         if R.world > 1 and args.scaling == "weak":
             n_strong = -(-cfg.envs // R.world)
-            s = R.measure(cfg, n_strong, args.steps, 3, max_blocks=15, budget_s=0.15)
+            s = R.measure(cfg, n_strong, args.steps, 3)
             line["strong_scaling"] = {"envs_total": n_strong * R.world, "envs_per_gpu": n_strong, "value": s["value"],
                                       "ms_per_step": s["ms_per_step"], "roofline_frac": s["roofline"]["frac"], "blocks": s["blocks"]}
         for name in ("c2", "c3", "c4"):
             if name == args.config:
                 continue
             c = CONFIGS[name]
-            m = R.measure(c, c.envs, args.steps, 3, max_blocks=15, budget_s=0.15)
+            m = R.measure(c, c.envs, args.steps, 3)
             extra[name] = {"value": m["value"], "unit": UNIT, "ms_per_step": m["ms_per_step"],
                            "config": workload_config(c, R.world, c.envs), "roofline": m["roofline"], "blocks": m["blocks"],
                            "gpu_launches": m["gpu_launches"]}
@@ -629,11 +664,14 @@ def main() -> int:
     ap.add_argument("--no-extra", action="store_true", help="headline config only (no `configs`, no strong-scaling figure)")
     ap.add_argument("--no-graph", dest="graph", action="store_false",
                     help="launch every step from Python instead of replaying CUDA graphs")
-    ap.add_argument("--ramp-ms", type=float, default=RAMP_MS, help="GPU-busy time before the timed blocks (profiling runs: 0)")
-    ap.add_argument("--max-blocks", type=int, default=30, help="upper bound on the timed blocks (profiling runs: 5)")
+    ap.add_argument("--ramp-ms", type=float, default=RAMP_MS, help="GPU-busy time before the timed steps (profiling runs: 0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the headline config returned "
+                    "(a fixed sample of envs) to DIR/<name>.npy, to compare two builds output for output")
     ap.add_argument("--bfs-puzzles", type=int, default=65_536, help="c5: puzzles per GPU")
     ap.add_argument("--bfs-check", type=int, default=1024, help="c5: puzzles cross-checked against the CPU oracle's BFS")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     if args.envs is None:
         world = int(os.environ.get("WORLD_SIZE", "1"))

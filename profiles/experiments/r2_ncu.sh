@@ -2,7 +2,7 @@
 # Round-2 ncu captures (one gpurun call).  Every command first runs plain; ncu only after it exited 0.
 set -x
 O=gpurun_out
-B="python bench.py --steps 20 --warmup 5 --no-extra --no-cpu --ramp-ms 0 --max-blocks 5 --e2e-steps 0"
+B="python bench.py --steps 20 --warmup 5 --no-extra --no-cpu --ramp-ms 0 --e2e-steps 0"
 NCU="ncu --set full --clock-control none --import-source on"
 $B --config c3 > $O/r2_plain_c3.log 2>&1 || exit 1
 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/r2_launches_c3.csv $B --config c3 > $O/r2_ncu_launches.log 2>&1

@@ -71,7 +71,8 @@ class Tally:
 def main() -> int:
     ap = argparse.ArgumentParser()
     ap.add_argument("--impl", choices=["adapter", "reference"], default="adapter")
-    ap.add_argument("--reference", default=os.environ.get("TS_REFERENCE", "/root/reference"))
+    ap.add_argument("--reference", default=os.environ.get("TS_REFERENCE"), required=not os.environ.get("TS_REFERENCE"),
+                    help="checkout of the reference (default: $TS_REFERENCE)")
     args = ap.parse_args()
     install(args.impl, args.reference)
     import pytest
