@@ -387,6 +387,64 @@ int ts_bfs_local_ctas_per_sm(const ts_bfs_local_args *a, int *ctas_per_sm, int *
 int ts_bfs_local(const ts_bfs_local_args *a, int grid, void *stream);
 
 /* ---------------------------------------------------------------------------------------
+ * K7 ts_synth_candidates: candidate puzzles for a generator that keeps the ones K6 grades into a
+ * band of shortest-solution lengths (csrc/ts_generate.cu; no reference counterpart).  One thread
+ * per listed env: puzzle of env slot d_env_ids[i] (i < n_items; NULL: slot i; ids outside
+ * [0, capacity) are skipped) written to walls / targets / init / pos.  The random stream is a
+ * function of (seed, attempt, global env index = env_index_base + slot) only.
+ *   recipe TS_RECIPE_UNIFORM: K0's draw.  attempt 0 writes exactly the puzzle ts_synth writes for
+ *          that env; attempt a > 0 draws with the seed splitmix64(seed ^ a * 0xA0761D6478BD642F).
+ *   recipe TS_RECIPE_WALK: walls and tiles as K0 (the first n_walls + n_tiles cells of the same
+ *          permutation, same seed rule), then walk_len moves, each drawn uniformly among the moves
+ *          that change the state (one 32-bit draw of the same stream per move: the k-th of the n
+ *          such moves in UP, DOWN, LEFT, RIGHT order, k = draw * n >> 32); the walk stops early
+ *          when no move changes the state.  Targets = the final positions (ordered goal: tile i's;
+ *          set goal: the cells).  Every such puzzle is solvable.
+ * Domain: size <= 8, 1 <= n_tiles <= 4 (what K6 grades).
+ * ------------------------------------------------------------------------------------- */
+#define TS_RECIPE_UNIFORM 0
+#define TS_RECIPE_WALK 1
+#define TS_MAX_WALK 65535
+typedef struct ts_synth_candidates_args {
+    int32_t size, n_tiles, n_walls, goal_mode;
+    int32_t recipe, walk_len, attempt, reserved0;
+    int64_t n_items, capacity, env_index_base;
+    uint64_t seed;
+    const int32_t *d_env_ids;
+    uint8_t *d_walls, *d_targets_packed, *d_init, *d_pos;
+} ts_synth_candidates_args;
+int ts_synth_candidates(const ts_synth_candidates_args *a, void *stream);
+
+/* ---------------------------------------------------------------------------------------
+ * K8 ts_pool_reset: auto-reset into a pool of puzzles (csrc/ts_generate.cu; no reference
+ * counterpart -- TilerSliderEnv.reset, environment.py:89-97, restarts the same puzzle).  For every
+ * env of [first_env, first_env + n_envs) whose d_done byte is set (d_done = NULL: every env):
+ *   j = H(seed, env_index_base + env, d_episode[env]) in [0, n_pool), d_episode[env] += 1,
+ *   walls / targets / init <- pool puzzle j, pos <- init, step_count <- 0,
+ *   d_solve_depth[env] <- d_pool_depth[j] (when both are given).
+ * H(seed, g, e) = (mix(mix(seed ^ (g + 1) * 0xD1B54A32D192ED03) ^ (e + 1) * 0x9E3779B97F4A7C15) * n_pool) >> 64
+ * with mix the splitmix64 finaliser (64x64 -> high 64 bits).  The pool is a packed batch of the
+ * same size, tile count and goal mode (any board class, any tile count up to TS_MAX_TILES) with
+ * stride pool_capacity.  Meant to run right after ts_step (it reads the done bytes the step wrote);
+ * it is launched with programmatic dependent launch like the step.  Touches nothing outside the
+ * range.
+ * ------------------------------------------------------------------------------------- */
+typedef struct ts_pool_reset_args {
+    int32_t size, n_tiles, goal_mode, count_bytes;
+    int64_t first_env, n_envs, capacity, env_index_base;
+    uint64_t seed;
+    const uint8_t *d_done;
+    uint32_t *d_episode;
+    uint8_t *d_walls, *d_targets_packed, *d_init, *d_pos;
+    void *d_step_count;
+    int32_t *d_solve_depth;
+    int64_t n_pool, pool_capacity;
+    const uint8_t *d_pool_walls, *d_pool_targets, *d_pool_init;
+    const int32_t *d_pool_depth;
+} ts_pool_reset_args;
+int ts_pool_reset(const ts_pool_reset_args *a, void *stream);
+
+/* ---------------------------------------------------------------------------------------
  * ts_step_host: the same step through HOST buffers (the call a host-side driver makes):
  * h_actions (pinned) -> device, ts_step, reward/done -> h_reward/h_done (pinned), pipelined in
  * chunks over the context's streams; returns after everything has landed.

@@ -20,6 +20,8 @@ MAX_SIZE = 16
 MAX_TILES = 32        # 0..8: register kernels; 9..32: per-env generic kernels
 F_DONE, F_WON, F_INVALID, F_TIMEOUT, F_STALE = 1, 2, 4, 8, 16
 GOAL_ORDERED, GOAL_SET = 0, 1
+RECIPE_UNIFORM, RECIPE_WALK = 0, 1
+MAX_WALK = 65535
 
 _vp, _i32, _i64, _f32 = C.c_void_p, C.c_int32, C.c_int64, C.c_float
 
@@ -91,6 +93,22 @@ class BfsLocalArgs(C.Structure):
                 ("d_levels", _vp), ("d_counters", _vp), ("d_moves", _vp), ("d_lengths", _vp), ("max_moves", _i64)]
 
 
+class SynthCandidatesArgs(C.Structure):
+    _fields_ = [("size", _i32), ("n_tiles", _i32), ("n_walls", _i32), ("goal_mode", _i32),
+                ("recipe", _i32), ("walk_len", _i32), ("attempt", _i32), ("reserved0", _i32),
+                ("n_items", _i64), ("capacity", _i64), ("env_index_base", _i64), ("seed", C.c_uint64),
+                ("d_env_ids", _vp), ("d_walls", _vp), ("d_targets_packed", _vp), ("d_init", _vp), ("d_pos", _vp)]
+
+
+class PoolResetArgs(C.Structure):
+    _fields_ = [("size", _i32), ("n_tiles", _i32), ("goal_mode", _i32), ("count_bytes", _i32),
+                ("first_env", _i64), ("n_envs", _i64), ("capacity", _i64), ("env_index_base", _i64),
+                ("seed", C.c_uint64), ("d_done", _vp), ("d_episode", _vp),
+                ("d_walls", _vp), ("d_targets_packed", _vp), ("d_init", _vp), ("d_pos", _vp),
+                ("d_step_count", _vp), ("d_solve_depth", _vp), ("n_pool", _i64), ("pool_capacity", _i64),
+                ("d_pool_walls", _vp), ("d_pool_targets", _vp), ("d_pool_init", _vp), ("d_pool_depth", _vp)]
+
+
 # every symbol include/tiler_slider.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "ts_version": (C.c_int, []),
@@ -123,6 +141,8 @@ SYMBOLS = {
     "ts_bfs_local_smem_bytes": (C.c_int, [C.POINTER(BfsLocalArgs)]),
     "ts_bfs_local_ctas_per_sm": (C.c_int, [C.POINTER(BfsLocalArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_bfs_local": (C.c_int, [C.POINTER(BfsLocalArgs), C.c_int, _vp]),
+    "ts_synth_candidates": (C.c_int, [C.POINTER(SynthCandidatesArgs), _vp]),
+    "ts_pool_reset": (C.c_int, [C.POINTER(PoolResetArgs), _vp]),
     "ts_host_ctx_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "ts_host_ctx_destroy": (C.c_int, [_vp]),
     "ts_step_host": (C.c_int, [_vp, C.POINTER(StepArgs), _vp, _vp, _vp, _vp, _i64]),

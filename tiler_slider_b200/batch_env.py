@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from ._lib import (CAP_ALIGN, F_WON, GOAL_ORDERED, GOAL_SET, MAX_SIZE, MAX_TILES, EncodeArgs, GoalArgs, ObserveArgs,
-                   StepArgs, SynthArgs, ValidArgs, check, lib)
+                   PoolResetArgs, StepArgs, SynthArgs, ValidArgs, check, lib)
 from .puzzle import Puzzle, as_puzzle, uniform_shape
 
 DEFAULT_REWARDS = (1.0, -0.01, -0.05)   # r_win, r_step, r_invalid -- repo-defined (the reference has no reward)
@@ -110,6 +110,10 @@ class BatchedTilerSliderEnv:
         self._cached_obs_args = None
         self._io_np = None
         self._loaded = False
+        self._pool = None             # set_reset_pool: the batch finished envs draw their next puzzle from
+        self._pool_args = None
+        self._episodes = None         # uint32 per env: puzzles drawn from a pool so far
+        self._solve_depth = None      # int32 per env: shortest solution of the current puzzle (-1: not known)
 
     # ------------------------------------------------------------------ construction
     @classmethod
@@ -159,6 +163,21 @@ class BatchedTilerSliderEnv:
         env._loaded = True
         env.reset()
         return env
+
+    @classmethod
+    def solvable(cls, n_envs: int, size: int, n_tiles: int, n_walls: int, multi_color: bool = False, *,
+                 min_depth: int = 1, max_depth: int = 30, recipe: str = "walk", walk_len: int | None = None,
+                 seed: int = 0, env_index_base: int = 0, max_attempts: int | None = None, **kw) -> "BatchedTilerSliderEnv":
+        """Solvable puzzles whose shortest solution takes between `min_depth` and `max_depth` steps,
+        generated and graded on the device (K7 candidates, K6 search; tiler_slider_b200/generate.py).
+        `solve_depth` holds each env's shortest-solution length.  recipe "walk": targets where a
+        random walk of `walk_len` (default max(8, 2 * max_depth)) state-changing moves leaves the
+        tiles; "uniform": synthetic()'s draw, redrawn until it lands in the band.  Env i's puzzle
+        depends on (seed, recipe, walk_len, band, env_index_base + i) only.  Sizes up to 8, 1..4 tiles."""
+        from .generate import DEFAULT_MAX_ATTEMPTS, solvable
+        return solvable(cls, n_envs, size, n_tiles, n_walls, multi_color, min_depth=min_depth, max_depth=max_depth,
+                        recipe=recipe, walk_len=walk_len, seed=seed, env_index_base=env_index_base,
+                        max_attempts=DEFAULT_MAX_ATTEMPTS if max_attempts is None else max_attempts, **kw)
 
     def encode(self, blocked: torch.Tensor, tiles: torch.Tensor, targets: torch.Tensor) -> None:
         """K1: dense description -> packed planes (GameState.__init__, state.py:61-73)."""
@@ -238,13 +257,21 @@ class BatchedTilerSliderEnv:
             n = self.n_envs
             self._cached_out = (self._pos[:n], self._reward[:n], self._done[:n].view(torch.bool))
         a.d_actions = ptr
+        pool = self._pool_args
         if torch.cuda.current_device() == self.device.index:      # skip the device-guard round trip (host-bound small batches)
-            rc = self._lib.ts_step(C.byref(a), torch.cuda.current_stream().cuda_stream)
+            stream = torch.cuda.current_stream().cuda_stream
+            rc = self._lib.ts_step(C.byref(a), stream)
+            if pool is not None and not rc:   # finished envs draw their next puzzle (K8 reads the done bytes K2 just wrote)
+                rc_pool = self._lib.ts_pool_reset(C.byref(pool), stream)
         else:
             with torch.cuda.device(self.device):
                 rc = self._lib.ts_step(C.byref(a), self._stream())
+                if pool is not None and not rc:
+                    rc_pool = self._lib.ts_pool_reset(C.byref(pool), self._stream())
         if rc:
             check(rc, "ts_step")
+        if pool is not None and rc_pool:
+            check(rc_pool, "ts_pool_reset")
         if self.host_io:          # the outputs are host memory: they are valid once the stream has drained
             torch.cuda.current_stream(self.device).synchronize()
         return self._cached_out
@@ -292,8 +319,12 @@ class BatchedTilerSliderEnv:
         with torch.cuda.device(self.device):
             side = torch.cuda.Stream(self.device)
             side.wait_stream(torch.cuda.current_stream(self.device))
-            with torch.cuda.stream(side):
-                self.step(action_rows[0])                      # warm-up outside capture (lazy init)
+            pool_args, self._pool_args = self._pool_args, None   # the warm-up must not draw puzzles: reset() cannot undo that
+            try:
+                with torch.cuda.stream(side):
+                    self.step(action_rows[0])                  # warm-up outside capture (lazy init)
+            finally:
+                self._pool_args = pool_args
             torch.cuda.current_stream(self.device).wait_stream(side)
             self.reset()
             with torch.cuda.graph(graph):
@@ -329,6 +360,8 @@ class BatchedTilerSliderEnv:
         comes back instead of 5: bit 0 is done, and the reward follows from the WON / INVALID
         bits (`rewards`)."""
         self._require_loaded()
+        if self._pool is not None:
+            raise ValueError("step_host does not draw from a reset pool: use step() or detach the pool")
         if h_flags is None and (h_reward is None or h_done is None):
             raise ValueError("step_host needs h_reward and h_done, or h_flags")
         if h_flags is not None and not self.track_flags:
@@ -348,6 +381,73 @@ class BatchedTilerSliderEnv:
             torch.cuda.current_stream().synchronize()
             check(self._lib.ts_step_host(self._host_ctx, C.byref(a), h_actions.data_ptr(), _ptr(h_reward), _ptr(h_done),
                                          _ptr(h_flags), _round_up(chunk_envs, CAP_ALIGN)), "ts_step_host")
+
+    # ------------------------------------------------------------------ reset pool
+    def set_reset_pool(self, pool: "BatchedTilerSliderEnv | None", *, seed: int = 0, draw_now: bool = False) -> None:
+        """Auto-reset into a pool of puzzles: from now on every step() is followed by K8 (ts_pool_reset),
+        which gives each env that finished in that step pool puzzle H(seed, global env index, episode)
+        (include/tiler_slider.h), so the returned state already shows the new puzzle (`terminal_pos`
+        keeps the positions before the reset); inside capture_steps too.  `pool`: a batch of the same
+        size, tile count, goal mode and target count on the same device (e.g. from solvable() or
+        from_puzzles()); None detaches it.  draw_now: every env draws a pool puzzle now and starts a new
+        episode.  `episodes` counts the draws per env; `solve_depth` follows the pool's depths (None
+        when the pool has none).  Needs auto_reset; not available for host_io batches or step_host."""
+        self._require_loaded()
+        if pool is None:
+            self._pool, self._pool_args = None, None
+            return
+        if not isinstance(pool, BatchedTilerSliderEnv):
+            raise ValueError("the reset pool must be a BatchedTilerSliderEnv")
+        if not self.auto_reset:
+            raise ValueError("a reset pool needs auto_reset=True")
+        if self.host_io:
+            raise ValueError("host_io batches do not support a reset pool")
+        if (pool.size, pool.n_tiles, pool.goal_mode, pool.n_targets) != (self.size, self.n_tiles, self.goal_mode, self.n_targets):
+            raise ValueError(f"the pool holds size {pool.size} / {pool.n_tiles} tiles / goal mode {pool.goal_mode} / {pool.n_targets} "
+                             f"targets, this batch size {self.size} / {self.n_tiles} / {self.goal_mode} / {self.n_targets}")
+        if pool.never_win:
+            raise ValueError("a never_win pool (target count != tile count, ordered goal) cannot be won")
+        if pool.device != self.device:
+            raise ValueError(f"the pool is on {pool.device}, this batch on {self.device}")
+        pool._require_loaded()
+        cap = self.capacity
+        if self._episodes is None:
+            self._episodes = torch.zeros(cap, dtype=torch.int32, device=self.device)
+        if pool._solve_depth is None:
+            self._solve_depth = None
+        elif self._solve_depth is None:
+            self._solve_depth = torch.full((cap,), -1, dtype=torch.int32, device=self.device)
+        self._pool = pool
+        self._pool_args = PoolResetArgs(
+            size=self.size, n_tiles=self.n_tiles, goal_mode=self.goal_mode, count_bytes=self.count_bytes,
+            first_env=0, n_envs=self.n_envs, capacity=cap, env_index_base=0, seed=seed & (2 ** 64 - 1),
+            d_done=_ptr(self._done), d_episode=_ptr(self._episodes), d_walls=_ptr(self._walls),
+            d_targets_packed=_ptr(self._targets), d_init=_ptr(self._init), d_pos=_ptr(self._pos),
+            d_step_count=_ptr(self._count), d_solve_depth=_ptr(self._solve_depth), n_pool=pool.n_envs,
+            pool_capacity=pool.capacity, d_pool_walls=_ptr(pool._walls), d_pool_targets=_ptr(pool._targets),
+            d_pool_init=_ptr(pool._init), d_pool_depth=_ptr(pool._solve_depth))
+        if draw_now:
+            a = PoolResetArgs.from_buffer_copy(self._pool_args)
+            a.d_done = None
+            with torch.cuda.device(self.device):
+                check(self._lib.ts_pool_reset(C.byref(a), self._stream()), "ts_pool_reset")
+            self._flags.zero_()
+            self._done.zero_()
+
+    @property
+    def episodes(self) -> torch.Tensor:
+        """uint32[N]: puzzles each env has drawn from a reset pool (one per finished episode while a
+        pool is attached, plus one for set_reset_pool(draw_now=True))."""
+        if self._episodes is None:
+            self._episodes = torch.zeros(self.capacity, dtype=torch.int32, device=self.device)
+        return self._episodes[: self.n_envs].view(torch.uint32)
+
+    @property
+    def solve_depth(self) -> torch.Tensor | None:
+        """int32[N]: the fewest steps that win the current puzzle from its reset state (K6's solve
+        depth; the goal is checked after every move), -1 where not known; None when the puzzles
+        were not graded (synthetic / from_puzzles batches, or a reset pool without depths)."""
+        return None if self._solve_depth is None else self._solve_depth[: self.n_envs]
 
     def __del__(self):
         h, self._host_ctx = getattr(self, "_host_ctx", None), None

@@ -733,19 +733,29 @@ class CudaLocalKernels:
     def puzzle(self, i: int) -> Puzzle:
         return self.t.puzzle(i)
 
-    def search(self, lo: int, hi: int, max_depth: int, out: dict) -> None:
+    def search(self, lo: int, hi: int, max_depth: int, out: dict, ids: torch.Tensor | None = None) -> None:
         """Search puzzles [lo, hi) into out = {states, depth, status, levels, counters[, moves, lengths]}
-        (tensors over ALL puzzles of the table); puzzles that do not fit get status != 0."""
+        (tensors over ALL puzzles of the table); puzzles that do not fit get status != 0.  ids: search
+        only these puzzles (int32 on the device, each in [lo, hi); the plan is that of the range)."""
         plan = self.plan(lo, hi)
         if plan is None:
-            out["status"][lo:hi] = 1                           # nothing fits on chip
+            if ids is None:
+                out["status"][lo:hi] = 1                       # nothing fits on chip
+            else:
+                out["status"][ids.long()] = 1
             return
-        if hi <= lo:
+        if hi <= lo or (ids is not None and ids.numel() == 0):
             return
         dev = self.device
-        ids = torch.arange(lo, hi, dtype=torch.int32, device=dev) if lo else None
+        if ids is None:
+            ids = torch.arange(lo, hi, dtype=torch.int32, device=dev) if lo else None
+            n_puzzles = hi - lo
+        else:
+            if ids.dtype != torch.int32 or ids.device != dev or not ids.is_contiguous():
+                raise ValueError("ids must be a contiguous int32 tensor on the table's device")
+            n_puzzles = ids.numel()
         with_paths = out.get("lengths") is not None
-        a = self._args(n_puzzles=hi - lo, d_puzzle_ids=None if ids is None else ids.data_ptr(),
+        a = self._args(n_puzzles=n_puzzles, d_puzzle_ids=None if ids is None else ids.data_ptr(),
                        max_depth=min(int(max_depth), (1 << 31) - 1), bitmap_words=plan["bitmap_words"],
                        queue_smem=plan["queue_smem"], spill_per_cta=plan["spill_per_cta"],
                        d_spill=self._buf("spill", plan["grid"] * max(plan["spill_per_cta"], 1), torch.int32).data_ptr(),

@@ -8,8 +8,7 @@
 //   ts_step     see ts_step.cuh;  ts_valid_moves see ts_valid.cuh
 #include <cstdarg>
 #include <cstdio>
-#include "ts_common.cuh"
-#include "../../include/tiler_slider.h"
+#include "ts_synth.cuh"
 
 namespace ts {
 #define TS_DECL(S)                                                              \
@@ -25,6 +24,8 @@ cudaError_t wide_goal_dispatch(const ts_goal_args&, cudaStream_t);
 cudaError_t generic_step_dispatch(const ts_step_args&, cudaStream_t);
 cudaError_t generic_goal_dispatch(const ts_goal_args&, cudaStream_t);
 cudaError_t generic_valid_dispatch(const ts_valid_args&, cudaStream_t);
+cudaError_t candidates_dispatch(const ts_synth_candidates_args&, cudaStream_t);
+cudaError_t pool_reset_dispatch(const ts_pool_reset_args&, cudaStream_t);
 
 static thread_local char g_err[256] = "ok";
 static int fail(int code, const char* fmt, ...) {
@@ -50,70 +51,6 @@ static int check_shape(int size, int n_tiles, int64_t first, int64_t n, int64_t 
         return fail(TS_E_BAD_RANGE, "env range [%lld, %lld) invalid for capacity %lld (first_env must be a multiple of %d)",
                     (long long)first, (long long)(first + n), (long long)cap, GROUP);
     return 0;
-}
-
-// value of bit `bit` of a stored WALL board: blocked cells, plus (padded boards) the sentinel
-// column S of every row and every bit past the last row
-__device__ __forceinline__ int wall_bit(const uint8_t* blocked_cells, int S, int bit) {
-    const int bs = board_stride(S);
-    const int r = bit / bs, c = bit % bs;
-    if (r >= S) return padded_board(S) ? 1 : 0;
-    if (c >= S) return 1;
-    return blocked_cells[r * S + c] ? 1 : 0;
-}
-
-// Write the wall board(s) of one env from a 0/1 cell map (all three board classes).
-__device__ void store_walls(uint8_t* d_walls, size_t cap, size_t env, int S, const uint8_t* cellmap) {
-    if (wide_board(S)) {
-        const int lines = 2 * wide_line_words(S);      // S rounded up to even
-        uint16_t* w = reinterpret_cast<uint16_t*>(d_walls) + env * lines;   // [axis][env][line]
-        const size_t plane = cap * lines;
-        const int lead = wide_line_lead(S);           // S <= 14: cells at bits 1..S between two sentinels
-        for (int l = 0; l < lines; ++l) {
-            uint32_t col = 0, row = 0;
-            if (l < S && lead) col = row = 1u | (1u << (S + 1));   // edge sentinels (ts_wide.cu)
-            if (l < S)
-                for (int k = 0; k < S; ++k) {
-                    if (cellmap[k * S + l]) col |= 1u << (k + lead);    // column l, bit = row
-                    if (cellmap[l * S + k]) row |= 1u << (k + lead);    // row l, bit = column
-                }
-            w[0 * plane + l] = (uint16_t)col;
-            w[1 * plane + l] = (uint16_t)row;
-        }
-        return;
-    }
-    const int nb = board_bytes(S);
-    for (int b = 0; b < nb; ++b) {
-        uint32_t v = 0;
-        for (int k = 0; k < 8; ++k) v |= (uint32_t)wall_bit(cellmap, S, 8 * b + k) << k;
-        d_walls[board_byte_addr(nb, cap, env, b)] = (uint8_t)v;
-    }
-}
-
-// Write the set-goal target board of one env from its target cells (row*S+col each).
-__device__ void store_target_board(uint8_t* d_tb, size_t cap, size_t env, int S, int T, const int* cells, int n) {
-    if (wide_board(S)) {
-        uint16_t rows[16];
-        for (int r = 0; r < 16; ++r) rows[r] = 0;
-        for (int t = 0; t < n; ++t) rows[cells[t] / S] |= (uint16_t)(1u << (cells[t] % S));
-        int distinct = 0;
-        for (int r = 0; r < 16; ++r) distinct += __popc((uint32_t)rows[r]);
-        // the wide kernels test "every tile on a target cell"; that is set equality only when
-        // there are exactly T distinct targets (state.py:185-186): the count travels in word 16
-        uint16_t* o = reinterpret_cast<uint16_t*>(d_tb) + env * WIDE_TARGET_WORDS;
-        for (int r = 0; r < 16; ++r) o[r] = rows[r];
-        o[16] = (uint16_t)distinct;
-        return;
-    }
-    const int nb = board_bytes(S), bs = board_stride(S);
-    for (int b = 0; b < nb; ++b) {
-        uint32_t v = 0;
-        for (int t = 0; t < n; ++t) {
-            const int bit = (cells[t] / S) * bs + (cells[t] % S);
-            if ((bit >> 3) == b) v |= 1u << (bit & 7);
-        }
-        d_tb[board_byte_addr(nb, cap, env, b)] = (uint8_t)v;
-    }
 }
 
 // ---- K1 encode --------------------------------------------------------------------------------
@@ -142,52 +79,11 @@ __global__ void encode_kernel(const ts_encode_args a) {
 }
 
 // ---- K0 synth -----------------------------------------------------------------------------------
-__device__ __forceinline__ uint64_t splitmix64(uint64_t& s) {
-    uint64_t z = (s += 0x9E3779B97F4A7C15ull);
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-
 __global__ void synth_kernel(const ts_synth_args a) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n_envs) return;
-    const size_t env = (size_t)(a.first_env + i), cap = (size_t)a.capacity;
-    const int S = a.size, T = a.n_tiles, W = a.n_walls, pw = pos_bytes(T);
-    const int cells = S * S, draws = W + 2 * T;
-    uint64_t rng = a.seed ^ (0xD1B54A32D192ED03ull * (uint64_t)(a.env_index_base + i + 1));
-    splitmix64(rng);
-    uint8_t perm[MAX_SIZE * MAX_SIZE];
-    for (int c = 0; c < cells; ++c) perm[c] = (uint8_t)c;
-    for (int d = 0; d < draws; ++d) {  // partial Fisher-Yates: prefix of a uniform permutation
-        const uint32_t r = (uint32_t)(splitmix64(rng) >> 32);
-        const int j = d + (int)(((uint64_t)r * (uint32_t)(cells - d)) >> 32);
-        const uint8_t t = perm[d];
-        perm[d] = perm[j];
-        perm[j] = t;
-    }
-    const int ps = pos_stride(S);
-    uint8_t cellmap[MAX_SIZE * MAX_SIZE];
-    for (int c = 0; c < cells; ++c) cellmap[c] = 0;
-    for (int d = 0; d < W; ++d) cellmap[perm[d]] = 1;
-    store_walls(a.d_walls, cap, env, S, cellmap);
-    for (int t = 0; t < pw; ++t) {
-        uint8_t v = 0;
-        if (t < T) { const int c = perm[W + t]; v = (uint8_t)((c / S) * ps + (c % S)); }
-        a.d_init[env * pw + t] = v;
-        a.d_pos[env * pw + t] = v;
-    }
-    if (a.goal_mode == TS_GOAL_ORDERED) {
-        for (int t = 0; t < pw; ++t) {
-            uint8_t v = 0;
-            if (t < T) { const int c = perm[W + T + t]; v = (uint8_t)((c / S) * ps + (c % S)); }
-            a.d_targets_packed[env * pw + t] = v;
-        }
-    } else {
-        int tcells[MAX_TILES_ANY];
-        for (int t = 0; t < T; ++t) tcells[t] = perm[W + T + t];
-        store_target_board(a.d_targets_packed, cap, env, S, T, tcells, T);
-    }
+    synth_env(a.size, a.n_tiles, a.n_walls, a.goal_mode, a.seed, (uint64_t)(a.env_index_base + i), (size_t)a.capacity,
+              (size_t)(a.first_env + i), a.d_walls, a.d_targets_packed, a.d_init, a.d_pos);
 }
 
 }  // namespace ts
@@ -233,6 +129,47 @@ int ts_synth(const ts_synth_args* a, void* stream) {
     const unsigned blocks = (unsigned)((a->n_envs + 127) / 128);
     synth_kernel<<<blocks, 128, 0, (cudaStream_t)stream>>>(*a);
     return cuda_result(cudaGetLastError(), "ts_synth launch");
+}
+
+int ts_synth_candidates(const ts_synth_candidates_args* a, void* stream) {
+    if (!a) return fail(TS_E_NULL_POINTER, "null args");
+    if (int rc = check_shape(a->size, a->n_tiles, 0, 0, a->capacity)) return rc;
+    if (a->size > 8 || a->n_tiles < 1 || a->n_tiles > 4)
+        return fail(TS_E_UNSUPPORTED, "candidates cover sizes up to 8 with 1 to 4 tiles (size %d, n_tiles %d)", a->size, a->n_tiles);
+    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
+    if (a->recipe != TS_RECIPE_UNIFORM && a->recipe != TS_RECIPE_WALK) return fail(TS_E_BAD_ARGUMENT, "recipe %d", a->recipe);
+    if (a->walk_len < 0 || a->walk_len > TS_MAX_WALK) return fail(TS_E_BAD_ARGUMENT, "walk_len %d outside 0..%d", a->walk_len, TS_MAX_WALK);
+    if (a->attempt < 0) return fail(TS_E_BAD_ARGUMENT, "attempt %d", a->attempt);
+    const int need = a->n_walls + (a->recipe == TS_RECIPE_UNIFORM ? 2 : 1) * a->n_tiles;
+    if (a->n_walls < 0 || need > a->size * a->size)
+        return fail(TS_E_BAD_ARGUMENT, "the recipe needs %d distinct cells, the board has %d", need, a->size * a->size);
+    if (a->env_index_base < 0) return fail(TS_E_BAD_RANGE, "env_index_base %lld", (long long)a->env_index_base);
+    if (a->n_items < 0 || (!a->d_env_ids && a->n_items > a->capacity))
+        return fail(TS_E_BAD_RANGE, "n_items %lld invalid for capacity %lld", (long long)a->n_items, (long long)a->capacity);
+    if (!a->d_walls || !a->d_targets_packed || !a->d_init || !a->d_pos) return fail(TS_E_NULL_POINTER, "null device pointer");
+    if (a->n_items == 0) return 0;
+    return cuda_result(candidates_dispatch(*a, (cudaStream_t)stream), "ts_synth_candidates launch");
+}
+
+int ts_pool_reset(const ts_pool_reset_args* a, void* stream) {
+    if (!a) return fail(TS_E_NULL_POINTER, "null args");
+    if (int rc = check_shape(a->size, a->n_tiles, a->first_env, a->n_envs, a->capacity)) return rc;
+    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
+    if (a->count_bytes != 1 && a->count_bytes != 4) return fail(TS_E_BAD_ARGUMENT, "count_bytes %d (1 or 4)", a->count_bytes);
+    if (a->n_pool < 1) return fail(TS_E_BAD_ARGUMENT, "n_pool %lld: the pool needs at least one puzzle", (long long)a->n_pool);
+    if (a->pool_capacity <= 0 || a->pool_capacity % CAP_ALIGN != 0 || a->pool_capacity < a->n_pool || a->pool_capacity >= (int64_t)1 << 33)
+        return fail(TS_E_BAD_CAPACITY, "pool_capacity %lld invalid for %lld puzzles (a positive multiple of %d)",
+                    (long long)a->pool_capacity, (long long)a->n_pool, CAP_ALIGN);
+    if (a->env_index_base < 0) return fail(TS_E_BAD_RANGE, "env_index_base %lld", (long long)a->env_index_base);
+    if (!a->d_episode || !a->d_walls || !a->d_targets_packed || !a->d_init || !a->d_pos || !a->d_step_count ||
+        !a->d_pool_walls || !a->d_pool_targets || !a->d_pool_init)
+        return fail(TS_E_NULL_POINTER, "null device pointer");
+    const void* ptrs[] = {a->d_done, a->d_episode, a->d_walls, a->d_targets_packed, a->d_init, a->d_pos, a->d_step_count,
+                          a->d_solve_depth, a->d_pool_walls, a->d_pool_targets, a->d_pool_init, a->d_pool_depth};
+    for (const void* p : ptrs)
+        if (p && !aligned16(p)) return fail(TS_E_MISALIGNED, "device pointer %p is not 16-byte aligned", p);
+    if (a->n_envs == 0) return 0;
+    return cuda_result(pool_reset_dispatch(*a, (cudaStream_t)stream), "ts_pool_reset launch");
 }
 
 int ts_step(const ts_step_args* a, void* stream) {
