@@ -445,6 +445,55 @@ typedef struct ts_pool_reset_args {
 int ts_pool_reset(const ts_pool_reset_args *a, void *stream);
 
 /* ---------------------------------------------------------------------------------------
+ * K9 ts_optimal_moves: exact distance to the goal and the set of optimal first moves of the
+ * CURRENT positions of listed envs (csrc/ts_optimal.cu; no reference counterpart -- defined
+ * through a BFS over GameState.move, state.py:120-170, with the goal test is_won,
+ * state.py:172-186, checked after every move).  Boards of size <= 8 with 1..4 tiles.  For item
+ * i < n_items, env e = d_env_ids[i] (NULL: e = i), positions s = d_pos[e]:
+ *   d_distance[i]  the fewest moves that win from s (>= 1: a state already on the goal is at 1,
+ *                  through any move that leaves the tiles on the goal, one that changes nothing
+ *                  included); max_steps and step counters play no part.  Otherwise
+ *                  TS_OPT_UNSOLVABLE (-1) no winning state reachable (never_win: always),
+ *                  TS_OPT_CUTOFF (-2) none within max_depth moves, TS_OPT_NOT_SEARCHED (-3)
+ *                  the state space exceeds bitmap_words*32 bits or the slab, or e is outside
+ *                  [0, capacity).
+ *   d_mask[i]      bit m (UP=0, DOWN=1, LEFT=2, RIGHT=3, as ts_valid_moves) set iff move m starts
+ *                  a shortest solution: distance 1: m wins; else distance(succ_m(s)) ==
+ *                  distance(s) - 1.  0 whenever d_distance[i] < 0.
+ * Both in item order, deterministic.  One CTA per env, persistent grid drawing envs from the
+ * ticket counter; visited set and optimal-state set: a shared-memory bitmap over the perfect hash
+ * of K6; frontier: a ring of queue_smem states (a power of two >= 32) in shared memory, and every
+ * state also in d_spill[cta][spill_per_cta] (it is read again by the backward pass), so
+ * spill_per_cta bounds the states a search may reach.  1 <= max_depth <= TS_OPT_MAX_DEPTH.
+ *   d_counters     [0] ticket (zero on entry), [1] += states expanded by the forward search,
+ *                  [2] += states re-expanded by the backward pass
+ * ts_optimal_moves_smem_bytes / ts_optimal_moves_ctas_per_sm: as for K6.
+ * ts_optimal_max_free_cells: atomically raises *d_max_free (int32, device) to the most free cells
+ * of any listed env (ids outside [0, capacity) skipped), which sizes bitmap_words; reads
+ * size, n_items, capacity, d_env_ids and d_walls only (d_targets_packed and d_pos must be set).
+ * ------------------------------------------------------------------------------------- */
+#define TS_OPT_UNSOLVABLE (-1)
+#define TS_OPT_CUTOFF (-2)
+#define TS_OPT_NOT_SEARCHED (-3)
+#define TS_OPT_MAX_DEPTH 254
+typedef struct ts_optimal_moves_args {
+    int32_t size, n_tiles, goal_mode, never_win;
+    int64_t n_items, capacity;
+    const int32_t *d_env_ids;
+    const uint8_t *d_walls, *d_targets_packed, *d_pos;
+    int32_t max_depth, bitmap_words, queue_smem, reserved0;
+    uint32_t *d_spill;
+    int64_t spill_per_cta;
+    uint64_t *d_counters;
+    int32_t *d_distance;
+    uint8_t *d_mask;
+} ts_optimal_moves_args;
+int ts_optimal_moves_smem_bytes(const ts_optimal_moves_args *a);
+int ts_optimal_moves_ctas_per_sm(const ts_optimal_moves_args *a, int *ctas_per_sm, int *n_sm);
+int ts_optimal_max_free_cells(const ts_optimal_moves_args *a, int32_t *d_max_free, void *stream);
+int ts_optimal_moves(const ts_optimal_moves_args *a, int grid, void *stream);
+
+/* ---------------------------------------------------------------------------------------
  * ts_step_host: the same step through HOST buffers (the call a host-side driver makes):
  * h_actions (pinned) -> device, ts_step, reward/done -> h_reward/h_done (pinned), pipelined in
  * chunks over the context's streams; returns after everything has landed.

@@ -22,6 +22,8 @@ F_DONE, F_WON, F_INVALID, F_TIMEOUT, F_STALE = 1, 2, 4, 8, 16
 GOAL_ORDERED, GOAL_SET = 0, 1
 RECIPE_UNIFORM, RECIPE_WALK = 0, 1
 MAX_WALK = 65535
+OPT_UNSOLVABLE, OPT_CUTOFF, OPT_NOT_SEARCHED = -1, -2, -3
+OPT_MAX_DEPTH = 254
 
 _vp, _i32, _i64, _f32 = C.c_void_p, C.c_int32, C.c_int64, C.c_float
 
@@ -109,6 +111,14 @@ class PoolResetArgs(C.Structure):
                 ("d_pool_walls", _vp), ("d_pool_targets", _vp), ("d_pool_init", _vp), ("d_pool_depth", _vp)]
 
 
+class OptimalMovesArgs(C.Structure):
+    _fields_ = [("size", _i32), ("n_tiles", _i32), ("goal_mode", _i32), ("never_win", _i32),
+                ("n_items", _i64), ("capacity", _i64),
+                ("d_env_ids", _vp), ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp),
+                ("max_depth", _i32), ("bitmap_words", _i32), ("queue_smem", _i32), ("reserved0", _i32),
+                ("d_spill", _vp), ("spill_per_cta", _i64), ("d_counters", _vp), ("d_distance", _vp), ("d_mask", _vp)]
+
+
 # every symbol include/tiler_slider.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "ts_version": (C.c_int, []),
@@ -143,6 +153,10 @@ SYMBOLS = {
     "ts_bfs_local": (C.c_int, [C.POINTER(BfsLocalArgs), C.c_int, _vp]),
     "ts_synth_candidates": (C.c_int, [C.POINTER(SynthCandidatesArgs), _vp]),
     "ts_pool_reset": (C.c_int, [C.POINTER(PoolResetArgs), _vp]),
+    "ts_optimal_moves_smem_bytes": (C.c_int, [C.POINTER(OptimalMovesArgs)]),
+    "ts_optimal_moves_ctas_per_sm": (C.c_int, [C.POINTER(OptimalMovesArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ts_optimal_max_free_cells": (C.c_int, [C.POINTER(OptimalMovesArgs), _vp, _vp]),
+    "ts_optimal_moves": (C.c_int, [C.POINTER(OptimalMovesArgs), C.c_int, _vp]),
     "ts_host_ctx_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "ts_host_ctx_destroy": (C.c_int, [_vp]),
     "ts_step_host": (C.c_int, [_vp, C.POINTER(StepArgs), _vp, _vp, _vp, _vp, _i64]),

@@ -114,6 +114,7 @@ class BatchedTilerSliderEnv:
         self._pool_args = None
         self._episodes = None         # uint32 per env: puzzles drawn from a pool so far
         self._solve_depth = None      # int32 per env: shortest solution of the current puzzle (-1: not known)
+        self._optimal = None          # optimal_moves(): the K9 driver (plans and scratch)
 
     # ------------------------------------------------------------------ construction
     @classmethod
@@ -577,6 +578,32 @@ class BatchedTilerSliderEnv:
         with torch.cuda.device(self.device):
             check(self._lib.ts_valid_moves(C.byref(a), self._stream()), "ts_valid_moves")
         return mask[: self.n_envs]
+
+    def optimal_moves(self, ids=None, *, max_depth: int = 254) -> tuple[torch.Tensor, torch.Tensor]:
+        """Exact solver answers for the CURRENT positions (K9, ts_optimal_moves), as supervision for
+        imitation learning, optimality gaps, reward shaping or an exact expert policy.  Returns
+        (distance int32[n], mask uint8[n]) for every env or for `ids` (in ids order):
+          distance: the fewest steps that win from the current state (>= 1; the goal is checked after
+                    every move, as solve_depth; max_steps and the step counter play no part), or
+                    -1 no win reachable (also every env of a never_win batch), -2 none within
+                    max_depth steps, -3 state space too large for the on-chip search;
+          mask:     bit a (valid_moves() order) set iff move a starts a shortest solution; 0 when
+                    distance < 0.
+        Runs on the current stream after the steps queued before it and changes no env state.
+        Sizes up to 8, 1..4 tiles, device-memory batches (not host_io)."""
+        from .bfs import CudaOptimalMoves, check_optimal_moves
+        check_optimal_moves(self.size, self.n_tiles, self.host_io, int(max_depth))
+        self._require_loaded()
+        if ids is not None:
+            ids = torch.as_tensor(ids).to(device=self.device, dtype=torch.int32).reshape(-1).contiguous()
+            if ids.numel():
+                lo, hi = torch.aminmax(ids)
+                lo, hi = int(lo), int(hi)
+                if lo < 0 or hi >= self.n_envs:
+                    raise IndexError(f"env ids must lie in [0, {self.n_envs}), got [{lo}, {hi}]")
+        if self._optimal is None:
+            self._optimal = CudaOptimalMoves(self)
+        return self._optimal.query(ids, int(max_depth))
 
     def set_positions(self, tiles) -> None:
         """Overwrite current positions from uint8[N,T,2] (row, col) -- e.g. to expand a search

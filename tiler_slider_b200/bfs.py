@@ -25,7 +25,9 @@ Two searches, same results (states per puzzle, level histogram, solve depths, sh
   Single-rank and peer-memory searches keep the frontier sizes on the device and launch 16 levels
   between host read-backs.  with_paths records parents (over several ranks they travel with the
   keys) and walks the chains back from the recorded last link of every solution.
-`solve_batch` picks the search that fits a batch.
+`solve_batch` picks the search that fits a batch.  `CudaOptimalMoves` (K9, csrc/ts_optimal.cu) is
+K6's sibling for the envs of a batch as they stand: the distance of their current positions to a win
+and the moves that start a shortest solution (BatchedTilerSliderEnv.optimal_moves).
 
 The device kernels sit behind `CudaBfsKernels`; tests run the same driver logic on CPU
 tensors over gloo with a CPU stand-in for the kernels (tests/test_bfs_gloo.py).
@@ -40,7 +42,7 @@ from typing import Sequence
 import torch
 import torch.distributed as dist
 
-from ._lib import BfsArgs, BfsLocalArgs, check, lib
+from ._lib import OPT_MAX_DEPTH, OPT_NOT_SEARCHED, BfsArgs, BfsLocalArgs, OptimalMovesArgs, check, lib
 from .batch_env import BatchedTilerSliderEnv, shard_range
 from .puzzle import Puzzle
 
@@ -766,6 +768,105 @@ class CudaLocalKernels:
                        d_lengths=out["lengths"].data_ptr() if with_paths else None, max_moves=self.MAX_MOVES)
         with torch.cuda.device(dev):
             check(self.lib.ts_bfs_local(C.byref(a), plan["grid"], torch.cuda.current_stream(dev).cuda_stream), "ts_bfs_local")
+
+
+def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int) -> None:
+    """The shapes ts_optimal_moves covers; raised before anything touches the device."""
+    if size > 8:
+        raise ValueError(f"optimal_moves covers board sizes up to 8 (got {size})")
+    if not 1 <= n_tiles <= 4:
+        raise ValueError(f"optimal_moves covers 1 to 4 tiles (got {n_tiles})")
+    if host_io:
+        raise ValueError("optimal_moves is not available for host_io batches")
+    if not 1 <= max_depth <= OPT_MAX_DEPTH:
+        raise ValueError(f"max_depth {max_depth} outside 1..{OPT_MAX_DEPTH}")
+
+
+class CudaOptimalMoves:
+    """ctypes front-end of ts_optimal_moves (K9, csrc/ts_optimal.cu) for one batch: the distance to
+    the goal and the optimal first moves of the envs' current positions.  The bitmap is sized per
+    call from the most free cells among the queried envs, counted on the device (a reset pool changes
+    the walls of a batch between calls); shared-memory split and grid follow K6's plan
+    (CudaLocalKernels.plan), cached per free-cell count."""
+
+    SMEM_PER_SM, STATIC_SMEM, MAX_SCRATCH_BYTES = CudaLocalKernels.SMEM_PER_SM, CudaLocalKernels.STATIC_SMEM, CudaLocalKernels.MAX_SCRATCH_BYTES
+
+    def __init__(self, env: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
+        self.t, self.lib, self.device = env, lib(), env.device
+        self.want_ctas = ctas_per_sm
+        self.want_queue = queue_smem        # cap on the ring entries kept in shared memory (tests: force slab reads)
+        self._plans: dict[int, dict] = {}
+        self._scratch: dict[str, torch.Tensor] = {}
+        self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)   # of the last call: see include/tiler_slider.h
+
+    def _args(self, **kw) -> OptimalMovesArgs:
+        t = self.t
+        base = dict(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win), capacity=t.capacity,
+                    d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(), d_pos=t._pos.data_ptr())
+        base.update(kw)
+        return OptimalMovesArgs(**base)
+
+    def plan(self, f_max: int) -> dict | None:
+        """Shared-memory split and grid for states of T tiles on up to f_max free cells (None: the
+        bitmap does not fit one CTA per SM)."""
+        if f_max in self._plans:
+            return self._plans[f_max] or None
+        bits = 1
+        for i in range(self.t.n_tiles):
+            bits *= max(f_max - i, 1)
+        bitmap_bytes = max(16, -(-bits // 128) * 16)
+        plan = None
+        for k in ([self.want_ctas] if self.want_ctas else [8, 6, 5, 4, 3, 2, 1]):
+            budget = self.SMEM_PER_SM // k - self.STATIC_SMEM
+            if bitmap_bytes + 1024 > budget:
+                continue
+            queue = 1 << (min(budget - bitmap_bytes, 64 * 1024) // 4).bit_length() - 1     # ring entries: a power of two
+            if self.want_queue is not None:
+                queue = max(32, 1 << (min(queue, self.want_queue).bit_length() - 1))
+            a = self._args(bitmap_words=bitmap_bytes // 4, queue_smem=queue)
+            got, n_sm = C.c_int(0), C.c_int(0)
+            with torch.cuda.device(self.device):
+                rc = self.lib.ts_optimal_moves_ctas_per_sm(C.byref(a), C.byref(got), C.byref(n_sm))
+            if rc == 0 and got.value >= (k if self.want_ctas is None else 1):
+                grid = got.value * n_sm.value
+                plan = dict(bitmap_words=bitmap_bytes // 4, queue_smem=queue, grid=grid, ctas_per_sm=got.value,
+                            spill_per_cta=int(min(bits + 1, self.MAX_SCRATCH_BYTES // 4 // grid)), f_max=f_max)
+                break
+        self._plans[f_max] = plan or {}
+        return plan
+
+    def _buf(self, name: str, n: int, dtype) -> torch.Tensor:
+        b = self._scratch.get(name)
+        if b is None or b.numel() < n or b.dtype != dtype:
+            b = torch.empty(n, dtype=dtype, device=self.device)
+            self._scratch[name] = b
+        return b[:n]
+
+    def query(self, ids: torch.Tensor | None, max_depth: int) -> tuple[torch.Tensor, torch.Tensor]:
+        """(distance int32[n], mask uint8[n]) of envs `ids` (int32 on the device, each in [0, n_envs);
+        None: every env), on the current stream."""
+        t, dev = self.t, self.device
+        n = t.n_envs if ids is None else ids.numel()
+        distance = torch.full((n,), OPT_NOT_SEARCHED, dtype=torch.int32, device=dev)
+        mask = torch.zeros(n, dtype=torch.uint8, device=dev)
+        self.counters.zero_()
+        if n == 0:
+            return distance, mask
+        ids_ptr = None if ids is None else ids.data_ptr()
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        f_max = torch.zeros(1, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            a = self._args(n_items=n, d_env_ids=ids_ptr)
+            check(self.lib.ts_optimal_max_free_cells(C.byref(a), f_max.data_ptr(), stream), "ts_optimal_max_free_cells")
+            plan = self.plan(int(f_max.item()))
+            if plan is None:                     # not even one env's state space fits on chip
+                return distance, mask
+            a = self._args(n_items=n, d_env_ids=ids_ptr, max_depth=int(max_depth), bitmap_words=plan["bitmap_words"],
+                           queue_smem=plan["queue_smem"], spill_per_cta=plan["spill_per_cta"],
+                           d_spill=self._buf("spill", plan["grid"] * plan["spill_per_cta"], torch.int32).data_ptr(),
+                           d_counters=self.counters.data_ptr(), d_distance=distance.data_ptr(), d_mask=mask.data_ptr())
+            check(self.lib.ts_optimal_moves(C.byref(a), plan["grid"], stream), "ts_optimal_moves")
+        return distance, mask
 
 
 class LocalBfs:

@@ -1,0 +1,349 @@
+// ts_optimal.cu -- K9: exact distance to the goal and the set of optimal first moves of the CURRENT
+// state of many envs, one CTA per env, on chip.  A sibling of K6 (ts_bfs_local.cu): same launch shape
+// (persistent CTAs drawing envs from a ticket counter), same visited set (a shared-memory bitmap over
+// the perfect hash of a state among the free cells of its puzzle, ts_bfs_local.cuh), same frontier
+// ring with a per-CTA HBM slab, same successor function slide_env<S,T> and goal test as the step.
+//
+//   1. Forward: BFS from the env's positions (set goal: states canonicalised by sorting), stopped
+//      after the level in which a successor first meets the goal; that level number is d.  Every
+//      state appended is also written to the slab (the ring only holds the levels in flight), so
+//      that levels 1 .. d-1 can be read again; their boundaries stay in shared memory.
+//   2. Backward: the bitmap is cleared and keyed again by the same hash, now as the set of "good"
+//      states, those from which a shortest solution continues.  Level d-1: good when some move
+//      wins.  Level k = d-2 .. 1: good when some successor that differs from it is marked.  A
+//      successor of a level-k state lies at level <= k+1, so only level k+1's marks can be hit; the
+//      marks of level k itself must not be (a same-level successor is one step farther from the
+//      goal), so all flags of level k are computed first (written over the level's slab entries)
+//      and set after a barrier.  One bitmap serves every level without clearing.
+//   3. Root: d == 1: the moves that win; otherwise the moves whose successor is marked (the root is
+//      never marked, so a move that changes nothing is never optimal there).
+// The forward pass stops at the goal level instead of enumerating the reachable set, and the
+// backward pass slides each state of levels 1 .. d-1 once more.  No reference counterpart (parity
+// unpinned; results pinned to a plain CPU BFS, tests/test_gpu_optimal.py).
+#include "ts_bfs_local.cuh"
+#include "../../include/tiler_slider.h"
+
+namespace ts {
+
+constexpr int OPT_THREADS = 256;
+constexpr int OPT_LEVELS = 256;              // level boundaries: max_depth <= 254
+constexpr uint32_t OPT_NONE = 0xFFFFFFFFu;
+constexpr uint32_t WON = 1u, OVER = 2u;
+
+template <int S, int T>
+__global__ void __launch_bounds__(OPT_THREADS) optimal_moves_kernel(const ts_optimal_moves_args a) {
+    constexpr int PW = pos_bytes(T), NB = board_bytes(S);
+    static_assert(T >= 1 && T <= 4, "32-bit states");
+    extern __shared__ __align__(16) uint32_t dyn[];
+    uint32_t* const bitmap = dyn;
+    uint32_t* const queue = dyn + a.bitmap_words;
+    __shared__ uint8_t lut[128];                 // position byte -> rank among the free cells
+    __shared__ uint32_t lstart[OPT_LEVELS];      // level k = discovery indices [lstart[k], lstart[k+1])
+    __shared__ uint32_t cnt[3];                  // entries appended during level L: cnt[L % 3]
+    __shared__ uint32_t lflag[3];                // ... and whether a successor met the goal (WON) / the slab overflowed (OVER)
+    __shared__ long long s_ticket;
+
+    const uint32_t tid = threadIdx.x, lane = tid & 31u;
+    // ring over discovery indices as in K6: entry p is in ring[p % R] when it was appended within R of
+    // the start of the level being expanded, and in the slab in any case
+    const uint32_t R = (uint32_t)a.queue_smem, RMASK = R - 1u;
+    uint32_t* const slab = a.d_spill + (size_t)blockIdx.x * (size_t)a.spill_per_cta;
+    const uint32_t q_cap = (uint32_t)a.spill_per_cta;
+    const size_t cap = (size_t)a.capacity;
+    unsigned long long fwd = 0, bwd = 0;         // states expanded forward / re-expanded backward (thread 0's count is added)
+
+    for (;;) {
+        __syncthreads();                         // the previous env is finished with shared memory
+        if (tid == 0) s_ticket = (long long)atomicAdd((unsigned long long*)&a.d_counters[0], 1ull);
+        __syncthreads();
+        const long long ticket = s_ticket;
+        if (ticket >= a.n_items) break;
+        const long long env = a.d_env_ids ? (long long)a.d_env_ids[ticket] : ticket;
+        const bool listed = env >= 0 && env < a.capacity;
+        if (!listed || a.never_win) {             // never_win: no state meets the goal
+            if (tid == 0) { a.d_distance[ticket] = listed ? TS_OPT_UNSOLVABLE : TS_OPT_NOT_SEARCHED; a.d_mask[ticket] = 0; }
+            continue;
+        }
+        const size_t pid = (size_t)env;
+
+        // ---- the env: walls, goal, current state, free-cell ranks -----------------------------
+        const uint64_t walls = load_board_elem<NB>(a.d_walls, cap, pid);
+        uint64_t tboard = 0;
+        uint32_t tq = 0, root = 0;
+        if (a.goal_mode == TS_GOAL_SET) tboard = load_board_elem<NB>(a.d_targets_packed, cap, pid);
+        else static_for<0, T>([&](auto I) { constexpr int t = decltype(I)::value; tq |= (uint32_t)a.d_targets_packed[pid * PW + t] << (8 * t); });
+        static_for<0, T>([&](auto I) { constexpr int t = decltype(I)::value; root |= (uint32_t)a.d_pos[pid * PW + t] << (8 * t); });
+        if (a.goal_mode == TS_GOAL_SET) sort_bytes4<T>(root);
+        const uint64_t free_cells = ~walls & cell_mask<S>();
+        const uint32_t F = (uint32_t)__popcll(free_cells);
+        if (tid < 128) {
+            const uint32_t bit = pos_to_bit<S>(tid);
+            lut[tid] = bit < 64 ? (uint8_t)__popcll(free_cells & ((1ull << bit) - 1ull)) : 0;
+        }
+        unsigned long long bits = 1;
+#pragma unroll
+        for (int t = 0; t < T; ++t) bits *= (F > (uint32_t)t ? F - (uint32_t)t : 1u);
+        const uint32_t words = (uint32_t)((bits + 31) / 32);
+        if (words > (uint32_t)a.bitmap_words) {
+            if (tid == 0) { a.d_distance[ticket] = TS_OPT_NOT_SEARCHED; a.d_mask[ticket] = 0; }
+            continue;
+        }
+        for (uint32_t k = tid; k < (words + 3) / 4; k += OPT_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+        if (tid == 0) { cnt[0] = cnt[1] = cnt[2] = 0; lflag[0] = lflag[1] = lflag[2] = 0; }
+        __syncthreads();
+
+        // state after move m (set goal: canonical); *won = it meets the goal
+        auto successor = [&](uint32_t q0, uint32_t m, bool& won) {
+            uint32_t q[1] = {q0};
+            slide_env<S, T>(q, walls, m >> 1, (m & 1u) ^ 1u);
+            if (a.goal_mode == TS_GOAL_SET) {
+                won = occupancy<S, T>(q) == tboard;
+                sort_bytes4<T>(q[0]);
+            } else {
+                won = q[0] == tq;
+            }
+            return q[0];
+        };
+        auto marked = [&](uint32_t q) {
+            const uint32_t idx = state_index<T>(lut, F, q);
+            return (bitmap[idx >> 5] >> (idx & 31u)) & 1u;
+        };
+
+        if (tid == 0) {
+            const uint32_t idx = state_index<T>(lut, F, root);
+            bitmap[idx >> 5] |= 1u << (idx & 31u);
+            queue[0] = root;
+            slab[0] = root;
+            lstart[0] = 0;
+        }
+        __syncthreads();
+
+        // ---- 1. forward: BFS levels until a successor meets the goal ---------------------------
+        uint32_t lo = 0, hi = 1, depth = 0, prev_lo = 0;
+        int32_t dist = TS_OPT_CUTOFF;
+        for (;;) {
+            if (lo == hi) { dist = TS_OPT_UNSOLVABLE; break; }
+            if (depth == (uint32_t)a.max_depth) break;
+            uint32_t* const my_cnt = &cnt[depth % 3u];
+            uint32_t* const my_flag = &lflag[depth % 3u];
+            if (tid == 0) cnt[(depth + 1u) % 3u] = lflag[(depth + 1u) % 3u] = 0;
+            const uint32_t n_items = (hi - lo) * 4u;
+            for (uint32_t base = 0; base < n_items; base += OPT_THREADS) {
+                const uint32_t j = base + tid;
+                const bool live = j < n_items;
+                const uint32_t src = lo + (j >> 2), d = j & 3u;
+                bool is_new = false;
+                uint32_t qn = 0;
+                if (live) {
+                    const uint32_t q0 = (src - prev_lo) < R ? queue[src & RMASK] : slab[src];
+                    bool won;
+                    qn = successor(q0, d, won);
+                    if (won) atomicOr(my_flag, WON);
+                    // once this level has met the goal its successors are never read: skip the appends
+                    if (qn != q0 && !(*(volatile uint32_t*)my_flag & WON)) {
+                        const uint32_t idx = state_index<T>(lut, F, qn);
+                        const uint32_t bit = 1u << (idx & 31u);
+                        is_new = (atomicOr(&bitmap[idx >> 5], bit) & bit) == 0;
+                    }
+                }
+                const unsigned m = __ballot_sync(0xFFFFFFFFu, is_new);
+                if (m) {
+                    uint32_t pos = 0;
+                    if (lane == (uint32_t)(__ffs(m) - 1)) pos = atomicAdd(my_cnt, (uint32_t)__popc(m));
+                    pos = __shfl_sync(0xFFFFFFFFu, pos, __ffs(m) - 1);
+                    if (is_new) {
+                        pos += hi + (uint32_t)__popc(m & ((1u << lane) - 1u));
+                        if (pos - lo < R) queue[pos & RMASK] = qn;
+                        if (pos < q_cap) slab[pos] = qn;
+                        else atomicOr(my_flag, OVER);
+                    }
+                }
+            }
+            __syncthreads();
+            const uint32_t n_new = *my_cnt, flag = *my_flag;
+            fwd += hi - lo;
+            prev_lo = lo;
+            lo = hi;
+            hi += n_new;
+            ++depth;
+            if (tid == 0) lstart[depth] = lo;
+            if (flag & WON) { dist = (int32_t)depth; break; }
+            if (flag & OVER) { dist = TS_OPT_NOT_SEARCHED; break; }     // slab exhausted before the goal level
+        }
+        if (dist < 0) {
+            if (tid == 0) { a.d_distance[ticket] = dist; a.d_mask[ticket] = 0; }
+            continue;
+        }
+
+        // ---- 2. backward: mark the states of levels d-1 .. 1 that start a shortest solution ------
+        const uint32_t D = (uint32_t)dist;
+        if (D >= 2) {
+            for (uint32_t k = tid; k < (words + 3) / 4; k += OPT_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+            __syncthreads();                      // bitmap clear, lstart complete
+            for (uint32_t k = D - 1u; k >= 1u; --k) {
+                const uint32_t l0 = lstart[k], l1 = lstart[k + 1u];
+                const uint32_t n_items = (l1 - l0) * 4u;
+                for (uint32_t base = 0; base < n_items; base += OPT_THREADS) {
+                    const uint32_t j = base + tid;
+                    const bool live = j < n_items;
+                    const uint32_t src = l0 + (j >> 2);
+                    bool hit = false;
+                    uint32_t q0 = 0;
+                    if (live) {
+                        q0 = slab[src];
+                        bool won;
+                        const uint32_t qn = successor(q0, j & 3u, won);
+                        hit = k == D - 1u ? won : (qn != q0 && marked(qn));
+                    }
+                    // the four lanes of a state are lanes 4i .. 4i+3 of one warp
+                    const unsigned m = __ballot_sync(0xFFFFFFFFu, hit);
+                    if (live && (j & 3u) == 0u) slab[src] = (m >> lane) & 0xFu ? state_index<T>(lut, F, q0) : OPT_NONE;
+                }
+                __syncthreads();                  // every flag of level k computed
+                for (uint32_t s = l0 + tid; s < l1; s += OPT_THREADS) {
+                    const uint32_t idx = slab[s];
+                    if (idx != OPT_NONE) atomicOr(&bitmap[idx >> 5], 1u << (idx & 31u));
+                }
+                __syncthreads();                  // level k marked
+                if (tid == 0) bwd += l1 - l0;
+            }
+        }
+
+        // ---- 3. root: its optimal moves ---------------------------------------------------------
+        if (tid < 32) {
+            bool hit = false;
+            if (lane < 4) {
+                bool won;
+                const uint32_t qn = successor(root, lane, won);
+                hit = D == 1u ? won : (qn != root && marked(qn));
+            }
+            const unsigned m = __ballot_sync(0xFFFFFFFFu, hit);
+            if (tid == 0) { a.d_distance[ticket] = dist; a.d_mask[ticket] = (uint8_t)(m & 0xFu); }
+        }
+    }
+    if (tid == 0) {
+        atomicAdd((unsigned long long*)&a.d_counters[1], fwd);
+        atomicAdd((unsigned long long*)&a.d_counters[2], bwd);
+    }
+}
+
+// the most free cells among the listed envs (sizes the bitmap of a launch)
+template <int S>
+__global__ void max_free_cells_kernel(const ts_optimal_moves_args a, int32_t* out) {
+    constexpr int NB = board_bytes(S);
+    uint32_t best = 0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < a.n_items; i += (long long)gridDim.x * blockDim.x) {
+        const long long env = a.d_env_ids ? (long long)a.d_env_ids[i] : i;
+        if (env < 0 || env >= a.capacity) continue;
+        const uint64_t walls = load_board_elem<NB>(a.d_walls, (size_t)a.capacity, (size_t)env);
+        best = max(best, (uint32_t)__popcll(~walls & cell_mask<S>()));
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) best = max(best, __shfl_xor_sync(0xFFFFFFFFu, best, o));
+    if ((threadIdx.x & 31u) == 0u && best) atomicMax(out, (int32_t)best);
+}
+
+// op 0: launch; op 1: occupancy query; op 2: free-cell maximum
+template <int S, int T>
+static cudaError_t optimal_op(int op, const ts_optimal_moves_args& a, int grid, size_t smem, int* out, cudaStream_t st) {
+    auto kernel = optimal_moves_kernel<S, T>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    if (op == 1) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(out, kernel, OPT_THREADS, smem);
+    kernel<<<grid, OPT_THREADS, smem, st>>>(a);
+    return cudaGetLastError();
+}
+
+template <int S> static cudaError_t optimal_dispatch_T(int op, const ts_optimal_moves_args& a, int grid, size_t smem, int* out, cudaStream_t st) {
+    if (op == 2) {
+        const long long blocks = (a.n_items + 255) / 256;
+        max_free_cells_kernel<S><<<(unsigned)(blocks < 4096 ? (blocks ? blocks : 1) : 4096), 256, 0, st>>>(a, out);
+        return cudaGetLastError();
+    }
+    switch (a.n_tiles) {
+        case 1: return optimal_op<S, 1>(op, a, grid, smem, out, st);
+        case 2: return optimal_op<S, 2>(op, a, grid, smem, out, st);
+        case 3: return optimal_op<S, 3>(op, a, grid, smem, out, st);
+        case 4: return optimal_op<S, 4>(op, a, grid, smem, out, st);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+static cudaError_t optimal_dispatch(int op, const ts_optimal_moves_args& a, int grid, size_t smem, int* out, cudaStream_t st) {
+    switch (a.size) {
+        case 1: return optimal_dispatch_T<1>(op, a, grid, smem, out, st);
+        case 2: return optimal_dispatch_T<2>(op, a, grid, smem, out, st);
+        case 3: return optimal_dispatch_T<3>(op, a, grid, smem, out, st);
+        case 4: return optimal_dispatch_T<4>(op, a, grid, smem, out, st);
+        case 5: return optimal_dispatch_T<5>(op, a, grid, smem, out, st);
+        case 6: return optimal_dispatch_T<6>(op, a, grid, smem, out, st);
+        case 7: return optimal_dispatch_T<7>(op, a, grid, smem, out, st);
+        case 8: return optimal_dispatch_T<8>(op, a, grid, smem, out, st);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+}  // namespace ts
+
+using namespace ts;
+
+// shape and shared-memory plan
+static int optimal_check_plan(const ts_optimal_moves_args* a) {
+    if (!a) return TS_E_NULL_POINTER;
+    if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
+    if (a->size > 8) return TS_E_UNSUPPORTED;                                 // wide boards: no 64-bit board word
+    if (a->n_tiles < 1 || a->n_tiles > 4) return TS_E_UNSUPPORTED;            // 32-bit states
+    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return TS_E_BAD_ARGUMENT;
+    if (a->bitmap_words < 4 || a->bitmap_words % 4 || a->queue_smem < 32 || (a->queue_smem & (a->queue_smem - 1)))
+        return TS_E_BAD_ARGUMENT;      // the shared-memory queue is a power-of-two ring
+    return 0;
+}
+
+// the env table the listed envs are read from
+static int optimal_check_table(const ts_optimal_moves_args* a) {
+    if (a->capacity <= 0 || a->capacity % TS_CAP_ALIGN) return TS_E_BAD_CAPACITY;
+    if (a->n_items < 0 || (!a->d_env_ids && a->n_items > a->capacity)) return TS_E_BAD_RANGE;
+    if (!a->d_walls || !a->d_targets_packed || !a->d_pos) return TS_E_NULL_POINTER;
+    return 0;
+}
+
+extern "C" {
+
+int ts_optimal_moves_smem_bytes(const ts_optimal_moves_args* a) {
+    if (int rc = optimal_check_plan(a)) return rc;
+    return (int)(((size_t)a->bitmap_words + (size_t)a->queue_smem) * sizeof(uint32_t));
+}
+
+int ts_optimal_moves_ctas_per_sm(const ts_optimal_moves_args* a, int* ctas_per_sm, int* n_sm) {
+    if (int rc = optimal_check_plan(a)) return rc;
+    if (!ctas_per_sm || !n_sm) return TS_E_NULL_POINTER;
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(n_sm, cudaDevAttrMultiProcessorCount, dev);
+    if (e == cudaSuccess) e = optimal_dispatch(1, *a, 0, (size_t)ts_optimal_moves_smem_bytes(a), ctas_per_sm, nullptr);
+    if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
+    return 0;
+}
+
+int ts_optimal_max_free_cells(const ts_optimal_moves_args* a, int32_t* d_max_free, void* stream) {
+    if (!a) return TS_E_NULL_POINTER;
+    if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
+    if (a->size > 8) return TS_E_UNSUPPORTED;
+    if (int rc = optimal_check_table(a)) return rc;
+    if (!d_max_free) return TS_E_NULL_POINTER;
+    if (a->n_items == 0) return 0;
+    return (int)optimal_dispatch(2, *a, 0, 0, d_max_free, (cudaStream_t)stream);
+}
+
+int ts_optimal_moves(const ts_optimal_moves_args* a, int grid, void* stream) {
+    if (int rc = optimal_check_plan(a)) return rc;
+    if (int rc = optimal_check_table(a)) return rc;
+    if (a->max_depth < 1 || a->max_depth > TS_OPT_MAX_DEPTH || a->spill_per_cta < 1 || a->spill_per_cta > 0xFFFFFFFFll)
+        return TS_E_BAD_ARGUMENT;
+    if (!a->d_spill || !a->d_counters || !a->d_distance || !a->d_mask) return TS_E_NULL_POINTER;
+    if (a->n_items == 0) return 0;
+    if (grid < 1) return TS_E_BAD_ARGUMENT;
+    return (int)optimal_dispatch(0, *a, grid, (size_t)ts_optimal_moves_smem_bytes(a), nullptr, (cudaStream_t)stream);
+}
+
+}  // extern "C"
