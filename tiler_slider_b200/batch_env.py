@@ -586,7 +586,9 @@ class BatchedTilerSliderEnv:
           distance: the fewest steps that win from the current state (>= 1; the goal is checked after
                     every move, as solve_depth; max_steps and the step counter play no part), or
                     -1 no win reachable (also every env of a never_win batch), -2 none within
-                    max_depth steps, -3 state space too large for the on-chip search;
+                    max_depth steps, -3 this env's state space is larger than the largest bitmap
+                    one CTA can hold, or than the slab of the launch (it does not depend on the
+                    other envs of the query);
           mask:     bit a (valid_moves() order) set iff move a starts a shortest solution; 0 when
                     distance < 0.
         Runs on the current stream after the steps queued before it and changes no env state.

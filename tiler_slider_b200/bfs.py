@@ -786,8 +786,9 @@ class CudaOptimalMoves:
     """ctypes front-end of ts_optimal_moves (K9, csrc/ts_optimal.cu) for one batch: the distance to
     the goal and the optimal first moves of the envs' current positions.  The bitmap is sized per
     call from the most free cells among the queried envs, counted on the device (a reset pool changes
-    the walls of a batch between calls); shared-memory split and grid follow K6's plan
-    (CudaLocalKernels.plan), cached per free-cell count."""
+    the walls of a batch between calls), or from the most free cells one CTA can hold when that is
+    fewer; shared-memory split and grid follow K6's plan (CudaLocalKernels.plan), cached per
+    free-cell count."""
 
     SMEM_PER_SM, STATIC_SMEM, MAX_SCRATCH_BYTES = CudaLocalKernels.SMEM_PER_SM, CudaLocalKernels.STATIC_SMEM, CudaLocalKernels.MAX_SCRATCH_BYTES
 
@@ -835,6 +836,15 @@ class CudaOptimalMoves:
         self._plans[f_max] = plan or {}
         return plan
 
+    def fitting_free_cells(self, f_max: int) -> int:
+        """The largest F <= f_max whose plan fits (down to F = n_tiles): the free-cell count a launch
+        for envs of up to f_max free cells is planned for.  The kernel reports -3 for each env whose
+        own state space exceeds that bitmap, so an env's answer never depends on the other envs."""
+        f = f_max
+        while f > self.t.n_tiles and self.plan(f) is None:
+            f -= 1
+        return f
+
     def _buf(self, name: str, n: int, dtype) -> torch.Tensor:
         b = self._scratch.get(name)
         if b is None or b.numel() < n or b.dtype != dtype:
@@ -858,8 +868,8 @@ class CudaOptimalMoves:
         with torch.cuda.device(dev):
             a = self._args(n_items=n, d_env_ids=ids_ptr)
             check(self.lib.ts_optimal_max_free_cells(C.byref(a), f_max.data_ptr(), stream), "ts_optimal_max_free_cells")
-            plan = self.plan(int(f_max.item()))
-            if plan is None:                     # not even one env's state space fits on chip
+            plan = self.plan(self.fitting_free_cells(int(f_max.item())))
+            if plan is None:                     # not even T free cells fit on chip
                 return distance, mask
             a = self._args(n_items=n, d_env_ids=ids_ptr, max_depth=int(max_depth), bitmap_words=plan["bitmap_words"],
                            queue_smem=plan["queue_smem"], spill_per_cta=plan["spill_per_cta"],
