@@ -52,7 +52,7 @@ def lib() -> ctypes.CDLL:
                                   ctypes.c_float, ctypes.c_float, ctypes.c_float,
                                   vp, vp, vp, vp, vp, vp]
         L.tso_bfs.restype = cl
-        L.tso_bfs.argtypes = [vp, ci, cl, vp, vp, vp]
+        L.tso_bfs.argtypes = [vp, ci, cl, vp, vp, vp, vp]
         _lib = L
     return _lib
 
@@ -115,21 +115,24 @@ class OracleState:
         mask = lib().tso_valid_moves(self._h)
         return [d for d in range(4) if mask >> d & 1]
 
-    def bfs(self, max_depth: int = 256, max_states: int = 1 << 22):
-        """CPU BFS over tso_move.  Returns (n_states, level_counts, solve_depth, sorted keys)."""
+    def bfs(self, max_depth: int = 256, max_states: int = 1 << 22, by_level: bool = False):
+        """CPU BFS over tso_move.  Returns (n_states, level_counts, solve_depth, sorted keys);
+        by_level: the keys in the order their levels were reached instead (depth 0 first, each
+        level sorted), so that level d is the level_counts[d] keys after those of depths < d."""
         levels = np.zeros(max_depth + 2, dtype=np.int64)
         depth = ctypes.c_int(-1)
         states = np.zeros(max_states + 4, dtype=np.uint64)
+        ordered = np.zeros(max_states + 4, dtype=np.uint64) if by_level else None
         saved = self.current_locations
         n = lib().tso_bfs(self._h, max_depth, max_states, levels.ctypes.data, ctypes.byref(depth),
-                          states.ctypes.data)
+                          states.ctypes.data, None if ordered is None else ordered.ctypes.data)
         self.set_locations(saved)
         if n < 0:
             raise RuntimeError("oracle BFS overflow (raise max_states)")
         lv = levels.tolist()
         while lv and lv[-1] == 0:
             lv.pop()
-        return int(n), lv, int(depth.value), states[:n].copy()
+        return int(n), lv, int(depth.value), (states if ordered is None else ordered)[:n].copy()
 
 
 def rollout(S: int, multi_color: bool, blocked: np.ndarray, tiles: np.ndarray, targets: np.ndarray,

@@ -337,7 +337,9 @@ int tso_rollout(int S, int T, int NT, int multi_color, long N, int K, const uint
  * Canonical key: ordered positions (multi) or sorted positions (single), cell index
  * r*S+c, 8 bits per tile (T <= 8).  Returns the number of reachable states; fills
  * level_counts[d] with the number of NEW states first seen at depth d and *solve_depth
- * with the first depth holding a won state reached by a move (-1 if none).
+ * with the first depth holding a won state reached by a move (-1 if none).  out_states
+ * gets the visited keys sorted; out_by_level (optional) gets them level after level, so
+ * the keys of depth d are the level_counts[d] that follow those of depths 0..d-1.
  * ---------------------------------------------------------------------------------- */
 static uint64_t bfs_key(const tso_state *st) {
     int T = st->n_tiles, S = st->size;
@@ -369,7 +371,7 @@ static int cmp_u64(const void *a, const void *b) {
 }
 
 long tso_bfs(tso_state *st, int max_depth, long max_states, long *level_counts, int *solve_depth,
-             uint64_t *out_states) {
+             uint64_t *out_states, uint64_t *out_by_level) {
     if (st->n_tiles > 8) return -1;
     uint64_t *visited = (uint64_t *)malloc(sizeof(uint64_t) * (size_t)(max_states + 4));
     uint64_t *frontier = (uint64_t *)malloc(sizeof(uint64_t) * (size_t)(max_states + 4));
@@ -378,6 +380,7 @@ long tso_bfs(tso_state *st, int max_depth, long max_states, long *level_counts, 
     *solve_depth = -1;
     frontier[n_front++] = bfs_key(st);
     visited[n_vis++] = frontier[0];
+    if (out_by_level) out_by_level[0] = frontier[0];
     level_counts[0] = 1;
     int depth = 0;
     while (n_front > 0 && depth < max_depth) {
@@ -400,6 +403,7 @@ long tso_bfs(tso_state *st, int max_depth, long max_states, long *level_counts, 
             frontier[n_new++] = next[i];
         }
         if (n_new < 0) { n_vis = -2; break; }
+        if (out_by_level) memcpy(out_by_level + n_vis, frontier, sizeof(uint64_t) * (size_t)n_new);
         memcpy(visited + n_vis, frontier, sizeof(uint64_t) * (size_t)n_new);
         n_vis += n_new;
         qsort(visited, (size_t)n_vis, sizeof(uint64_t), cmp_u64);

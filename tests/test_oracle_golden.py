@@ -235,6 +235,22 @@ def test_bfs_known_answers(golden_misc):
     assert by["puzzle_single_151"]["n_states"] == 51 and by["puzzle_single_151"]["solve_depth"] == 7
 
 
+def test_bfs_keys_by_level(golden_misc):
+    """bfs(by_level=True) lists the visited keys level after level: level d is exactly what a
+    search cut at depth d has visited and one cut at depth d-1 has not."""
+    for b in golden_misc["bfs"]:
+        st = orc.OracleState(b["size"], b["blocked"], b["tiles"], b["targets"], b["multi_color"])
+        n, levels, depth, keys = st.bfs()
+        n2, levels2, depth2, ordered = st.bfs(by_level=True)
+        assert (n2, levels2, depth2) == (n, levels, depth)
+        assert np.array_equal(np.sort(ordered), keys)
+        start = 0
+        for d, count in enumerate(levels):
+            want = np.setdiff1d(st.bfs(max_depth=d)[3], st.bfs(max_depth=d - 1)[3] if d else [])
+            assert np.array_equal(np.sort(ordered[start:start + count]), want), (b["name"], d)
+            start += count
+
+
 def test_success_and_timeout_same_step():
     """SURVEY 7.0 probe: max_steps=1 and a winning move set both flags."""
     blocked = np.zeros((1, 9), np.uint8)
