@@ -1,6 +1,6 @@
 """CPU tests of the optimal-move query (K9 ts_optimal_moves): the C-ABI struct against its ctypes
-mirror, the argument checks of the new entry points, the free-cell count a launch is planned for,
-and the ValueErrors BatchedTilerSliderEnv.optimal_moves raises before it needs a device."""
+mirror, the argument checks of the new entry points, and the ValueErrors
+BatchedTilerSliderEnv.optimal_moves raises before it needs a device (the shared-memory plan: test_on_chip_host.py)."""
 import ctypes as C
 import os
 import subprocess
@@ -80,51 +80,6 @@ def test_optimal_moves_queries_check_their_arguments_without_gpu():
         assert lib.ts_optimal_max_free_cells(C.byref(b), 16, None) == code, kw
     assert lib.ts_optimal_max_free_cells(C.byref(a), None, None) == -4
     assert lib.ts_optimal_max_free_cells(None, 16, None) == -4
-
-
-class _SmemArithmetic:
-    """Stand-in for the library's occupancy query: CTAs per SM from the shared-memory arithmetic alone
-    (the bitmap and ring plus the kernel's static part and the per-CTA reservation), 148 SMs."""
-
-    def ts_optimal_moves_ctas_per_sm(self, a_ref, got_ref, n_sm_ref):
-        from tiler_slider_b200.bfs import CudaOptimalMoves
-        a = a_ref._obj
-        got_ref._obj.value = CudaOptimalMoves.SMEM_PER_SM // (4 * (a.bitmap_words + a.queue_smem) + CudaOptimalMoves.STATIC_SMEM)
-        n_sm_ref._obj.value = 148
-        return 0
-
-
-def _planner(monkeypatch, size, n_tiles):
-    """A CudaOptimalMoves whose plans come from _SmemArithmetic (no device, no buffers read)."""
-    import contextlib
-    import torch
-    from tiler_slider_b200.bfs import CudaOptimalMoves
-    monkeypatch.setattr(torch.cuda, "device", lambda d: contextlib.nullcontext())
-    p = object.__new__(CudaOptimalMoves)
-    z = torch.zeros(16, dtype=torch.uint8)
-    p.t = types.SimpleNamespace(size=size, n_tiles=n_tiles, goal_mode=0, never_win=False, capacity=128, _walls=z, _targets=z, _pos=z)
-    p.lib, p.device, p.want_ctas, p.want_queue, p._plans = _SmemArithmetic(), None, None, None, {}
-    return p
-
-
-@pytest.mark.parametrize("n_tiles", [1, 2, 3, 4])
-def test_optimal_moves_plans_for_the_most_free_cells_that_fit(monkeypatch, n_tiles):
-    """A launch for envs of up to f_max free cells is planned for the largest F <= f_max whose bitmap
-    fits one CTA, never a larger one.  With 4 tiles that is F = 38: 38*37*36*35 bits = 221,456 B of
-    bitmap next to a 1,024-entry ring in one CTA per SM, while F = 39 needs 246,752 B.  With fewer
-    tiles every 8x8 board fits."""
-    p = _planner(monkeypatch, 8, n_tiles)
-    fits = [f for f in range(n_tiles, 65) if p.plan(f) is not None]
-    f_star = fits[-1]
-    assert fits == list(range(n_tiles, f_star + 1))              # a larger board never fits where a smaller one does not
-    assert f_star == (38 if n_tiles == 4 else 64)
-    for f_max in range(n_tiles, 65):
-        assert p.fitting_free_cells(f_max) == min(f_max, f_star), f_max
-    if n_tiles == 4:
-        plan = p.plan(38)
-        assert (plan["bitmap_words"], plan["queue_smem"], plan["ctas_per_sm"], plan["grid"]) == (221456 // 4, 1024, 1, 148)
-        assert plan["spill_per_cta"] == 38 * 37 * 36 * 35 + 1
-        assert p.plan(30)["ctas_per_sm"] == 2 and p.plan(39) is None and p.plan(64) is None
 
 
 @pytest.mark.parametrize("size,n_tiles,host_io,max_depth", [

@@ -664,44 +664,33 @@ class BfsSolver:
                          solve_depth_per_puzzle=depth_pp, generated=generated, solutions=solutions)
 
 
-class CudaLocalKernels:
-    """ctypes front-end of ts_bfs_local for one puzzle table: the shared-memory plan and the launch
-    that searches a contiguous range of puzzles into caller-provided result tensors."""
+class OnChipSearch:
+    """What the front-ends of the two on-chip searches (K6 `CudaLocalKernels`, K9 `CudaOptimalMoves`)
+    share: the shared-memory plan of a launch and the per-CTA scratch slabs.  `want_ctas` fixes the
+    CTAs per SM; `want_queue` caps the ring entries kept in shared memory (tests: force the slab)."""
 
-    N_LEVELS = 256
+    N_LEVELS = 256                  # levels a search may have on chip (the kernels' level buffers)
     SMEM_PER_SM = 228 * 1024
     STATIC_SMEM = 4 * 1024          # the kernel's static shared memory + the per-CTA reservation
     MAX_SCRATCH_BYTES = 4 << 30
-    MAX_MOVES = 255
+    CTAS_PER_SM = ""                # the library's occupancy query of the front-end's kernel
 
     def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
-        if table.size > 8 or not 1 <= table.n_tiles <= 4:
-            raise ValueError("the on-chip BFS covers board sizes up to 8 with 1 to 4 tiles")
         self.t, self.lib, self.device = table, lib(), table.device
         self.want_ctas = ctas_per_sm
-        self.want_queue = queue_smem        # cap on the ring entries kept in shared memory (tests: force the spill path)
-        self._plans: dict[tuple[int, int], dict] = {}
+        self.want_queue = queue_smem
+        self._plans: dict = {}
         self._scratch: dict[str, torch.Tensor] = {}
 
-    def _args(self, **kw) -> BfsLocalArgs:
-        t = self.t
-        base = dict(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win),
-                    puzzle_capacity=t.capacity, d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(),
-                    d_init=t._init.data_ptr(), n_levels=self.N_LEVELS)
-        base.update(kw)
-        return BfsLocalArgs(**base)
-
-    def plan(self, lo: int, hi: int) -> dict | None:
-        """Shared-memory split and grid for puzzles [lo, hi): the bitmap must hold F!/(F-T)! bits for
-        F = the most free cells of any of them; the more CTAs fit an SM next to it, the better the
-        level-synchronisation latency of one puzzle hides behind the others."""
-        if (lo, hi) in self._plans:
-            return self._plans[(lo, hi)] or None
-        t = self.t
-        blocked = t.blocked_cells()[lo:hi]
-        f_max = int(t.size * t.size - blocked.sum(1).min()) if hi > lo else 1
+    def _plan(self, key, f_max: int) -> dict | None:
+        """Shared-memory split and grid for states of T tiles on up to f_max free cells, cached under
+        `key` (None: the bitmap does not fit one CTA per SM).  The bitmap must hold F!/(F-T)! bits;
+        the more CTAs fit an SM next to it, the better the level-synchronisation latency of one
+        puzzle hides behind the others, so the ring gets what is left of the CTA's share."""
+        if key in self._plans:
+            return self._plans[key] or None
         bits = 1
-        for i in range(t.n_tiles):                               # arrangements of T distinct tiles on F_max cells
+        for i in range(self.t.n_tiles):                          # arrangements of T distinct tiles on f_max cells
             bits *= max(f_max - i, 1)
         bitmap_bytes = max(16, -(-bits // 128) * 16)
         plan = None
@@ -712,17 +701,16 @@ class CudaLocalKernels:
             queue = 1 << (min(budget - bitmap_bytes, 64 * 1024) // 4).bit_length() - 1     # ring entries: a power of two
             if self.want_queue is not None:
                 queue = max(32, 1 << (min(queue, self.want_queue).bit_length() - 1))
-            a = self._args(bitmap_words=bitmap_bytes // 4, queue_smem=queue, n_puzzles=0)
+            a = self._args(bitmap_words=bitmap_bytes // 4, queue_smem=queue)
             got, n_sm = C.c_int(0), C.c_int(0)
             with torch.cuda.device(self.device):
-                rc = self.lib.ts_bfs_local_ctas_per_sm(C.byref(a), C.byref(got), C.byref(n_sm))
+                rc = getattr(self.lib, self.CTAS_PER_SM)(C.byref(a), C.byref(got), C.byref(n_sm))
             if rc == 0 and got.value >= (k if self.want_ctas is None else 1):
                 grid = got.value * n_sm.value
-                spill = int(min(bits + 1, self.MAX_SCRATCH_BYTES // 4 // grid))
                 plan = dict(bitmap_words=bitmap_bytes // 4, queue_smem=queue, grid=grid, ctas_per_sm=got.value,
-                            spill_per_cta=spill, f_max=f_max, smem_bytes=bitmap_bytes + 4 * queue)
+                            spill_per_cta=int(min(bits + 1, self.MAX_SCRATCH_BYTES // 4 // grid)), f_max=f_max)
                 break
-        self._plans[(lo, hi)] = plan or {}
+        self._plans[key] = plan or {}
         return plan
 
     def _buf(self, name: str, n: int, dtype) -> torch.Tensor:
@@ -731,6 +719,38 @@ class CudaLocalKernels:
             b = torch.empty(n, dtype=dtype, device=self.device)
             self._scratch[name] = b
         return b[:n]
+
+
+class CudaLocalKernels(OnChipSearch):
+    """ctypes front-end of ts_bfs_local for one puzzle table: the shared-memory plan and the launch
+    that searches a contiguous range of puzzles into caller-provided result tensors."""
+
+    MAX_MOVES = 255
+    CTAS_PER_SM = "ts_bfs_local_ctas_per_sm"
+
+    def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
+        if table.size > 8 or not 1 <= table.n_tiles <= 4:
+            raise ValueError("the on-chip BFS covers board sizes up to 8 with 1 to 4 tiles")
+        super().__init__(table, ctas_per_sm, queue_smem)
+
+    def _args(self, **kw) -> BfsLocalArgs:
+        t = self.t
+        base = dict(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win),
+                    puzzle_capacity=t.capacity, d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(),
+                    d_init=t._init.data_ptr(), n_levels=self.N_LEVELS)
+        base.update(kw)
+        return BfsLocalArgs(**base)
+
+    def plan(self, lo: int, hi: int) -> dict | None:
+        """The plan for puzzles [lo, hi): F = the most free cells of any of them."""
+        t = self.t
+        if (lo, hi) not in self._plans:
+            blocked = t.blocked_cells()[lo:hi]
+            f_max = int(t.size * t.size - blocked.sum(1).min()) if hi > lo else 1
+            plan = self._plan((lo, hi), f_max)
+            if plan:
+                plan["smem_bytes"] = 4 * (plan["bitmap_words"] + plan["queue_smem"])
+        return self._plans[(lo, hi)] or None
 
     def puzzle(self, i: int) -> Puzzle:
         return self.t.puzzle(i)
@@ -782,22 +802,17 @@ def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int) 
         raise ValueError(f"max_depth {max_depth} outside 1..{OPT_MAX_DEPTH}")
 
 
-class CudaOptimalMoves:
+class CudaOptimalMoves(OnChipSearch):
     """ctypes front-end of ts_optimal_moves (K9, csrc/ts_optimal.cu) for one batch: the distance to
     the goal and the optimal first moves of the envs' current positions.  The bitmap is sized per
     call from the most free cells among the queried envs, counted on the device (a reset pool changes
     the walls of a batch between calls), or from the most free cells one CTA can hold when that is
-    fewer; shared-memory split and grid follow K6's plan (CudaLocalKernels.plan), cached per
-    free-cell count."""
+    fewer; the plan is cached per free-cell count."""
 
-    SMEM_PER_SM, STATIC_SMEM, MAX_SCRATCH_BYTES = CudaLocalKernels.SMEM_PER_SM, CudaLocalKernels.STATIC_SMEM, CudaLocalKernels.MAX_SCRATCH_BYTES
+    CTAS_PER_SM = "ts_optimal_moves_ctas_per_sm"
 
     def __init__(self, env: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
-        self.t, self.lib, self.device = env, lib(), env.device
-        self.want_ctas = ctas_per_sm
-        self.want_queue = queue_smem        # cap on the ring entries kept in shared memory (tests: force slab reads)
-        self._plans: dict[int, dict] = {}
-        self._scratch: dict[str, torch.Tensor] = {}
+        super().__init__(env, ctas_per_sm, queue_smem)
         self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)   # of the last call: see include/tiler_slider.h
 
     def _args(self, **kw) -> OptimalMovesArgs:
@@ -808,33 +823,8 @@ class CudaOptimalMoves:
         return OptimalMovesArgs(**base)
 
     def plan(self, f_max: int) -> dict | None:
-        """Shared-memory split and grid for states of T tiles on up to f_max free cells (None: the
-        bitmap does not fit one CTA per SM)."""
-        if f_max in self._plans:
-            return self._plans[f_max] or None
-        bits = 1
-        for i in range(self.t.n_tiles):
-            bits *= max(f_max - i, 1)
-        bitmap_bytes = max(16, -(-bits // 128) * 16)
-        plan = None
-        for k in ([self.want_ctas] if self.want_ctas else [8, 6, 5, 4, 3, 2, 1]):
-            budget = self.SMEM_PER_SM // k - self.STATIC_SMEM
-            if bitmap_bytes + 1024 > budget:
-                continue
-            queue = 1 << (min(budget - bitmap_bytes, 64 * 1024) // 4).bit_length() - 1     # ring entries: a power of two
-            if self.want_queue is not None:
-                queue = max(32, 1 << (min(queue, self.want_queue).bit_length() - 1))
-            a = self._args(bitmap_words=bitmap_bytes // 4, queue_smem=queue)
-            got, n_sm = C.c_int(0), C.c_int(0)
-            with torch.cuda.device(self.device):
-                rc = self.lib.ts_optimal_moves_ctas_per_sm(C.byref(a), C.byref(got), C.byref(n_sm))
-            if rc == 0 and got.value >= (k if self.want_ctas is None else 1):
-                grid = got.value * n_sm.value
-                plan = dict(bitmap_words=bitmap_bytes // 4, queue_smem=queue, grid=grid, ctas_per_sm=got.value,
-                            spill_per_cta=int(min(bits + 1, self.MAX_SCRATCH_BYTES // 4 // grid)), f_max=f_max)
-                break
-        self._plans[f_max] = plan or {}
-        return plan
+        """The plan for states on up to f_max free cells."""
+        return self._plan(f_max, f_max)
 
     def fitting_free_cells(self, f_max: int) -> int:
         """The largest F <= f_max whose plan fits (down to F = n_tiles): the free-cell count a launch
@@ -844,13 +834,6 @@ class CudaOptimalMoves:
         while f > self.t.n_tiles and self.plan(f) is None:
             f -= 1
         return f
-
-    def _buf(self, name: str, n: int, dtype) -> torch.Tensor:
-        b = self._scratch.get(name)
-        if b is None or b.numel() < n or b.dtype != dtype:
-            b = torch.empty(n, dtype=dtype, device=self.device)
-            self._scratch[name] = b
-        return b[:n]
 
     def query(self, ids: torch.Tensor | None, max_depth: int) -> tuple[torch.Tensor, torch.Tensor]:
         """(distance int32[n], mask uint8[n]) of envs `ids` (int32 on the device, each in [0, n_envs);

@@ -1,10 +1,19 @@
-// ts_bfs_local.cuh -- device helpers of the on-chip searches (K6 ts_bfs_local.cu, K9 ts_optimal.cu):
-// canonical set-goal states, position byte -> bitboard bit, and the perfect hash of a state over the
-// free cells of its puzzle that keys the shared-memory bitmap.
+// ts_bfs_local.cuh -- what the two on-chip searches, K6 (ts_bfs_local.cu, the batched BFS) and K9
+// (ts_optimal.cu, the optimal-move query), share: the CTA shape, canonical set-goal states, position
+// byte -> bitboard bit, the perfect hash of a state over the free cells of its puzzle that keys the
+// shared-memory bitmap, and on the host the plan check, the shared-memory size and the launch.
 #pragma once
 #include "ts_common.cuh"
+#include "../../include/tiler_slider.h"
 
 namespace ts {
+
+// threads of a search CTA, one (state, move) pair each (384 and 512 measured within noise: DESIGN.md)
+constexpr int SEARCH_THREADS = 256;
+// entries of a search's per-level buffers: K6 leaves a puzzle of more levels to the hash-partitioned
+// search, K9 takes max_depth <= TS_OPT_MAX_DEPTH
+constexpr int SEARCH_LEVELS = 256;
+static_assert(TS_OPT_MAX_DEPTH + 2 <= SEARCH_LEVELS, "K9 keeps the start of levels 0 .. max_depth + 1");
 
 // canonical form of a set-goal state: its T position bytes sorted ascending (tiles are interchangeable)
 template <int T> __device__ __forceinline__ void sort_bytes4(uint32_t& q) {
@@ -48,6 +57,46 @@ template <int T> __device__ __forceinline__ uint32_t state_index(const uint8_t (
         idx = idx * (F - (uint32_t)i) + d;
     });
     return idx;
+}
+
+// ---- host side -------------------------------------------------------------------------------------
+// tile count, goal mode and shared-memory plan of a search launch: a bitmap of whole 16-byte units,
+// a power-of-two ring of at least 32 entries
+template <class A> int check_search_plan(const A& a) {
+    if (a.n_tiles < 1 || a.n_tiles > 4) return TS_E_UNSUPPORTED;            // 32-bit states
+    if (a.goal_mode != TS_GOAL_ORDERED && a.goal_mode != TS_GOAL_SET) return TS_E_BAD_ARGUMENT;
+    if (a.bitmap_words < 4 || a.bitmap_words % 4 || a.queue_smem < 32 || (a.queue_smem & (a.queue_smem - 1))) return TS_E_BAD_ARGUMENT;
+    return 0;
+}
+
+template <class A> size_t search_smem_bytes(const A& a) { return ((size_t)a.bitmap_words + (size_t)a.queue_smem) * sizeof(uint32_t); }
+
+// Instance <a.size, a.n_tiles> of a search kernel (kernel_of(IC<S>, IC<T>) returns it) with a's
+// dynamic shared memory: launched on `grid` CTAs, or, when ctas_per_sm is given, asked how many of
+// its CTAs fit an SM.
+template <class KernelOf, class A>
+cudaError_t search_kernel(KernelOf&& kernel_of, const A& a, int grid, int* ctas_per_sm, cudaStream_t st) {
+    const size_t smem = search_smem_bytes(a);
+    return dispatch_small(a.size, a.n_tiles, [&](auto S, auto T) {
+        const auto kernel = kernel_of(S, T);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        if (ctas_per_sm) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kernel, SEARCH_THREADS, smem);
+        kernel<<<grid, SEARCH_THREADS, smem, st>>>(a);
+        return cudaGetLastError();
+    });
+}
+
+// resident CTAs per SM of a's search kernel and the SM count of the current device
+template <class KernelOf, class A>
+int search_ctas_per_sm(KernelOf&& kernel_of, const A& a, int* ctas_per_sm, int* n_sm) {
+    if (!ctas_per_sm || !n_sm) return TS_E_NULL_POINTER;
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(n_sm, cudaDevAttrMultiProcessorCount, dev);
+    if (e == cudaSuccess) e = search_kernel(kernel_of, a, 0, ctas_per_sm, nullptr);
+    if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
+    return 0;
 }
 
 }  // namespace ts

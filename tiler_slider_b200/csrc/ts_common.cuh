@@ -84,6 +84,33 @@ template <int B, int E, class F> __device__ __forceinline__ void static_for(F&& 
     if constexpr (B < E) { f(IC<B>{}); static_for<B + 1, E>(f); }
 }
 
+// host: f(IC<S>{}) for the board sizes of one 64-bit board, 1..8
+template <class F> cudaError_t dispatch_size(int size, F&& f) {
+    switch (size) {
+        case 1: return f(IC<1>{});
+        case 2: return f(IC<2>{});
+        case 3: return f(IC<3>{});
+        case 4: return f(IC<4>{});
+        case 5: return f(IC<5>{});
+        case 6: return f(IC<6>{});
+        case 7: return f(IC<7>{});
+        case 8: return f(IC<8>{});
+        default: return cudaErrorInvalidValue;
+    }
+}
+// host: f(IC<S>{}, IC<T>{}) for those sizes and the tile counts of one 32-bit state, 1..4
+template <class F> cudaError_t dispatch_small(int size, int n_tiles, F&& f) {
+    return dispatch_size(size, [&](auto S) {
+        switch (n_tiles) {
+            case 1: return f(S, IC<1>{});
+            case 2: return f(S, IC<2>{});
+            case 3: return f(S, IC<3>{});
+            case 4: return f(S, IC<4>{});
+            default: return cudaErrorInvalidValue;
+        }
+    });
+}
+
 // cache policy of the streaming accesses (overridable for experiments: -D'TS_LD(p)=__ldg(p)')
 #ifndef TS_LD
 #define TS_LD(p) __ldcs(p)

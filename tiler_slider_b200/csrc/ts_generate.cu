@@ -93,30 +93,12 @@ __global__ void __launch_bounds__(GEN_THREADS) synth_candidates_kernel(const ts_
     }
 }
 
-template <int S> static cudaError_t candidates_T(const ts_synth_candidates_args& a, unsigned blocks, cudaStream_t st) {
-    switch (a.n_tiles) {
-        case 1: synth_candidates_kernel<S, 1><<<blocks, GEN_THREADS, 0, st>>>(a); break;
-        case 2: synth_candidates_kernel<S, 2><<<blocks, GEN_THREADS, 0, st>>>(a); break;
-        case 3: synth_candidates_kernel<S, 3><<<blocks, GEN_THREADS, 0, st>>>(a); break;
-        case 4: synth_candidates_kernel<S, 4><<<blocks, GEN_THREADS, 0, st>>>(a); break;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
-}
-
 cudaError_t candidates_dispatch(const ts_synth_candidates_args& a, cudaStream_t st) {
     const unsigned blocks = (unsigned)((a.n_items + GEN_THREADS - 1) / GEN_THREADS);
-    switch (a.size) {
-        case 1: return candidates_T<1>(a, blocks, st);
-        case 2: return candidates_T<2>(a, blocks, st);
-        case 3: return candidates_T<3>(a, blocks, st);
-        case 4: return candidates_T<4>(a, blocks, st);
-        case 5: return candidates_T<5>(a, blocks, st);
-        case 6: return candidates_T<6>(a, blocks, st);
-        case 7: return candidates_T<7>(a, blocks, st);
-        case 8: return candidates_T<8>(a, blocks, st);
-        default: return cudaErrorInvalidValue;
-    }
+    return dispatch_small(a.size, a.n_tiles, [&](auto S, auto T) {
+        synth_candidates_kernel<decltype(S)::value, decltype(T)::value><<<blocks, GEN_THREADS, 0, st>>>(a);
+        return cudaGetLastError();
+    });
 }
 
 // ---- K8 pool reset -------------------------------------------------------------------------------

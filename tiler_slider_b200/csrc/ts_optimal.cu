@@ -1,8 +1,9 @@
 // ts_optimal.cu -- K9: exact distance to the goal and the set of optimal first moves of the CURRENT
-// state of many envs, one CTA per env, on chip.  A sibling of K6 (ts_bfs_local.cu): same launch shape
-// (persistent CTAs drawing envs from a ticket counter), same visited set (a shared-memory bitmap over
-// the perfect hash of a state among the free cells of its puzzle, ts_bfs_local.cuh), same frontier
-// ring with a per-CTA HBM slab, same successor function slide_env<S,T> and goal test as the step.
+// state of many envs, one CTA per env, on chip.  Built on K6's machinery (ts_bfs_local.cu; the CTA
+// shape, hash, plan check and launch are in ts_bfs_local.cuh): persistent CTAs drawing envs from a
+// ticket counter, the visited set a shared-memory bitmap over the perfect hash of a state among the
+// free cells of its puzzle, the frontier ring with a per-CTA HBM slab, the successor function
+// slide_env<S,T> and goal test of the step.
 //
 //   1. Forward: BFS from the env's positions (set goal: states canonicalised by sorting), stopped
 //      after the level in which a successor first meets the goal; that level number is d.  Every
@@ -21,24 +22,21 @@
 // backward pass slides each state of levels 1 .. d-1 once more.  No reference counterpart (parity
 // unpinned; results pinned to a plain CPU BFS, tests/test_gpu_optimal.py).
 #include "ts_bfs_local.cuh"
-#include "../../include/tiler_slider.h"
 
 namespace ts {
 
-constexpr int OPT_THREADS = 256;
-constexpr int OPT_LEVELS = 256;              // level boundaries: max_depth <= 254
 constexpr uint32_t OPT_NONE = 0xFFFFFFFFu;
 constexpr uint32_t WON = 1u, OVER = 2u;
 
 template <int S, int T>
-__global__ void __launch_bounds__(OPT_THREADS) optimal_moves_kernel(const ts_optimal_moves_args a) {
+__global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_optimal_moves_args a) {
     constexpr int PW = pos_bytes(T), NB = board_bytes(S);
     static_assert(T >= 1 && T <= 4, "32-bit states");
     extern __shared__ __align__(16) uint32_t dyn[];
     uint32_t* const bitmap = dyn;
     uint32_t* const queue = dyn + a.bitmap_words;
     __shared__ uint8_t lut[128];                 // position byte -> rank among the free cells
-    __shared__ uint32_t lstart[OPT_LEVELS];      // level k = discovery indices [lstart[k], lstart[k+1])
+    __shared__ uint32_t lstart[SEARCH_LEVELS];   // level k = discovery indices [lstart[k], lstart[k+1])
     __shared__ uint32_t cnt[3];                  // entries appended during level L: cnt[L % 3]
     __shared__ uint32_t lflag[3];                // ... and whether a successor met the goal (WON) / the slab overflowed (OVER)
     __shared__ long long s_ticket;
@@ -88,7 +86,7 @@ __global__ void __launch_bounds__(OPT_THREADS) optimal_moves_kernel(const ts_opt
             if (tid == 0) { a.d_distance[ticket] = TS_OPT_NOT_SEARCHED; a.d_mask[ticket] = 0; }
             continue;
         }
-        for (uint32_t k = tid; k < (words + 3) / 4; k += OPT_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+        for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
         if (tid == 0) { cnt[0] = cnt[1] = cnt[2] = 0; lflag[0] = lflag[1] = lflag[2] = 0; }
         __syncthreads();
 
@@ -128,7 +126,7 @@ __global__ void __launch_bounds__(OPT_THREADS) optimal_moves_kernel(const ts_opt
             uint32_t* const my_flag = &lflag[depth % 3u];
             if (tid == 0) cnt[(depth + 1u) % 3u] = lflag[(depth + 1u) % 3u] = 0;
             const uint32_t n_items = (hi - lo) * 4u;
-            for (uint32_t base = 0; base < n_items; base += OPT_THREADS) {
+            for (uint32_t base = 0; base < n_items; base += SEARCH_THREADS) {
                 const uint32_t j = base + tid;
                 const bool live = j < n_items;
                 const uint32_t src = lo + (j >> 2), d = j & 3u;
@@ -178,12 +176,12 @@ __global__ void __launch_bounds__(OPT_THREADS) optimal_moves_kernel(const ts_opt
         // ---- 2. backward: mark the states of levels d-1 .. 1 that start a shortest solution ------
         const uint32_t D = (uint32_t)dist;
         if (D >= 2) {
-            for (uint32_t k = tid; k < (words + 3) / 4; k += OPT_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+            for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
             __syncthreads();                      // bitmap clear, lstart complete
             for (uint32_t k = D - 1u; k >= 1u; --k) {
                 const uint32_t l0 = lstart[k], l1 = lstart[k + 1u];
                 const uint32_t n_items = (l1 - l0) * 4u;
-                for (uint32_t base = 0; base < n_items; base += OPT_THREADS) {
+                for (uint32_t base = 0; base < n_items; base += SEARCH_THREADS) {
                     const uint32_t j = base + tid;
                     const bool live = j < n_items;
                     const uint32_t src = l0 + (j >> 2);
@@ -200,7 +198,7 @@ __global__ void __launch_bounds__(OPT_THREADS) optimal_moves_kernel(const ts_opt
                     if (live && (j & 3u) == 0u) slab[src] = (m >> lane) & 0xFu ? state_index<T>(lut, F, q0) : OPT_NONE;
                 }
                 __syncthreads();                  // every flag of level k computed
-                for (uint32_t s = l0 + tid; s < l1; s += OPT_THREADS) {
+                for (uint32_t s = l0 + tid; s < l1; s += SEARCH_THREADS) {
                     const uint32_t idx = slab[s];
                     if (idx != OPT_NONE) atomicOr(&bitmap[idx >> 5], 1u << (idx & 31u));
                 }
@@ -243,45 +241,7 @@ __global__ void max_free_cells_kernel(const ts_optimal_moves_args a, int32_t* ou
     if ((threadIdx.x & 31u) == 0u && best) atomicMax(out, (int32_t)best);
 }
 
-// op 0: launch; op 1: occupancy query; op 2: free-cell maximum
-template <int S, int T>
-static cudaError_t optimal_op(int op, const ts_optimal_moves_args& a, int grid, size_t smem, int* out, cudaStream_t st) {
-    auto kernel = optimal_moves_kernel<S, T>;
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    if (op == 1) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(out, kernel, OPT_THREADS, smem);
-    kernel<<<grid, OPT_THREADS, smem, st>>>(a);
-    return cudaGetLastError();
-}
-
-template <int S> static cudaError_t optimal_dispatch_T(int op, const ts_optimal_moves_args& a, int grid, size_t smem, int* out, cudaStream_t st) {
-    if (op == 2) {
-        const long long blocks = (a.n_items + 255) / 256;
-        max_free_cells_kernel<S><<<(unsigned)(blocks < 4096 ? (blocks ? blocks : 1) : 4096), 256, 0, st>>>(a, out);
-        return cudaGetLastError();
-    }
-    switch (a.n_tiles) {
-        case 1: return optimal_op<S, 1>(op, a, grid, smem, out, st);
-        case 2: return optimal_op<S, 2>(op, a, grid, smem, out, st);
-        case 3: return optimal_op<S, 3>(op, a, grid, smem, out, st);
-        case 4: return optimal_op<S, 4>(op, a, grid, smem, out, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-static cudaError_t optimal_dispatch(int op, const ts_optimal_moves_args& a, int grid, size_t smem, int* out, cudaStream_t st) {
-    switch (a.size) {
-        case 1: return optimal_dispatch_T<1>(op, a, grid, smem, out, st);
-        case 2: return optimal_dispatch_T<2>(op, a, grid, smem, out, st);
-        case 3: return optimal_dispatch_T<3>(op, a, grid, smem, out, st);
-        case 4: return optimal_dispatch_T<4>(op, a, grid, smem, out, st);
-        case 5: return optimal_dispatch_T<5>(op, a, grid, smem, out, st);
-        case 6: return optimal_dispatch_T<6>(op, a, grid, smem, out, st);
-        case 7: return optimal_dispatch_T<7>(op, a, grid, smem, out, st);
-        case 8: return optimal_dispatch_T<8>(op, a, grid, smem, out, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
+static constexpr auto K9 = [](auto S, auto T) { return optimal_moves_kernel<decltype(S)::value, decltype(T)::value>; };
 
 }  // namespace ts
 
@@ -292,11 +252,7 @@ static int optimal_check_plan(const ts_optimal_moves_args* a) {
     if (!a) return TS_E_NULL_POINTER;
     if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
     if (a->size > 8) return TS_E_UNSUPPORTED;                                 // wide boards: no 64-bit board word
-    if (a->n_tiles < 1 || a->n_tiles > 4) return TS_E_UNSUPPORTED;            // 32-bit states
-    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return TS_E_BAD_ARGUMENT;
-    if (a->bitmap_words < 4 || a->bitmap_words % 4 || a->queue_smem < 32 || (a->queue_smem & (a->queue_smem - 1)))
-        return TS_E_BAD_ARGUMENT;      // the shared-memory queue is a power-of-two ring
-    return 0;
+    return check_search_plan(*a);
 }
 
 // the env table the listed envs are read from
@@ -311,18 +267,12 @@ extern "C" {
 
 int ts_optimal_moves_smem_bytes(const ts_optimal_moves_args* a) {
     if (int rc = optimal_check_plan(a)) return rc;
-    return (int)(((size_t)a->bitmap_words + (size_t)a->queue_smem) * sizeof(uint32_t));
+    return (int)search_smem_bytes(*a);
 }
 
 int ts_optimal_moves_ctas_per_sm(const ts_optimal_moves_args* a, int* ctas_per_sm, int* n_sm) {
     if (int rc = optimal_check_plan(a)) return rc;
-    if (!ctas_per_sm || !n_sm) return TS_E_NULL_POINTER;
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (e == cudaSuccess) e = optimal_dispatch(1, *a, 0, (size_t)ts_optimal_moves_smem_bytes(a), ctas_per_sm, nullptr);
-    if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
-    return 0;
+    return search_ctas_per_sm(K9, *a, ctas_per_sm, n_sm);
 }
 
 int ts_optimal_max_free_cells(const ts_optimal_moves_args* a, int32_t* d_max_free, void* stream) {
@@ -332,7 +282,11 @@ int ts_optimal_max_free_cells(const ts_optimal_moves_args* a, int32_t* d_max_fre
     if (int rc = optimal_check_table(a)) return rc;
     if (!d_max_free) return TS_E_NULL_POINTER;
     if (a->n_items == 0) return 0;
-    return (int)optimal_dispatch(2, *a, 0, 0, d_max_free, (cudaStream_t)stream);
+    const long long blocks = (a->n_items + 255) / 256;
+    return (int)dispatch_size(a->size, [&](auto S) {
+        max_free_cells_kernel<decltype(S)::value><<<(unsigned)(blocks < 4096 ? blocks : 4096), 256, 0, (cudaStream_t)stream>>>(*a, d_max_free);
+        return cudaGetLastError();
+    });
 }
 
 int ts_optimal_moves(const ts_optimal_moves_args* a, int grid, void* stream) {
@@ -343,7 +297,7 @@ int ts_optimal_moves(const ts_optimal_moves_args* a, int grid, void* stream) {
     if (!a->d_spill || !a->d_counters || !a->d_distance || !a->d_mask) return TS_E_NULL_POINTER;
     if (a->n_items == 0) return 0;
     if (grid < 1) return TS_E_BAD_ARGUMENT;
-    return (int)optimal_dispatch(0, *a, grid, (size_t)ts_optimal_moves_smem_bytes(a), nullptr, (cudaStream_t)stream);
+    return (int)search_kernel(K9, *a, grid, nullptr, (cudaStream_t)stream);
 }
 
 }  // extern "C"
