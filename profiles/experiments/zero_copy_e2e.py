@@ -1,3 +1,4 @@
+# Needs commit 71e789f (the TS_HOST_ZERO_COPY switch was removed afterwards; results: profiles/r2_zero_copy_e2e.txt).
 """ts_step_host with the step's outputs written by the kernel straight into pinned host memory
 (TS_HOST_ZERO_COPY=1) against the default (HBM + device-to-host copy per chunk):
     TS_HOST_ZERO_COPY=0 python profiles/experiments/zero_copy_e2e.py; TS_HOST_ZERO_COPY=1 python profiles/experiments/zero_copy_e2e.py"""

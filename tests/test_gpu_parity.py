@@ -218,23 +218,28 @@ def test_limits_are_value_errors_not_fallbacks(ts):
 
 def test_sub_range_steps_touch_nothing_outside_the_range(ts):
     """The capacity contract of include/tiler_slider.h: ts_step reads and writes exactly
-    [first_env, first_env + n_envs).  A batch of 1,021 envs (capacity 1,024) has its padding
-    poisoned, and is stepped (a) whole and (b) through the ragged sub-range [0, 510) only -- the
-    envs outside the range, padding included, must stay bit for bit as they were, the envs
-    inside must match the oracle.  Covers the bitboard kernels (4-env groups + the per-env
-    kernel for the ragged end) and the wide kernel."""
+    [first_env, first_env + n_envs).  A batch of 3,001 envs (capacity 3,072) has its padding
+    poisoned, and is stepped (a) whole, (b) through the ragged sub-range [0, 510) or [0, 3) only --
+    the envs outside the range, padding included, must stay bit for bit as they were, the envs
+    inside must match the oracle -- and (c) through the consecutive sub-ranges [0, 128),
+    [128, 512), [512, 2048) and the ragged [2048, 3001): every buffer must equal the whole-batch
+    step bit for bit, so ranges that start at a non-zero first_env step exactly their own envs.
+    Covers the bitboard kernels (4-env groups + the per-env kernel for the ragged end) and the
+    wide kernel."""
     import ctypes as C
     for S, T, W, multi, auto_reset in [(6, 4, 8, True, True), (6, 4, 8, False, False), (5, 1, 5, False, True),
-                                       (8, 6, 12, True, False), (12, 8, 36, True, True), (3, 2, 1, True, True)]:
-        N, K, max_steps = 1021, 10, 6
+                                       (8, 6, 12, True, False), (12, 8, 36, True, True), (3, 2, 1, True, True),
+                                       (4, 2, 2, True, True), (8, 8, 12, True, True), (6, 3, 4, True, False)]:
+        N, K, max_steps = 3001, 10, 6
         rng = np.random.default_rng(S * 100 + T)
         blocked, tiles, targets = random_puzzles(rng, N, S, T, W)
         actions = rng.integers(0, 4, size=(K, N), dtype=np.uint8)
         want = orc.rollout(S, multi, blocked, tiles, targets, actions, max_steps=max_steps, auto_reset=auto_reset)
-        for n_range in (N, 510, 3):
+        whole = []                            # every buffer after each whole-batch step
+        for ends in ((N,), (510,), (3,), (128, 512, 2048, N)):
             env = ts.BatchedTilerSliderEnv.from_arrays(S, blocked, tiles, targets, multi, max_steps=max_steps,
                                                        auto_reset=auto_reset, track_terminal=True)
-            cap = env.capacity
+            cap, n_range = env.capacity, ends[-1]
             bufs = {k: getattr(env, k) for k in ("_pos", "_count", "_reward", "_done", "_flags", "_terminal")}
             poison = {"_pos": 0xA5, "_count": 0x5A, "_reward": -123.5, "_done": 0x77, "_flags": 0, "_terminal": 0xC3}
             for k, buf in bufs.items():       # the padding envs (flags stay 0: a set DONE bit would mean "frozen")
@@ -244,10 +249,16 @@ def test_sub_range_steps_touch_nothing_outside_the_range(ts):
             for k in range(K):
                 before = {name: buf.clone() for name, buf in bufs.items()}
                 a = env._step_args(acts[k].data_ptr())
-                a.first_env, a.n_envs = 0, n_range
-                assert ts.lib().ts_step(C.byref(a), torch.cuda.current_stream().cuda_stream) == 0
+                for lo, hi in zip((0,) + ends[:-1], ends):
+                    a.first_env, a.n_envs = lo, hi - lo
+                    assert ts.lib().ts_step(C.byref(a), torch.cuda.current_stream().cuda_stream) == 0
                 for name, buf in bufs.items():
-                    assert torch.equal(buf[n_range:], before[name][n_range:]), (S, T, name, n_range, k)
+                    assert torch.equal(buf[n_range:], before[name][n_range:]), (S, T, name, ends, k)
+                if ends == (N,):
+                    whole.append({name: buf.clone() for name, buf in bufs.items()})
+                elif n_range == N:
+                    for name, buf in bufs.items():
+                        assert torch.equal(buf, whole[k][name]), (S, T, name, ends, k)
                 d = env._done[:n_range].bool()
                 post = env.positions(env._pos[:n_range])
                 if auto_reset:
@@ -376,25 +387,6 @@ def test_synthetic_rollout_vs_oracle(ts):
             assert np.array_equal(post.cpu().numpy(), want["pos"][k])
             assert np.array_equal(env.flags.cpu().numpy(), want["flags"][k])
             assert np.array_equal(r.cpu().numpy(), want["reward"][k])
-
-
-def test_pipelined_kernel_matches_direct_kernel_and_oracle(ts):
-    """The persistent bulk-async (cp.async.bulk + mbarrier) step kernel is an opt-in experiment that
-    the product library does not carry (-DTS_WITH_PIPE; it measured 5-25 % slower).  A variant
-    library with it is built into variants/ and driven in a subprocess (TS_LIB_PATH, TS_STEP_PIPE=1):
-    batches of >= 2^18 envs stepped by the pipelined kernel against the same batches stepped by the
-    direct kernel through 65,536-env sub-ranges, bit for bit, and against the oracle."""
-    import os
-    import subprocess
-    import sys
-    from tiler_slider_b200 import _lib
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    variant = _lib.build_variant("pipe", "-DTS_WITH_PIPE")
-    env = dict(os.environ, TS_LIB_PATH=variant, TS_STEP_PIPE="1", PYTHONPATH=root)
-    out = subprocess.run([sys.executable, os.path.join(root, "tests", "pipe_variant_check.py")], env=env,
-                         capture_output=True, text=True, timeout=1500)
-    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
-    assert "pipe variant ok" in out.stdout
 
 
 def test_full_size_properties(ts):

@@ -176,30 +176,6 @@ def build(force: bool = False, jobs: int | None = None) -> str:
     return LIB_PATH
 
 
-def build_variant(name: str, extra: str, jobs: int | None = None) -> str:
-    """Compile a variant of the library (kernel experiments, e.g. the opt-in pipelined step kernel:
-    extra = "-DTS_WITH_PIPE") into variants/libts_<name>.so; load it with TS_LIB_PATH."""
-    import hashlib
-    out_dir = os.path.join(os.path.dirname(_HERE), "variants")
-    os.makedirs(out_dir, exist_ok=True)
-    out = os.path.join(out_dir, f"libts_{name}.so")
-    # a content stamp, not mtimes: the prebuilt variant travels to the GPU box without its objects
-    h = hashlib.sha256(extra.encode())
-    for fn in sorted(os.listdir(CSRC)) + [os.path.join(os.path.dirname(_HERE), "include", "tiler_slider.h")]:
-        path = fn if os.path.isabs(fn) else os.path.join(CSRC, fn)
-        if os.path.isfile(path) and path.endswith((".cu", ".cuh", ".h", "Makefile")):
-            with open(path, "rb") as f:
-                h.update(f.read())
-    stamp = out + ".stamp"
-    if os.path.exists(out) and os.path.exists(stamp) and open(stamp).read() == h.hexdigest():
-        return out
-    subprocess.check_call(["make", "-C", CSRC, f"-j{jobs or os.cpu_count() or 4}", f"EXTRA={extra}",
-                           f"BUILD=build_{name}", f"OUT={out}"], stdout=subprocess.DEVNULL)
-    with open(stamp, "w") as f:
-        f.write(h.hexdigest())
-    return out
-
-
 _lib = None
 
 

@@ -27,7 +27,6 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <type_traits>
 
 namespace ts {
@@ -111,41 +110,33 @@ template <class F> cudaError_t dispatch_small(int size, int n_tiles, F&& f) {
     });
 }
 
-// cache policy of the streaming accesses (overridable for experiments: -D'TS_LD(p)=__ldg(p)')
-#ifndef TS_LD
-#define TS_LD(p) __ldcs(p)
-#endif
-#ifndef TS_ST
-#define TS_ST(p, v) __stcs(p, v)
-#endif
-
 // ---- streaming global access ---------------------------------------------------------------
 // Every stream is touched once per step and the working set (>=400 MB at 16M envs) exceeds
 // the 126 MB L2, so loads/stores carry the evict-first (.cs) policy.
 template <int WORDS> __device__ __forceinline__ void ld_words(const void* p, uint32_t (&r)[WORDS]) {
     if constexpr (WORDS == 1) {
-        r[0] = TS_LD(reinterpret_cast<const unsigned int*>(p));
+        r[0] = __ldcs(reinterpret_cast<const unsigned int*>(p));
     } else if constexpr (WORDS == 2) {
-        uint2 v = TS_LD(reinterpret_cast<const uint2*>(p));
+        uint2 v = __ldcs(reinterpret_cast<const uint2*>(p));
         r[0] = v.x; r[1] = v.y;
     } else {
         static_assert(WORDS % 4 == 0, "group loads are 4, 8 or 16*k bytes");
 #pragma unroll
         for (int k = 0; k < WORDS / 4; ++k) {
-            uint4 v = TS_LD(reinterpret_cast<const uint4*>(p) + k);
+            uint4 v = __ldcs(reinterpret_cast<const uint4*>(p) + k);
             r[4 * k] = v.x; r[4 * k + 1] = v.y; r[4 * k + 2] = v.z; r[4 * k + 3] = v.w;
         }
     }
 }
 template <int WORDS> __device__ __forceinline__ void st_words(void* p, const uint32_t (&r)[WORDS]) {
     if constexpr (WORDS == 1) {
-        TS_ST(reinterpret_cast<unsigned int*>(p), r[0]);
+        __stcs(reinterpret_cast<unsigned int*>(p), r[0]);
     } else if constexpr (WORDS == 2) {
-        TS_ST(reinterpret_cast<uint2*>(p), make_uint2(r[0], r[1]));
+        __stcs(reinterpret_cast<uint2*>(p), make_uint2(r[0], r[1]));
     } else {
 #pragma unroll
         for (int k = 0; k < WORDS / 4; ++k)
-            TS_ST(reinterpret_cast<uint4*>(p) + k, make_uint4(r[4 * k], r[4 * k + 1], r[4 * k + 2], r[4 * k + 3]));
+            __stcs(reinterpret_cast<uint4*>(p) + k, make_uint4(r[4 * k], r[4 * k + 1], r[4 * k + 2], r[4 * k + 3]));
     }
 }
 
@@ -493,7 +484,7 @@ constexpr uint32_t F_DONE = 1, F_WON = 2, F_INVALID = 4, F_TIMEOUT = 8, F_STALE 
 // launch latency of back-to-back steps (measured, Python loop without a CUDA graph: 73.9 -> 71.9 us
 // per 16.7M-env step, 14.3 -> 12.6 us per 1M-env step; same as a graph replay).  The kernels execute
 // griddepcontrol.wait before their first global access, so whatever ran ahead of them in the
-// stream has completed and is visible.  TS_STEP_PDL=0 switches back to plain launches.
+// stream has completed and is visible.
 __device__ __forceinline__ void dependent_launch_sync() {
     asm volatile("griddepcontrol.launch_dependents;");
     asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -501,11 +492,6 @@ __device__ __forceinline__ void dependent_launch_sync() {
 
 template <typename K, typename A>
 inline void launch_dependent(K kernel, unsigned blocks, unsigned threads, cudaStream_t stream, const A& args) {
-    static const bool plain = [] { const char* e = getenv("TS_STEP_PDL"); return e && e[0] == '0'; }();   // read once
-    if (plain) {
-        kernel<<<blocks, threads, 0, stream>>>(args);
-        return;
-    }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(blocks);
     cfg.blockDim = dim3(threads);

@@ -6,7 +6,6 @@
 // so the PCIe uploads, the kernel and the downloads of neighbouring chunks overlap
 // (H2D and D2H use separate copy engines).  The call returns after all streams drained.
 #include <cstdio>
-#include <cstdlib>
 #include <vector>
 #include "ts_common.cuh"
 #include "../../include/tiler_slider.h"
@@ -51,11 +50,6 @@ int ts_step_host(ts_host_ctx* ctx, const ts_step_args* a, const uint8_t* h_actio
     const int ns = (int)ctx->streams.size();
     int rc = 0;
     int c = 0;
-    // TS_HOST_ZERO_COPY=1 (experiment): the step kernel stores reward / done / flags straight into the
-    // pinned host buffers (unified addressing: posted writes over PCIe from inside the kernel) instead of
-    // into HBM followed by a device-to-host copy per chunk
-    static const bool zero_copy = [] { const char* e = getenv("TS_HOST_ZERO_COPY"); return e && e[0] == '1'; }();
-    const bool zc = zero_copy && a->auto_reset && a->first_env % 16 == 0;   // without auto-reset the status byte is state the kernel reads back: it stays in HBM
     for (int64_t off = 0; off < a->n_envs && rc == 0; off += chunk_envs, ++c) {
         const int64_t n = (a->n_envs - off < chunk_envs) ? a->n_envs - off : chunk_envs;
         const int64_t e0 = a->first_env + off;
@@ -66,15 +60,6 @@ int ts_step_host(ts_host_ctx* ctx, const ts_step_args* a, const uint8_t* h_actio
         ts_step_args sub = *a;
         sub.first_env = e0;
         sub.n_envs = n;
-        if (zc) {                                  // arrays are indexed by absolute env: element first_env is host element 0
-            if (h_reward) sub.d_reward = h_reward - a->first_env;
-            sub.d_done = h_done ? h_done - a->first_env : nullptr;
-            sub.d_flags = h_flags ? h_flags - a->first_env : nullptr;
-            if (!sub.d_done && !sub.d_flags) sub.d_done = a->d_done;
-            rc = ts_step(&sub, s);
-            if (rc) break;
-            continue;
-        }
         rc = ts_step(&sub, s);
         if (rc) break;
         e = cudaSuccess;

@@ -83,7 +83,6 @@ __global__ void __launch_bounds__(OBS_THREADS) observe_kernel(const ts_observe_a
         }
     }
     float* out = a.d_obs + env0 * PER_ENV;          // 16-byte aligned: E * PER_ENV is a multiple of 4
-#ifndef TS_OBS_NO_BULK
     // Stream-out by the copy engine of the SM: one elected thread hands the whole staged image
     // (up to 28 KB, contiguous in HBM) to cp.async.bulk (TMA 1-D, SASS UBLKCP) instead of 256 threads
     // looping over 16-byte stores.  The writers publish their shared-memory stores to the async
@@ -100,7 +99,6 @@ __global__ void __launch_bounds__(OBS_THREADS) observe_kernel(const ts_observe_a
         }
         return;
     }
-#endif
     __syncthreads();
     for (int k = threadIdx.x; k * 4 < n_floats; k += OBS_THREADS) {
         if (k * 4 + 3 < n_floats) __stcs(reinterpret_cast<float4*>(out) + k, reinterpret_cast<const float4*>(stage)[k]);

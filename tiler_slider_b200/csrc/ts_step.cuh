@@ -10,16 +10,12 @@
 // coalesced.  The kernel is bound by the integer ALU pipe, not by HBM (profiles/), so the
 // per-env bookkeeping is done SWAR on the four packed status bytes of the thread's envs.
 #pragma once
-#include <cstdlib>
 #include "ts_common.cuh"
 #include "../../include/tiler_slider.h"
 
 namespace ts {
 
-#ifndef TS_STEP_THREADS
-#define TS_STEP_THREADS 256
-#endif
-constexpr int STEP_THREADS = TS_STEP_THREADS;
+constexpr int STEP_THREADS = 256;
 
 // Resident CTAs per SM requested from ptxas.  The kernel needs every warp it can get to
 // cover the load latency at the top of each thread (measured: 8 CTAs x 256 threads = full
@@ -27,13 +23,9 @@ constexpr int STEP_THREADS = TS_STEP_THREADS;
 // variants that fit 32 registers without spilling are forced there.
 template <int S, int T, int GOAL, bool AR, int CW>
 constexpr int step_min_blocks() {
-#ifdef TS_STEP_MINBLOCKS
-    return TS_STEP_MINBLOCKS;
-#else
     if (padded_board(S) && T <= 4 && GOAL == TS_GOAL_ORDERED && CW == 1) return 8;
     if (T <= 4) return 6;
     return 4;
-#endif
 }
 
 // bit 7 of every byte of the result = (byte of a) >= (byte of b); b given as its low 7 bits
@@ -171,11 +163,11 @@ __device__ __forceinline__ void step_group(const ts_step_args& a, uint32_t g, St
 
     // ---- stores --------------------------------------------------------------------------------
     st_words<PW>(a.d_pos + e0 * PW, pnew);
-    if constexpr (CW == 1) TS_ST(reinterpret_cast<unsigned int*>(a.d_step_count) + g, c1);
-    else TS_ST(reinterpret_cast<uint4*>(a.d_step_count) + g, make_uint4(cntw[0], cntw[1], cntw[2], cntw[3]));
-    TS_ST(reinterpret_cast<float4*>(a.d_reward) + g, make_float4(rew[0], rew[1], rew[2], rew[3]));
-    if (a.d_done) TS_ST(reinterpret_cast<unsigned int*>(a.d_done + e0), done1);
-    if (a.d_flags) TS_ST(reinterpret_cast<unsigned int*>(a.d_flags + e0), flags4);
+    if constexpr (CW == 1) __stcs(reinterpret_cast<unsigned int*>(a.d_step_count) + g, c1);
+    else __stcs(reinterpret_cast<uint4*>(a.d_step_count) + g, make_uint4(cntw[0], cntw[1], cntw[2], cntw[3]));
+    __stcs(reinterpret_cast<float4*>(a.d_reward) + g, make_float4(rew[0], rew[1], rew[2], rew[3]));
+    if (a.d_done) __stcs(reinterpret_cast<unsigned int*>(a.d_done + e0), done1);
+    if (a.d_flags) __stcs(reinterpret_cast<unsigned int*>(a.d_flags + e0), flags4);
 }
 
 // fill the per-block table of direction parameters (threads 0..3) -- call before any early return
@@ -216,258 +208,26 @@ __global__ void __launch_bounds__(STEP_THREADS, (step_min_blocks<S, T, GOAL, AR,
     in.walls.load(a.d_walls, cap, g);
     if constexpr (GOAL == TS_GOAL_ORDERED) ld_words<PW>(a.d_targets_packed + e0 * PW, in.traw);
     else in.tboard.load(a.d_targets_packed, cap, g);
-    in.act4 = TS_LD(reinterpret_cast<const unsigned int*>(a.d_actions + e0));
+    in.act4 = __ldcs(reinterpret_cast<const unsigned int*>(a.d_actions + e0));
     in.cnt4 = 0;
     if constexpr (CW == 1) {
-        in.cnt4 = TS_LD(reinterpret_cast<const unsigned int*>(a.d_step_count) + g);
+        in.cnt4 = __ldcs(reinterpret_cast<const unsigned int*>(a.d_step_count) + g);
     } else {
-        const uint4 c = TS_LD(reinterpret_cast<const uint4*>(a.d_step_count) + g);
+        const uint4 c = __ldcs(reinterpret_cast<const uint4*>(a.d_step_count) + g);
         in.cntw[0] = c.x; in.cntw[1] = c.y; in.cntw[2] = c.z; in.cntw[3] = c.w;
     }
     in.prev_flags = 0;
-    if constexpr (!AR) in.prev_flags = TS_LD(reinterpret_cast<const unsigned int*>(a.d_flags + e0));
+    if constexpr (!AR) in.prev_flags = __ldcs(reinterpret_cast<const unsigned int*>(a.d_flags + e0));
     step_group<S, T, GOAL, AR, CW>(a, g, in, dir_tab);
-}
-
-// ---- OPT-IN experiment, compiled only with -DTS_WITH_PIPE (make EXTRA=-DTS_WITH_PIPE OUT=...): the
-// product library does not carry it (it doubled the size of the .so for a kernel measured slower).
-#ifdef TS_WITH_PIPE
-// ---- pipelined kernel: persistent CTAs, bulk-async (TMA 1-D) staging through shared memory -----
-// A tile is PIPE_THREADS groups (4*PIPE_THREADS envs).  Every input stream of a tile is one
-// contiguous run of bytes in HBM (env-innermost planes), so one elected thread fetches a whole
-// tile with a handful of cp.async.bulk copies that complete on an mbarrier; PIPE_STAGES tiles
-// are in flight per CTA, so no warp ever waits on a global load (the direct kernel loses about
-// a third of its issue slots to exactly that, profiles/).  Consumers read their 16 bytes per
-// stream from shared memory (conflict-free), hand the stage back with one __syncthreads, and
-// compute while the next tiles land.  Narrow step counter only (CW == 1).
-#ifndef TS_PIPE_THREADS
-#define TS_PIPE_THREADS 256
-#endif
-#ifndef TS_PIPE_STAGES
-#define TS_PIPE_STAGES 2
-#endif
-#ifndef TS_PIPE_MINBLOCKS
-#define TS_PIPE_MINBLOCKS 1
-#endif
-constexpr int PIPE_THREADS = TS_PIPE_THREADS;
-constexpr int PIPE_STAGES = TS_PIPE_STAGES;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "TS_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra TS_DONE;\n"
-        "bra TS_WAIT;\n"
-        "TS_DONE:\n"
-        "}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-
-template <int S, int T, int GOAL, bool AR>
-struct PipeLayout {
-    static constexpr int PW = pos_bytes(T), NB = board_bytes(S);
-    static constexpr int TB = (GOAL == TS_GOAL_ORDERED) ? PW : NB;              // target bytes per env
-    // byte offsets inside one stage, per stream, for a full tile (GROUP*PIPE_THREADS envs)
-    static constexpr int ENVS = GROUP * PIPE_THREADS;
-    static constexpr int OFF_POS = 0;
-    static constexpr int OFF_TGT = OFF_POS + ENVS * PW;
-    static constexpr int OFF_WALLS = OFF_TGT + ENVS * TB;
-    static constexpr int OFF_CNT = OFF_WALLS + ENVS * NB;
-    static constexpr int OFF_ACT = OFF_CNT + ENVS;
-    static constexpr int OFF_FLG = OFF_ACT + ENVS;
-    static constexpr int STAGE_BYTES = OFF_FLG + (AR ? 0 : ENVS);
-    static constexpr int SMEM_BYTES = STAGE_BYTES * PIPE_STAGES;
-};
-
-// one board buffer (plane layout) of a tile: global -> shared, plane by plane
-template <int NB>
-__device__ __forceinline__ uint32_t bulk_board(uint8_t* sdst, const uint8_t* gbase, size_t cap, size_t env0, uint32_t n_envs, uint64_t* bar) {
-    uint32_t bytes = 0;
-    static_for<0, plane_count(NB)>([&](auto I) {
-        constexpr int k = decltype(I)::value;
-        constexpr int w = plane_width(NB, k), off = plane_offset(NB, k);
-        bulk_g2s(sdst + (size_t)off * (GROUP * PIPE_THREADS), gbase + (size_t)off * cap + env0 * w, n_envs * w, bar);
-        bytes += n_envs * w;
-    });
-    return bytes;
-}
-template <int NB>
-__device__ __forceinline__ void board_from_smem(BoardGroup<NB>& b, const uint8_t* s, uint32_t t) {
-    static_for<0, plane_count(NB)>([&](auto I) {
-        constexpr int k = decltype(I)::value;
-        constexpr int w = plane_width(NB, k), off = plane_offset(NB, k);
-        const uint8_t* p = s + (size_t)off * (GROUP * PIPE_THREADS) + (size_t)t * (GROUP * w);
-        if constexpr (w == 1) b.raw[off] = *reinterpret_cast<const uint32_t*>(p);
-        else if constexpr (w == 2) { const uint2 v = *reinterpret_cast<const uint2*>(p); b.raw[off] = v.x; b.raw[off + 1] = v.y; }
-        else {
-#pragma unroll
-            for (int j = 0; j < w / 4; ++j) {
-                const uint4 v = reinterpret_cast<const uint4*>(p)[j];
-                b.raw[off + 4 * j] = v.x; b.raw[off + 4 * j + 1] = v.y; b.raw[off + 4 * j + 2] = v.z; b.raw[off + 4 * j + 3] = v.w;
-            }
-        }
-    });
-}
-template <int W> __device__ __forceinline__ void words_from_smem(uint32_t (&r)[W], const uint8_t* s, uint32_t t) {
-    const uint8_t* p = s + (size_t)t * (GROUP * W);
-    if constexpr (W == 1) r[0] = *reinterpret_cast<const uint32_t*>(p);
-    else if constexpr (W == 2) { const uint2 v = *reinterpret_cast<const uint2*>(p); r[0] = v.x; r[1] = v.y; }
-    else {
-#pragma unroll
-        for (int j = 0; j < W / 4; ++j) {
-            const uint4 v = reinterpret_cast<const uint4*>(p)[j];
-            r[4 * j] = v.x; r[4 * j + 1] = v.y; r[4 * j + 2] = v.z; r[4 * j + 3] = v.w;
-        }
-    }
-}
-
-template <int S, int T, int GOAL, bool AR>
-__global__ void __launch_bounds__(PIPE_THREADS, TS_PIPE_MINBLOCKS) step_kernel_pipe(const __grid_constant__ ts_step_args a) {
-    using L = PipeLayout<S, T, GOAL, AR>;
-    constexpr int PW = L::PW, NB = L::NB;
-    extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ __align__(8) uint64_t full_bar[PIPE_STAGES];
-    __shared__ uint4 dir_tab[4];
-    fill_dir_tab<S>(dir_tab);
-
-    const uint32_t tid = threadIdx.x;
-    const size_t cap = (size_t)a.capacity;
-    // groups rounded up to 32 (= 128 envs, the capacity granularity): every bulk copy is then a
-    // multiple of 16 bytes; the few padding envs past n_envs lie inside the allocation
-    const uint32_t n_groups = (((uint32_t)((a.n_envs + GROUP - 1) / GROUP)) + 31u) & ~31u;
-    const uint32_t g_first = (uint32_t)(a.first_env / GROUP);
-    const uint32_t n_tiles = (n_groups + PIPE_THREADS - 1) / PIPE_THREADS;
-
-    auto issue = [&](uint32_t tile, uint32_t stage) {   // one elected thread
-        const uint32_t ng = min((uint32_t)PIPE_THREADS, n_groups - tile * PIPE_THREADS);
-        const uint32_t ne = ng * GROUP;
-        const size_t env0 = ((size_t)g_first + (size_t)tile * PIPE_THREADS) * GROUP;
-        uint8_t* s = smem + (size_t)stage * L::STAGE_BYTES;
-        uint64_t* bar = &full_bar[stage];
-        uint32_t bytes = ne * PW + ne + ne + ne * NB + (GOAL == TS_GOAL_ORDERED ? ne * PW : ne * NB) + (AR ? 0u : ne);
-        mbar_expect_tx(bar, bytes);
-        bulk_g2s(s + L::OFF_POS, a.d_pos + env0 * PW, ne * PW, bar);
-        if constexpr (GOAL == TS_GOAL_ORDERED) bulk_g2s(s + L::OFF_TGT, a.d_targets_packed + env0 * PW, ne * PW, bar);
-        else bulk_board<NB>(s + L::OFF_TGT, a.d_targets_packed, cap, env0, ne, bar);
-        bulk_board<NB>(s + L::OFF_WALLS, a.d_walls, cap, env0, ne, bar);
-        bulk_g2s(s + L::OFF_CNT, reinterpret_cast<const uint8_t*>(a.d_step_count) + env0, ne, bar);
-        bulk_g2s(s + L::OFF_ACT, a.d_actions + env0, ne, bar);
-        if constexpr (!AR) bulk_g2s(s + L::OFF_FLG, a.d_flags + env0, ne, bar);
-    };
-
-    if (tid == 0) {
-#pragma unroll
-        for (int s = 0; s < PIPE_STAGES; ++s) mbar_init(&full_bar[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (tid == 0) {
-#pragma unroll
-        for (int s = 0; s < PIPE_STAGES; ++s) {
-            const uint32_t tile = blockIdx.x + (uint32_t)s * gridDim.x;
-            if (tile < n_tiles) issue(tile, s);
-        }
-    }
-
-    uint32_t it = 0;
-    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-        const uint32_t stage = it % PIPE_STAGES;
-        const uint32_t parity = (it / PIPE_STAGES) & 1u;
-        const uint32_t ng = min((uint32_t)PIPE_THREADS, n_groups - tile * PIPE_THREADS);
-        const uint8_t* s = smem + (size_t)stage * L::STAGE_BYTES;
-        mbar_wait(&full_bar[stage], parity);
-
-        StepInputs<S, T, GOAL, 1> in;
-        const bool active = tid < ng;
-        if (active) {
-            words_from_smem<PW>(in.praw, s + L::OFF_POS, tid);
-            if constexpr (GOAL == TS_GOAL_ORDERED) words_from_smem<PW>(in.traw, s + L::OFF_TGT, tid);
-            else board_from_smem<NB>(in.tboard, s + L::OFF_TGT, tid);
-            board_from_smem<NB>(in.walls, s + L::OFF_WALLS, tid);
-            in.cnt4 = reinterpret_cast<const uint32_t*>(s + L::OFF_CNT)[tid];
-            in.act4 = reinterpret_cast<const uint32_t*>(s + L::OFF_ACT)[tid];
-            in.prev_flags = 0;
-            if constexpr (!AR) in.prev_flags = reinterpret_cast<const uint32_t*>(s + L::OFF_FLG)[tid];
-        }
-        __syncthreads();                                   // every thread has taken its inputs out of the stage
-        if (tid == 0) {
-            const uint32_t next = tile + (uint32_t)PIPE_STAGES * gridDim.x;
-            if (next < n_tiles) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                issue(next, stage);
-            }
-        }
-        if (active) step_group<S, T, GOAL, AR, 1>(a, g_first + tile * PIPE_THREADS + tid, in, dir_tab);
-    }
-}
-
-// persistent grid of the pipelined kernel: as many CTAs per SM as shared memory allows
-template <int S, int T, int GOAL, bool AR>
-inline bool launch_step_pipe(const ts_step_args& a, cudaStream_t stream) {
-    using L = PipeLayout<S, T, GOAL, AR>;
-    static int ctas_per_sm = -1, n_sm = 0;      // per template instantiation; same answer on every device of a box
-    auto kernel = step_kernel_pipe<S, T, GOAL, AR>;
-    if (ctas_per_sm < 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L::SMEM_BYTES) != cudaSuccess) { cudaGetLastError(); ctas_per_sm = 0; return false; }
-        int occ = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, PIPE_THREADS, L::SMEM_BYTES) != cudaSuccess) { cudaGetLastError(); occ = 0; }
-        ctas_per_sm = occ;
-    }
-    if (ctas_per_sm <= 0) return false;
-    const uint32_t n_groups = (((uint32_t)((a.n_envs + GROUP - 1) / GROUP)) + 31u) & ~31u;
-    const uint32_t n_tiles = (n_groups + PIPE_THREADS - 1) / PIPE_THREADS;
-    const uint32_t grid = min(n_tiles, (uint32_t)(ctas_per_sm * n_sm));
-    kernel<<<grid, PIPE_THREADS, L::SMEM_BYTES, stream>>>(a);
-    return true;
-}
-
-// The pipelined kernel is OPT-IN (environment variable TS_STEP_PIPE=1): measured on B200 it is
-// 5-25 % slower than the direct kernel at every (threads, stages) setting tried (78.7-96 us vs
-// 74.7 us per 16.7M-env step, DESIGN.md section 5) -- the step is bound by instruction issue, the
-// direct kernel already hides its load latency with 8 resident CTAs per SM, and the staging
-// buffers cap the pipelined kernel at fewer warps.  It needs 128-env aligned ranges and the
-// 1-byte step counter.
-inline bool use_pipe(const ts_step_args& a) {
-    const char* e = getenv("TS_STEP_PIPE");     // read per call: tests switch it on for one test only
-    const bool enabled = e && e[0] == '1';
-    // whole 128-env tiles only: the kernel steps every env of a tile it touches
-    return enabled && a.count_bytes == 1 && a.first_env % CAP_ALIGN == 0 && a.n_envs % CAP_ALIGN == 0 && a.n_envs >= (int64_t)1 << 18;
-}
-#endif  // TS_WITH_PIPE
-
-template <typename K>
-inline void launch_direct(K kernel, const ts_step_args& a, unsigned blocks, cudaStream_t stream) {
-    launch_dependent(kernel, blocks, STEP_THREADS, stream, a);
 }
 
 template <int S, int T, int GOAL>
 inline void launch_step_goal(const ts_step_args& a, unsigned blocks, cudaStream_t stream) {
     const bool ar = a.auto_reset != 0, narrow = a.count_bytes == 1;
-#ifdef TS_WITH_PIPE
-    if (use_pipe(a)) {
-        const bool ok = ar ? launch_step_pipe<S, T, GOAL, true>(a, stream) : launch_step_pipe<S, T, GOAL, false>(a, stream);
-        if (ok) return;
-    }
-#endif
-    if (ar && narrow) launch_direct(step_kernel<S, T, GOAL, true, 1>, a, blocks, stream);
-    else if (ar) launch_direct(step_kernel<S, T, GOAL, true, 4>, a, blocks, stream);
-    else if (narrow) launch_direct(step_kernel<S, T, GOAL, false, 1>, a, blocks, stream);
-    else launch_direct(step_kernel<S, T, GOAL, false, 4>, a, blocks, stream);
+    if (ar && narrow) launch_dependent(step_kernel<S, T, GOAL, true, 1>, blocks, STEP_THREADS, stream, a);
+    else if (ar) launch_dependent(step_kernel<S, T, GOAL, true, 4>, blocks, STEP_THREADS, stream, a);
+    else if (narrow) launch_dependent(step_kernel<S, T, GOAL, false, 1>, blocks, STEP_THREADS, stream, a);
+    else launch_dependent(step_kernel<S, T, GOAL, false, 4>, blocks, STEP_THREADS, stream, a);
 }
 
 template <int S, int T>

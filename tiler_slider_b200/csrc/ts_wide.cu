@@ -36,9 +36,7 @@
 namespace ts {
 
 constexpr int WIDE_THREADS = 256;
-#ifndef WIDE_MIN_BLOCKS
-#define WIDE_MIN_BLOCKS 8
-#endif
+constexpr int WIDE_MIN_BLOCKS = 8;
 
 struct WideSmem {
     uint32_t w[8][WIDE_THREADS];   // wall lines, two 16-bit lines per word
