@@ -27,13 +27,22 @@
  *    defined for blocked start cells, therefore probes on a board whose start cell is open.
  *
  * Packed layout (struct-of-arrays, environment index innermost):
- *  - capacity: allocation stride in environments, a multiple of TS_CAP_ALIGN.  EVERY per-env
- *    array handed to the library (state, actions, reward, done, flags, ...) must hold
- *    `capacity` elements.  ts_step reads and writes exactly the envs of its range
- *    [first_env, first_env + n_envs): whole 4-env groups go through the vectorised kernel, the
- *    ragged end (n_envs % 4 envs) through a per-env kernel.  The pure queries ts_valid_moves and
- *    ts_goal_check may also WRITE their (correct) result for the up-to-3 envs that share the last
- *    4-env group of the range.
+ *  - capacity: allocation stride in environments, a multiple of TS_CAP_ALIGN, below 2^33.  EVERY
+ *    per-env array handed to the library (state, actions, reward, done, flags, ...) must hold
+ *    `capacity` elements.  A call covers the env range [first_env, first_env + n_envs), first_env a
+ *    multiple of 4; ts_step on boards of size 9..16 with 1..8 tiles needs first_env + n_envs < 2^32
+ *    (32-bit env index; TS_E_BAD_RANGE otherwise).
+ *  - write set of each entry point (everything else is left as it was, bit for bit):
+ *      ts_encode, ts_synth, ts_step, ts_pool_reset: exactly the envs of the range (ts_step: whole
+ *        4-env groups through the vectorised kernel, the ragged end, n_envs % 4 envs, through a
+ *        per-env kernel);
+ *      ts_observe: d_obs[0 .. n_envs) -- d_obs is RELATIVE to the range: env first_env + i is
+ *        written to d_obs[i];
+ *      ts_valid_moves, ts_goal_check: d_mask / d_won are ABSOLUTE (env e at [e]); the range, and on
+ *        boards up to 8x8 with 1..8 tiles also the (correct) result of the up-to-3 envs after the
+ *        range that share its last 4-env group;
+ *      ts_step_host: the device buffers as ts_step; the host buffers are RELATIVE to the range,
+ *        elements [0, n_envs).
  *  - position word: ts_pos_bytes(T) in {1,2,4,8,16,32} bytes per env, byte i = row*PS + col of tile
  *    i (PS = ts_pos_stride(S)), unused bytes zero.  Arrays: pos (in/out), init, targets
  *    (ordered mode).
@@ -184,7 +193,9 @@ int ts_step(const ts_step_args *a, void *stream);
  *   1 (set mode), ch2 target index+1 or 1.  In set mode targets come from the bitboard.
  *   n_targets (ordered mode): 0 = as many targets as tiles, d_targets_packed as ts_step reads it;
  *   k > 0 = k targets in words of ts_pos_bytes(k) bytes per env (a board whose target count
- *   differs from its tile count, which ts_step's packed word cannot hold); -1 = no targets.
+ *   differs from its tile count, which ts_step's packed word cannot hold); -1 = no targets;
+ *   outside -1..32: TS_E_BAD_TILES.  goal_mode other than TS_GOAL_ORDERED / TS_GOAL_SET:
+ *   TS_E_BAD_ARGUMENT.  d_obs must be 16-byte aligned and hold n_envs*size*size*3 floats.
  * ------------------------------------------------------------------------------------- */
 typedef struct ts_observe_args {
     int32_t size, n_tiles, goal_mode, n_targets;

@@ -224,12 +224,15 @@ def test_sub_range_steps_touch_nothing_outside_the_range(ts):
     inside must match the oracle -- and (c) through the consecutive sub-ranges [0, 128),
     [128, 512), [512, 2048) and the ragged [2048, 3001): every buffer must equal the whole-batch
     step bit for bit, so ranges that start at a non-zero first_env step exactly their own envs.
-    Covers the bitboard kernels (4-env groups + the per-env kernel for the ragged end) and the
-    wide kernel."""
+    Covers the bitboard kernels (4-env groups + the per-env kernel for the ragged end), the wide
+    kernel, and the generic kernels (9..32 tiles on narrow and wide boards, and boards without
+    tiles)."""
     import ctypes as C
     for S, T, W, multi, auto_reset in [(6, 4, 8, True, True), (6, 4, 8, False, False), (5, 1, 5, False, True),
                                        (8, 6, 12, True, False), (12, 8, 36, True, True), (3, 2, 1, True, True),
-                                       (4, 2, 2, True, True), (8, 8, 12, True, True), (6, 3, 4, True, False)]:
+                                       (4, 2, 2, True, True), (8, 8, 12, True, True), (6, 3, 4, True, False),
+                                       (6, 12, 6, True, True), (10, 20, 12, False, False), (5, 0, 3, False, True),
+                                       (9, 4, 20, False, False), (16, 8, 60, True, True)]:
         N, K, max_steps = 3001, 10, 6
         rng = np.random.default_rng(S * 100 + T)
         blocked, tiles, targets = random_puzzles(rng, N, S, T, W)

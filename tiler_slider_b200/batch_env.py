@@ -301,6 +301,7 @@ class BatchedTilerSliderEnv:
             if obs_out is not None:
                 o = self._cached_obs_args
                 if o is None or o.d_obs != obs_out.data_ptr():
+                    self._check_obs_out(obs_out)
                     o = self._cached_obs_args = self._observe_args(obs_out)
                 rc = self._lib.ts_observe(C.byref(o), stream.cuda_stream)
                 if rc:
@@ -549,16 +550,31 @@ class BatchedTilerSliderEnv:
         return self._board_cells(self._targets)
 
     def observe(self, out: torch.Tensor | None = None) -> torch.Tensor:
-        """K3: float32[N,S,S,3] observation, GameState.get_state_array (state.py:188-211)."""
+        """K3: float32[N,S,S,3] observation, GameState.get_state_array (state.py:188-211).  `out`:
+        a contiguous float32[N,S,S,3] tensor on the batch's device or in pinned host memory, 16-byte
+        aligned; anything else raises ValueError (misalignment: TilerSliderError) before a launch."""
         self._require_loaded()
         S, n = self.size, self.n_envs
         if out is None:
             out = torch.empty(n, S, S, 3, dtype=torch.float32, device=self.device)
+        else:
+            self._check_obs_out(out)
         # single colour with one tile is stored as an ordered batch: index+1 == 1, same values
         a = self._observe_args(out)
         with torch.cuda.device(self.device):
             check(self._lib.ts_observe(C.byref(a), self._stream()), "ts_observe")
         return out
+
+    def _check_obs_out(self, out: torch.Tensor) -> None:
+        # the kernel writes n*S*S*3 floats from out.data_ptr() on and cannot check a size: a wrong
+        # tensor would be written past its end (16-byte alignment is checked by ts_observe)
+        S, n = self.size, self.n_envs
+        if not isinstance(out, torch.Tensor) or tuple(out.shape) != (n, S, S, 3) or out.dtype != torch.float32:
+            raise ValueError(f"observe(out): out must be a float32 tensor of shape ({n}, {S}, {S}, 3)")
+        if not out.is_contiguous():
+            raise ValueError("observe(out): out must be contiguous")
+        if out.device != self.device and not (out.device.type == "cpu" and out.is_pinned()):
+            raise ValueError(f"observe(out): out must live on {self.device} (or in pinned host memory), not on {out.device}")
 
     def _observe_args(self, out: torch.Tensor) -> ObserveArgs:
         # a never_win batch draws its ordered targets from their own buffer (count != tile count)

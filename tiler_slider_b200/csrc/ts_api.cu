@@ -188,6 +188,10 @@ int ts_step(const ts_step_args* a, void* stream) {
                           a->d_reward, a->d_done, a->d_flags, a->d_terminal_pos};
     for (const void* p : ptrs)
         if (p && !aligned16(p)) return fail(TS_E_MISALIGNED, "device pointer %p is not 16-byte aligned", p);
+    // the wide kernel (S >= 9, 1..8 tiles) indexes envs with 32 bits (ts_wide.cu)
+    if (wide_board(a->size) && a->n_tiles >= 1 && a->n_tiles <= MAX_TILES && a->first_env + a->n_envs >= ((int64_t)1 << 32))
+        return fail(TS_E_BAD_RANGE, "env range [%lld, %lld) exceeds the 2^32-env limit of boards of size 9..16 with 1..%d tiles",
+                    (long long)a->first_env, (long long)(a->first_env + a->n_envs), MAX_TILES);
     if (a->n_envs == 0) return 0;
     ts_step_args args = *a;
     if (args.max_steps < 1) args.max_steps = 1;   // step_count >= max_steps holds on the first step either way
@@ -222,6 +226,10 @@ int ts_step(const ts_step_args* a, void* stream) {
 int ts_observe(const ts_observe_args* a, void* stream) {
     if (!a) return fail(TS_E_NULL_POINTER, "null args");
     if (int rc = check_shape(a->size, a->n_tiles, a->first_env, a->n_envs, a->capacity)) return rc;
+    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
+    // ordered targets are read as a position word of ts_pos_bytes(n_targets) bytes, which holds at most 32
+    if (a->goal_mode == TS_GOAL_ORDERED && (a->n_targets < -1 || a->n_targets > MAX_TILES_ANY))
+        return fail(TS_E_BAD_TILES, "n_targets %d outside -1..%d", a->n_targets, MAX_TILES_ANY);
     if (!a->d_walls || !a->d_targets_packed || !a->d_pos || !a->d_obs) return fail(TS_E_NULL_POINTER, "null device pointer");
     if (a->n_envs == 0) return 0;
     if (!aligned16(a->d_obs)) return fail(TS_E_MISALIGNED, "d_obs %p is not 16-byte aligned", (const void*)a->d_obs);

@@ -377,7 +377,8 @@ template <int T, int GOAL> static void launch_wide_step_goal(const ts_step_args&
     }
 }
 template <int T> static cudaError_t launch_wide_step(const ts_step_args& a, cudaStream_t st) {
-    if (a.first_env + a.n_envs >= ((int64_t)1 << 32)) return cudaErrorInvalidValue;   // 32-bit env index
+    // 32-bit env index: ts_step refuses such a range with TS_E_BAD_RANGE before it gets here; kept as a backstop
+    if (a.first_env + a.n_envs >= ((int64_t)1 << 32)) return cudaErrorInvalidValue;
     const unsigned blocks = (unsigned)((a.n_envs + WIDE_THREADS - 1) / WIDE_THREADS);
     if (a.goal_mode == TS_GOAL_ORDERED) launch_wide_step_goal<T, TS_GOAL_ORDERED>(a, blocks, st);
     else launch_wide_step_goal<T, TS_GOAL_SET>(a, blocks, st);
