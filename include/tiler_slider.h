@@ -38,6 +38,8 @@
  *        per-env kernel);
  *      ts_observe: d_obs[0 .. n_envs) -- d_obs is RELATIVE to the range: env first_env + i is
  *        written to d_obs[i];
+ *      ts_observe_planes: d_out[0 .. n_envs*C*size*size) elements, RELATIVE to the range as
+ *        ts_observe's;
  *      ts_valid_moves, ts_goal_check: d_mask / d_won are ABSOLUTE (env e at [e]); the range, and on
  *        boards up to 8x8 with 1..8 tiles also the (correct) result of the up-to-3 envs after the
  *        range that share its last 4-env group;
@@ -204,6 +206,37 @@ typedef struct ts_observe_args {
     float *d_obs;
 } ts_observe_args;
 int ts_observe(const ts_observe_args *a, void *stream);
+
+/* ---------------------------------------------------------------------------------------
+ * ts_observe_planes: the observation as a network input (csrc/ts_observe_planes.cu; no
+ * reference counterpart).  d_out [n_envs][C][size][size], channel first, contiguous, every
+ * element 0 or 1 in the type `dtype` names (TS_OBS_U8 / BF16 / F16 / F32: 1, 2, 2, 4 bytes).
+ *   plane 0            blocked cells
+ *   ordered goal       plane 1+i: tile i's cell (i < n_tiles); plane 1+n_tiles+j: target j's cell
+ *                      (j < NT; NT from n_targets as in ts_observe: 0 = n_tiles, k > 0 = k, -1 = 0;
+ *                      duplicate targets each keep their own plane);  C = 1 + n_tiles + NT
+ *   set goal           plane 1: the tile cells; plane 2: the target cells (the bitboard);  C = 3
+ * (single colour with one tile and one target gives the same 3 planes under either rule.)
+ * Relation to ts_observe (channels last, HWC): set goal -- the planes are its three channels;
+ * ordered goal -- ch0 = plane 0, ch1 = sum_i (i+1) plane(1+i), ch2 = max_j (j+1) plane(1+n_tiles+j).
+ * ts_observe_planes_channels: C for these arguments (pure host arithmetic), or a negative
+ * TS_E_* code when goal_mode, n_tiles or n_targets is out of range.  Argument errors as
+ * ts_observe's, plus an unknown dtype (TS_E_BAD_ARGUMENT); d_out must be 16-byte aligned and hold
+ * n_envs*C*size*size elements.
+ * ------------------------------------------------------------------------------------- */
+#define TS_OBS_U8 0
+#define TS_OBS_BF16 1
+#define TS_OBS_F16 2
+#define TS_OBS_F32 3
+typedef struct ts_observe_planes_args {
+    int32_t size, n_tiles, goal_mode, n_targets;
+    int64_t first_env, n_envs, capacity;
+    const uint8_t *d_walls, *d_targets_packed, *d_pos;
+    int32_t dtype, reserved0;
+    void *d_out;
+} ts_observe_planes_args;
+int ts_observe_planes_channels(const ts_observe_planes_args *a);
+int ts_observe_planes(const ts_observe_planes_args *a, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * ts_valid_moves: bit d of d_mask[env] set when move d changes any tile position

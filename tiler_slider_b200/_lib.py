@@ -24,6 +24,7 @@ RECIPE_UNIFORM, RECIPE_WALK = 0, 1
 MAX_WALK = 65535
 OPT_UNSOLVABLE, OPT_CUTOFF, OPT_NOT_SEARCHED = -1, -2, -3
 OPT_MAX_DEPTH = 254
+OBS_U8, OBS_BF16, OBS_F16, OBS_F32 = 0, 1, 2, 3
 
 _vp, _i32, _i64, _f32 = C.c_void_p, C.c_int32, C.c_int64, C.c_float
 
@@ -57,6 +58,13 @@ class ObserveArgs(C.Structure):
     _fields_ = [("size", _i32), ("n_tiles", _i32), ("goal_mode", _i32), ("n_targets", _i32),
                 ("first_env", _i64), ("n_envs", _i64), ("capacity", _i64),
                 ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp), ("d_obs", _vp)]
+
+
+class ObservePlanesArgs(C.Structure):
+    _fields_ = [("size", _i32), ("n_tiles", _i32), ("goal_mode", _i32), ("n_targets", _i32),
+                ("first_env", _i64), ("n_envs", _i64), ("capacity", _i64),
+                ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp),
+                ("dtype", _i32), ("reserved0", _i32), ("d_out", _vp)]
 
 
 class ValidArgs(C.Structure):
@@ -137,6 +145,8 @@ SYMBOLS = {
     "ts_synth": (C.c_int, [C.POINTER(SynthArgs), _vp]),
     "ts_step": (C.c_int, [C.POINTER(StepArgs), _vp]),
     "ts_observe": (C.c_int, [C.POINTER(ObserveArgs), _vp]),
+    "ts_observe_planes_channels": (C.c_int, [C.POINTER(ObservePlanesArgs)]),
+    "ts_observe_planes": (C.c_int, [C.POINTER(ObservePlanesArgs), _vp]),
     "ts_valid_moves": (C.c_int, [C.POINTER(ValidArgs), _vp]),
     "ts_goal_check": (C.c_int, [C.POINTER(GoalArgs), _vp]),
     "ts_bfs_seed": (C.c_int, [C.POINTER(BfsArgs), _vp]),

@@ -17,11 +17,14 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (CAP_ALIGN, F_WON, GOAL_ORDERED, GOAL_SET, MAX_SIZE, MAX_TILES, EncodeArgs, GoalArgs, ObserveArgs,
-                   PoolResetArgs, StepArgs, SynthArgs, ValidArgs, check, lib)
+from ._lib import (CAP_ALIGN, F_WON, GOAL_ORDERED, GOAL_SET, MAX_SIZE, MAX_TILES, OBS_BF16, OBS_F16, OBS_F32, OBS_U8,
+                   EncodeArgs, GoalArgs, ObserveArgs, ObservePlanesArgs, PoolResetArgs, StepArgs, SynthArgs, ValidArgs,
+                   check, lib)
 from .puzzle import Puzzle, as_puzzle, uniform_shape
 
 DEFAULT_REWARDS = (1.0, -0.01, -0.05)   # r_win, r_step, r_invalid -- repo-defined (the reference has no reward)
+# element types observe_planes() writes, and their codes in include/tiler_slider.h
+PLANE_DTYPES = {torch.uint8: OBS_U8, torch.bfloat16: OBS_BF16, torch.float16: OBS_F16, torch.float32: OBS_F32}
 
 
 def _round_up(n: int, m: int) -> int:
@@ -576,13 +579,55 @@ class BatchedTilerSliderEnv:
         if out.device != self.device and not (out.device.type == "cpu" and out.is_pinned()):
             raise ValueError(f"observe(out): out must live on {self.device} (or in pinned host memory), not on {out.device}")
 
-    def _observe_args(self, out: torch.Tensor) -> ObserveArgs:
+    def _observe_args(self, out: torch.Tensor | None) -> ObserveArgs:
         # a never_win batch draws its ordered targets from their own buffer (count != tile count)
         nt = 0 if self._obs_targets is None else (self.n_targets or -1)
         tg = self._targets if self._obs_targets is None else self._obs_targets
         return ObserveArgs(size=self.size, n_tiles=self.n_tiles, goal_mode=self.goal_mode, n_targets=nt,
                            first_env=0, n_envs=self.n_envs, capacity=self.capacity, d_walls=_ptr(self._walls),
                            d_targets_packed=_ptr(tg), d_pos=_ptr(self._pos), d_obs=_ptr(out))
+
+    @property
+    def plane_count(self) -> int:
+        """C of observe_planes(): 1 + T + NT with multi colour (the walls, one plane per tile and one
+        per target), 3 with single colour (walls, tile cells, target cells)."""
+        c = self._lib.ts_observe_planes_channels(C.byref(self._observe_planes_args(None, torch.float32)))
+        if c < 0:
+            check(c, "ts_observe_planes_channels")
+        return c
+
+    def observe_planes(self, out: torch.Tensor | None = None, *, dtype: torch.dtype = torch.float32) -> torch.Tensor:
+        """Network input [N, C, S, S] (C = plane_count), channel first, every element 0 or 1 in
+        `dtype` (uint8, bfloat16, float16 or float32), written by one kernel (ts_observe_planes).
+        Plane 0: blocked cells; multi colour: plane 1+i tile i, plane 1+T+j target j; single
+        colour: plane 1 the tile cells, plane 2 the target cells.  No host synchronisation, and
+        with `out` no allocation, so it can be captured in a CUDA graph beside step().  `out`: a
+        contiguous `dtype` tensor of that shape on the batch's device or in pinned host memory,
+        16-byte aligned; anything else raises ValueError (misalignment: TilerSliderError) before a
+        launch."""
+        self._require_loaded()
+        if dtype not in PLANE_DTYPES:
+            raise ValueError(f"observe_planes: dtype {dtype} is not one of uint8, bfloat16, float16, float32")
+        shape = (self.n_envs, self.plane_count, self.size, self.size)
+        if out is None:
+            out = torch.empty(shape, dtype=dtype, device=self.device)
+        elif not isinstance(out, torch.Tensor) or tuple(out.shape) != shape or out.dtype != dtype:
+            raise ValueError(f"observe_planes(out): out must be a {dtype} tensor of shape {shape}")
+        elif not out.is_contiguous():
+            raise ValueError("observe_planes(out): out must be contiguous")
+        elif out.device != self.device and not (out.device.type == "cpu" and out.is_pinned()):
+            raise ValueError(f"observe_planes(out): out must live on {self.device} (or in pinned host memory), not on {out.device}")
+        a = self._observe_planes_args(out, dtype)
+        with torch.cuda.device(self.device):
+            check(self._lib.ts_observe_planes(C.byref(a), self._stream()), "ts_observe_planes")
+        return out
+
+    def _observe_planes_args(self, out: torch.Tensor | None, dtype: torch.dtype) -> ObservePlanesArgs:
+        o = self._observe_args(None)      # the same targets and n_targets convention as observe()
+        return ObservePlanesArgs(size=o.size, n_tiles=o.n_tiles, goal_mode=o.goal_mode, n_targets=o.n_targets,
+                                 first_env=o.first_env, n_envs=o.n_envs, capacity=o.capacity, d_walls=o.d_walls,
+                                 d_targets_packed=o.d_targets_packed, d_pos=o.d_pos, dtype=PLANE_DTYPES[dtype],
+                                 d_out=_ptr(out))
 
     def valid_moves(self) -> torch.Tensor:
         """uint8[N]: bit d set when move d changes the state (get_valid_moves,

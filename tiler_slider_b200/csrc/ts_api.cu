@@ -1,5 +1,6 @@
 // ts_api.cu -- C-ABI entry points (include/tiler_slider.h), argument validation, and the
-// load-time kernels: K1 ts_encode, K0 ts_synth (K3 ts_observe lives in ts_observe.cu).
+// load-time kernels: K1 ts_encode, K0 ts_synth (K3 ts_observe lives in ts_observe.cu,
+// ts_observe_planes in ts_observe_planes.cu).
 //
 // Reference map (paths relative to the reference checkout):
 //   ts_encode   explainrl/environment/state.py:61-73        GameState.__init__ (is_blocked + lists)
@@ -18,6 +19,8 @@ namespace ts {
 TS_DECL(1) TS_DECL(2) TS_DECL(3) TS_DECL(4) TS_DECL(5) TS_DECL(6) TS_DECL(7) TS_DECL(8)
 #undef TS_DECL
 cudaError_t observe_dispatch(const ts_observe_args&, cudaStream_t);
+cudaError_t observe_planes_dispatch(const ts_observe_planes_args&, cudaStream_t);
+int observe_planes_channels(const ts_observe_planes_args&);
 cudaError_t wide_step_dispatch(const ts_step_args&, cudaStream_t);
 cudaError_t wide_valid_dispatch(const ts_valid_args&, cudaStream_t);
 cudaError_t wide_goal_dispatch(const ts_goal_args&, cudaStream_t);
@@ -234,6 +237,32 @@ int ts_observe(const ts_observe_args* a, void* stream) {
     if (a->n_envs == 0) return 0;
     if (!aligned16(a->d_obs)) return fail(TS_E_MISALIGNED, "d_obs %p is not 16-byte aligned", (const void*)a->d_obs);
     return cuda_result(observe_dispatch(*a, (cudaStream_t)stream), "ts_observe launch");
+}
+
+// the checks of ts_observe_planes that do not involve the range or the buffers
+static int check_planes_kind(const ts_observe_planes_args* a) {
+    if (a->n_tiles < 0 || a->n_tiles > MAX_TILES_ANY) return fail(TS_E_BAD_TILES, "n_tiles %d outside 0..%d", a->n_tiles, MAX_TILES_ANY);
+    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
+    if (a->goal_mode == TS_GOAL_ORDERED && (a->n_targets < -1 || a->n_targets > MAX_TILES_ANY))
+        return fail(TS_E_BAD_TILES, "n_targets %d outside -1..%d", a->n_targets, MAX_TILES_ANY);
+    if (a->dtype < TS_OBS_U8 || a->dtype > TS_OBS_F32) return fail(TS_E_BAD_ARGUMENT, "dtype %d (TS_OBS_U8 .. TS_OBS_F32)", a->dtype);
+    return 0;
+}
+
+int ts_observe_planes_channels(const ts_observe_planes_args* a) {
+    if (!a) return fail(TS_E_NULL_POINTER, "null args");
+    if (int rc = check_planes_kind(a)) return rc;
+    return observe_planes_channels(*a);
+}
+
+int ts_observe_planes(const ts_observe_planes_args* a, void* stream) {
+    if (!a) return fail(TS_E_NULL_POINTER, "null args");
+    if (int rc = check_shape(a->size, a->n_tiles, a->first_env, a->n_envs, a->capacity)) return rc;
+    if (int rc = check_planes_kind(a)) return rc;
+    if (!a->d_walls || !a->d_targets_packed || !a->d_pos || !a->d_out) return fail(TS_E_NULL_POINTER, "null device pointer");
+    if (a->n_envs == 0) return 0;
+    if (!aligned16(a->d_out)) return fail(TS_E_MISALIGNED, "d_out %p is not 16-byte aligned", a->d_out);
+    return cuda_result(observe_planes_dispatch(*a, (cudaStream_t)stream), "ts_observe_planes launch");
 }
 
 int ts_valid_moves(const ts_valid_args* a, void* stream) {
