@@ -40,6 +40,9 @@
  *        written to d_obs[i];
  *      ts_observe_planes: d_out[0 .. n_envs*C*size*size) elements, RELATIVE to the range as
  *        ts_observe's;
+ *      ts_observe_planes_items: d_out[0 .. n_items*C*size*size) elements, in item order;
+ *      ts_expand: d_succ[0 .. 4*n_items*pos_bytes) bytes, d_moved[0 .. n_items) and
+ *        d_won[0 .. n_items) (when given), in item order -- no env buffer;
  *      ts_valid_moves, ts_goal_check: d_mask / d_won are ABSOLUTE (env e at [e]); the range, and on
  *        boards up to 8x8 with 1..8 tiles also the (correct) result of the up-to-3 envs after the
  *        range that share its last 4-env group;
@@ -237,6 +240,46 @@ typedef struct ts_observe_planes_args {
 } ts_observe_planes_args;
 int ts_observe_planes_channels(const ts_observe_planes_args *a);
 int ts_observe_planes(const ts_observe_planes_args *a, void *stream);
+/* ts_observe_planes_items: the same planes for n_items ITEMS instead of an env range (first_env and
+ * n_envs of *a are not read).  Item i shows env e = d_env_ids[i] (NULL: e = i) -- its walls and
+ * targets -- with the tiles of the position word d_item_pos[i] (NULL: d_pos[e]); d_out holds
+ * n_items*C*size*size elements, item i at [i].  An e outside [0, capacity) gives an all-zero image and
+ * nothing of it is read.  Argument errors as ts_observe_planes's, plus n_items < 0 or, without
+ * d_env_ids, n_items > capacity (TS_E_BAD_RANGE); d_pos may be NULL when d_item_pos is given;
+ * d_out and d_item_pos must be 16-byte aligned (checked only when n_items > 0). */
+int ts_observe_planes_items(const ts_observe_planes_args *a, const int32_t *d_env_ids, const uint8_t *d_item_pos,
+                            int64_t n_items, void *stream);
+
+/* ---------------------------------------------------------------------------------------
+ * ts_expand: the four successors of many states (csrc/ts_expand.cu, ts_wide.cu, ts_generic.cu;
+ * GameState.move, state.py:120-170, and is_won, state.py:172-186, once per move), for search:
+ * beam search, A* with a learned heuristic, MCTS expansion, value-iteration targets.  An ITEM is
+ * a pair (env id, position word): the env supplies the puzzle (walls and targets), the word the
+ * tiles.  For item i < n_items, env e = d_env_ids[i] (NULL: e = i), positions p = d_item_pos[i]
+ * (NULL: d_pos[e]; words of ts_pos_bytes(n_tiles) bytes, unused bytes zero):
+ *   d_succ[i][a]  [n_items][4][pos_bytes], item-major: the positions after move a from p (0 UP,
+ *                 1 DOWN, 2 LEFT, 3 RIGHT) -- bit for bit what ts_step leaves in pos for that action
+ *                 before any reset; tile order kept (no sorting in set mode), so d_succ read as
+ *                 [4*n_items][pos_bytes] is the item list of the next level, with ids repeated 4 times
+ *   d_moved[i]    optional: bit a set iff move a changes the positions (the step's !INVALID;
+ *                 ts_valid_moves of p)
+ *   d_won[i]      optional: bit a set iff the positions after move a meet the goal (the step's WON:
+ *                 0 with never_win; n_tiles = 0: the rule of ts_step)
+ * An e outside [0, capacity) gives zero successors and masks, and nothing of it is read.  No env
+ * buffer is written.  Argument errors (all before the n_items = 0 return): size, n_tiles,
+ * capacity, goal_mode, never_win outside 0/1 (TS_E_BAD_ARGUMENT), a NULL d_walls /
+ * d_targets_packed / d_succ, or d_pos when d_item_pos is NULL (TS_E_NULL_POINTER), n_items < 0 or,
+ * without d_env_ids, n_items > capacity (TS_E_BAD_RANGE); then, with n_items > 0, d_succ and
+ * d_item_pos must be 16-byte aligned (TS_E_MISALIGNED).
+ * ------------------------------------------------------------------------------------- */
+typedef struct ts_expand_args {
+    int32_t size, n_tiles, goal_mode, never_win;
+    int64_t n_items, capacity;
+    const int32_t *d_env_ids;
+    const uint8_t *d_walls, *d_targets_packed, *d_pos, *d_item_pos;
+    uint8_t *d_succ, *d_moved, *d_won;
+} ts_expand_args;
+int ts_expand(const ts_expand_args *a, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * ts_valid_moves: bit d of d_mask[env] set when move d changes any tile position

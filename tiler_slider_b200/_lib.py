@@ -67,6 +67,13 @@ class ObservePlanesArgs(C.Structure):
                 ("dtype", _i32), ("reserved0", _i32), ("d_out", _vp)]
 
 
+class ExpandArgs(C.Structure):
+    _fields_ = [("size", _i32), ("n_tiles", _i32), ("goal_mode", _i32), ("never_win", _i32),
+                ("n_items", _i64), ("capacity", _i64),
+                ("d_env_ids", _vp), ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp), ("d_item_pos", _vp),
+                ("d_succ", _vp), ("d_moved", _vp), ("d_won", _vp)]
+
+
 class ValidArgs(C.Structure):
     _fields_ = [("size", _i32), ("n_tiles", _i32),
                 ("first_env", _i64), ("n_envs", _i64), ("capacity", _i64),
@@ -147,6 +154,8 @@ SYMBOLS = {
     "ts_observe": (C.c_int, [C.POINTER(ObserveArgs), _vp]),
     "ts_observe_planes_channels": (C.c_int, [C.POINTER(ObservePlanesArgs)]),
     "ts_observe_planes": (C.c_int, [C.POINTER(ObservePlanesArgs), _vp]),
+    "ts_observe_planes_items": (C.c_int, [C.POINTER(ObservePlanesArgs), _vp, _vp, _i64, _vp]),
+    "ts_expand": (C.c_int, [C.POINTER(ExpandArgs), _vp]),
     "ts_valid_moves": (C.c_int, [C.POINTER(ValidArgs), _vp]),
     "ts_goal_check": (C.c_int, [C.POINTER(GoalArgs), _vp]),
     "ts_bfs_seed": (C.c_int, [C.POINTER(BfsArgs), _vp]),

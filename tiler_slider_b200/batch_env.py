@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from ._lib import (CAP_ALIGN, F_WON, GOAL_ORDERED, GOAL_SET, MAX_SIZE, MAX_TILES, OBS_BF16, OBS_F16, OBS_F32, OBS_U8,
-                   EncodeArgs, GoalArgs, ObserveArgs, ObservePlanesArgs, PoolResetArgs, StepArgs, SynthArgs, ValidArgs,
+                   EncodeArgs, ExpandArgs, GoalArgs, ObserveArgs, ObservePlanesArgs, PoolResetArgs, StepArgs, SynthArgs, ValidArgs,
                    check, lib)
 from .puzzle import Puzzle, as_puzzle, uniform_shape
 
@@ -596,7 +596,8 @@ class BatchedTilerSliderEnv:
             check(c, "ts_observe_planes_channels")
         return c
 
-    def observe_planes(self, out: torch.Tensor | None = None, *, dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    def observe_planes(self, out: torch.Tensor | None = None, *, dtype: torch.dtype = torch.float32, ids=None,
+                       pos: torch.Tensor | None = None) -> torch.Tensor:
         """Network input [N, C, S, S] (C = plane_count), channel first, every element 0 or 1 in
         `dtype` (uint8, bfloat16, float16 or float32), written by one kernel (ts_observe_planes).
         Plane 0: blocked cells; multi colour: plane 1+i tile i, plane 1+T+j target j; single
@@ -604,11 +605,20 @@ class BatchedTilerSliderEnv:
         with `out` no allocation, so it can be captured in a CUDA graph beside step().  `out`: a
         contiguous `dtype` tensor of that shape on the batch's device or in pinned host memory,
         16-byte aligned; anything else raises ValueError (misalignment: TilerSliderError) before a
-        launch."""
+        launch.
+
+        With `ids` and / or `pos` the images are of ITEMS, as expand() takes them
+        (ts_observe_planes_items): image i shows env ids[i]'s walls and targets with the tiles of
+        pos[i], so [n, C, S, S] for n items -- e.g. the successors expand() returned, with
+        ids.repeat_interleave(4) and pos = succ.reshape(-1, pos_bytes)."""
         self._require_loaded()
         if dtype not in PLANE_DTYPES:
             raise ValueError(f"observe_planes: dtype {dtype} is not one of uint8, bfloat16, float16, float32")
-        shape = (self.n_envs, self.plane_count, self.size, self.size)
+        items = ids is not None or pos is not None
+        n = self.n_envs
+        if items:
+            n, ids, pos = self._items("observe_planes", ids, pos)
+        shape = (n, self.plane_count, self.size, self.size)
         if out is None:
             out = torch.empty(shape, dtype=dtype, device=self.device)
         elif not isinstance(out, torch.Tensor) or tuple(out.shape) != shape or out.dtype != dtype:
@@ -619,7 +629,98 @@ class BatchedTilerSliderEnv:
             raise ValueError(f"observe_planes(out): out must live on {self.device} (or in pinned host memory), not on {out.device}")
         a = self._observe_planes_args(out, dtype)
         with torch.cuda.device(self.device):
-            check(self._lib.ts_observe_planes(C.byref(a), self._stream()), "ts_observe_planes")
+            if not items:
+                check(self._lib.ts_observe_planes(C.byref(a), self._stream()), "ts_observe_planes")
+            elif n:
+                check(self._lib.ts_observe_planes_items(C.byref(a), _ptr(ids), _ptr(pos), n, self._stream()),
+                      "ts_observe_planes_items")
+        return out
+
+    def _items(self, what: str, ids, pos: torch.Tensor | None) -> tuple[int, torch.Tensor | None, torch.Tensor | None]:
+        """(n, int32 ids on the device or None, pos or None) of an item call; raises ValueError /
+        IndexError before any launch.  Host ids are range-checked against [0, n_envs); device ids
+        are not (that would cost a synchronisation): the kernels give an id outside [0, capacity)
+        an all-zero result and read nothing of it."""
+        if self.host_io:
+            raise ValueError(f"{what}: not available for host_io batches (their positions live in host memory)")
+        n = self.n_envs
+        if ids is not None:
+            if isinstance(ids, torch.Tensor) and ids.is_cuda:
+                if ids.device != self.device:
+                    raise ValueError(f"{what}: ids are on {ids.device}, the batch on {self.device}")
+                if ids.is_floating_point() or ids.is_complex() or ids.dtype == torch.bool:
+                    raise ValueError(f"{what}: ids must be integers, not {ids.dtype}")
+                if ids.dtype != torch.int32 or not ids.is_contiguous():
+                    ids = ids.to(torch.int32).contiguous()
+                ids = ids.reshape(-1)
+            else:
+                t = torch.as_tensor(ids).reshape(-1)
+                if t.numel() and (t.is_floating_point() or t.is_complex() or t.dtype == torch.bool):
+                    raise ValueError(f"{what}: ids must be integers, not {t.dtype}")
+                if t.numel():
+                    lo, hi = int(t.min()), int(t.max())
+                    if lo < 0 or hi >= self.n_envs:
+                        raise IndexError(f"{what}: env ids must lie in [0, {self.n_envs}), got [{lo}, {hi}]")
+                ids = t.to(torch.int32)          # copied to the device once pos has passed its checks too
+            n = ids.numel()
+        if pos is not None:
+            want = (n, self.pos_bytes)
+            if not isinstance(pos, torch.Tensor) or pos.dtype != torch.uint8 or pos.dim() != 2 or pos.shape[1] != self.pos_bytes:
+                raise ValueError(f"{what}: pos must be a uint8 tensor [n, {self.pos_bytes}]")
+            if tuple(pos.shape) != want:
+                raise ValueError(f"{what}: pos has {pos.shape[0]} rows, expected {n} "
+                                 f"({'one per id' if ids is not None else 'one per env without ids'})")
+            if pos.device != self.device:
+                raise ValueError(f"{what}: pos is on {pos.device}, the batch on {self.device}")
+            if not pos.is_contiguous():
+                raise ValueError(f"{what}: pos must be contiguous")
+        if ids is not None and not ids.is_cuda:
+            ids = ids.to(self.device)
+        return n, ids, pos
+
+    def expand(self, ids=None, pos: torch.Tensor | None = None, *,
+               out: tuple[torch.Tensor, torch.Tensor, torch.Tensor] | None = None) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """The four successors of many states, for search (beam search, A* with a learned heuristic,
+        MCTS expansion, value-iteration targets), in one kernel (ts_expand).  An item is (env id,
+        positions): the env gives the puzzle (walls and targets), the position word the tiles.
+        ids: any integer sequence or tensor of env ids (default: every env); pos: uint8 [n, pos_bytes]
+        on the device (default: each listed env's current positions; without ids it needs n_envs
+        rows).  Returns (succ uint8[n, 4, pos_bytes], moved uint8[n], won uint8[n]):
+          succ[i, a]  the positions after move a (0 UP, 1 DOWN, 2 LEFT, 3 RIGHT) -- what step()
+                      would leave, before any reset, with the tile order kept (no sorting with a
+                      single colour); succ.reshape(-1, pos_bytes) with ids.repeat_interleave(4) is
+                      the next level's item list;
+          moved[i]    bit a set iff move a changes the positions (valid_moves() of the item);
+          won[i]      bit a set iff the positions after move a meet the goal (the step's is_won).
+        `out`: preallocated (succ, moved, won) of those shapes, contiguous uint8 on the device; with it
+        and device ids (int32, contiguous, passed as they are) or none, the call neither allocates nor
+        synchronises, so it can be captured in a CUDA graph beside step().  Host ids outside
+        [0, n_envs) raise IndexError; device ids are not checked: one outside [0, capacity) gets
+        zero successors and masks.  Runs on the current stream and changes no env state.  Not
+        available for host_io batches."""
+        self._require_loaded()
+        n, ids, pos = self._items("expand", ids, pos)
+        shapes = ((n, 4, self.pos_bytes), (n,), (n,))
+        if out is None:
+            out = tuple(torch.empty(s, dtype=torch.uint8, device=self.device) for s in shapes)
+        else:
+            if not isinstance(out, (tuple, list)) or len(out) != 3:
+                raise ValueError("expand(out): out must be a tuple (succ, moved, won)")
+            for t, s in zip(out, shapes):
+                if not isinstance(t, torch.Tensor) or t.dtype != torch.uint8 or tuple(t.shape) != s:
+                    raise ValueError(f"expand(out): expected uint8 tensors of shapes {shapes}")
+                if t.device != self.device:
+                    raise ValueError(f"expand(out): out must live on {self.device}, not on {t.device}")
+                if not t.is_contiguous():
+                    raise ValueError("expand(out): out must be contiguous")
+            out = tuple(out)
+        if n:
+            a = ExpandArgs(size=self.size, n_tiles=self.n_tiles, goal_mode=self.goal_mode, never_win=int(self.never_win),
+                           n_items=n, capacity=self.capacity, d_env_ids=_ptr(ids), d_walls=_ptr(self._walls),
+                           d_targets_packed=_ptr(self._targets), d_pos=_ptr(self._pos), d_item_pos=_ptr(pos),
+                           d_succ=_ptr(out[0]), d_moved=_ptr(out[1]), d_won=_ptr(out[2]))
+            with torch.cuda.device(self.device):
+                check(self._lib.ts_expand(C.byref(a), self._stream()), "ts_expand")
         return out
 
     def _observe_planes_args(self, out: torch.Tensor | None, dtype: torch.dtype) -> ObservePlanesArgs:

@@ -1,6 +1,6 @@
 // ts_api.cu -- C-ABI entry points (include/tiler_slider.h), argument validation, and the
 // load-time kernels: K1 ts_encode, K0 ts_synth (K3 ts_observe lives in ts_observe.cu,
-// ts_observe_planes in ts_observe_planes.cu).
+// ts_observe_planes in ts_observe_planes.cu, ts_expand in ts_expand.cu / ts_wide.cu / ts_generic.cu).
 //
 // Reference map (paths relative to the reference checkout):
 //   ts_encode   explainrl/environment/state.py:61-73        GameState.__init__ (is_blocked + lists)
@@ -20,7 +20,11 @@ TS_DECL(1) TS_DECL(2) TS_DECL(3) TS_DECL(4) TS_DECL(5) TS_DECL(6) TS_DECL(7) TS_
 #undef TS_DECL
 cudaError_t observe_dispatch(const ts_observe_args&, cudaStream_t);
 cudaError_t observe_planes_dispatch(const ts_observe_planes_args&, cudaStream_t);
+cudaError_t observe_planes_items_dispatch(const ts_observe_planes_args&, const int32_t*, const uint8_t*, int64_t, cudaStream_t);
 int observe_planes_channels(const ts_observe_planes_args&);
+cudaError_t expand_dispatch(const ts_expand_args&, cudaStream_t);
+cudaError_t wide_expand_dispatch(const ts_expand_args&, cudaStream_t);
+cudaError_t generic_expand_dispatch(const ts_expand_args&, cudaStream_t);
 cudaError_t wide_step_dispatch(const ts_step_args&, cudaStream_t);
 cudaError_t wide_valid_dispatch(const ts_valid_args&, cudaStream_t);
 cudaError_t wide_goal_dispatch(const ts_goal_args&, cudaStream_t);
@@ -263,6 +267,47 @@ int ts_observe_planes(const ts_observe_planes_args* a, void* stream) {
     if (a->n_envs == 0) return 0;
     if (!aligned16(a->d_out)) return fail(TS_E_MISALIGNED, "d_out %p is not 16-byte aligned", a->d_out);
     return cuda_result(observe_planes_dispatch(*a, (cudaStream_t)stream), "ts_observe_planes launch");
+}
+
+// the item list of ts_observe_planes_items / ts_expand: n_items items, ids from d_env_ids or 0 .. n_items-1
+static int check_items(int64_t n_items, const int32_t* d_env_ids, int64_t cap) {
+    if (n_items < 0 || (!d_env_ids && n_items > cap))
+        return fail(TS_E_BAD_RANGE, "n_items %lld invalid for capacity %lld (without env ids item i is env i)", (long long)n_items,
+                    (long long)cap);
+    return 0;
+}
+
+int ts_observe_planes_items(const ts_observe_planes_args* a, const int32_t* d_env_ids, const uint8_t* d_item_pos, int64_t n_items,
+                            void* stream) {
+    if (!a) return fail(TS_E_NULL_POINTER, "null args");
+    if (int rc = check_shape(a->size, a->n_tiles, 0, 0, a->capacity)) return rc;
+    if (int rc = check_planes_kind(a)) return rc;
+    if (int rc = check_items(n_items, d_env_ids, a->capacity)) return rc;
+    if (!a->d_walls || !a->d_targets_packed || (!a->d_pos && !d_item_pos) || !a->d_out) return fail(TS_E_NULL_POINTER, "null device pointer");
+    if (n_items == 0) return 0;
+    if (!aligned16(a->d_out)) return fail(TS_E_MISALIGNED, "d_out %p is not 16-byte aligned", a->d_out);
+    if (d_item_pos && !aligned16(d_item_pos)) return fail(TS_E_MISALIGNED, "d_item_pos %p is not 16-byte aligned", (const void*)d_item_pos);
+    return cuda_result(observe_planes_items_dispatch(*a, d_env_ids, d_item_pos, n_items, (cudaStream_t)stream), "ts_observe_planes_items launch");
+}
+
+int ts_expand(const ts_expand_args* a, void* stream) {
+    if (!a) return fail(TS_E_NULL_POINTER, "null args");
+    if (int rc = check_shape(a->size, a->n_tiles, 0, 0, a->capacity)) return rc;
+    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
+    if (a->never_win != 0 && a->never_win != 1) return fail(TS_E_BAD_ARGUMENT, "never_win %d (0 or 1)", a->never_win);
+    if (int rc = check_items(a->n_items, a->d_env_ids, a->capacity)) return rc;
+    if (!a->d_walls || !a->d_targets_packed || (!a->d_pos && !a->d_item_pos) || !a->d_succ)
+        return fail(TS_E_NULL_POINTER, "null device pointer");
+    if (a->n_items == 0) return 0;
+    if (!aligned16(a->d_succ)) return fail(TS_E_MISALIGNED, "d_succ %p is not 16-byte aligned", (const void*)a->d_succ);
+    if (a->d_item_pos && !aligned16(a->d_item_pos))
+        return fail(TS_E_MISALIGNED, "d_item_pos %p is not 16-byte aligned", (const void*)a->d_item_pos);
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e;
+    if (a->n_tiles == 0 || a->n_tiles > MAX_TILES) e = generic_expand_dispatch(*a, st);   // the kernel classes of ts_step
+    else if (wide_board(a->size)) e = wide_expand_dispatch(*a, st);
+    else e = expand_dispatch(*a, st);
+    return cuda_result(e, "ts_expand launch");
 }
 
 int ts_valid_moves(const ts_valid_args* a, void* stream) {

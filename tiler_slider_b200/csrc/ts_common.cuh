@@ -97,17 +97,16 @@ template <class F> cudaError_t dispatch_size(int size, F&& f) {
         default: return cudaErrorInvalidValue;
     }
 }
-// host: f(IC<S>{}, IC<T>{}) for those sizes and the tile counts of one 32-bit state, 1..4
-template <class F> cudaError_t dispatch_small(int size, int n_tiles, F&& f) {
-    return dispatch_size(size, [&](auto S) {
-        switch (n_tiles) {
-            case 1: return f(S, IC<1>{});
-            case 2: return f(S, IC<2>{});
-            case 3: return f(S, IC<3>{});
-            case 4: return f(S, IC<4>{});
-            default: return cudaErrorInvalidValue;
-        }
-    });
+// host: f(IC<T>{}) for the tile counts T0..MAXT
+template <int T0, int MAXT, class F> cudaError_t dispatch_tiles(int n_tiles, F&& f) {
+    if constexpr (T0 > MAXT) return cudaErrorInvalidValue;
+    else return n_tiles == T0 ? f(IC<T0>{}) : dispatch_tiles<T0 + 1, MAXT>(n_tiles, f);
+}
+// host: f(IC<S>{}, IC<T>{}) for those sizes and the tile counts 1..MAXT (default: those of one
+// 32-bit state, 1..4; MAX_TILES: every tile count of the register kernels)
+template <int MAXT = 4, class F> cudaError_t dispatch_small(int size, int n_tiles, F&& f) {
+    static_assert(MAXT >= 1 && MAXT <= MAX_TILES, "register kernels hold 1..8 tiles");
+    return dispatch_size(size, [&](auto S) { return dispatch_tiles<1, MAXT>(n_tiles, [&](auto T) { return f(S, T); }); });
 }
 
 // ---- streaming global access ---------------------------------------------------------------
@@ -258,6 +257,33 @@ template <int NB> __device__ __forceinline__ uint64_t load_board_elem(const uint
         b |= v << (8 * off);
     });
     return b;
+}
+
+// position word `idx` of a packed position array (T <= 8: 1, 2, 4 or 8 bytes) into PR words, and back
+template <int PW> __device__ __forceinline__ void ld_pos(const uint8_t* p, size_t idx, uint32_t (&q)[(PW + 3) / 4]) {
+    if constexpr (PW == 1) q[0] = p[idx];
+    else if constexpr (PW == 2) q[0] = reinterpret_cast<const uint16_t*>(p)[idx];
+    else if constexpr (PW == 4) q[0] = reinterpret_cast<const uint32_t*>(p)[idx];
+    else { const uint2 v = reinterpret_cast<const uint2*>(p)[idx]; q[0] = v.x; q[1] = v.y; }
+}
+template <int PW> __device__ __forceinline__ void st_pos(uint8_t* p, size_t idx, const uint32_t (&q)[(PW + 3) / 4]) {
+    if constexpr (PW == 1) p[idx] = (uint8_t)q[0];
+    else if constexpr (PW == 2) reinterpret_cast<uint16_t*>(p)[idx] = (uint16_t)q[0];
+    else if constexpr (PW == 4) reinterpret_cast<uint32_t*>(p)[idx] = q[0];
+    else reinterpret_cast<uint2*>(p)[idx] = make_uint2(q[0], q[1]);
+}
+
+// the four successor words s[move][word] of one item (ts_expand) to its 4*PW-byte output row, as
+// vector stores: one u32 (T = 1), one u64 (T = 2), one 16-byte store (T = 3, 4), two (T = 5..8).
+// The row is 16-byte aligned for PW >= 4 (the caller checks the buffer), 4*PW-aligned below.
+template <int PW> __device__ __forceinline__ void st_succ4(uint8_t* row, const uint32_t (&s)[4][(PW + 3) / 4]) {
+    if constexpr (PW == 1) __stcs(reinterpret_cast<unsigned int*>(row), s[0][0] | s[1][0] << 8 | s[2][0] << 16 | s[3][0] << 24);
+    else if constexpr (PW == 2) __stcs(reinterpret_cast<uint2*>(row), make_uint2(s[0][0] | s[1][0] << 16, s[2][0] | s[3][0] << 16));
+    else if constexpr (PW == 4) __stcs(reinterpret_cast<uint4*>(row), make_uint4(s[0][0], s[1][0], s[2][0], s[3][0]));
+    else {
+        __stcs(reinterpret_cast<uint4*>(row), make_uint4(s[0][0], s[0][1], s[1][0], s[1][1]));
+        __stcs(reinterpret_cast<uint4*>(row) + 1, make_uint4(s[2][0], s[2][1], s[3][0], s[3][1]));
+    }
 }
 
 // ---- SWAR helpers on 4 packed position bytes -------------------------------------------------

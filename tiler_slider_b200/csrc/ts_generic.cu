@@ -1,4 +1,4 @@
-// ts_generic.cu -- step / valid-move / goal kernels for everything the specialised kernels do not cover:
+// ts_generic.cu -- step / valid-move / goal / expand kernels for everything the specialised kernels do not cover:
 //   (a) the ragged end of a range on bitboard-class boards (S <= 8): step_kernel works on whole
 //       4-env groups, so ts_step hands the last n_envs % 4 envs of a call to generic_step_kernel --
 //       nothing outside [first_env, first_env + n_envs) is ever read-modified-written;
@@ -78,20 +78,25 @@ __device__ __forceinline__ bool goal_met(const uint8_t* p, int S, int T, int goa
     return true;
 }
 
-__global__ void __launch_bounds__(128) generic_step_kernel(const ts_step_args a) {
-    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
-    if (i >= a.n_envs) return;
-    const size_t env = (size_t)(a.first_env + i), cap = (size_t)a.capacity;
-    const int S = a.size, T = a.n_tiles, pw = pos_bytes(T), ps = pos_stride(S);
-    const uint32_t action = a.d_actions[env] & 3u;
-    const int dr = action == 0 ? -1 : action == 1 ? 1 : 0, dc = action == 2 ? -1 : action == 3 ? 1 : 0;   // state.py:31-34
+// the env's walls in the form generic_slide reads: the 64-bit board on boards up to 8x8, rows on wide ones
+struct GenericWalls {
+    uint64_t b;
+    uint32_t rows[MAX_SIZE];
+};
+__device__ __forceinline__ void load_generic_walls(GenericWalls& w, const uint8_t* d_walls, int S, int T, size_t cap, size_t env) {
+    if (T > 0 && !wide_board(S)) w.b = load_board64(d_walls, S, cap, env);
+    else if (T > 0) wall_rows(w.rows, d_walls, S, cap, env);
+}
 
-    uint8_t p0[MAX_TILES_ANY], p[MAX_TILES_ANY];
-    for (int t = 0; t < T; ++t) p[t] = p0[t] = a.d_pos[env * pw + t];
+// One slide of the T tiles p0 -> p under `action` (state.py:137-170), cell by cell; true iff a tile moved.
+// T = 0: nothing moves.
+__device__ __forceinline__ bool generic_slide(const uint8_t* p0, uint8_t* p, int S, int T, uint32_t action, const GenericWalls& wl) {
+    const int ps = pos_stride(S);
+    const int dr = action == 0 ? -1 : action == 1 ? 1 : 0, dc = action == 2 ? -1 : action == 3 ? 1 : 0;   // state.py:31-34
     bool moved = false;
     if (T > 0 && !wide_board(S)) {             // the whole board in one word: register bit tests (ragged ends, the single-env adapter)
         const int bs = board_stride(S);
-        const uint64_t walls = load_board64(a.d_walls, S, cap, env);
+        const uint64_t walls = wl.b;
         uint64_t occ = 0;
         for (int t = 0; t < T; ++t) occ |= 1ull << ((p0[t] / ps) * bs + p0[t] % ps);
         for (int t = 0; t < T; ++t) {
@@ -106,8 +111,8 @@ __global__ void __launch_bounds__(128) generic_step_kernel(const ts_step_args a)
             moved |= n != 0;
         }
     } else if (T > 0) {                        // wide boards with more than 8 tiles: row words in local arrays
-        uint32_t walls[MAX_SIZE], occ[MAX_SIZE];
-        wall_rows(walls, a.d_walls, S, cap, env);
+        const uint32_t* walls = wl.rows;
+        uint32_t occ[MAX_SIZE];
         for (int r = 0; r < S; ++r) occ[r] = 0;
         for (int t = 0; t < T; ++t) occ[p0[t] / ps] |= 1u << (p0[t] % ps);
         for (int t = 0; t < T; ++t) {
@@ -121,6 +126,21 @@ __global__ void __launch_bounds__(128) generic_step_kernel(const ts_step_args a)
             moved |= n != 0;
         }
     }
+    return moved;
+}
+
+__global__ void __launch_bounds__(128) generic_step_kernel(const ts_step_args a) {
+    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (i >= a.n_envs) return;
+    const size_t env = (size_t)(a.first_env + i), cap = (size_t)a.capacity;
+    const int S = a.size, T = a.n_tiles, pw = pos_bytes(T);
+    const uint32_t action = a.d_actions[env] & 3u;
+
+    uint8_t p0[MAX_TILES_ANY], p[MAX_TILES_ANY];
+    for (int t = 0; t < T; ++t) p[t] = p0[t] = a.d_pos[env * pw + t];
+    GenericWalls wl;
+    load_generic_walls(wl, a.d_walls, S, T, cap, env);
+    const bool moved = generic_slide(p0, p, S, T, action, wl);
     const bool won = a.never_win == 0 && goal_met(p, S, T, a.goal_mode, a.d_targets_packed, cap, env);
     // bookkeeping (environment.py:126-141)
     const bool narrow = a.count_bytes == 1;
@@ -189,6 +209,40 @@ __global__ void __launch_bounds__(128) generic_valid_kernel(const ts_valid_args 
         if (c + 1 < S && ((open[r] >> (c + 1)) & 1u)) mask |= 8u;
     }
     a.d_mask[env] = (uint8_t)mask;
+}
+
+// ts_expand for 0 and 9..32 tiles (any S): the step's slide and goal test once per move.  An id
+// outside [0, capacity) reads nothing and writes zero successors and masks.
+__global__ void __launch_bounds__(128) generic_expand_kernel(const ts_expand_args a) {
+    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (i >= a.n_items) return;
+    const int S = a.size, T = a.n_tiles, pw = pos_bytes(T);
+    const int64_t e = a.d_env_ids ? (int64_t)a.d_env_ids[i] : i;
+    uint8_t* out = a.d_succ + (size_t)i * (4 * pw);
+    uint32_t moved = 0, won = 0;
+    if (e >= 0 && e < a.capacity) {
+        const size_t env = (size_t)e, cap = (size_t)a.capacity;
+        const uint8_t* src = a.d_item_pos ? a.d_item_pos + (size_t)i * pw : a.d_pos + env * pw;
+        uint8_t p0[MAX_TILES_ANY], p[MAX_TILES_ANY];
+        for (int t = 0; t < T; ++t) p0[t] = src[t];
+        GenericWalls wl;
+        load_generic_walls(wl, a.d_walls, S, T, cap, env);
+        for (uint32_t d = 0; d < 4; ++d) {
+            if (generic_slide(p0, p, S, T, d, wl)) moved |= 1u << d;
+            if (a.never_win == 0 && goal_met(p, S, T, a.goal_mode, a.d_targets_packed, cap, env)) won |= 1u << d;
+            for (int t = 0; t < pw; ++t) out[d * pw + t] = t < T ? p[t] : 0;
+        }
+    } else {
+        for (int t = 0; t < 4 * pw; ++t) out[t] = 0;
+    }
+    if (a.d_moved) a.d_moved[i] = (uint8_t)moved;
+    if (a.d_won) a.d_won[i] = (uint8_t)won;
+}
+
+cudaError_t generic_expand_dispatch(const ts_expand_args& a, cudaStream_t st) {
+    if (a.n_items <= 0) return cudaSuccess;
+    generic_expand_kernel<<<(unsigned)((a.n_items + 127) / 128), 128, 0, st>>>(a);
+    return cudaGetLastError();
 }
 
 cudaError_t generic_step_dispatch(const ts_step_args& a, cudaStream_t st) {

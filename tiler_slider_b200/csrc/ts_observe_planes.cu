@@ -32,14 +32,31 @@ struct PlanesParams {
     int64_t env_bytes, total_bytes;     // C*S*S << wshift; n_envs * env_bytes
 };
 
+// ts_observe_planes_items: image e shows env ids[e] (NULL: e) with the tiles of item_pos[e] (NULL:
+// that env's pos); a.first_env = 0 and a.n_envs = the item count
+struct PlanesItemsParams : PlanesParams {
+    const int32_t* ids;
+    const uint8_t* item_pos;
+};
+
 __device__ __forceinline__ void put_one(uint8_t* stage, int off, int wshift, uint32_t one) {
     if (wshift == 0) stage[off] = (uint8_t)one;
     else if (wshift == 1) *reinterpret_cast<uint16_t*>(stage + off) = (uint16_t)one;
     else *reinterpret_cast<uint32_t*>(stage + off) = one;
 }
 
-template <int S>
-__global__ void __launch_bounds__(PLANES_THREADS) observe_planes_kernel(const PlanesParams p) {
+// env shown by image `item` of an item call; false: its id lies outside [0, capacity) and the image stays zero
+__device__ __forceinline__ bool item_env(const PlanesItemsParams& p, int64_t item, size_t& env) {
+    const int64_t e = p.ids ? (int64_t)p.ids[item] : item;
+    env = (size_t)e;
+    return e >= 0 && e < p.a.capacity;
+}
+
+// PP = PlanesParams: images of the env range; PP = PlanesItemsParams: images of items (a compile-time
+// variant, so the range instantiations are the kernels they were)
+template <int S, class PP = PlanesParams>
+__global__ void __launch_bounds__(PLANES_THREADS) observe_planes_kernel(const PP p) {
+    constexpr bool ITEMS = std::is_same<PP, PlanesItemsParams>::value;
     constexpr int CELLS = S * S, NB = board_bytes(S), PS = pos_stride(S);
     __shared__ __align__(16) uint8_t stage[PLANES_STAGE];
     const ts_observe_planes_args& a = p.a;
@@ -63,11 +80,14 @@ __global__ void __launch_bounds__(PLANES_THREADS) observe_planes_kernel(const Pl
     constexpr uint32_t ROW = (1u << S) - 1u;      // drops the sentinels past column S-1
     for (int j = threadIdx.x; j < n_e * S; j += PLANES_THREADS) {
         const int e = j / S, r = j - e * S;
-        const size_t env = (size_t)(a.first_env + e_first + e);
+        size_t env;
+        bool live = true;
+        if constexpr (ITEMS) live = item_env(p, e_first + e, env);
+        else env = (size_t)(a.first_env + e_first + e);
         const int o0 = base + e * env_bytes + ((r * S) << ws);              // plane 0, cell (r, 0)
         const int o2 = o0 + ((2 * CELLS) << ws);                            // plane 2, cell (r, 0)
-        const bool in0 = o0 + (S << ws) > 0 && o0 < len;
-        const bool in2 = !ordered && o2 + (S << ws) > 0 && o2 < len;
+        const bool in0 = live && o0 + (S << ws) > 0 && o0 < len;
+        const bool in2 = live && !ordered && o2 + (S << ws) > 0 && o2 < len;
         uint32_t wrow = 0, trow = 0;
         if constexpr (wide_board(S)) {
             if (in0) wrow = (uint32_t)reinterpret_cast<const uint16_t*>(a.d_walls)[(cap + env) * (2 * wide_line_words(S)) + r] >> wide_line_lead(S);   // plane 1 = rows
@@ -90,11 +110,17 @@ __global__ void __launch_bounds__(PLANES_THREADS) observe_planes_kernel(const Pl
     // so the items are independent; duplicate targets each keep their own plane.
     for (int j = threadIdx.x; j < n_e * P; j += PLANES_THREADS) {
         const int e = j / P, k = j - e * P;
-        const size_t env = (size_t)(a.first_env + e_first + e);
+        size_t env;
+        if constexpr (ITEMS) {
+            if (!item_env(p, e_first + e, env)) continue;
+        } else {
+            env = (size_t)(a.first_env + e_first + e);
+        }
         int plane, b;
         if (k < T) {
             plane = ordered ? 1 + k : 1;
-            b = a.d_pos[env * pw + k];
+            if constexpr (ITEMS) b = p.item_pos ? p.item_pos[(size_t)(e_first + e) * pw + k] : a.d_pos[env * pw + k];
+            else b = a.d_pos[env * pw + k];
         } else {
             plane = 1 + k;
             b = a.d_targets_packed[env * tpw + (k - T)];
@@ -121,9 +147,9 @@ __global__ void __launch_bounds__(PLANES_THREADS) observe_planes_kernel(const Pl
     if (threadIdx.x >= 32 && t < len) out[t] = stage[t];
 }
 
-template <int S> static void launch_observe_planes(const PlanesParams& p, cudaStream_t st) {
+template <int S, class PP> static void launch_observe_planes(const PP& p, cudaStream_t st) {
     const unsigned blocks = (unsigned)((p.total_bytes + PLANES_STAGE - 1) / PLANES_STAGE);
-    observe_planes_kernel<S><<<blocks, PLANES_THREADS, 0, st>>>(p);
+    observe_planes_kernel<S, PP><<<blocks, PLANES_THREADS, 0, st>>>(p);
 }
 
 // channels of the planes observation; the arguments have been checked (ts_api.cu)
@@ -133,10 +159,9 @@ int observe_planes_channels(const ts_observe_planes_args& a) {
     return 1 + a.n_tiles + nt;
 }
 
-cudaError_t observe_planes_dispatch(const ts_observe_planes_args& a, cudaStream_t st) {
+static void fill_planes_params(PlanesParams& p, const ts_observe_planes_args& a) {
     static const uint32_t ONE[4] = {1u, 0x3F80u, 0x3C00u, 0x3F800000u};    // u8, bf16, f16, f32
     static const int32_t SHIFT[4] = {0, 1, 1, 2};
-    PlanesParams p;
     p.a = a;
     const int C = observe_planes_channels(a);
     p.n_targets = a.goal_mode == TS_GOAL_ORDERED ? C - 1 - a.n_tiles : 0;
@@ -144,7 +169,10 @@ cudaError_t observe_planes_dispatch(const ts_observe_planes_args& a, cudaStream_
     p.one = ONE[a.dtype];
     p.env_bytes = (int64_t)C * a.size * a.size << p.wshift;
     p.total_bytes = a.n_envs * p.env_bytes;
-    switch (a.size) {
+}
+
+template <class PP> static cudaError_t launch_planes_size(const PP& p, cudaStream_t st) {
+    switch (p.a.size) {
 #define TS_OBSP(S) case S: launch_observe_planes<S>(p, st); break;
         TS_OBSP(1) TS_OBSP(2) TS_OBSP(3) TS_OBSP(4) TS_OBSP(5) TS_OBSP(6) TS_OBSP(7) TS_OBSP(8)
         TS_OBSP(9) TS_OBSP(10) TS_OBSP(11) TS_OBSP(12) TS_OBSP(13) TS_OBSP(14) TS_OBSP(15) TS_OBSP(16)
@@ -152,6 +180,24 @@ cudaError_t observe_planes_dispatch(const ts_observe_planes_args& a, cudaStream_
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
+}
+
+cudaError_t observe_planes_dispatch(const ts_observe_planes_args& a, cudaStream_t st) {
+    PlanesParams p;
+    fill_planes_params(p, a);
+    return launch_planes_size(p, st);
+}
+
+cudaError_t observe_planes_items_dispatch(const ts_observe_planes_args& a, const int32_t* ids, const uint8_t* item_pos,
+                                          int64_t n_items, cudaStream_t st) {
+    ts_observe_planes_args r = a;
+    r.first_env = 0;
+    r.n_envs = n_items;
+    PlanesItemsParams p;
+    fill_planes_params(p, r);
+    p.ids = ids;
+    p.item_pos = item_pos;
+    return launch_planes_size(p, st);
 }
 
 }  // namespace ts

@@ -43,19 +43,6 @@ struct WideSmem {
     uint32_t o[8][WIDE_THREADS];   // occupancy lines of the current move
 };
 
-template <int PW> __device__ __forceinline__ void ld_pos(const uint8_t* p, size_t env, uint32_t (&q)[(PW + 3) / 4]) {
-    if constexpr (PW == 1) q[0] = p[env];
-    else if constexpr (PW == 2) q[0] = reinterpret_cast<const uint16_t*>(p)[env];
-    else if constexpr (PW == 4) q[0] = reinterpret_cast<const uint32_t*>(p)[env];
-    else { const uint2 v = reinterpret_cast<const uint2*>(p)[env]; q[0] = v.x; q[1] = v.y; }
-}
-template <int PW> __device__ __forceinline__ void st_pos(uint8_t* p, size_t env, const uint32_t (&q)[(PW + 3) / 4]) {
-    if constexpr (PW == 1) p[env] = (uint8_t)q[0];
-    else if constexpr (PW == 2) reinterpret_cast<uint16_t*>(p)[env] = (uint16_t)q[0];
-    else if constexpr (PW == 4) reinterpret_cast<uint32_t*>(p)[env] = q[0];
-    else reinterpret_cast<uint2*>(p)[env] = make_uint2(q[0], q[1]);
-}
-
 // S = 15, 16 (plain lines, 8 pair words).  Fetch the env's 32-byte wall record of the move's axis (plane 1 =
 // rows for LEFT/RIGHT, plane 0 = columns for UP/DOWN), turn it toward the move direction and park
 // it in the thread's smem column.  Stored lines run toward DOWN / RIGHT; for UP / LEFT (f = 1)
@@ -364,6 +351,53 @@ __global__ void __launch_bounds__(WIDE_THREADS) wide_goal_kernel(const __grid_co
     a.d_won[env] = won ? 1 : 0;
 }
 
+// ts_expand on wide boards: thread = one item (env id, position word); the four moves are four
+// slides of the step's, each reading the wall record of its axis, and the step's goal compare.
+// An id outside [0, capacity) reads nothing and writes zero successors and masks.
+template <int T, int LW>
+__global__ void __launch_bounds__(WIDE_THREADS) wide_expand_kernel(const __grid_constant__ ts_expand_args a) {
+    constexpr int PW = pos_bytes(T), PR = (T + 3) / 4;
+    __shared__ WideSmem sm;
+    const int64_t i = (int64_t)blockIdx.x * WIDE_THREADS + threadIdx.x;
+    if (i >= a.n_items) return;
+    const int64_t e = a.d_env_ids ? (int64_t)a.d_env_ids[i] : i;
+    uint32_t s[4][PR] = {};
+    uint32_t moved = 0, won = 0;
+    if (e >= 0 && e < a.capacity) {
+        const size_t env = (size_t)e, cap = (size_t)a.capacity;
+        uint32_t q0[PR], tq[PR];
+        if (a.d_item_pos) ld_pos<PW>(a.d_item_pos, (size_t)i, q0);
+        else ld_pos<PW>(a.d_pos, env, q0);
+        const bool ordered = a.goal_mode == TS_GOAL_ORDERED, can_win = a.never_win == 0;
+        if (ordered) ld_pos<PW>(a.d_targets_packed, env, tq);
+#pragma unroll
+        for (uint32_t d = 0; d < 4; ++d) {
+            uint32_t q[PR];
+#pragma unroll
+            for (int w = 0; w < PR; ++w) q[w] = q0[w];
+            const uint32_t* rec = reinterpret_cast<const uint32_t*>(a.d_walls) + ((size_t)(d >> 1) * cap + env) * LW;
+            if constexpr (LW == 8) slide_wide16<T>(sm, q, reinterpret_cast<const uint4*>(rec), a.size, d);
+            else slide_wide<T, LW>(sm, q, rec, d);
+            bool mv = false, w_ = can_win;
+#pragma unroll
+            for (int w = 0; w < PR; ++w) mv |= q[w] != q0[w];
+            if (ordered) {
+#pragma unroll
+                for (int w = 0; w < PR; ++w) w_ &= q[w] == tq[w];
+            } else {
+                w_ &= on_targets_wide<T>(q, a.d_targets_packed, env);
+            }
+            moved |= (mv ? 1u : 0u) << d;
+            won |= (w_ ? 1u : 0u) << d;
+#pragma unroll
+            for (int w = 0; w < PR; ++w) s[d][w] = q[w];
+        }
+    }
+    st_succ4<PW>(a.d_succ + (size_t)i * (4 * PW), s);
+    if (a.d_moved) a.d_moved[i] = (uint8_t)moved;
+    if (a.d_won) a.d_won[i] = (uint8_t)won;
+}
+
 template <int T, int GOAL, int LW> static void launch_wide_step_lw(const ts_step_args& a, unsigned blocks, cudaStream_t st) {
     if (a.auto_reset != 0) launch_dependent(wide_step_kernel<T, GOAL, true, LW>, blocks, WIDE_THREADS, st, a);
     else launch_dependent(wide_step_kernel<T, GOAL, false, LW>, blocks, WIDE_THREADS, st, a);
@@ -404,6 +438,23 @@ cudaError_t wide_step_dispatch(const ts_step_args& a, cudaStream_t st) {
 cudaError_t wide_valid_dispatch(const ts_valid_args& a, cudaStream_t st) {
     const unsigned blocks = (unsigned)((a.n_envs + WIDE_THREADS - 1) / WIDE_THREADS);
 #define CALL(T) wide_valid_kernel<T><<<blocks, WIDE_THREADS, 0, st>>>(a)
+    TS_WIDE_SWITCH(CALL)
+#undef CALL
+    return cudaGetLastError();
+}
+
+template <int T> static void launch_wide_expand(const ts_expand_args& a, unsigned blocks, cudaStream_t st) {
+    switch (wide_line_words(a.size)) {
+        case 5: wide_expand_kernel<T, 5><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+        case 6: wide_expand_kernel<T, 6><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+        case 7: wide_expand_kernel<T, 7><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+        default: wide_expand_kernel<T, 8><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+    }
+}
+
+cudaError_t wide_expand_dispatch(const ts_expand_args& a, cudaStream_t st) {
+    const unsigned blocks = (unsigned)((a.n_items + WIDE_THREADS - 1) / WIDE_THREADS);
+#define CALL(T) launch_wide_expand<T>(a, blocks, st)
     TS_WIDE_SWITCH(CALL)
 #undef CALL
     return cudaGetLastError();
