@@ -43,6 +43,9 @@
  *      ts_observe_planes_items: d_out[0 .. n_items*C*size*size) elements, in item order;
  *      ts_expand: d_succ[0 .. 4*n_items*pos_bytes) bytes, d_moved[0 .. n_items) and
  *        d_won[0 .. n_items) (when given), in item order -- no env buffer;
+ *      ts_playout: d_final[0 .. n_items*pos_bytes) bytes, d_steps[0 .. n_items), d_won[0 .. n_items)
+ *        and, when given, d_moves[0 .. n_steps*n_items) and d_traj[0 .. n_steps*n_items*pos_bytes)
+ *        bytes, in item order (step-major for the last two) -- no env buffer;
  *      ts_valid_moves, ts_goal_check: d_mask / d_won are ABSOLUTE (env e at [e]); the range, and on
  *        boards up to 8x8 with 1..8 tiles also the (correct) result of the up-to-3 envs after the
  *        range that share its last 4-env group;
@@ -280,6 +283,55 @@ typedef struct ts_expand_args {
     uint8_t *d_succ, *d_moved, *d_won;
 } ts_expand_args;
 int ts_expand(const ts_expand_args *a, void *stream);
+
+/* ---------------------------------------------------------------------------------------
+ * ts_playout: up to n_steps moves from many states in one launch (csrc/ts_playout.cu, ts_wide.cu,
+ * ts_generic.cu; GameState.move, state.py:120-170, and is_won, state.py:172-186, once per move),
+ * for MCTS simulation, replaying plans and recording trajectories.  Items as ts_expand's: item
+ * i < n_items plays on env e = d_env_ids[i] (NULL: e = i) from positions d_item_pos[i] (NULL:
+ * d_pos[e]).  The moves come from `policy`:
+ *   TS_PLAYOUT_PLAN    d_plan u8 [n_steps][n_items], step-major: move k of item i is
+ *                      d_plan[k*n_items + i] (0 UP, 1 DOWN, 2 LEFT, 3 RIGHT); a byte >= 4 ends the
+ *                      plan (255: padding of ragged move strings).  A move that changes nothing is
+ *                      still played and counted, as ts_step counts it.
+ *   TS_PLAYOUT_RANDOM  each move drawn uniformly among the moves that change the positions (the
+ *                      mask of ts_valid_moves), by K7's walk rule: item i's stream is K0's
+ *                      synth_stream(seed, i), each move takes one draw r = splitmix64 >> 32 and is
+ *                      the floor(r*n / 2^32)-th set bit, lowest first, of the n-bit mask; an empty
+ *                      mask ends the playout.
+ * The goal is checked after every move, as ts_step does: the playout stops after the first move that
+ * meets it.  So a plan of moves 0..3 gives what n_steps ts_step calls with auto_reset = 0 and
+ * max_steps > n_steps leave.  Outputs, for every item:
+ *   d_final[i]      [n_items][pos_bytes]: the positions after the last move played (tile order kept)
+ *   d_steps[i]      int32: moves played
+ *   d_won[i]        1 iff the last move played met the goal (never 1 with never_win)
+ *   d_moves[k][i]   optional u8 [n_steps][n_items]: the move played as move k; 255 for k >= steps
+ *   d_traj[k][i]    optional [n_steps][n_items][pos_bytes]: the positions after move k; 0 for k >= steps
+ * An e outside [0, capacity) reads nothing: zero positions, 0 moves, not won, 255 moves.
+ * n_tiles = 0: nothing moves; a plan plays its moves as no-ops and the first one wins iff the board
+ * has no targets (the rule of ts_step); a random playout plays none.  n_steps = 0: the start
+ * positions, 0 moves, not won.  Argument errors (all before the n_items = 0 return): size, n_tiles,
+ * capacity, goal_mode, never_win outside 0/1, an unknown policy, n_steps < 0 (TS_E_BAD_ARGUMENT);
+ * n_items < 0 or, without d_env_ids, n_items > capacity (TS_E_BAD_RANGE); a NULL d_walls /
+ * d_targets_packed / d_final / d_steps / d_won, d_pos when d_item_pos is NULL, or d_plan under
+ * TS_PLAYOUT_PLAN (TS_E_NULL_POINTER); n_steps*n_items*pos_bytes beyond int64, or n_items beyond
+ * (2^31 - 1) * 128, the items one launch covers (TS_E_BAD_RANGE);
+ * then, with n_items > 0, d_final, d_item_pos and d_traj must be 16-byte aligned (TS_E_MISALIGNED).
+ * ------------------------------------------------------------------------------------- */
+#define TS_PLAYOUT_PLAN 0
+#define TS_PLAYOUT_RANDOM 1
+typedef struct ts_playout_args {
+    int32_t size, n_tiles, goal_mode, never_win;
+    int32_t policy, n_steps;
+    int64_t n_items, capacity;
+    uint64_t seed;
+    const int32_t *d_env_ids;
+    const uint8_t *d_walls, *d_targets_packed, *d_pos, *d_item_pos, *d_plan;
+    uint8_t *d_final;
+    int32_t *d_steps;
+    uint8_t *d_won, *d_moves, *d_traj;
+} ts_playout_args;
+int ts_playout(const ts_playout_args *a, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * ts_valid_moves: bit d of d_mask[env] set when move d changes any tile position

@@ -25,6 +25,7 @@ MAX_WALK = 65535
 OPT_UNSOLVABLE, OPT_CUTOFF, OPT_NOT_SEARCHED = -1, -2, -3
 OPT_MAX_DEPTH = 254
 OBS_U8, OBS_BF16, OBS_F16, OBS_F32 = 0, 1, 2, 3
+PLAYOUT_PLAN, PLAYOUT_RANDOM = 0, 1
 
 _vp, _i32, _i64, _f32 = C.c_void_p, C.c_int32, C.c_int64, C.c_float
 
@@ -72,6 +73,13 @@ class ExpandArgs(C.Structure):
                 ("n_items", _i64), ("capacity", _i64),
                 ("d_env_ids", _vp), ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp), ("d_item_pos", _vp),
                 ("d_succ", _vp), ("d_moved", _vp), ("d_won", _vp)]
+
+
+class PlayoutArgs(C.Structure):
+    _fields_ = [("size", _i32), ("n_tiles", _i32), ("goal_mode", _i32), ("never_win", _i32),
+                ("policy", _i32), ("n_steps", _i32), ("n_items", _i64), ("capacity", _i64), ("seed", C.c_uint64),
+                ("d_env_ids", _vp), ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp), ("d_item_pos", _vp),
+                ("d_plan", _vp), ("d_final", _vp), ("d_steps", _vp), ("d_won", _vp), ("d_moves", _vp), ("d_traj", _vp)]
 
 
 class ValidArgs(C.Structure):
@@ -156,6 +164,7 @@ SYMBOLS = {
     "ts_observe_planes": (C.c_int, [C.POINTER(ObservePlanesArgs), _vp]),
     "ts_observe_planes_items": (C.c_int, [C.POINTER(ObservePlanesArgs), _vp, _vp, _i64, _vp]),
     "ts_expand": (C.c_int, [C.POINTER(ExpandArgs), _vp]),
+    "ts_playout": (C.c_int, [C.POINTER(PlayoutArgs), _vp]),
     "ts_valid_moves": (C.c_int, [C.POINTER(ValidArgs), _vp]),
     "ts_goal_check": (C.c_int, [C.POINTER(GoalArgs), _vp]),
     "ts_bfs_seed": (C.c_int, [C.POINTER(BfsArgs), _vp]),

@@ -18,8 +18,8 @@ import torch
 
 from . import _lib
 from ._lib import (CAP_ALIGN, F_WON, GOAL_ORDERED, GOAL_SET, MAX_SIZE, MAX_TILES, OBS_BF16, OBS_F16, OBS_F32, OBS_U8,
-                   EncodeArgs, ExpandArgs, GoalArgs, ObserveArgs, ObservePlanesArgs, PoolResetArgs, StepArgs, SynthArgs, ValidArgs,
-                   check, lib)
+                   PLAYOUT_PLAN, PLAYOUT_RANDOM, EncodeArgs, ExpandArgs, GoalArgs, ObserveArgs, ObservePlanesArgs, PlayoutArgs,
+                   PoolResetArgs, StepArgs, SynthArgs, ValidArgs, check, lib)
 from .puzzle import Puzzle, as_puzzle, uniform_shape
 
 DEFAULT_REWARDS = (1.0, -0.01, -0.05)   # r_win, r_step, r_invalid -- repo-defined (the reference has no reward)
@@ -721,6 +721,77 @@ class BatchedTilerSliderEnv:
                            d_succ=_ptr(out[0]), d_moved=_ptr(out[1]), d_won=_ptr(out[2]))
             with torch.cuda.device(self.device):
                 check(self._lib.ts_expand(C.byref(a), self._stream()), "ts_expand")
+        return out
+
+    def playout(self, ids=None, pos: torch.Tensor | None = None, *, actions: torch.Tensor | None = None,
+                n_steps: int | None = None, seed: int = 0, record: bool = False, out=None) -> tuple[torch.Tensor, ...]:
+        """Up to L moves from many states in one kernel (ts_playout), for MCTS simulation, replaying
+        plans and recording trajectories.  Items as expand() takes them: ids (default every env) give
+        the puzzles, pos (default each listed env's current positions) the start positions.
+          actions   a plan: contiguous uint8 [L, n] on the batch's device, step-major (row k = move k
+                    of every item; 0 UP, 1 DOWN, 2 LEFT, 3 RIGHT); a byte >= 4 ends the item's plan
+                    (pad ragged move strings with 255).  L = actions.shape[0]; `n_steps` must not be
+                    given.  A move that changes nothing is played and counted, as step() counts it.
+          otherwise random moves: `n_steps` (required) moves, each drawn uniformly among the moves
+                    that change the positions (valid_moves()); item i's draws depend on (seed, i) only
+                    (K7's walk rule, include/tiler_slider.h); a state where nothing can move ends it.
+        The goal is checked after every move and a win ends the item's playout.  Returns (final uint8
+        [n, pos_bytes], steps int32 [n], won uint8 [n]): the positions after the last move played, the
+        moves played and 1 iff the last one won; with record=True also (moves uint8 [L, n], traj uint8
+        [L, n, pos_bytes]): the move played as move k (255 for k >= steps) and the positions after it
+        (zero for k >= steps).  `out`: preallocated tensors of those shapes and dtypes, contiguous on
+        the device (3 of them, 5 with record); with it and device ids (int32, contiguous) or none,
+        the call neither allocates nor synchronises, so it can be captured in a CUDA graph beside
+        step() -- the seed is then fixed at capture.  Host ids outside [0, n_envs) raise IndexError;
+        a device id outside [0, capacity) gets zero positions, 0 steps, not won.  Runs on the current
+        stream and changes no env state.  Not available for host_io batches."""
+        self._require_loaded()
+        n, ids, pos = self._items("playout", ids, pos)
+        if actions is not None:
+            if n_steps is not None:
+                raise ValueError("playout: give either actions (a plan) or n_steps (random moves), not both")
+            if not isinstance(actions, torch.Tensor) or actions.dtype != torch.uint8 or actions.dim() != 2 or actions.shape[1] != n:
+                raise ValueError(f"playout: actions must be a uint8 tensor [L, {n}] (step-major: row k = move k of every item)")
+            if actions.device != self.device:
+                raise ValueError(f"playout: actions are on {actions.device}, the batch on {self.device}")
+            if not actions.is_contiguous():
+                raise ValueError("playout: actions must be contiguous")
+            # an empty plan plays no move: the random policy with no moves gives the same result and
+            # needs no plan buffer (an empty tensor has no data pointer)
+            L, policy = actions.shape[0], PLAYOUT_PLAN if actions.shape[0] else PLAYOUT_RANDOM
+        else:
+            if n_steps is None:
+                raise ValueError("playout: random playouts need n_steps (or pass actions, a plan)")
+            L, policy = int(n_steps), PLAYOUT_RANDOM
+        if not 0 <= L < 2 ** 31:
+            raise ValueError(f"playout: {L} moves outside 0 .. 2^31 - 1")
+        PW = self.pos_bytes
+        specs = [((n, PW), torch.uint8), ((n,), torch.int32), ((n,), torch.uint8)]
+        if record:
+            specs += [((L, n), torch.uint8), ((L, n, PW), torch.uint8)]
+        if out is None:
+            out = tuple(torch.empty(s, dtype=dt, device=self.device) for s, dt in specs)
+        else:
+            if not isinstance(out, (tuple, list)) or len(out) != len(specs):
+                raise ValueError(f"playout(out): out must be a tuple of {len(specs)} tensors "
+                                 f"({'final, steps, won, moves, traj' if record else 'final, steps, won'})")
+            for t, (s, dt) in zip(out, specs):
+                if not isinstance(t, torch.Tensor) or t.dtype != dt or tuple(t.shape) != s:
+                    raise ValueError(f"playout(out): expected tensors of shapes and dtypes {[(s, str(dt)) for s, dt in specs]}")
+                if t.device != self.device:
+                    raise ValueError(f"playout(out): out must live on {self.device}, not on {t.device}")
+                if not t.is_contiguous():
+                    raise ValueError("playout(out): out must be contiguous")
+            out = tuple(out)
+        if n:
+            a = PlayoutArgs(size=self.size, n_tiles=self.n_tiles, goal_mode=self.goal_mode, never_win=int(self.never_win),
+                            policy=policy, n_steps=L, n_items=n, capacity=self.capacity, seed=int(seed) & (2 ** 64 - 1),
+                            d_env_ids=_ptr(ids), d_walls=_ptr(self._walls), d_targets_packed=_ptr(self._targets),
+                            d_pos=_ptr(self._pos), d_item_pos=_ptr(pos), d_plan=_ptr(actions), d_final=_ptr(out[0]),
+                            d_steps=_ptr(out[1]), d_won=_ptr(out[2]), d_moves=_ptr(out[3]) if record else None,
+                            d_traj=_ptr(out[4]) if record else None)
+            with torch.cuda.device(self.device):
+                check(self._lib.ts_playout(C.byref(a), self._stream()), "ts_playout")
         return out
 
     def _observe_planes_args(self, out: torch.Tensor | None, dtype: torch.dtype) -> ObservePlanesArgs:

@@ -1,6 +1,7 @@
 // ts_api.cu -- C-ABI entry points (include/tiler_slider.h), argument validation, and the
 // load-time kernels: K1 ts_encode, K0 ts_synth (K3 ts_observe lives in ts_observe.cu,
-// ts_observe_planes in ts_observe_planes.cu, ts_expand in ts_expand.cu / ts_wide.cu / ts_generic.cu).
+// ts_observe_planes in ts_observe_planes.cu, ts_expand in ts_expand.cu / ts_wide.cu / ts_generic.cu, ts_playout in
+// ts_playout.cu / ts_wide.cu / ts_generic.cu).
 //
 // Reference map (paths relative to the reference checkout):
 //   ts_encode   explainrl/environment/state.py:61-73        GameState.__init__ (is_blocked + lists)
@@ -25,6 +26,9 @@ int observe_planes_channels(const ts_observe_planes_args&);
 cudaError_t expand_dispatch(const ts_expand_args&, cudaStream_t);
 cudaError_t wide_expand_dispatch(const ts_expand_args&, cudaStream_t);
 cudaError_t generic_expand_dispatch(const ts_expand_args&, cudaStream_t);
+cudaError_t playout_dispatch(const ts_playout_args&, cudaStream_t);
+cudaError_t wide_playout_dispatch(const ts_playout_args&, cudaStream_t);
+cudaError_t generic_playout_dispatch(const ts_playout_args&, cudaStream_t);
 cudaError_t wide_step_dispatch(const ts_step_args&, cudaStream_t);
 cudaError_t wide_valid_dispatch(const ts_valid_args&, cudaStream_t);
 cudaError_t wide_goal_dispatch(const ts_goal_args&, cudaStream_t);
@@ -308,6 +312,39 @@ int ts_expand(const ts_expand_args* a, void* stream) {
     else if (wide_board(a->size)) e = wide_expand_dispatch(*a, st);
     else e = expand_dispatch(*a, st);
     return cuda_result(e, "ts_expand launch");
+}
+
+int ts_playout(const ts_playout_args* a, void* stream) {
+    if (!a) return fail(TS_E_NULL_POINTER, "null args");
+    if (int rc = check_shape(a->size, a->n_tiles, 0, 0, a->capacity)) return rc;
+    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
+    if (a->never_win != 0 && a->never_win != 1) return fail(TS_E_BAD_ARGUMENT, "never_win %d (0 or 1)", a->never_win);
+    if (a->policy != TS_PLAYOUT_PLAN && a->policy != TS_PLAYOUT_RANDOM)
+        return fail(TS_E_BAD_ARGUMENT, "policy %d (TS_PLAYOUT_PLAN or TS_PLAYOUT_RANDOM)", a->policy);
+    if (a->n_steps < 0) return fail(TS_E_BAD_ARGUMENT, "n_steps %d", a->n_steps);
+    if (int rc = check_items(a->n_items, a->d_env_ids, a->capacity)) return rc;
+    if (!a->d_walls || !a->d_targets_packed || (!a->d_pos && !a->d_item_pos) || !a->d_final || !a->d_steps || !a->d_won ||
+        (a->policy == TS_PLAYOUT_PLAN && !a->d_plan))
+        return fail(TS_E_NULL_POINTER, "null device pointer");
+    // the step-major records hold n_steps * n_items elements, indexed with 64 bits
+    const int64_t per_item = (int64_t)a->n_steps * pos_bytes(a->n_tiles);
+    if (per_item > 0 && a->n_items > INT64_MAX / per_item)
+        return fail(TS_E_BAD_RANGE, "n_steps %d x n_items %lld x pos_bytes overflows 64 bits", a->n_steps, (long long)a->n_items);
+    // one launch of 128-thread blocks (the smallest of the three kernels) covers at most 2^31 - 1 blocks
+    if (a->n_items > (int64_t)INT32_MAX * 128)
+        return fail(TS_E_BAD_RANGE, "n_items %lld exceeds the %lld items of one launch", (long long)a->n_items,
+                    (long long)INT32_MAX * 128);
+    if (a->n_items == 0) return 0;
+    if (!aligned16(a->d_final)) return fail(TS_E_MISALIGNED, "d_final %p is not 16-byte aligned", (const void*)a->d_final);
+    if (a->d_item_pos && !aligned16(a->d_item_pos))
+        return fail(TS_E_MISALIGNED, "d_item_pos %p is not 16-byte aligned", (const void*)a->d_item_pos);
+    if (a->d_traj && !aligned16(a->d_traj)) return fail(TS_E_MISALIGNED, "d_traj %p is not 16-byte aligned", (const void*)a->d_traj);
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e;
+    if (a->n_tiles == 0 || a->n_tiles > MAX_TILES) e = generic_playout_dispatch(*a, st);   // the kernel classes of ts_step
+    else if (wide_board(a->size)) e = wide_playout_dispatch(*a, st);
+    else e = playout_dispatch(*a, st);
+    return cuda_result(e, "ts_playout launch");
 }
 
 int ts_valid_moves(const ts_valid_args* a, void* stream) {

@@ -1,4 +1,4 @@
-// ts_generic.cu -- step / valid-move / goal / expand kernels for everything the specialised kernels do not cover:
+// ts_generic.cu -- step / valid-move / goal / expand / playout kernels for everything the specialised kernels do not cover:
 //   (a) the ragged end of a range on bitboard-class boards (S <= 8): step_kernel works on whole
 //       4-env groups, so ts_step hands the last n_envs % 4 envs of a call to generic_step_kernel --
 //       nothing outside [first_env, first_env + n_envs) is ever read-modified-written;
@@ -15,6 +15,7 @@
 // bookkeeping of TilerSliderEnv.step (explainrl/environment/environment.py:119-143) and reset
 // (:89-97) exactly as step_group (ts_step.cuh) does it.  Not a fast path.
 #include "ts_common.cuh"
+#include "ts_playout.cuh"
 #include "../../include/tiler_slider.h"
 
 namespace ts {
@@ -242,6 +243,64 @@ __global__ void __launch_bounds__(128) generic_expand_kernel(const ts_expand_arg
 cudaError_t generic_expand_dispatch(const ts_expand_args& a, cudaStream_t st) {
     if (a.n_items <= 0) return cudaSuccess;
     generic_expand_kernel<<<(unsigned)((a.n_items + 127) / 128), 128, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+// ts_playout for 0 and 9..32 tiles (any S): the step's slide and goal test once per move.  The random
+// policy takes its mask from the four slides of the current positions, then plays the drawn one.  An
+// id outside [0, capacity) reads nothing: zero positions, 0 moves, not won.
+__global__ void __launch_bounds__(128) generic_playout_kernel(const ts_playout_args a) {
+    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (i >= a.n_items) return;
+    const int S = a.size, T = a.n_tiles, pw = pos_bytes(T);
+    const int64_t e = a.d_env_ids ? (int64_t)a.d_env_ids[i] : i;
+    uint8_t p[MAX_TILES_ANY], nxt[MAX_TILES_ANY];
+    for (int t = 0; t < MAX_TILES_ANY; ++t) p[t] = 0;
+    int steps = 0;
+    bool won = false;
+    if (e >= 0 && e < a.capacity) {
+        const size_t env = (size_t)e, cap = (size_t)a.capacity;
+        const uint8_t* src = a.d_item_pos ? a.d_item_pos + (size_t)i * pw : a.d_pos + env * pw;
+        for (int t = 0; t < T; ++t) p[t] = src[t];
+        GenericWalls wl;
+        load_generic_walls(wl, a.d_walls, S, T, cap, env);
+        uint64_t rng = a.policy == TS_PLAYOUT_RANDOM ? synth_stream(a.seed, (uint64_t)i) : 0;
+        while (steps < a.n_steps && !won) {
+            uint32_t d;
+            if (a.policy == TS_PLAYOUT_RANDOM) {
+                uint32_t mask = 0;
+                for (uint32_t m = 0; m < 4; ++m)
+                    if (generic_slide(p, nxt, S, T, m, wl)) mask |= 1u << m;
+                if (!mask) break;
+                d = draw_move(rng, mask);
+            } else {
+                d = a.d_plan[playout_row(a, steps, i)];
+                if (d >= 4) break;
+            }
+            generic_slide(p, nxt, S, T, d, wl);
+            for (int t = 0; t < T; ++t) p[t] = nxt[t];
+            won = a.never_win == 0 && goal_met(p, S, T, a.goal_mode, a.d_targets_packed, cap, env);
+            const size_t row = playout_row(a, steps, i);
+            if (a.d_moves) a.d_moves[row] = (uint8_t)d;
+            if (a.d_traj)
+                for (int t = 0; t < pw; ++t) a.d_traj[row * pw + t] = t < T ? p[t] : 0;
+            ++steps;
+        }
+    }
+    for (int t = 0; t < pw; ++t) a.d_final[(size_t)i * pw + t] = t < T ? p[t] : 0;
+    a.d_steps[i] = steps;
+    a.d_won[i] = won ? 1 : 0;
+    for (int k = steps; k < a.n_steps && (a.d_moves || a.d_traj); ++k) {
+        const size_t row = playout_row(a, k, i);
+        if (a.d_moves) a.d_moves[row] = 255;
+        if (a.d_traj)
+            for (int t = 0; t < pw; ++t) a.d_traj[row * pw + t] = 0;
+    }
+}
+
+cudaError_t generic_playout_dispatch(const ts_playout_args& a, cudaStream_t st) {
+    if (a.n_items <= 0) return cudaSuccess;
+    generic_playout_kernel<<<(unsigned)((a.n_items + 127) / 128), 128, 0, st>>>(a);
     return cudaGetLastError();
 }
 

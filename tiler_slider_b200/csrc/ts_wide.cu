@@ -31,6 +31,7 @@
 // only ever touches its own column, so the dynamic line index costs no bank conflict
 // (bank = thread % 32 whatever the line) and needs no barrier.
 #include "ts_common.cuh"
+#include "ts_playout.cuh"
 #include "../../include/tiler_slider.h"
 
 namespace ts {
@@ -398,6 +399,63 @@ __global__ void __launch_bounds__(WIDE_THREADS) wide_expand_kernel(const __grid_
     if (a.d_won) a.d_won[i] = (uint8_t)won;
 }
 
+// ts_playout on wide boards: thread = one item (env id, position word), positions in registers for
+// every move; a move is the step's slide on the wall record of its axis and the step's goal compare.
+// The random policy takes the mask of ts_valid_moves (valid_mask_wide, rows record) before each move.
+// The records are re-read every move (a thread reads the same 4*LW bytes again, which is expected to hit
+// L1; not measured against records held in registers or shared memory).
+// An id outside [0, capacity) reads nothing: zero positions, 0 moves, not won.
+template <int T, int LW, int POLICY>
+__global__ void __launch_bounds__(WIDE_THREADS) wide_playout_kernel(const __grid_constant__ ts_playout_args a) {
+    constexpr int PW = pos_bytes(T), PR = (T + 3) / 4;
+    __shared__ WideSmem sm;
+    const int64_t i = (int64_t)blockIdx.x * WIDE_THREADS + threadIdx.x;
+    if (i >= a.n_items) return;
+    const int64_t e = a.d_env_ids ? (int64_t)a.d_env_ids[i] : i;
+    uint32_t q[PR] = {};
+    int steps = 0;
+    bool won = false;
+    if (e >= 0 && e < a.capacity) {
+        const size_t env = (size_t)e, cap = (size_t)a.capacity;
+        if (a.d_item_pos) ld_pos<PW>(a.d_item_pos, (size_t)i, q);
+        else ld_pos<PW>(a.d_pos, env, q);
+        const bool ordered = a.goal_mode == TS_GOAL_ORDERED, can_win = a.never_win == 0;
+        uint32_t tq[PR] = {};
+        if (ordered) ld_pos<PW>(a.d_targets_packed, env, tq);
+        const uint32_t* cols = reinterpret_cast<const uint32_t*>(a.d_walls) + env * LW;           // plane 0: UP / DOWN
+        const uint32_t* rows = reinterpret_cast<const uint32_t*>(a.d_walls) + (cap + env) * LW;   // plane 1: LEFT / RIGHT
+        uint64_t rng = 0;
+        if constexpr (POLICY == TS_PLAYOUT_RANDOM) rng = synth_stream(a.seed, (uint64_t)i);
+        while (steps < a.n_steps && !won) {
+            uint32_t d;
+            if constexpr (POLICY == TS_PLAYOUT_RANDOM) {
+                const uint32_t mask = valid_mask_wide<T, LW>(sm, q, rows, a.size);
+                if (!mask) break;
+                d = draw_move(rng, mask);
+            } else {
+                d = __ldcs(a.d_plan + playout_row(a, steps, i));
+                if (d >= 4) break;
+            }
+            const uint32_t* rec = d >> 1 ? rows : cols;
+            if constexpr (LW == 8) slide_wide16<T>(sm, q, reinterpret_cast<const uint4*>(rec), a.size, d);
+            else slide_wide<T, LW>(sm, q, rec, d);
+            won = can_win;
+            if (ordered) {
+#pragma unroll
+                for (int w = 0; w < PR; ++w) won &= q[w] == tq[w];
+            } else {
+                won &= on_targets_wide<T>(q, a.d_targets_packed, env);
+            }
+            playout_record<PW>(a, steps, i, d, q);
+            ++steps;
+        }
+    }
+    st_pos<PW>(a.d_final, (size_t)i, q);
+    a.d_steps[i] = steps;
+    a.d_won[i] = won ? 1 : 0;
+    playout_tail<PW>(a, steps, i);
+}
+
 template <int T, int GOAL, int LW> static void launch_wide_step_lw(const ts_step_args& a, unsigned blocks, cudaStream_t st) {
     if (a.auto_reset != 0) launch_dependent(wide_step_kernel<T, GOAL, true, LW>, blocks, WIDE_THREADS, st, a);
     else launch_dependent(wide_step_kernel<T, GOAL, false, LW>, blocks, WIDE_THREADS, st, a);
@@ -455,6 +513,25 @@ template <int T> static void launch_wide_expand(const ts_expand_args& a, unsigne
 cudaError_t wide_expand_dispatch(const ts_expand_args& a, cudaStream_t st) {
     const unsigned blocks = (unsigned)((a.n_items + WIDE_THREADS - 1) / WIDE_THREADS);
 #define CALL(T) launch_wide_expand<T>(a, blocks, st)
+    TS_WIDE_SWITCH(CALL)
+#undef CALL
+    return cudaGetLastError();
+}
+
+template <int T, int POLICY> static void launch_wide_playout(const ts_playout_args& a, unsigned blocks, cudaStream_t st) {
+    switch (wide_line_words(a.size)) {
+        case 5: wide_playout_kernel<T, 5, POLICY><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+        case 6: wide_playout_kernel<T, 6, POLICY><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+        case 7: wide_playout_kernel<T, 7, POLICY><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+        default: wide_playout_kernel<T, 8, POLICY><<<blocks, WIDE_THREADS, 0, st>>>(a); break;
+    }
+}
+
+cudaError_t wide_playout_dispatch(const ts_playout_args& a, cudaStream_t st) {
+    const unsigned blocks = (unsigned)((a.n_items + WIDE_THREADS - 1) / WIDE_THREADS);
+#define CALL(T)                                                                                              \
+    if (a.policy == TS_PLAYOUT_RANDOM) launch_wide_playout<T, TS_PLAYOUT_RANDOM>(a, blocks, st);             \
+    else launch_wide_playout<T, TS_PLAYOUT_PLAN>(a, blocks, st)
     TS_WIDE_SWITCH(CALL)
 #undef CALL
     return cudaGetLastError();
