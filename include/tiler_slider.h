@@ -180,6 +180,10 @@ int ts_synth(const ts_synth_args *a, void *stream);
  *   n_tiles = 0: nothing moves (every step is INVALID); won iff the board has no targets either
  *             (ordered mode: the caller says so through never_win).
  *   count_bytes = 1 needs max_steps <= 255 with auto_reset, <= 254 without.
+ *   order   : the order in which the launch walks the range; 0 = ascending, 1 = descending.
+ *             Results do not depend on it.  Alternating it on back-to-back steps over one
+ *             range makes each step start on the envs the previous one left in L2 (DESIGN
+ *             section 3).  Other values: TS_E_BAD_ARGUMENT.
  * ------------------------------------------------------------------------------------- */
 typedef struct ts_step_args {
     int32_t size, n_tiles, goal_mode, never_win;
@@ -187,7 +191,7 @@ typedef struct ts_step_args {
     const uint8_t *d_walls, *d_targets_packed, *d_init;
     uint8_t *d_pos;
     void *d_step_count;
-    int32_t count_bytes, max_steps, auto_reset, reserved0;
+    int32_t count_bytes, max_steps, auto_reset, order;
     const uint8_t *d_actions;
     float r_win, r_step, r_invalid, reserved1;
     float *d_reward;

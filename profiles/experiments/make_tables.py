@@ -1,6 +1,7 @@
 """Regenerate the measured tables of README.md and DESIGN.md from the kept bench lines
-(profiles/r2_bench_n{1,2,4,8}.json), between the <!-- BEGIN/END ... --> markers, so that every
-number in the docs is a number of an artifact:   python profiles/experiments/make_tables.py"""
+(profiles/r8_bench_n1.json for one GPU, profiles/r2_bench_n{2,4,8}.json for several), between the
+<!-- BEGIN/END ... --> markers, so that every number in the docs is a number of an artifact:
+    python profiles/experiments/make_tables.py"""
 import json
 import os
 import re
@@ -14,8 +15,9 @@ def f(x):
 
 def load():
     out = {}
-    for n in (1, 2, 4, 8):
-        p = os.path.join(ROOT, "profiles", f"r2_bench_n{n}.json")
+    # one GPU: the step with alternating traversal order (round 8); several GPUs: round 2's lines
+    for n, name in ((1, "r8_bench_n1.json"), (2, "r2_bench_n2.json"), (4, "r2_bench_n4.json"), (8, "r2_bench_n8.json")):
+        p = os.path.join(ROOT, "profiles", name)
         if os.path.exists(p):
             with open(p) as fh:
                 out[n] = json.loads(fh.read().strip().splitlines()[-1])
@@ -41,7 +43,7 @@ def scaling_table(d):
 
 def config_table(d):
     x = d[1]
-    t = ("| Config (1×B200) | env-steps/s | µs/step | fraction of the algorithmic HBM roofline (6534 GB/s measured copy) | "
+    t = (f"| Config (1×B200) | env-steps/s | µs/step | fraction of the algorithmic HBM roofline ({x['roofline']['peak']:.0f} GB/s) | "
          "bytes moved / algorithmic per env-step | steady-state DRAM traffic per launch (ncu) | parity (env-steps vs the C oracle, mismatches) |\n"
          "|---|---|---|---|---|---|---|\n")
     rows = [("c3: 6×6, 4 coloured tiles, 8 walls, 16,777,216 envs (headline)", x, x["parity"])]

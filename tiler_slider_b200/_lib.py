@@ -49,7 +49,7 @@ class StepArgs(C.Structure):
                 ("first_env", _i64), ("n_envs", _i64), ("capacity", _i64),
                 ("d_walls", _vp), ("d_targets_packed", _vp), ("d_init", _vp), ("d_pos", _vp),
                 ("d_step_count", _vp),
-                ("count_bytes", _i32), ("max_steps", _i32), ("auto_reset", _i32), ("reserved0", _i32),
+                ("count_bytes", _i32), ("max_steps", _i32), ("auto_reset", _i32), ("order", _i32),
                 ("d_actions", _vp),
                 ("r_win", _f32), ("r_step", _f32), ("r_invalid", _f32), ("reserved1", _f32),
                 ("d_reward", _vp), ("d_done", _vp), ("d_flags", _vp), ("d_terminal_pos", _vp)]

@@ -252,7 +252,9 @@ class BatchedTilerSliderEnv:
         the device.  Returns (state, reward, done): the packed positions uint8[N,pos_bytes],
         float32[N], bool[N] -- views of buffers that the next step overwrites.  `flags`
         holds is_won / invalid_move / timeout; with auto_reset the state of a finished env is
-        already its reset state (its last positions are in `terminal_pos` if tracked)."""
+        already its reset state (its last positions are in `terminal_pos` if tracked).
+        Successive calls walk the envs in alternating order (ts_step_args.order), which changes no
+        result and lets each step start on what the previous one left in L2."""
         self._require_loaded()
         ptr = self._stage_actions(actions)
         a = self._cached_args
@@ -272,6 +274,7 @@ class BatchedTilerSliderEnv:
                 rc = self._lib.ts_step(C.byref(a), self._stream())
                 if pool is not None and not rc:
                     rc_pool = self._lib.ts_pool_reset(C.byref(pool), self._stream())
+        a.order ^= 1              # the next step walks the envs the other way and starts on what this one left in L2
         if rc:
             check(rc, "ts_step")
         if pool is not None and rc_pool:

@@ -189,6 +189,7 @@ int ts_step(const ts_step_args* a, void* stream) {
     if (!ts_supported(a->size, a->n_tiles)) return fail(TS_E_UNSUPPORTED, "no step kernel for size %d, n_tiles %d", a->size, a->n_tiles);
     if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
     if (a->count_bytes != 1 && a->count_bytes != 4) return fail(TS_E_BAD_ARGUMENT, "count_bytes %d (1 or 4)", a->count_bytes);
+    if (a->order != 0 && a->order != 1) return fail(TS_E_BAD_ARGUMENT, "order %d (0 ascending, 1 descending)", a->order);
     // 1-byte counters are bumped SWAR, four to a word: a frozen env (auto_reset = 0) resting at 255 would carry into its neighbour
     if (a->count_bytes == 1 && a->max_steps > (a->auto_reset ? 255 : 254)) return fail(TS_E_BAD_ARGUMENT, "max_steps %d needs count_bytes 4", a->max_steps);
     if (!a->d_walls || !a->d_targets_packed || !a->d_init || !a->d_pos || !a->d_step_count || !a->d_actions || !a->d_reward)

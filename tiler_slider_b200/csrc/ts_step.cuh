@@ -191,10 +191,15 @@ __global__ void __launch_bounds__(STEP_THREADS, (step_min_blocks<S, T, GOAL, AR,
     // (ts_step rejects capacities of 2^32 groups or more)
     // whole 4-env groups only: ts_step hands the ragged end of a range (n_envs % 4 envs) to
     // generic_step_kernel (ts_generic.cu), so nothing outside [first_env, first_env + n_envs) is touched
-    const uint32_t n_groups = (uint32_t)(a.n_envs / GROUP);
-    uint32_t g = blockIdx.x * STEP_THREADS + threadIdx.x;
-    if (g >= n_groups) return;
-    g += (uint32_t)(a.first_env / GROUP);
+    // order 1 walks the range from its end, so a step that follows an ascending one starts on the
+    // groups it left in L2 (ts_step_args.order): i -> n_groups - 1 - i = (i ^ m) + n_groups with
+    // m = ~0, the form under which the kernels of boards up to 6x6 fit their registers without spills.
+    // ts_step has checked first_env, n_envs >= 0.
+    const uint32_t n_groups = (uint32_t)((uint64_t)a.n_envs / GROUP);
+    const uint32_t i = blockIdx.x * STEP_THREADS + threadIdx.x;
+    if (i >= n_groups) return;
+    const uint32_t m = 0u - (uint32_t)a.order;
+    const uint32_t g = (i ^ m) + ((uint32_t)((uint64_t)a.first_env / GROUP) + (n_groups & m));
     const size_t cap = (size_t)a.capacity;
     const size_t e0 = (size_t)g * GROUP;
     dependent_launch_sync();     // nothing is read before the launch ahead of us has completed (ts_common.cuh)
@@ -203,7 +208,9 @@ __global__ void __launch_bounds__(STEP_THREADS, (step_min_blocks<S, T, GOAL, AR,
     // targets and step counters are only needed after the slide; under the 32-register cap the
     // compiler sinks their loads to that point, so pull the lines into L2 now (no register cost)
     if constexpr (GOAL == TS_GOAL_ORDERED) asm volatile("prefetch.global.L2 [%0];" ::"l"(a.d_targets_packed + e0 * PW));
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const uint8_t*>(a.d_step_count) + (size_t)g * (GROUP * CW)));
+    // (the counter's address is formed inside the asm, so the compiler forms it again for the load
+    // instead of keeping it live across the slide: that register is what keeps the kernel spill-free)
+    asm volatile("{ .reg .u64 p; mad.wide.u32 p, %1, %2, %0; prefetch.global.L2 [p]; }" ::"l"(a.d_step_count), "r"(g), "n"(GROUP * CW));
     ld_words<PW>(a.d_pos + e0 * PW, in.praw);
     in.walls.load(a.d_walls, cap, g);
     if constexpr (GOAL == TS_GOAL_ORDERED) ld_words<PW>(a.d_targets_packed + e0 * PW, in.traw);

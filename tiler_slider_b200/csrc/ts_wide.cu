@@ -214,9 +214,10 @@ template <int T, int GOAL, bool AR, int LW>
 __global__ void __launch_bounds__(WIDE_THREADS, WIDE_MIN_BLOCKS) wide_step_kernel(const __grid_constant__ ts_step_args a) {
     constexpr int PW = pos_bytes(T), PR = (T + 3) / 4;
     __shared__ WideSmem sm;
+    const uint32_t n = (uint32_t)a.n_envs;
     const uint32_t i = blockIdx.x * WIDE_THREADS + threadIdx.x;
-    if (i >= (uint32_t)a.n_envs) return;
-    const uint32_t env = (uint32_t)a.first_env + i;
+    if (i >= n) return;
+    const uint32_t env = (uint32_t)a.first_env + (a.order ? n - 1u - i : i);   // ts_step_args.order
     dependent_launch_sync();
     const uint32_t action = a.d_actions[env] & 3u;
     uint32_t q0[PR], q[PR];
