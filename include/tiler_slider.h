@@ -588,22 +588,33 @@ typedef struct ts_pool_reset_args {
 int ts_pool_reset(const ts_pool_reset_args *a, void *stream);
 
 /* ---------------------------------------------------------------------------------------
- * K9 ts_optimal_moves: exact distance to the goal and the set of optimal first moves of the
- * CURRENT positions of listed envs (csrc/ts_optimal.cu; no reference counterpart -- defined
+ * K9 ts_optimal_moves: exact distance to the goal, the set of optimal first moves and optionally
+ * a shortest solution of items (env id, positions), for the CURRENT positions of listed envs or
+ * for any position words (csrc/ts_optimal.cu; no reference counterpart -- defined
  * through a BFS over GameState.move, state.py:120-170, with the goal test is_won,
  * state.py:172-186, checked after every move).  Boards of size <= 8 with 1..4 tiles.  For item
- * i < n_items, env e = d_env_ids[i] (NULL: e = i), positions s = d_pos[e]:
+ * i < n_items, env e = d_env_ids[i] (NULL: e = i), positions s = d_item_pos[i * pos_bytes ..]
+ * (d_item_pos NULL: s = d_pos[e]); the env gives the walls and the goal:
  *   d_distance[i]  the fewest moves that win from s (>= 1: a state already on the goal is at 1,
  *                  through any move that leaves the tiles on the goal, one that changes nothing
  *                  included); max_steps and step counters play no part.  Otherwise
  *                  TS_OPT_UNSOLVABLE (-1) no winning state reachable (never_win: always),
  *                  TS_OPT_CUTOFF (-2) none within max_depth moves, TS_OPT_NOT_SEARCHED (-3)
  *                  the state space exceeds bitmap_words*32 bits or the slab, or e is outside
- *                  [0, capacity).
+ *                  [0, capacity), TS_OPT_BAD_STATE (-4) s is not a well-formed state of env e:
+ *                  a tile byte on no in-board free cell (a wall, off the board, >= 128) or two
+ *                  tiles on one cell (checked for every listed item, env positions included,
+ *                  before never_win and the state-space size).
  *   d_mask[i]      bit m (UP=0, DOWN=1, LEFT=2, RIGHT=3, as ts_valid_moves) set iff move m starts
  *                  a shortest solution: distance 1: m wins; else distance(succ_m(s)) ==
  *                  distance(s) - 1.  0 whenever d_distance[i] < 0.
- * Both in item order, deterministic.  One CTA per env, persistent grid drawing envs from the
+ *   d_plan         (NULL: no paths) uint8 [max_depth][n_items], step-major as ts_playout's plan:
+ *                  d_plan[k * n_items + i] for k < d_distance[i] is move k of the
+ *                  lexicographically smallest shortest solution from s (UP < DOWN < LEFT < RIGHT:
+ *                  each move the lowest bit of the mask of the state it is played from); every
+ *                  other entry, all rows of an item with d_distance[i] < 0 included, is 255.  The
+ *                  kernel writes every entry.  d_distance and d_mask do not depend on d_plan.
+ * All in item order, deterministic.  One CTA per item, persistent grid drawing items from the
  * ticket counter; visited set and optimal-state set: a shared-memory bitmap over the perfect hash
  * of K6; frontier: a ring of queue_smem states (a power of two >= 32) in shared memory, and every
  * state also in d_spill[cta][spill_per_cta] (it is read again by the backward pass), so
@@ -618,6 +629,7 @@ int ts_pool_reset(const ts_pool_reset_args *a, void *stream);
 #define TS_OPT_UNSOLVABLE (-1)
 #define TS_OPT_CUTOFF (-2)
 #define TS_OPT_NOT_SEARCHED (-3)
+#define TS_OPT_BAD_STATE (-4)
 #define TS_OPT_MAX_DEPTH 254
 typedef struct ts_optimal_moves_args {
     int32_t size, n_tiles, goal_mode, never_win;
@@ -630,6 +642,8 @@ typedef struct ts_optimal_moves_args {
     uint64_t *d_counters;
     int32_t *d_distance;
     uint8_t *d_mask;
+    const uint8_t *d_item_pos;      /* [n_items][pos_bytes] roots; NULL: the envs' positions */
+    uint8_t *d_plan;                /* [max_depth][n_items] shortest solutions; NULL: none */
 } ts_optimal_moves_args;
 int ts_optimal_moves_smem_bytes(const ts_optimal_moves_args *a);
 int ts_optimal_moves_ctas_per_sm(const ts_optimal_moves_args *a, int *ctas_per_sm, int *n_sm);

@@ -22,7 +22,7 @@ F_DONE, F_WON, F_INVALID, F_TIMEOUT, F_STALE = 1, 2, 4, 8, 16
 GOAL_ORDERED, GOAL_SET = 0, 1
 RECIPE_UNIFORM, RECIPE_WALK = 0, 1
 MAX_WALK = 65535
-OPT_UNSOLVABLE, OPT_CUTOFF, OPT_NOT_SEARCHED = -1, -2, -3
+OPT_UNSOLVABLE, OPT_CUTOFF, OPT_NOT_SEARCHED, OPT_BAD_STATE = -1, -2, -3, -4
 OPT_MAX_DEPTH = 254
 OBS_U8, OBS_BF16, OBS_F16, OBS_F32 = 0, 1, 2, 3
 PLAYOUT_PLAN, PLAYOUT_RANDOM = 0, 1
@@ -139,7 +139,8 @@ class OptimalMovesArgs(C.Structure):
                 ("n_items", _i64), ("capacity", _i64),
                 ("d_env_ids", _vp), ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp),
                 ("max_depth", _i32), ("bitmap_words", _i32), ("queue_smem", _i32), ("reserved0", _i32),
-                ("d_spill", _vp), ("spill_per_cta", _i64), ("d_counters", _vp), ("d_distance", _vp), ("d_mask", _vp)]
+                ("d_spill", _vp), ("spill_per_cta", _i64), ("d_counters", _vp), ("d_distance", _vp), ("d_mask", _vp),
+                ("d_item_pos", _vp), ("d_plan", _vp)]
 
 
 # every symbol include/tiler_slider.h declares: name -> (restype, argtypes)

@@ -667,16 +667,7 @@ class BatchedTilerSliderEnv:
                 ids = t.to(torch.int32)          # copied to the device once pos has passed its checks too
             n = ids.numel()
         if pos is not None:
-            want = (n, self.pos_bytes)
-            if not isinstance(pos, torch.Tensor) or pos.dtype != torch.uint8 or pos.dim() != 2 or pos.shape[1] != self.pos_bytes:
-                raise ValueError(f"{what}: pos must be a uint8 tensor [n, {self.pos_bytes}]")
-            if tuple(pos.shape) != want:
-                raise ValueError(f"{what}: pos has {pos.shape[0]} rows, expected {n} "
-                                 f"({'one per id' if ids is not None else 'one per env without ids'})")
-            if pos.device != self.device:
-                raise ValueError(f"{what}: pos is on {pos.device}, the batch on {self.device}")
-            if not pos.is_contiguous():
-                raise ValueError(f"{what}: pos must be contiguous")
+            check_item_pos(what, pos, n, ids is not None, self.pos_bytes, self.device)
         if ids is not None and not ids.is_cuda:
             ids = ids.to(self.device)
         return n, ids, pos
@@ -815,33 +806,53 @@ class BatchedTilerSliderEnv:
             check(self._lib.ts_valid_moves(C.byref(a), self._stream()), "ts_valid_moves")
         return mask[: self.n_envs]
 
-    def optimal_moves(self, ids=None, *, max_depth: int = 254) -> tuple[torch.Tensor, torch.Tensor]:
-        """Exact solver answers for the CURRENT positions (K9, ts_optimal_moves), as supervision for
-        imitation learning, optimality gaps, reward shaping or an exact expert policy.  Returns
-        (distance int32[n], mask uint8[n]) for every env or for `ids` (in ids order):
-          distance: the fewest steps that win from the current state (>= 1; the goal is checked after
+    def optimal_moves(self, ids=None, pos: torch.Tensor | None = None, *, max_depth: int = 254,
+                      paths: bool = False) -> tuple[torch.Tensor, ...]:
+        """Exact solver answers for items (K9, ts_optimal_moves), as supervision for imitation
+        learning, value targets, optimality gaps, reward shaping or an exact expert policy.  Items as
+        expand() takes them: ids (default every env) give the puzzles, pos (default each listed
+        env's CURRENT positions) the states to solve from; pos is a contiguous uint8 [n, pos_bytes]
+        on the batch's device (n_envs rows without ids).  Returns (distance int32[n], mask uint8[n])
+        in item order, and with paths=True also plan:
+          distance: the fewest steps that win from the item's state (>= 1; the goal is checked after
                     every move, as solve_depth; max_steps and the step counter play no part), or
                     -1 no win reachable (also every env of a never_win batch), -2 none within
                     max_depth steps, -3 this env's state space is larger than the largest bitmap
                     one CTA can hold, or than the slab of the launch (it does not depend on the
-                    other envs of the query);
+                    other items of the query), -4 the position word is not a well-formed state of
+                    its env (a tile on a wall or off the board, two tiles on one cell; e.g. the
+                    zero rows playout(record=True) writes past an item's end);
           mask:     bit a (valid_moves() order) set iff move a starts a shortest solution; 0 when
-                    distance < 0.
-        Runs on the current stream after the steps queued before it and changes no env state.
-        Sizes up to 8, 1..4 tiles, device-memory batches (not host_io)."""
+                    distance < 0;
+          plan:     uint8 [max_depth, n], step-major as playout(actions=) takes it: rows
+                    0 .. distance[i]-1 of column i hold the lexicographically smallest shortest
+                    solution of item i (UP < DOWN < LEFT < RIGHT: each move the lowest bit of the
+                    mask of the state it is played from), every other entry is 255.  So
+                    playout(ids, pos, actions=plan) wins every item with distance >= 1 in exactly
+                    distance moves.  distance and mask are the same with and without paths.
+        Ids are range-checked against [0, n_envs) (IndexError), host and device ids alike.  Runs on
+        the current stream after the steps queued before it, reads one scalar back, and changes no
+        env state.  Sizes up to 8, 1..4 tiles, device-memory batches (not host_io)."""
         from .bfs import CudaOptimalMoves, check_optimal_moves
         check_optimal_moves(self.size, self.n_tiles, self.host_io, int(max_depth))
         self._require_loaded()
         if ids is not None:
             ids = torch.as_tensor(ids).to(device=self.device, dtype=torch.int32).reshape(-1).contiguous()
-            if ids.numel():
-                lo, hi = torch.aminmax(ids)
-                lo, hi = int(lo), int(hi)
-                if lo < 0 or hi >= self.n_envs:
-                    raise IndexError(f"env ids must lie in [0, {self.n_envs}), got [{lo}, {hi}]")
+        if pos is not None:
+            check_item_pos("optimal_moves", pos, self.n_envs if ids is None else ids.numel(), ids is not None,
+                           self.pos_bytes, self.device)
+        if ids is not None and ids.numel():
+            lo, hi = torch.aminmax(ids)
+            lo, hi = int(lo), int(hi)
+            if lo < 0 or hi >= self.n_envs:
+                raise IndexError(f"env ids must lie in [0, {self.n_envs}), got [{lo}, {hi}]")
         if self._optimal is None:
             self._optimal = CudaOptimalMoves(self)
-        return self._optimal.query(ids, int(max_depth))
+        if not paths:
+            return self._optimal.query(ids, int(max_depth), pos)
+        n = self.n_envs if ids is None else ids.numel()
+        plan = torch.empty((int(max_depth), n), dtype=torch.uint8, device=self.device)
+        return (*self._optimal.query(ids, int(max_depth), pos, plan), plan)
 
     def set_positions(self, tiles) -> None:
         """Overwrite current positions from uint8[N,T,2] (row, col) -- e.g. to expand a search
@@ -861,6 +872,20 @@ class BatchedTilerSliderEnv:
         else:
             tg = [(int(c) // S, int(c) % S) for c in torch.nonzero(self.target_positions()[i]).flatten().tolist()]
         return Puzzle(S, blocked, tiles, tg, self.multi_color)
+
+
+def check_item_pos(what: str, pos, n: int, with_ids: bool, pos_bytes: int, device: torch.device) -> None:
+    """The position words of n items: a contiguous uint8 [n, pos_bytes] tensor on `device`, else
+    ValueError."""
+    if not isinstance(pos, torch.Tensor) or pos.dtype != torch.uint8 or pos.dim() != 2 or pos.shape[1] != pos_bytes:
+        raise ValueError(f"{what}: pos must be a uint8 tensor [n, {pos_bytes}]")
+    if pos.shape[0] != n:
+        raise ValueError(f"{what}: pos has {pos.shape[0]} rows, expected {n} "
+                         f"({'one per id' if with_ids else 'one per env without ids'})")
+    if pos.device != device:
+        raise ValueError(f"{what}: pos is on {pos.device}, the batch on {device}")
+    if not pos.is_contiguous():
+        raise ValueError(f"{what}: pos must be contiguous")
 
 
 def shard_range(n_total: int, rank: int, world_size: int) -> tuple[int, int]:

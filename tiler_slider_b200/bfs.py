@@ -804,7 +804,8 @@ def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int) 
 
 class CudaOptimalMoves(OnChipSearch):
     """ctypes front-end of ts_optimal_moves (K9, csrc/ts_optimal.cu) for one batch: the distance to
-    the goal and the optimal first moves of the envs' current positions.  The bitmap is sized per
+    the goal, the optimal first moves and optionally a shortest solution of items (env id, positions:
+    the env's current ones or given words).  The bitmap is sized per
     call from the most free cells among the queried envs, counted on the device (a reset pool changes
     the walls of a batch between calls), or from the most free cells one CTA can hold when that is
     fewer; the plan is cached per free-cell count."""
@@ -835,9 +836,13 @@ class CudaOptimalMoves(OnChipSearch):
             f -= 1
         return f
 
-    def query(self, ids: torch.Tensor | None, max_depth: int) -> tuple[torch.Tensor, torch.Tensor]:
-        """(distance int32[n], mask uint8[n]) of envs `ids` (int32 on the device, each in [0, n_envs);
-        None: every env), on the current stream."""
+    def query(self, ids: torch.Tensor | None, max_depth: int, pos: torch.Tensor | None = None,
+              plan: torch.Tensor | None = None) -> tuple[torch.Tensor, torch.Tensor]:
+        """(distance int32[n], mask uint8[n]) of items (env `ids[i]`, positions `pos[i]`) on the
+        current stream.  ids: int32 on the device, each in [0, n_envs) (None: every env); pos:
+        contiguous uint8 [n, pos_bytes] on the device (None: the envs' current positions); plan:
+        uint8 [max_depth, n] on the device that receives a shortest solution per item (every entry
+        is written)."""
         t, dev = self.t, self.device
         n = t.n_envs if ids is None else ids.numel()
         distance = torch.full((n,), OPT_NOT_SEARCHED, dtype=torch.int32, device=dev)
@@ -851,14 +856,20 @@ class CudaOptimalMoves(OnChipSearch):
         with torch.cuda.device(dev):
             a = self._args(n_items=n, d_env_ids=ids_ptr)
             check(self.lib.ts_optimal_max_free_cells(C.byref(a), f_max.data_ptr(), stream), "ts_optimal_max_free_cells")
-            plan = self.plan(self.fitting_free_cells(int(f_max.item())))
-            if plan is None:                     # not even T free cells fit on chip
+            # one plan with and without paths: the same grid and slab, so the same answers (the plan
+            # kernel instance may fit fewer CTAs per SM; the surplus CTAs find no ticket left)
+            sp = self.plan(self.fitting_free_cells(int(f_max.item())))
+            if sp is None:                       # not even T free cells fit on chip
+                if plan is not None:
+                    plan.fill_(255)
                 return distance, mask
-            a = self._args(n_items=n, d_env_ids=ids_ptr, max_depth=int(max_depth), bitmap_words=plan["bitmap_words"],
-                           queue_smem=plan["queue_smem"], spill_per_cta=plan["spill_per_cta"],
-                           d_spill=self._buf("spill", plan["grid"] * plan["spill_per_cta"], torch.int32).data_ptr(),
-                           d_counters=self.counters.data_ptr(), d_distance=distance.data_ptr(), d_mask=mask.data_ptr())
-            check(self.lib.ts_optimal_moves(C.byref(a), plan["grid"], stream), "ts_optimal_moves")
+            a = self._args(n_items=n, d_env_ids=ids_ptr, max_depth=int(max_depth), bitmap_words=sp["bitmap_words"],
+                           queue_smem=sp["queue_smem"], spill_per_cta=sp["spill_per_cta"],
+                           d_spill=self._buf("spill", sp["grid"] * sp["spill_per_cta"], torch.int32).data_ptr(),
+                           d_counters=self.counters.data_ptr(), d_distance=distance.data_ptr(), d_mask=mask.data_ptr(),
+                           d_item_pos=None if pos is None else pos.data_ptr(),
+                           d_plan=None if plan is None else plan.data_ptr())
+            check(self.lib.ts_optimal_moves(C.byref(a), sp["grid"], stream), "ts_optimal_moves")
         return distance, mask
 
 

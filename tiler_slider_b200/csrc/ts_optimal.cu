@@ -1,11 +1,14 @@
-// ts_optimal.cu -- K9: exact distance to the goal and the set of optimal first moves of the CURRENT
-// state of many envs, one CTA per env, on chip.  Built on K6's machinery (ts_bfs_local.cu; the CTA
-// shape, hash, plan check and launch are in ts_bfs_local.cuh): persistent CTAs drawing envs from a
+// ts_optimal.cu -- K9: exact distance to the goal and the set of optimal first moves of many items
+// (env id, positions: the env's current ones or a caller's word), one CTA per item, on chip, and
+// optionally a shortest solution per item.  Built on K6's machinery (ts_bfs_local.cu; the CTA
+// shape, hash, plan check and launch are in ts_bfs_local.cuh): persistent CTAs drawing items from a
 // ticket counter, the visited set a shared-memory bitmap over the perfect hash of a state among the
 // free cells of its puzzle, the frontier ring with a per-CTA HBM slab, the successor function
 // slide_env<S,T> and goal test of the step.
 //
-//   1. Forward: BFS from the env's positions (set goal: states canonicalised by sorting), stopped
+//   0. Root: the item's word must be a well-formed state (every tile on an in-board free cell, no
+//      two on one cell), else TS_OPT_BAD_STATE -- the hash below is only defined for those.
+//   1. Forward: BFS from the root (set goal: states canonicalised by sorting), stopped
 //      after the level in which a successor first meets the goal; that level number is d.  Every
 //      state appended is also written to the slab (the ring only holds the levels in flight), so
 //      that levels 1 .. d-1 can be read again; their boundaries stay in shared memory.
@@ -15,9 +18,14 @@
 //      successor of a level-k state lies at level <= k+1, so only level k+1's marks can be hit; the
 //      marks of level k itself must not be (a same-level successor is one step farther from the
 //      goal), so all flags of level k are computed first (written over the level's slab entries)
-//      and set after a barrier.  One bitmap serves every level without clearing.
+//      and set after a barrier.  One bitmap serves every level without clearing.  A good state's
+//      slab entry is its hash << 2 | the lowest of those moves (only levels > k are marked, so they
+//      are exactly its optimal moves); the mark loop reads entry >> 2.
 //   3. Root: d == 1: the moves that win; otherwise the moves whose successor is marked (the root is
 //      never marked, so a move that changes nothing is never optimal there).
+//   4. Plan (d_plan set): from the root, play the lowest optimal move; the state reached at level k
+//      is good, so level k's slab range holds its entry, and that entry's move is the next one.
+//      This gives the lexicographically smallest shortest solution (UP < DOWN < LEFT < RIGHT).
 // The forward pass stops at the goal level instead of enumerating the reachable set, and the
 // backward pass slides each state of levels 1 .. d-1 once more.  No reference counterpart (parity
 // unpinned; results pinned to a plain CPU BFS, tests/test_gpu_optimal.py).
@@ -28,9 +36,19 @@ namespace ts {
 constexpr uint32_t OPT_NONE = 0xFFFFFFFFu;
 constexpr uint32_t WON = 1u, OVER = 2u;
 
-template <int S, int T>
+// bitboard bit of position byte p as a mask, 0 when p is no cell of the board (so that a word of
+// T tiles is well-formed iff its T masks are distinct free cells: popcount T, all inside free_cells)
+template <int S> __device__ __forceinline__ uint64_t cell_bit(uint32_t p) {
+    if constexpr (padded_board(S)) return p < 64u ? (1ull << p) & cell_mask<S>() : 0ull;
+    else return (p >> 4) < (uint32_t)S && (p & 15u) < (uint32_t)S ? 1ull << pos_to_bit<S>(p) : 0ull;
+}
+
+// PLAN: the instance that writes d_plan (a compile-time parameter, so that the query without plans
+// carries none of the plan's code: its slab entries are bare hashes, as they were before plans)
+template <int S, int T, bool PLAN>
 __global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_optimal_moves_args a) {
     constexpr int PW = pos_bytes(T), NB = board_bytes(S);
+    constexpr uint32_t KEY_SHIFT = PLAN ? 2u : 0u;        // slab entry of a good state: hash << KEY_SHIFT | move
     static_assert(T >= 1 && T <= 4, "32-bit states");
     extern __shared__ __align__(16) uint32_t dyn[];
     uint32_t* const bitmap = dyn;
@@ -40,6 +58,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_
     __shared__ uint32_t cnt[3];                  // entries appended during level L: cnt[L % 3]
     __shared__ uint32_t lflag[3];                // ... and whether a successor met the goal (WON) / the slab overflowed (OVER)
     __shared__ long long s_ticket;
+    __shared__ uint32_t s_move;                  // plan: the move played from the current state
 
     const uint32_t tid = threadIdx.x, lane = tid & 31u;
     // ring over discovery indices as in K6: entry p is in ring[p % R] when it was appended within R of
@@ -56,23 +75,39 @@ __global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_
         __syncthreads();
         const long long ticket = s_ticket;
         if (ticket >= a.n_items) break;
+        // the item's column of the plan: row r
+        auto plan_at = [&](uint32_t r) -> uint8_t& { return a.d_plan[(size_t)r * (size_t)a.n_items + (size_t)ticket]; };
+        // no solution: distance `code`, mask 0, an all-255 plan column (every thread calls it)
+        auto no_solution = [&](int32_t code) {
+            if (tid == 0) { a.d_distance[ticket] = code; a.d_mask[ticket] = 0; }
+            if constexpr (PLAN)
+#pragma unroll 1
+                for (uint32_t r = tid; r < (uint32_t)a.max_depth; r += SEARCH_THREADS) plan_at(r) = 0xFF;
+        };
         const long long env = a.d_env_ids ? (long long)a.d_env_ids[ticket] : ticket;
-        const bool listed = env >= 0 && env < a.capacity;
-        if (!listed || a.never_win) {             // never_win: no state meets the goal
-            if (tid == 0) { a.d_distance[ticket] = listed ? TS_OPT_UNSOLVABLE : TS_OPT_NOT_SEARCHED; a.d_mask[ticket] = 0; }
-            continue;
-        }
+        if (env < 0 || env >= a.capacity) { no_solution(TS_OPT_NOT_SEARCHED); continue; }
         const size_t pid = (size_t)env;
 
-        // ---- the env: walls, goal, current state, free-cell ranks -----------------------------
+        // ---- the item: walls, goal, root state, free-cell ranks ---------------------------------
         const uint64_t walls = load_board_elem<NB>(a.d_walls, cap, pid);
+        const uint64_t free_cells = ~walls & cell_mask<S>();
+        const uint8_t* const root_pos = a.d_item_pos ? a.d_item_pos + (size_t)ticket * PW : a.d_pos + pid * PW;
+        uint32_t root = 0;
+        uint64_t occ = 0;
+        static_for<0, T>([&](auto I) {
+            constexpr int t = decltype(I)::value;
+            const uint32_t p = root_pos[t];
+            root |= p << (8 * t);
+            occ |= cell_bit<S>(p);
+        });
+        // each tile on its own free cell: an off-board byte adds no bit, two tiles on one cell one
+        if (__popcll(occ) != T || (occ & ~free_cells)) { no_solution(TS_OPT_BAD_STATE); continue; }
+        if (a.never_win) { no_solution(TS_OPT_UNSOLVABLE); continue; }   // no state meets the goal
         uint64_t tboard = 0;
-        uint32_t tq = 0, root = 0;
+        uint32_t tq = 0;
         if (a.goal_mode == TS_GOAL_SET) tboard = load_board_elem<NB>(a.d_targets_packed, cap, pid);
         else static_for<0, T>([&](auto I) { constexpr int t = decltype(I)::value; tq |= (uint32_t)a.d_targets_packed[pid * PW + t] << (8 * t); });
-        static_for<0, T>([&](auto I) { constexpr int t = decltype(I)::value; root |= (uint32_t)a.d_pos[pid * PW + t] << (8 * t); });
         if (a.goal_mode == TS_GOAL_SET) sort_bytes4<T>(root);
-        const uint64_t free_cells = ~walls & cell_mask<S>();
         const uint32_t F = (uint32_t)__popcll(free_cells);
         if (tid < 128) {
             const uint32_t bit = pos_to_bit<S>(tid);
@@ -82,10 +117,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_
 #pragma unroll
         for (int t = 0; t < T; ++t) bits *= (F > (uint32_t)t ? F - (uint32_t)t : 1u);
         const uint32_t words = (uint32_t)((bits + 31) / 32);
-        if (words > (uint32_t)a.bitmap_words) {
-            if (tid == 0) { a.d_distance[ticket] = TS_OPT_NOT_SEARCHED; a.d_mask[ticket] = 0; }
-            continue;
-        }
+        if (words > (uint32_t)a.bitmap_words) { no_solution(TS_OPT_NOT_SEARCHED); continue; }
         for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
         if (tid == 0) { cnt[0] = cnt[1] = cnt[2] = 0; lflag[0] = lflag[1] = lflag[2] = 0; }
         __syncthreads();
@@ -168,10 +200,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_
             if (flag & WON) { dist = (int32_t)depth; break; }
             if (flag & OVER) { dist = TS_OPT_NOT_SEARCHED; break; }     // slab exhausted before the goal level
         }
-        if (dist < 0) {
-            if (tid == 0) { a.d_distance[ticket] = dist; a.d_mask[ticket] = 0; }
-            continue;
-        }
+        if (dist < 0) { no_solution(dist); continue; }
 
         // ---- 2. backward: mark the states of levels d-1 .. 1 that start a shortest solution ------
         const uint32_t D = (uint32_t)dist;
@@ -195,12 +224,15 @@ __global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_
                     }
                     // the four lanes of a state are lanes 4i .. 4i+3 of one warp
                     const unsigned m = __ballot_sync(0xFFFFFFFFu, hit);
-                    if (live && (j & 3u) == 0u) slab[src] = (m >> lane) & 0xFu ? state_index<T>(lut, F, q0) : OPT_NONE;
+                    if (live && (j & 3u) == 0u) {
+                        const uint32_t hits = (m >> lane) & 0xFu;
+                        slab[src] = hits ? state_index<T>(lut, F, q0) << KEY_SHIFT | (PLAN ? (uint32_t)(__ffs(hits) - 1) : 0u) : OPT_NONE;
+                    }
                 }
                 __syncthreads();                  // every flag of level k computed
                 for (uint32_t s = l0 + tid; s < l1; s += SEARCH_THREADS) {
-                    const uint32_t idx = slab[s];
-                    if (idx != OPT_NONE) atomicOr(&bitmap[idx >> 5], 1u << (idx & 31u));
+                    const uint32_t e = slab[s];
+                    if (e != OPT_NONE) atomicOr(&bitmap[e >> (5 + KEY_SHIFT)], 1u << ((e >> KEY_SHIFT) & 31u));
                 }
                 __syncthreads();                  // level k marked
                 if (tid == 0) bwd += l1 - l0;
@@ -216,7 +248,35 @@ __global__ void __launch_bounds__(SEARCH_THREADS) optimal_moves_kernel(const ts_
                 hit = D == 1u ? won : (qn != root && marked(qn));
             }
             const unsigned m = __ballot_sync(0xFFFFFFFFu, hit);
-            if (tid == 0) { a.d_distance[ticket] = dist; a.d_mask[ticket] = (uint8_t)(m & 0xFu); }
+            if (tid == 0) {
+                a.d_distance[ticket] = dist;
+                a.d_mask[ticket] = (uint8_t)(m & 0xFu);
+                if constexpr (PLAN) s_move = (uint32_t)(__ffs(m) - 1);
+            }
+        }
+
+        // ---- 4. plan: the lowest optimal move from each state of the solution --------------------
+        if constexpr (PLAN) {
+#pragma unroll 1
+            for (uint32_t r = D + tid; r < (uint32_t)a.max_depth; r += SEARCH_THREADS) plan_at(r) = 0xFF;
+            __syncthreads();                      // s_move of the root
+            uint32_t q = root;
+            for (uint32_t k = 0;;) {
+                const uint32_t mv = s_move;
+                if (tid == 0) plan_at(k) = (uint8_t)mv;
+                if (++k == D) break;
+                bool won;
+                q = successor(q, mv, won);
+                const uint32_t key = state_index<T>(lut, F, q);
+                __syncthreads();                  // s_move read by every thread
+                // q is good at level k, appended there once: exactly one entry of the range is its own
+#pragma unroll 1
+                for (uint32_t s = lstart[k] + tid; s < lstart[k + 1u]; s += SEARCH_THREADS) {
+                    const uint32_t e = slab[s];
+                    if (e >> 2 == key) s_move = e & 3u;
+                }
+                __syncthreads();                  // s_move of q
+            }
         }
     }
     if (tid == 0) {
@@ -241,7 +301,8 @@ __global__ void max_free_cells_kernel(const ts_optimal_moves_args a, int32_t* ou
     if ((threadIdx.x & 31u) == 0u && best) atomicMax(out, (int32_t)best);
 }
 
-static constexpr auto K9 = [](auto S, auto T) { return optimal_moves_kernel<decltype(S)::value, decltype(T)::value>; };
+static constexpr auto K9 = [](auto S, auto T) { return optimal_moves_kernel<decltype(S)::value, decltype(T)::value, false>; };
+static constexpr auto K9_PLAN = [](auto S, auto T) { return optimal_moves_kernel<decltype(S)::value, decltype(T)::value, true>; };
 
 }  // namespace ts
 
@@ -272,7 +333,7 @@ int ts_optimal_moves_smem_bytes(const ts_optimal_moves_args* a) {
 
 int ts_optimal_moves_ctas_per_sm(const ts_optimal_moves_args* a, int* ctas_per_sm, int* n_sm) {
     if (int rc = optimal_check_plan(a)) return rc;
-    return search_ctas_per_sm(K9, *a, ctas_per_sm, n_sm);
+    return a->d_plan ? search_ctas_per_sm(K9_PLAN, *a, ctas_per_sm, n_sm) : search_ctas_per_sm(K9, *a, ctas_per_sm, n_sm);
 }
 
 int ts_optimal_max_free_cells(const ts_optimal_moves_args* a, int32_t* d_max_free, void* stream) {
@@ -297,7 +358,8 @@ int ts_optimal_moves(const ts_optimal_moves_args* a, int grid, void* stream) {
     if (!a->d_spill || !a->d_counters || !a->d_distance || !a->d_mask) return TS_E_NULL_POINTER;
     if (a->n_items == 0) return 0;
     if (grid < 1) return TS_E_BAD_ARGUMENT;
-    return (int)search_kernel(K9, *a, grid, nullptr, (cudaStream_t)stream);
+    return (int)(a->d_plan ? search_kernel(K9_PLAN, *a, grid, nullptr, (cudaStream_t)stream)
+                           : search_kernel(K9, *a, grid, nullptr, (cudaStream_t)stream));
 }
 
 }  // extern "C"
