@@ -651,6 +651,52 @@ int ts_optimal_max_free_cells(const ts_optimal_moves_args *a, int32_t *d_max_fre
 int ts_optimal_moves(const ts_optimal_moves_args *a, int grid, void *stream);
 
 /* ---------------------------------------------------------------------------------------
+ * K10 ts_state_table: every state reachable from items (env id, positions), each with K9's
+ * distance and optimal-move mask (csrc/ts_state_table.cu; no reference counterpart).  Items,
+ * domain and root check as K9 (size <= 8, 1..4 tiles; env e = d_env_ids[i] (NULL: e = i), root
+ * d_item_pos[i * pos_bytes ..] (NULL: d_pos[e])).  Two launches with the same arguments and grid:
+ *   ts_state_table_count  forward BFS from each root to exhaustion:
+ *     d_status[i]   0 enumerated; TS_OPT_NOT_SEARCHED (-3) the state space exceeds
+ *                   bitmap_words*32 bits, the reachable set exceeds spill_per_cta states (the
+ *                   slab the ring spills to), or e is outside [0, capacity); TS_OPT_BAD_STATE (-4)
+ *                   the root is not a well-formed state (K9's rule)
+ *     d_count[i]    int64: the states reachable from the root, the root included (0 if status != 0)
+ *     d_counters    [0] ticket (zero on entry)
+ *   the caller sets d_offsets (int64 [n_items + 1]) to the exclusive cumsum of d_count, then
+ *   ts_state_table_fill   for each item with status 0 (the others are skipped), rows
+ *     [d_offsets[i], d_offsets[i+1]) of:
+ *     d_rows        uint8 [rows][pos_bytes]: each reachable state exactly once (set goal: canonical,
+ *                   bytes ascending; padding bytes 0), in ascending order of the perfect hash
+ *                   the bitmap is keyed by (deterministic); the rows also serve as the BFS queue
+ *     d_distance    int32 [rows]: K9's distance of the row's state (>= 1), or -1 if no win is
+ *                   reachable from it (never_win: every row)
+ *     d_mask        uint8 [rows]: K9's mask of the row's state (0 where distance < 0)
+ *     d_counters    [1] ticket (zero on entry), [2] += rows swept by the retrograde rounds
+ * ts_state_table_ctas_per_sm: resident CTAs per SM of both kernels (the fewer) and the SM count.
+ * ts_optimal_max_free_cells sizes bitmap_words for these launches as for K9.
+ * ------------------------------------------------------------------------------------- */
+typedef struct ts_state_table_args {
+    int32_t size, n_tiles, goal_mode, never_win;
+    int64_t n_items, capacity;
+    const int32_t *d_env_ids;
+    const uint8_t *d_walls, *d_targets_packed, *d_pos;
+    const uint8_t *d_item_pos;      /* [n_items][pos_bytes] roots; NULL: the envs' positions */
+    int32_t bitmap_words, queue_smem;
+    uint32_t *d_spill;              /* count pass: [grid][spill_per_cta] */
+    int64_t spill_per_cta;
+    uint64_t *d_counters;
+    int64_t *d_count;               /* count pass output */
+    int32_t *d_status;              /* count pass output, fill pass input */
+    const int64_t *d_offsets;       /* fill pass input */
+    uint8_t *d_rows;                /* fill pass outputs */
+    int32_t *d_distance;
+    uint8_t *d_mask;
+} ts_state_table_args;
+int ts_state_table_ctas_per_sm(const ts_state_table_args *a, int *ctas_per_sm, int *n_sm);
+int ts_state_table_count(const ts_state_table_args *a, int grid, void *stream);
+int ts_state_table_fill(const ts_state_table_args *a, int grid, void *stream);
+
+/* ---------------------------------------------------------------------------------------
  * ts_step_host: the same step through HOST buffers (the call a host-side driver makes):
  * h_actions (pinned) -> device, ts_step, reward/done -> h_reward/h_done (pinned), pipelined in
  * chunks over the context's streams; returns after everything has landed.

@@ -14,11 +14,11 @@ include/tiler_slider.h); there is no CPU fallback.
 from ._lib import (F_DONE, F_INVALID, F_STALE, F_TIMEOUT, F_WON, GOAL_ORDERED, GOAL_SET, TilerSliderError, build, lib)
 from .moves import Move
 from .puzzle import Puzzle, load_puzzle_file, parse_board_text, parse_puzzle_file_text, puzzle_to_text
-from .batch_env import DEFAULT_REWARDS, BatchedTilerSliderEnv, shard_range
+from .batch_env import DEFAULT_REWARDS, BatchedTilerSliderEnv, StateTable, shard_range
 from .env import GameState, TilerSliderEnv, TilerSliderEnvFactory
 
 __version__ = "0.2.0"
-__all__ = ["GameState", "TilerSliderEnv", "TilerSliderEnvFactory", "Move", "BatchedTilerSliderEnv", "Puzzle",
+__all__ = ["GameState", "TilerSliderEnv", "TilerSliderEnvFactory", "Move", "BatchedTilerSliderEnv", "StateTable", "Puzzle",
            "parse_board_text", "parse_puzzle_file_text", "load_puzzle_file", "puzzle_to_text", "shard_range",
            "DEFAULT_REWARDS", "TilerSliderError", "build", "lib",
            "F_DONE", "F_WON", "F_INVALID", "F_TIMEOUT", "F_STALE", "GOAL_ORDERED", "GOAL_SET"]

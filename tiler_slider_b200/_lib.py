@@ -143,6 +143,15 @@ class OptimalMovesArgs(C.Structure):
                 ("d_item_pos", _vp), ("d_plan", _vp)]
 
 
+class StateTableArgs(C.Structure):
+    _fields_ = [("size", _i32), ("n_tiles", _i32), ("goal_mode", _i32), ("never_win", _i32),
+                ("n_items", _i64), ("capacity", _i64),
+                ("d_env_ids", _vp), ("d_walls", _vp), ("d_targets_packed", _vp), ("d_pos", _vp), ("d_item_pos", _vp),
+                ("bitmap_words", _i32), ("queue_smem", _i32), ("d_spill", _vp), ("spill_per_cta", _i64),
+                ("d_counters", _vp), ("d_count", _vp), ("d_status", _vp), ("d_offsets", _vp),
+                ("d_rows", _vp), ("d_distance", _vp), ("d_mask", _vp)]
+
+
 # every symbol include/tiler_slider.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "ts_version": (C.c_int, []),
@@ -186,6 +195,9 @@ SYMBOLS = {
     "ts_optimal_moves_ctas_per_sm": (C.c_int, [C.POINTER(OptimalMovesArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_optimal_max_free_cells": (C.c_int, [C.POINTER(OptimalMovesArgs), _vp, _vp]),
     "ts_optimal_moves": (C.c_int, [C.POINTER(OptimalMovesArgs), C.c_int, _vp]),
+    "ts_state_table_ctas_per_sm": (C.c_int, [C.POINTER(StateTableArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ts_state_table_count": (C.c_int, [C.POINTER(StateTableArgs), C.c_int, _vp]),
+    "ts_state_table_fill": (C.c_int, [C.POINTER(StateTableArgs), C.c_int, _vp]),
     "ts_host_ctx_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "ts_host_ctx_destroy": (C.c_int, [_vp]),
     "ts_step_host": (C.c_int, [_vp, C.POINTER(StepArgs), _vp, _vp, _vp, _vp, _i64]),

@@ -11,13 +11,14 @@ Packed state (see include/tiler_slider.h): `pos` is uint8[N, pos_bytes(T)], byte
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 from typing import Sequence
 
 import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (CAP_ALIGN, F_WON, GOAL_ORDERED, GOAL_SET, MAX_SIZE, MAX_TILES, OBS_BF16, OBS_F16, OBS_F32, OBS_U8,
+from ._lib import (CAP_ALIGN, F_WON, GOAL_ORDERED, GOAL_SET, MAX_SIZE, MAX_TILES, OBS_BF16, OBS_F16, OBS_F32, OBS_U8, OPT_MAX_DEPTH,
                    PLAYOUT_PLAN, PLAYOUT_RANDOM, EncodeArgs, ExpandArgs, GoalArgs, ObserveArgs, ObservePlanesArgs, PlayoutArgs,
                    PoolResetArgs, StepArgs, SynthArgs, ValidArgs, check, lib)
 from .puzzle import Puzzle, as_puzzle, uniform_shape
@@ -118,6 +119,7 @@ class BatchedTilerSliderEnv:
         self._episodes = None         # uint32 per env: puzzles drawn from a pool so far
         self._solve_depth = None      # int32 per env: shortest solution of the current puzzle (-1: not known)
         self._optimal = None          # optimal_moves(): the K9 driver (plans and scratch)
+        self._state_table = None      # state_table(): the K10 driver
 
     # ------------------------------------------------------------------ construction
     @classmethod
@@ -836,16 +838,7 @@ class BatchedTilerSliderEnv:
         from .bfs import CudaOptimalMoves, check_optimal_moves
         check_optimal_moves(self.size, self.n_tiles, self.host_io, int(max_depth))
         self._require_loaded()
-        if ids is not None:
-            ids = torch.as_tensor(ids).to(device=self.device, dtype=torch.int32).reshape(-1).contiguous()
-        if pos is not None:
-            check_item_pos("optimal_moves", pos, self.n_envs if ids is None else ids.numel(), ids is not None,
-                           self.pos_bytes, self.device)
-        if ids is not None and ids.numel():
-            lo, hi = torch.aminmax(ids)
-            lo, hi = int(lo), int(hi)
-            if lo < 0 or hi >= self.n_envs:
-                raise IndexError(f"env ids must lie in [0, {self.n_envs}), got [{lo}, {hi}]")
+        ids = self._search_items("optimal_moves", ids, pos)
         if self._optimal is None:
             self._optimal = CudaOptimalMoves(self)
         if not paths:
@@ -853,6 +846,47 @@ class BatchedTilerSliderEnv:
         n = self.n_envs if ids is None else ids.numel()
         plan = torch.empty((int(max_depth), n), dtype=torch.uint8, device=self.device)
         return (*self._optimal.query(ids, int(max_depth), pos, plan), plan)
+
+    def state_table(self, ids=None, pos: torch.Tensor | None = None) -> StateTable:
+        """Every state reachable from items, each with its exact distance to a win and its optimal
+        moves (K10, ts_state_table), for value / policy datasets over whole state spaces, reverse
+        curricula (states a chosen distance from the goal) and puzzle statistics (dead states, the
+        distance histogram).  Items as optimal_moves() takes them: ids (default every env) give the
+        walls and the goal, row i of pos (default each listed env's CURRENT positions) the root.
+        Returns a StateTable: item i owns rows offsets[i] .. offsets[i+1]-1, which hold every state
+        reachable from its root, the root included, each once, in ascending order of the perfect
+        hash the search keys states by (so the table is the same from call to call); set-goal
+        batches store the canonical word (bytes ascending).  distance and mask of a row are what
+        optimal_moves(ids=..., pos=row) answers for it (max_depth plays no part: every finite
+        distance is found), -1 and 0 where no win is reachable (every row of a never_win batch).
+        status[i] is 0, or -3 (the item's state space is larger than the largest bitmap one CTA can
+        hold) or -4 (a malformed root, as optimal_moves() reports it); such items own no rows.
+        Ids are range-checked as in optimal_moves() (IndexError).  Runs on the current stream,
+        changes no env state and reads back two scalars (the free-cell maximum and the row count,
+        to allocate), so it cannot be captured in a CUDA graph.  Sizes up to 8, 1..4 tiles,
+        device-memory batches (not host_io)."""
+        from .bfs import CudaStateTable, check_optimal_moves
+        check_optimal_moves(self.size, self.n_tiles, self.host_io, OPT_MAX_DEPTH, "state_table")
+        self._require_loaded()
+        ids = self._search_items("state_table", ids, pos)
+        if self._state_table is None:
+            self._state_table = CudaStateTable(self)
+        return StateTable(*self._state_table.build(ids, pos))
+
+    def _search_items(self, what: str, ids, pos: torch.Tensor | None) -> torch.Tensor | None:
+        """The ids of a solver query as int32 on the device (None: every env), range-checked against
+        [0, n_envs) (IndexError), and its pos validated (ValueError)."""
+        if ids is not None:
+            ids = torch.as_tensor(ids).to(device=self.device, dtype=torch.int32).reshape(-1).contiguous()
+        if pos is not None:
+            check_item_pos(what, pos, self.n_envs if ids is None else ids.numel(), ids is not None,
+                           self.pos_bytes, self.device)
+        if ids is not None and ids.numel():
+            lo, hi = torch.aminmax(ids)
+            lo, hi = int(lo), int(hi)
+            if lo < 0 or hi >= self.n_envs:
+                raise IndexError(f"env ids must lie in [0, {self.n_envs}), got [{lo}, {hi}]")
+        return ids
 
     def set_positions(self, tiles) -> None:
         """Overwrite current positions from uint8[N,T,2] (row, col) -- e.g. to expand a search
@@ -872,6 +906,22 @@ class BatchedTilerSliderEnv:
         else:
             tg = [(int(c) // S, int(c) % S) for c in torch.nonzero(self.target_positions()[i]).flatten().tolist()]
         return Puzzle(S, blocked, tiles, tg, self.multi_color)
+
+
+@dataclass(frozen=True)
+class StateTable:
+    """The states reachable from items with their exact labels (BatchedTilerSliderEnv.state_table):
+    item i owns rows offsets[i] .. offsets[i+1]-1 of pos / distance / mask.
+      offsets   int64 [n+1]
+      status    int32 [n]: 0 enumerated, -3 the state space does not fit one CTA, -4 malformed root
+      pos       uint8 [M, pos_bytes]: the states, ascending by the search's perfect hash per item
+      distance  int32 [M]: fewest moves that win (>= 1), -1 if no win is reachable
+      mask      uint8 [M]: bit a set iff move a starts a shortest solution (0 where distance < 0)"""
+    offsets: torch.Tensor
+    status: torch.Tensor
+    pos: torch.Tensor
+    distance: torch.Tensor
+    mask: torch.Tensor
 
 
 def check_item_pos(what: str, pos, n: int, with_ids: bool, pos_bytes: int, device: torch.device) -> None:

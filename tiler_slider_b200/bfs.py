@@ -27,7 +27,9 @@ Two searches, same results (states per puzzle, level histogram, solve depths, sh
   keys) and walks the chains back from the recorded last link of every solution.
 `solve_batch` picks the search that fits a batch.  `CudaOptimalMoves` (K9, csrc/ts_optimal.cu) is
 K6's sibling for the envs of a batch as they stand: the distance of their current positions to a win
-and the moves that start a shortest solution (BatchedTilerSliderEnv.optimal_moves).
+and the moves that start a shortest solution (BatchedTilerSliderEnv.optimal_moves).  `CudaStateTable`
+(K10, csrc/ts_state_table.cu) enumerates every state reachable from items and labels each with K9's
+answer (BatchedTilerSliderEnv.state_table).
 
 The device kernels sit behind `CudaBfsKernels`; tests run the same driver logic on CPU
 tensors over gloo with a CPU stand-in for the kernels (tests/test_bfs_gloo.py).
@@ -42,7 +44,7 @@ from typing import Sequence
 import torch
 import torch.distributed as dist
 
-from ._lib import OPT_MAX_DEPTH, OPT_NOT_SEARCHED, BfsArgs, BfsLocalArgs, OptimalMovesArgs, check, lib
+from ._lib import OPT_MAX_DEPTH, OPT_NOT_SEARCHED, BfsArgs, BfsLocalArgs, OptimalMovesArgs, StateTableArgs, check, lib
 from .batch_env import BatchedTilerSliderEnv, shard_range
 from .puzzle import Puzzle
 
@@ -713,6 +715,28 @@ class OnChipSearch:
         self._plans[key] = plan or {}
         return plan
 
+    def fitting_free_cells(self, f_max: int) -> int:
+        """The largest F <= f_max whose plan fits (down to F = n_tiles): the free-cell count a launch
+        for envs of up to f_max free cells is planned for (K9, K10: plans keyed by free cells).  The
+        kernel reports -3 for each env whose own state space exceeds that bitmap, so an env's answer
+        never depends on the other envs."""
+        f = f_max
+        while f > self.t.n_tiles and self._plan(f, f) is None:
+            f -= 1
+        return f
+
+    def _max_free_cells(self, ids: torch.Tensor | None, n: int) -> int:
+        """The most free cells among the envs of n items (ts_optimal_max_free_cells; one read-back)."""
+        t, dev = self.t, self.device
+        f_max = torch.zeros(1, dtype=torch.int32, device=dev)
+        a = OptimalMovesArgs(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win), n_items=n,
+                             capacity=t.capacity, d_env_ids=None if ids is None else ids.data_ptr(),
+                             d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(), d_pos=t._pos.data_ptr())
+        with torch.cuda.device(dev):
+            check(self.lib.ts_optimal_max_free_cells(C.byref(a), f_max.data_ptr(), torch.cuda.current_stream(dev).cuda_stream),
+                  "ts_optimal_max_free_cells")
+        return int(f_max.item())
+
     def _buf(self, name: str, n: int, dtype) -> torch.Tensor:
         b = self._scratch.get(name)
         if b is None or b.numel() < n or b.dtype != dtype:
@@ -790,14 +814,15 @@ class CudaLocalKernels(OnChipSearch):
             check(self.lib.ts_bfs_local(C.byref(a), plan["grid"], torch.cuda.current_stream(dev).cuda_stream), "ts_bfs_local")
 
 
-def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int) -> None:
-    """The shapes ts_optimal_moves covers; raised before anything touches the device."""
+def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int, what: str = "optimal_moves") -> None:
+    """The shapes ts_optimal_moves (and ts_state_table, `what`) covers; raised before anything
+    touches the device."""
     if size > 8:
-        raise ValueError(f"optimal_moves covers board sizes up to 8 (got {size})")
+        raise ValueError(f"{what} covers board sizes up to 8 (got {size})")
     if not 1 <= n_tiles <= 4:
-        raise ValueError(f"optimal_moves covers 1 to 4 tiles (got {n_tiles})")
+        raise ValueError(f"{what} covers 1 to 4 tiles (got {n_tiles})")
     if host_io:
-        raise ValueError("optimal_moves is not available for host_io batches")
+        raise ValueError(f"{what} is not available for host_io batches")
     if not 1 <= max_depth <= OPT_MAX_DEPTH:
         raise ValueError(f"max_depth {max_depth} outside 1..{OPT_MAX_DEPTH}")
 
@@ -827,15 +852,6 @@ class CudaOptimalMoves(OnChipSearch):
         """The plan for states on up to f_max free cells."""
         return self._plan(f_max, f_max)
 
-    def fitting_free_cells(self, f_max: int) -> int:
-        """The largest F <= f_max whose plan fits (down to F = n_tiles): the free-cell count a launch
-        for envs of up to f_max free cells is planned for.  The kernel reports -3 for each env whose
-        own state space exceeds that bitmap, so an env's answer never depends on the other envs."""
-        f = f_max
-        while f > self.t.n_tiles and self.plan(f) is None:
-            f -= 1
-        return f
-
     def query(self, ids: torch.Tensor | None, max_depth: int, pos: torch.Tensor | None = None,
               plan: torch.Tensor | None = None) -> tuple[torch.Tensor, torch.Tensor]:
         """(distance int32[n], mask uint8[n]) of items (env `ids[i]`, positions `pos[i]`) on the
@@ -852,13 +868,10 @@ class CudaOptimalMoves(OnChipSearch):
             return distance, mask
         ids_ptr = None if ids is None else ids.data_ptr()
         stream = torch.cuda.current_stream(dev).cuda_stream
-        f_max = torch.zeros(1, dtype=torch.int32, device=dev)
         with torch.cuda.device(dev):
-            a = self._args(n_items=n, d_env_ids=ids_ptr)
-            check(self.lib.ts_optimal_max_free_cells(C.byref(a), f_max.data_ptr(), stream), "ts_optimal_max_free_cells")
             # one plan with and without paths: the same grid and slab, so the same answers (the plan
             # kernel instance may fit fewer CTAs per SM; the surplus CTAs find no ticket left)
-            sp = self.plan(self.fitting_free_cells(int(f_max.item())))
+            sp = self.plan(self.fitting_free_cells(self._max_free_cells(ids, n)))
             if sp is None:                       # not even T free cells fit on chip
                 if plan is not None:
                     plan.fill_(255)
@@ -871,6 +884,67 @@ class CudaOptimalMoves(OnChipSearch):
                            d_plan=None if plan is None else plan.data_ptr())
             check(self.lib.ts_optimal_moves(C.byref(a), sp["grid"], stream), "ts_optimal_moves")
         return distance, mask
+
+
+class CudaStateTable(OnChipSearch):
+    """ctypes front-end of ts_state_table_count / ts_state_table_fill (K10, csrc/ts_state_table.cu)
+    for one batch: every state reachable from items (env id, positions), each with K9's distance
+    and mask.  Planned per call as CudaOptimalMoves.query plans (the most free cells among the
+    queried envs); both launches share the plan, so they agree on the items that fit."""
+
+    CTAS_PER_SM = "ts_state_table_ctas_per_sm"
+
+    def __init__(self, env: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
+        super().__init__(env, ctas_per_sm, queue_smem)
+        self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)   # of the last call: see include/tiler_slider.h
+
+    def _args(self, **kw) -> StateTableArgs:
+        t = self.t
+        base = dict(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win), capacity=t.capacity,
+                    d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(), d_pos=t._pos.data_ptr())
+        base.update(kw)
+        return StateTableArgs(**base)
+
+    def plan(self, f_max: int) -> dict | None:
+        """The plan for states on up to f_max free cells."""
+        return self._plan(f_max, f_max)
+
+    def build(self, ids: torch.Tensor | None, pos: torch.Tensor | None = None) -> tuple[torch.Tensor, ...]:
+        """(offsets int64[n+1], status int32[n], pos uint8[M, pos_bytes], distance int32[M], mask
+        uint8[M]) of items (env `ids[i]`, root `pos[i]`) on the current stream; ids: int32 on the
+        device, each in [0, n_envs) (None: every env); pos: contiguous uint8 [n, pos_bytes] on the
+        device (None: the envs' current positions).  Reads back the free-cell maximum and the row
+        count."""
+        t, dev = self.t, self.device
+        n = t.n_envs if ids is None else ids.numel()
+        offsets = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+        status = torch.full((n,), OPT_NOT_SEARCHED, dtype=torch.int32, device=dev)
+        self.counters.zero_()
+        sp = self.plan(self.fitting_free_cells(self._max_free_cells(ids, n))) if n else None
+        if sp is None:                           # no items, or not even T free cells fit on chip
+            return (offsets, status, torch.empty((0, t.pos_bytes), dtype=torch.uint8, device=dev),
+                    torch.empty(0, dtype=torch.int32, device=dev), torch.empty(0, dtype=torch.uint8, device=dev))
+        count = torch.empty(n, dtype=torch.int64, device=dev)
+        # the count pass's slab (grid x spill_per_cta words, ~0.9 GB at the benchmark shape) lives for
+        # this call only: it goes back to the allocator's cache on return, for the rows or K9's slab
+        spill = torch.empty(sp["grid"] * sp["spill_per_cta"], dtype=torch.int32, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        a = self._args(n_items=n, d_env_ids=None if ids is None else ids.data_ptr(),
+                       d_item_pos=None if pos is None else pos.data_ptr(), bitmap_words=sp["bitmap_words"],
+                       queue_smem=sp["queue_smem"], spill_per_cta=sp["spill_per_cta"],
+                       d_spill=spill.data_ptr(), d_counters=self.counters.data_ptr(), d_count=count.data_ptr(),
+                       d_status=status.data_ptr())
+        with torch.cuda.device(dev):
+            check(self.lib.ts_state_table_count(C.byref(a), sp["grid"], stream), "ts_state_table_count")
+            torch.cumsum(count, 0, out=offsets[1:])
+            total = int(offsets[-1].item())
+            rows = torch.empty((total, t.pos_bytes), dtype=torch.uint8, device=dev)
+            distance = torch.empty(total, dtype=torch.int32, device=dev)
+            mask = torch.empty(total, dtype=torch.uint8, device=dev)
+            if total:
+                a.d_offsets, a.d_rows, a.d_distance, a.d_mask = offsets.data_ptr(), rows.data_ptr(), distance.data_ptr(), mask.data_ptr()
+                check(self.lib.ts_state_table_fill(C.byref(a), sp["grid"], stream), "ts_state_table_fill")
+        return offsets, status, rows, distance, mask
 
 
 class LocalBfs:

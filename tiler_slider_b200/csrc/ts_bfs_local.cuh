@@ -1,6 +1,6 @@
-// ts_bfs_local.cuh -- what the two on-chip searches, K6 (ts_bfs_local.cu, the batched BFS) and K9
-// (ts_optimal.cu, the optimal-move query), share: the CTA shape, canonical set-goal states, position
-// byte -> bitboard bit, the perfect hash of a state over the free cells of its puzzle that keys the
+// ts_bfs_local.cuh -- what the on-chip searches, K6 (ts_bfs_local.cu, the batched BFS), K9
+// (ts_optimal.cu, the optimal-move query) and K10 (ts_state_table.cu, the state tables), share: the
+// CTA shape, canonical set-goal states, position byte -> bitboard bit, the perfect hash of a state over the free cells of its puzzle that keys the
 // shared-memory bitmap, and on the host the plan check, the shared-memory size and the launch.
 #pragma once
 #include "ts_common.cuh"
@@ -40,6 +40,12 @@ template <int S> __host__ __device__ constexpr uint64_t cell_mask() {
     for (int r = 0; r < S; ++r)
         for (int c = 0; c < S; ++c) m |= 1ull << (r * board_stride(S) + c);
     return m;
+}
+// bitboard bit of position byte p as a mask, 0 when p is no cell of the board (so that a word of
+// T tiles is well-formed iff its T masks are distinct free cells: popcount T, all inside free_cells)
+template <int S> __device__ __forceinline__ uint64_t cell_bit(uint32_t p) {
+    if constexpr (padded_board(S)) return p < 64u ? (1ull << p) & cell_mask<S>() : 0ull;
+    else return (p >> 4) < (uint32_t)S && (p & 15u) < (uint32_t)S ? 1ull << pos_to_bit<S>(p) : 0ull;
 }
 
 // perfect hash of a state: its tiles stand on DISTINCT free cells, so digit i = rank of tile i

@@ -36,13 +36,6 @@ namespace ts {
 constexpr uint32_t OPT_NONE = 0xFFFFFFFFu;
 constexpr uint32_t WON = 1u, OVER = 2u;
 
-// bitboard bit of position byte p as a mask, 0 when p is no cell of the board (so that a word of
-// T tiles is well-formed iff its T masks are distinct free cells: popcount T, all inside free_cells)
-template <int S> __device__ __forceinline__ uint64_t cell_bit(uint32_t p) {
-    if constexpr (padded_board(S)) return p < 64u ? (1ull << p) & cell_mask<S>() : 0ull;
-    else return (p >> 4) < (uint32_t)S && (p & 15u) < (uint32_t)S ? 1ull << pos_to_bit<S>(p) : 0ull;
-}
-
 // PLAN: the instance that writes d_plan (a compile-time parameter, so that the query without plans
 // carries none of the plan's code: its slab entries are bare hashes, as they were before plans)
 template <int S, int T, bool PLAN>
