@@ -530,6 +530,23 @@ int ts_bfs_local_ctas_per_sm(const ts_bfs_local_args *a, int *ctas_per_sm, int *
 int ts_bfs_local(const ts_bfs_local_args *a, int grid, void *stream);
 
 /* ---------------------------------------------------------------------------------------
+ * Device-memory bitmaps (K6 here, K9 and K10 below).  With four tiles the bitmap of a board of
+ * more than 38 free cells does not fit one CTA's shared memory; only 7x7 and 8x8 boards have that
+ * many (up to 64*63*62*61 bits = 1.9 MB).  The *_gmem entry points run the same search with the
+ * bitmap in device memory: CTA b's bitmap is d_bitmap[b * bitmap_words ..], so d_bitmap holds
+ * grid * bitmap_words words and is 16-byte aligned; its contents on entry do not matter and are
+ * left undefined.  Dynamic shared memory holds the ring alone (queue_smem * 4 bytes).  Same
+ * arguments and results as the shared counterpart, as if shared memory were large enough.
+ * Argument checks: every check of the shared counterpart with the same code, in the same order;
+ * then TS_E_UNSUPPORTED unless (size, n_tiles) is (7, 4) or (8, 4), TS_E_NULL_POINTER for a NULL
+ * d_bitmap, TS_E_MISALIGNED for a misaligned one; all before the empty-batch return.
+ * *_gmem_ctas_per_sm: resident CTAs per SM of the device instance and the SM count (the shape is
+ * checked after the shared query's checks).
+ * ------------------------------------------------------------------------------------- */
+int ts_bfs_local_gmem_ctas_per_sm(const ts_bfs_local_args *a, int *ctas_per_sm, int *n_sm);
+int ts_bfs_local_gmem(const ts_bfs_local_args *a, uint32_t *d_bitmap, int grid, void *stream);
+
+/* ---------------------------------------------------------------------------------------
  * K7 ts_synth_candidates: candidate puzzles for a generator that keeps the ones K6 grades into a
  * band of shortest-solution lengths (csrc/ts_generate.cu; no reference counterpart).  One thread
  * per listed env: puzzle of env slot d_env_ids[i] (i < n_items; NULL: slot i; ids outside
@@ -649,6 +666,9 @@ int ts_optimal_moves_smem_bytes(const ts_optimal_moves_args *a);
 int ts_optimal_moves_ctas_per_sm(const ts_optimal_moves_args *a, int *ctas_per_sm, int *n_sm);
 int ts_optimal_max_free_cells(const ts_optimal_moves_args *a, int32_t *d_max_free, void *stream);
 int ts_optimal_moves(const ts_optimal_moves_args *a, int grid, void *stream);
+/* device-memory bitmap (see ts_bfs_local_gmem): the instance with plans when d_plan is set */
+int ts_optimal_moves_gmem_ctas_per_sm(const ts_optimal_moves_args *a, int *ctas_per_sm, int *n_sm);
+int ts_optimal_moves_gmem(const ts_optimal_moves_args *a, uint32_t *d_bitmap, int grid, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * K10 ts_state_table: every state reachable from items (env id, positions), each with K9's
@@ -695,6 +715,11 @@ typedef struct ts_state_table_args {
 int ts_state_table_ctas_per_sm(const ts_state_table_args *a, int *ctas_per_sm, int *n_sm);
 int ts_state_table_count(const ts_state_table_args *a, int grid, void *stream);
 int ts_state_table_fill(const ts_state_table_args *a, int grid, void *stream);
+/* device-memory bitmap (see ts_bfs_local_gmem): both passes of a table take the same plan, grid
+ * and d_bitmap; ts_state_table_gmem_ctas_per_sm gives the fewer CTAs per SM of the two */
+int ts_state_table_gmem_ctas_per_sm(const ts_state_table_args *a, int *ctas_per_sm, int *n_sm);
+int ts_state_table_count_gmem(const ts_state_table_args *a, uint32_t *d_bitmap, int grid, void *stream);
+int ts_state_table_fill_gmem(const ts_state_table_args *a, uint32_t *d_bitmap, int grid, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * ts_step_host: the same step through HOST buffers (the call a host-side driver makes):

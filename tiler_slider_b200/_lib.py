@@ -189,15 +189,22 @@ SYMBOLS = {
     "ts_bfs_local_smem_bytes": (C.c_int, [C.POINTER(BfsLocalArgs)]),
     "ts_bfs_local_ctas_per_sm": (C.c_int, [C.POINTER(BfsLocalArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_bfs_local": (C.c_int, [C.POINTER(BfsLocalArgs), C.c_int, _vp]),
+    "ts_bfs_local_gmem_ctas_per_sm": (C.c_int, [C.POINTER(BfsLocalArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ts_bfs_local_gmem": (C.c_int, [C.POINTER(BfsLocalArgs), _vp, C.c_int, _vp]),
     "ts_synth_candidates": (C.c_int, [C.POINTER(SynthCandidatesArgs), _vp]),
     "ts_pool_reset": (C.c_int, [C.POINTER(PoolResetArgs), _vp]),
     "ts_optimal_moves_smem_bytes": (C.c_int, [C.POINTER(OptimalMovesArgs)]),
     "ts_optimal_moves_ctas_per_sm": (C.c_int, [C.POINTER(OptimalMovesArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_optimal_max_free_cells": (C.c_int, [C.POINTER(OptimalMovesArgs), _vp, _vp]),
     "ts_optimal_moves": (C.c_int, [C.POINTER(OptimalMovesArgs), C.c_int, _vp]),
+    "ts_optimal_moves_gmem_ctas_per_sm": (C.c_int, [C.POINTER(OptimalMovesArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ts_optimal_moves_gmem": (C.c_int, [C.POINTER(OptimalMovesArgs), _vp, C.c_int, _vp]),
     "ts_state_table_ctas_per_sm": (C.c_int, [C.POINTER(StateTableArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_state_table_count": (C.c_int, [C.POINTER(StateTableArgs), C.c_int, _vp]),
     "ts_state_table_fill": (C.c_int, [C.POINTER(StateTableArgs), C.c_int, _vp]),
+    "ts_state_table_gmem_ctas_per_sm": (C.c_int, [C.POINTER(StateTableArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ts_state_table_count_gmem": (C.c_int, [C.POINTER(StateTableArgs), _vp, C.c_int, _vp]),
+    "ts_state_table_fill_gmem": (C.c_int, [C.POINTER(StateTableArgs), _vp, C.c_int, _vp]),
     "ts_host_ctx_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "ts_host_ctx_destroy": (C.c_int, [_vp]),
     "ts_step_host": (C.c_int, [_vp, C.POINTER(StepArgs), _vp, _vp, _vp, _vp, _i64]),

@@ -173,17 +173,22 @@ class BatchedTilerSliderEnv:
     @classmethod
     def solvable(cls, n_envs: int, size: int, n_tiles: int, n_walls: int, multi_color: bool = False, *,
                  min_depth: int = 1, max_depth: int = 30, recipe: str = "walk", walk_len: int | None = None,
-                 seed: int = 0, env_index_base: int = 0, max_attempts: int | None = None, **kw) -> "BatchedTilerSliderEnv":
+                 seed: int = 0, env_index_base: int = 0, max_attempts: int | None = None, device_bitmap: bool = False,
+                 **kw) -> "BatchedTilerSliderEnv":
         """Solvable puzzles whose shortest solution takes between `min_depth` and `max_depth` steps,
         generated and graded on the device (K7 candidates, K6 search; tiler_slider_b200/generate.py).
         `solve_depth` holds each env's shortest-solution length.  recipe "walk": targets where a
         random walk of `walk_len` (default max(8, 2 * max_depth)) state-changing moves leaves the
         tiles; "uniform": synthetic()'s draw, redrawn until it lands in the band.  Env i's puzzle
-        depends on (seed, recipe, walk_len, band, env_index_base + i) only.  Sizes up to 8, 1..4 tiles."""
+        depends on (seed, recipe, walk_len, band, env_index_base + i) only.  Sizes up to 8, 1..4 tiles.
+        A 7x7 board with four tiles and fewer than 11 walls, or an 8x8 one with fewer than 26, has a
+        state space too large for the shared-memory bitmap of the grading search: ValueError, unless
+        device_bitmap=True, which grades such boards with the bitmap in device memory."""
         from .generate import DEFAULT_MAX_ATTEMPTS, solvable
         return solvable(cls, n_envs, size, n_tiles, n_walls, multi_color, min_depth=min_depth, max_depth=max_depth,
                         recipe=recipe, walk_len=walk_len, seed=seed, env_index_base=env_index_base,
-                        max_attempts=DEFAULT_MAX_ATTEMPTS if max_attempts is None else max_attempts, **kw)
+                        max_attempts=DEFAULT_MAX_ATTEMPTS if max_attempts is None else max_attempts,
+                        device_bitmap=device_bitmap, **kw)
 
     def encode(self, blocked: torch.Tensor, tiles: torch.Tensor, targets: torch.Tensor) -> None:
         """K1: dense description -> packed planes (GameState.__init__, state.py:61-73)."""
@@ -809,7 +814,7 @@ class BatchedTilerSliderEnv:
         return mask[: self.n_envs]
 
     def optimal_moves(self, ids=None, pos: torch.Tensor | None = None, *, max_depth: int = 254,
-                      paths: bool = False) -> tuple[torch.Tensor, ...]:
+                      paths: bool = False, device_bitmap: bool = False) -> tuple[torch.Tensor, ...]:
         """Exact solver answers for items (K9, ts_optimal_moves), as supervision for imitation
         learning, value targets, optimality gaps, reward shaping or an exact expert policy.  Items as
         expand() takes them: ids (default every env) give the puzzles, pos (default each listed
@@ -820,8 +825,11 @@ class BatchedTilerSliderEnv:
                     every move, as solve_depth; max_steps and the step counter play no part), or
                     -1 no win reachable (also every env of a never_win batch), -2 none within
                     max_depth steps, -3 this env's state space is larger than the largest bitmap
-                    one CTA can hold, or than the slab of the launch (it does not depend on the
-                    other items of the query), -4 the position word is not a well-formed state of
+                    one CTA can hold in shared memory (4 tiles on a 7x7 board with fewer than 11
+                    walls or an 8x8 one with fewer than 26; with device_bitmap=True such boards
+                    are searched with the bitmap in device memory instead), or than the slab of
+                    the launch (it does not depend on the other items of the query), -4 the
+                    position word is not a well-formed state of
                     its env (a tile on a wall or off the board, two tiles on one cell; e.g. the
                     zero rows playout(record=True) writes past an item's end);
           mask:     bit a (valid_moves() order) set iff move a starts a shortest solution; 0 when
@@ -842,12 +850,12 @@ class BatchedTilerSliderEnv:
         if self._optimal is None:
             self._optimal = CudaOptimalMoves(self)
         if not paths:
-            return self._optimal.query(ids, int(max_depth), pos)
+            return self._optimal.query(ids, int(max_depth), pos, device_bitmap=bool(device_bitmap))
         n = self.n_envs if ids is None else ids.numel()
         plan = torch.empty((int(max_depth), n), dtype=torch.uint8, device=self.device)
-        return (*self._optimal.query(ids, int(max_depth), pos, plan), plan)
+        return (*self._optimal.query(ids, int(max_depth), pos, plan, bool(device_bitmap)), plan)
 
-    def state_table(self, ids=None, pos: torch.Tensor | None = None) -> StateTable:
+    def state_table(self, ids=None, pos: torch.Tensor | None = None, *, device_bitmap: bool = False) -> StateTable:
         """Every state reachable from items, each with its exact distance to a win and its optimal
         moves (K10, ts_state_table), for value / policy datasets over whole state spaces, reverse
         curricula (states a chosen distance from the goal) and puzzle statistics (dead states, the
@@ -860,7 +868,8 @@ class BatchedTilerSliderEnv:
         optimal_moves(ids=..., pos=row) answers for it (max_depth plays no part: every finite
         distance is found), -1 and 0 where no win is reachable (every row of a never_win batch).
         status[i] is 0, or -3 (the item's state space is larger than the largest bitmap one CTA can
-        hold) or -4 (a malformed root, as optimal_moves() reports it); such items own no rows.
+        hold in shared memory, unless device_bitmap=True: as in optimal_moves()) or -4 (a malformed
+        root, as optimal_moves() reports it); such items own no rows.
         Ids are range-checked as in optimal_moves() (IndexError).  Runs on the current stream,
         changes no env state and reads back two scalars (the free-cell maximum and the row count,
         to allocate), so it cannot be captured in a CUDA graph.  Sizes up to 8, 1..4 tiles,
@@ -871,7 +880,7 @@ class BatchedTilerSliderEnv:
         ids = self._search_items("state_table", ids, pos)
         if self._state_table is None:
             self._state_table = CudaStateTable(self)
-        return StateTable(*self._state_table.build(ids, pos))
+        return StateTable(*self._state_table.build(ids, pos, bool(device_bitmap)))
 
     def _search_items(self, what: str, ids, pos: torch.Tensor | None) -> torch.Tensor | None:
         """The ids of a solver query as int32 on the device (None: every env), range-checked against

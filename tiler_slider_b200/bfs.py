@@ -667,15 +667,18 @@ class BfsSolver:
 
 
 class OnChipSearch:
-    """What the front-ends of the two on-chip searches (K6 `CudaLocalKernels`, K9 `CudaOptimalMoves`)
-    share: the shared-memory plan of a launch and the per-CTA scratch slabs.  `want_ctas` fixes the
-    CTAs per SM; `want_queue` caps the ring entries kept in shared memory (tests: force the slab)."""
+    """What the front-ends of the on-chip searches (K6 `CudaLocalKernels`, K9 `CudaOptimalMoves`, K10
+    `CudaStateTable`) share: the plan of a launch, the rule that picks it and the per-CTA scratch
+    slabs.  `want_ctas` fixes the CTAs per SM; `want_queue` caps the ring entries kept in shared
+    memory (tests: force the slab)."""
 
     N_LEVELS = 256                  # levels a search may have on chip (the kernels' level buffers)
     SMEM_PER_SM = 228 * 1024
     STATIC_SMEM = 4 * 1024          # the kernel's static shared memory + the per-CTA reservation
     MAX_SCRATCH_BYTES = 4 << 30
     CTAS_PER_SM = ""                # the library's occupancy query of the front-end's kernel
+    GMEM_CTAS_PER_SM = ""           # ... of its device-memory-bitmap instance
+    GMEM_SHAPES = ((7, 4), (8, 4))  # (size, tiles) with device instances: boards a shared bitmap may not hold
 
     def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
         self.t, self.lib, self.device = table, lib(), table.device
@@ -689,31 +692,63 @@ class OnChipSearch:
         `key` (None: the bitmap does not fit one CTA per SM).  The bitmap must hold F!/(F-T)! bits;
         the more CTAs fit an SM next to it, the better the level-synchronisation latency of one
         puzzle hides behind the others, so the ring gets what is left of the CTA's share."""
-        if key in self._plans:
-            return self._plans[key] or None
+        if key not in self._plans:
+            self._plans[key] = self._fit(f_max, gmem=False) or {}
+        return self._plans[key] or None
+
+    def _plan_gmem(self, f_max: int) -> dict | None:
+        """The plan of the device-memory-bitmap instance for up to f_max free cells (None: no such
+        instance for this shape), marked gmem=True: the same CTA-per-SM loop as _plan with the ring
+        alone in shared memory, and the grid capped so that its bitmaps (grid x F!/(F-T)! bits, 1.9 MB
+        per CTA at F = 64) stay within MAX_SCRATCH_BYTES."""
+        key = ("gmem", f_max)
+        if key not in self._plans:
+            ok = (self.t.size, self.t.n_tiles) in self.GMEM_SHAPES
+            self._plans[key] = (self._fit(f_max, gmem=True) if ok else None) or {}
+        return self._plans[key] or None
+
+    def _fit(self, f_max: int, gmem: bool) -> dict | None:
         bits = 1
         for i in range(self.t.n_tiles):                          # arrangements of T distinct tiles on f_max cells
             bits *= max(f_max - i, 1)
         bitmap_bytes = max(16, -(-bits // 128) * 16)
-        plan = None
+        smem_bitmap = 0 if gmem else bitmap_bytes
+        query = getattr(self.lib, self.GMEM_CTAS_PER_SM if gmem else self.CTAS_PER_SM)
         for k in ([self.want_ctas] if self.want_ctas else [8, 6, 5, 4, 3, 2, 1]):
             budget = self.SMEM_PER_SM // k - self.STATIC_SMEM
-            if bitmap_bytes + 1024 > budget:
+            if smem_bitmap + 1024 > budget:
                 continue
-            queue = 1 << (min(budget - bitmap_bytes, 64 * 1024) // 4).bit_length() - 1     # ring entries: a power of two
+            queue = 1 << (min(budget - smem_bitmap, 64 * 1024) // 4).bit_length() - 1     # ring entries: a power of two
             if self.want_queue is not None:
                 queue = max(32, 1 << (min(queue, self.want_queue).bit_length() - 1))
             a = self._args(bitmap_words=bitmap_bytes // 4, queue_smem=queue)
             got, n_sm = C.c_int(0), C.c_int(0)
             with torch.cuda.device(self.device):
-                rc = getattr(self.lib, self.CTAS_PER_SM)(C.byref(a), C.byref(got), C.byref(n_sm))
+                rc = query(C.byref(a), C.byref(got), C.byref(n_sm))
             if rc == 0 and got.value >= (k if self.want_ctas is None else 1):
                 grid = got.value * n_sm.value
+                if gmem:
+                    grid = min(grid, self.MAX_SCRATCH_BYTES // bitmap_bytes)
                 plan = dict(bitmap_words=bitmap_bytes // 4, queue_smem=queue, grid=grid, ctas_per_sm=got.value,
                             spill_per_cta=int(min(bits + 1, self.MAX_SCRATCH_BYTES // 4 // grid)), f_max=f_max)
-                break
-        self._plans[key] = plan or {}
-        return plan
+                return {**plan, "gmem": True} if gmem else plan
+        return None
+
+    def search_plan(self, f_max: int, device_bitmap: bool = False) -> dict | None:
+        """The plan of a query whose envs have up to f_max free cells, one rule for K9 and K10: the
+        shared plan for f_max when it exists; else, with device_bitmap on a shape that has device
+        instances, the gmem plan for f_max (every item of the call then runs on the device instance);
+        else the plan of the most free cells that fit (fitting_free_cells), the larger envs getting
+        -3.  Both instances give the same answers, so an env's answer never depends on the others."""
+        if device_bitmap and self.plan(f_max) is None:
+            gp = self._plan_gmem(f_max)
+            if gp is not None:
+                return gp
+        return self.plan(self.fitting_free_cells(f_max))
+
+    def _bitmap(self, plan: dict) -> int:
+        """The device-memory bitmaps of a gmem plan (grid x bitmap_words words, contents undefined)."""
+        return self._buf("bitmap", plan["grid"] * plan["bitmap_words"], torch.int32).data_ptr()
 
     def fitting_free_cells(self, f_max: int) -> int:
         """The largest F <= f_max whose plan fits (down to F = n_tiles): the free-cell count a launch
@@ -751,11 +786,14 @@ class CudaLocalKernels(OnChipSearch):
 
     MAX_MOVES = 255
     CTAS_PER_SM = "ts_bfs_local_ctas_per_sm"
+    GMEM_CTAS_PER_SM = "ts_bfs_local_gmem_ctas_per_sm"
 
-    def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
+    def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None,
+                 device_bitmap: bool = False):
         if table.size > 8 or not 1 <= table.n_tiles <= 4:
             raise ValueError("the on-chip BFS covers board sizes up to 8 with 1 to 4 tiles")
         super().__init__(table, ctas_per_sm, queue_smem)
+        self.device_bitmap = bool(device_bitmap)   # plan(): fall back to the device-memory bitmap (7x7 / 8x8, 4 tiles)
 
     def _args(self, **kw) -> BfsLocalArgs:
         t = self.t
@@ -766,14 +804,18 @@ class CudaLocalKernels(OnChipSearch):
         return BfsLocalArgs(**base)
 
     def plan(self, lo: int, hi: int) -> dict | None:
-        """The plan for puzzles [lo, hi): F = the most free cells of any of them."""
+        """The plan for puzzles [lo, hi): F = the most free cells of any of them.  With device_bitmap,
+        a range whose bitmap does not fit shared memory gets the gmem plan of its shape, if any."""
         t = self.t
         if (lo, hi) not in self._plans:
             blocked = t.blocked_cells()[lo:hi]
             f_max = int(t.size * t.size - blocked.sum(1).min()) if hi > lo else 1
             plan = self._plan((lo, hi), f_max)
+            if plan is None and self.device_bitmap:
+                plan = self._plan_gmem(f_max)
+                self._plans[(lo, hi)] = plan or {}
             if plan:
-                plan["smem_bytes"] = 4 * (plan["bitmap_words"] + plan["queue_smem"])
+                plan["smem_bytes"] = 4 * (plan["queue_smem"] + (0 if plan.get("gmem") else plan["bitmap_words"]))
         return self._plans[(lo, hi)] or None
 
     def puzzle(self, i: int) -> Puzzle:
@@ -811,7 +853,11 @@ class CudaLocalKernels(OnChipSearch):
                        d_moves=out["moves"].data_ptr() if with_paths else None,
                        d_lengths=out["lengths"].data_ptr() if with_paths else None, max_moves=self.MAX_MOVES)
         with torch.cuda.device(dev):
-            check(self.lib.ts_bfs_local(C.byref(a), plan["grid"], torch.cuda.current_stream(dev).cuda_stream), "ts_bfs_local")
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            if plan.get("gmem"):
+                check(self.lib.ts_bfs_local_gmem(C.byref(a), self._bitmap(plan), plan["grid"], stream), "ts_bfs_local_gmem")
+            else:
+                check(self.lib.ts_bfs_local(C.byref(a), plan["grid"], stream), "ts_bfs_local")
 
 
 def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int, what: str = "optimal_moves") -> None:
@@ -836,6 +882,7 @@ class CudaOptimalMoves(OnChipSearch):
     fewer; the plan is cached per free-cell count."""
 
     CTAS_PER_SM = "ts_optimal_moves_ctas_per_sm"
+    GMEM_CTAS_PER_SM = "ts_optimal_moves_gmem_ctas_per_sm"
 
     def __init__(self, env: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
         super().__init__(env, ctas_per_sm, queue_smem)
@@ -853,12 +900,13 @@ class CudaOptimalMoves(OnChipSearch):
         return self._plan(f_max, f_max)
 
     def query(self, ids: torch.Tensor | None, max_depth: int, pos: torch.Tensor | None = None,
-              plan: torch.Tensor | None = None) -> tuple[torch.Tensor, torch.Tensor]:
+              plan: torch.Tensor | None = None, device_bitmap: bool = False) -> tuple[torch.Tensor, torch.Tensor]:
         """(distance int32[n], mask uint8[n]) of items (env `ids[i]`, positions `pos[i]`) on the
         current stream.  ids: int32 on the device, each in [0, n_envs) (None: every env); pos:
         contiguous uint8 [n, pos_bytes] on the device (None: the envs' current positions); plan:
         uint8 [max_depth, n] on the device that receives a shortest solution per item (every entry
-        is written)."""
+        is written); device_bitmap: envs too large for a shared-memory bitmap are searched with one
+        in device memory (search_plan)."""
         t, dev = self.t, self.device
         n = t.n_envs if ids is None else ids.numel()
         distance = torch.full((n,), OPT_NOT_SEARCHED, dtype=torch.int32, device=dev)
@@ -871,7 +919,7 @@ class CudaOptimalMoves(OnChipSearch):
         with torch.cuda.device(dev):
             # one plan with and without paths: the same grid and slab, so the same answers (the plan
             # kernel instance may fit fewer CTAs per SM; the surplus CTAs find no ticket left)
-            sp = self.plan(self.fitting_free_cells(self._max_free_cells(ids, n)))
+            sp = self.search_plan(self._max_free_cells(ids, n), device_bitmap)
             if sp is None:                       # not even T free cells fit on chip
                 if plan is not None:
                     plan.fill_(255)
@@ -882,7 +930,10 @@ class CudaOptimalMoves(OnChipSearch):
                            d_counters=self.counters.data_ptr(), d_distance=distance.data_ptr(), d_mask=mask.data_ptr(),
                            d_item_pos=None if pos is None else pos.data_ptr(),
                            d_plan=None if plan is None else plan.data_ptr())
-            check(self.lib.ts_optimal_moves(C.byref(a), sp["grid"], stream), "ts_optimal_moves")
+            if sp.get("gmem"):
+                check(self.lib.ts_optimal_moves_gmem(C.byref(a), self._bitmap(sp), sp["grid"], stream), "ts_optimal_moves_gmem")
+            else:
+                check(self.lib.ts_optimal_moves(C.byref(a), sp["grid"], stream), "ts_optimal_moves")
         return distance, mask
 
 
@@ -893,6 +944,7 @@ class CudaStateTable(OnChipSearch):
     queried envs); both launches share the plan, so they agree on the items that fit."""
 
     CTAS_PER_SM = "ts_state_table_ctas_per_sm"
+    GMEM_CTAS_PER_SM = "ts_state_table_gmem_ctas_per_sm"
 
     def __init__(self, env: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
         super().__init__(env, ctas_per_sm, queue_smem)
@@ -909,18 +961,19 @@ class CudaStateTable(OnChipSearch):
         """The plan for states on up to f_max free cells."""
         return self._plan(f_max, f_max)
 
-    def build(self, ids: torch.Tensor | None, pos: torch.Tensor | None = None) -> tuple[torch.Tensor, ...]:
+    def build(self, ids: torch.Tensor | None, pos: torch.Tensor | None = None,
+              device_bitmap: bool = False) -> tuple[torch.Tensor, ...]:
         """(offsets int64[n+1], status int32[n], pos uint8[M, pos_bytes], distance int32[M], mask
         uint8[M]) of items (env `ids[i]`, root `pos[i]`) on the current stream; ids: int32 on the
         device, each in [0, n_envs) (None: every env); pos: contiguous uint8 [n, pos_bytes] on the
-        device (None: the envs' current positions).  Reads back the free-cell maximum and the row
-        count."""
+        device (None: the envs' current positions); device_bitmap as in CudaOptimalMoves.query.
+        Reads back the free-cell maximum and the row count."""
         t, dev = self.t, self.device
         n = t.n_envs if ids is None else ids.numel()
         offsets = torch.zeros(n + 1, dtype=torch.int64, device=dev)
         status = torch.full((n,), OPT_NOT_SEARCHED, dtype=torch.int32, device=dev)
         self.counters.zero_()
-        sp = self.plan(self.fitting_free_cells(self._max_free_cells(ids, n))) if n else None
+        sp = self.search_plan(self._max_free_cells(ids, n), device_bitmap) if n else None
         if sp is None:                           # no items, or not even T free cells fit on chip
             return (offsets, status, torch.empty((0, t.pos_bytes), dtype=torch.uint8, device=dev),
                     torch.empty(0, dtype=torch.int32, device=dev), torch.empty(0, dtype=torch.uint8, device=dev))
@@ -934,8 +987,13 @@ class CudaStateTable(OnChipSearch):
                        queue_smem=sp["queue_smem"], spill_per_cta=sp["spill_per_cta"],
                        d_spill=spill.data_ptr(), d_counters=self.counters.data_ptr(), d_count=count.data_ptr(),
                        d_status=status.data_ptr())
+        # both passes: the same plan and, with a gmem plan, the same bitmaps
+        bitmap = self._bitmap(sp) if sp.get("gmem") else None
         with torch.cuda.device(dev):
-            check(self.lib.ts_state_table_count(C.byref(a), sp["grid"], stream), "ts_state_table_count")
+            if bitmap is None:
+                check(self.lib.ts_state_table_count(C.byref(a), sp["grid"], stream), "ts_state_table_count")
+            else:
+                check(self.lib.ts_state_table_count_gmem(C.byref(a), bitmap, sp["grid"], stream), "ts_state_table_count_gmem")
             torch.cumsum(count, 0, out=offsets[1:])
             total = int(offsets[-1].item())
             rows = torch.empty((total, t.pos_bytes), dtype=torch.uint8, device=dev)
@@ -943,7 +1001,10 @@ class CudaStateTable(OnChipSearch):
             mask = torch.empty(total, dtype=torch.uint8, device=dev)
             if total:
                 a.d_offsets, a.d_rows, a.d_distance, a.d_mask = offsets.data_ptr(), rows.data_ptr(), distance.data_ptr(), mask.data_ptr()
-                check(self.lib.ts_state_table_fill(C.byref(a), sp["grid"], stream), "ts_state_table_fill")
+                if bitmap is None:
+                    check(self.lib.ts_state_table_fill(C.byref(a), sp["grid"], stream), "ts_state_table_fill")
+                else:
+                    check(self.lib.ts_state_table_fill_gmem(C.byref(a), bitmap, sp["grid"], stream), "ts_state_table_fill_gmem")
         return offsets, status, rows, distance, mask
 
 
@@ -955,18 +1016,20 @@ class LocalBfs:
     searches its shard with no exchange at all, and the per-puzzle results are combined once at
     the end.  A puzzle that does not fit on chip (state space above the shared-memory bitmap,
     more than 255 levels) is searched by the hash-partitioned `BfsSolver` instead.  Same result
-    definitions as BfsSolver; boards of size <= 8 with 1..4 tiles.
+    definitions as BfsSolver; boards of size <= 8 with 1..4 tiles.  device_bitmap=True: 7x7 and 8x8
+    boards with four tiles whose bitmap outgrows shared memory are searched on chip all the same,
+    with the bitmap in device memory (same results, and per-puzzle levels rather than a fallback).
 
     The device work sits behind `CudaLocalKernels`; tests run this driver on CPU tensors over
     gloo with a stand-in (tests/test_bfs_gloo.py)."""
 
     def __init__(self, puzzles: Sequence[Puzzle] | BatchedTilerSliderEnv | None = None, *, device="cuda", group=None,
                  ctas_per_sm: int | None = None, queue_smem: int | None = None, fallback_table_capacity: int = 1 << 24,
-                 kernels=None, n_puzzles: int | None = None, fallback=None):
+                 kernels=None, n_puzzles: int | None = None, fallback=None, device_bitmap: bool = False):
         if kernels is None:
             table = puzzles if isinstance(puzzles, BatchedTilerSliderEnv) else \
                 BatchedTilerSliderEnv.from_puzzles(list(puzzles), device=device)
-            kernels = CudaLocalKernels(table, ctas_per_sm, queue_smem)
+            kernels = CudaLocalKernels(table, ctas_per_sm, queue_smem, device_bitmap)
             n_puzzles = table.n_envs
         self.k, self.device, self.group = kernels, kernels.device, group
         self.n_puzzles = int(n_puzzles)

@@ -50,11 +50,12 @@ def write_candidates(env: BatchedTilerSliderEnv, ids: torch.Tensor | None, n_wal
 
 
 def fill(env: BatchedTilerSliderEnv, n_walls: int, *, min_depth: int, max_depth: int, recipe: str, walk_len: int,
-         seed: int, env_index_base: int, max_attempts: int) -> dict:
+         seed: int, env_index_base: int, max_attempts: int, device_bitmap: bool = False) -> dict:
     """Run up to `max_attempts` rounds over the envs of `env`; accepted envs get their solve depth in
-    env._solve_depth.  Returns {rounds, candidates, accepted, unfilled}."""
+    env._solve_depth.  device_bitmap: grade boards whose bitmap outgrows shared memory with one in
+    device memory (7x7 / 8x8, 4 tiles).  Returns {rounds, candidates, accepted, unfilled}."""
     dev, n = env.device, env.n_envs
-    k = CudaLocalKernels(env)
+    k = CudaLocalKernels(env, device_bitmap=device_bitmap)
     depth = torch.full((env.capacity,), -1, dtype=torch.int32, device=dev)
     out = dict(states=torch.zeros(n, dtype=torch.int64, device=dev), depth=torch.zeros(n, dtype=torch.int32, device=dev),
                status=torch.zeros(n, dtype=torch.int32, device=dev),
@@ -66,7 +67,9 @@ def fill(env: BatchedTilerSliderEnv, n_walls: int, *, min_depth: int, max_depth:
         write_candidates(env, pending, n_walls, recipe, walk_len, rounds, seed, env_index_base)
         if rounds == 0 and k.plan(0, n) is None:      # every candidate has n_walls walls: one plan fits all
             raise ValueError(f"size {env.size} with {env.n_tiles} tiles and {n_walls} walls: the state bitmap does not fit "
-                             "the on-chip search that grades the puzzles")
+                             "the on-chip search that grades the puzzles"
+                             + ("" if device_bitmap or (env.size, env.n_tiles) not in k.GMEM_SHAPES else
+                                " (device_bitmap=True keeps it in device memory)"))
         out["counters"].zero_()                       # [0] is K6's ticket counter
         k.search(0, n, max_depth, out, ids=pending)
         idx = pending.long()
@@ -82,7 +85,8 @@ def fill(env: BatchedTilerSliderEnv, n_walls: int, *, min_depth: int, max_depth:
 
 def solvable(cls, n_envs: int, size: int, n_tiles: int, n_walls: int, multi_color: bool = False, *, min_depth: int = 1,
              max_depth: int = 30, recipe: str = "walk", walk_len: int | None = None, seed: int = 0,
-             env_index_base: int = 0, max_attempts: int = DEFAULT_MAX_ATTEMPTS, **kw) -> BatchedTilerSliderEnv:
+             env_index_base: int = 0, max_attempts: int = DEFAULT_MAX_ATTEMPTS, device_bitmap: bool = False,
+             **kw) -> BatchedTilerSliderEnv:
     """BatchedTilerSliderEnv.solvable (see there)."""
     if not (1 <= size <= 8 and 1 <= n_tiles <= 4):
         raise ValueError(f"graded generation covers sizes up to 8 with 1 to 4 tiles (got size {size}, {n_tiles} tiles)")
@@ -103,7 +107,7 @@ def solvable(cls, n_envs: int, size: int, n_tiles: int, n_walls: int, multi_colo
         raise ValueError("max_attempts must be positive")
     env = cls(size, n_tiles, n_envs, multi_color, **kw)
     stats = fill(env, n_walls, min_depth=min_depth, max_depth=max_depth, recipe=recipe, walk_len=walk_len, seed=seed,
-                 env_index_base=env_index_base, max_attempts=max_attempts)
+                 env_index_base=env_index_base, max_attempts=max_attempts, device_bitmap=device_bitmap)
     if stats["unfilled"]:
         raise RuntimeError(f"{stats['unfilled']} of {n_envs} envs unfilled after {stats['rounds']} rounds: "
                            f"{stats['accepted']} of {stats['candidates']} candidates were in the band "
