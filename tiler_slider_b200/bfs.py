@@ -668,8 +668,8 @@ class BfsSolver:
 
 class OnChipSearch:
     """What the front-ends of the on-chip searches (K6 `CudaLocalKernels`, K9 `CudaOptimalMoves`, K10
-    `CudaStateTable`) share: the plan of a launch, the rule that picks it and the per-CTA scratch
-    slabs.  `want_ctas` fixes the CTAs per SM; `want_queue` caps the ring entries kept in shared
+    `CudaStateTable`) share: the plan of a launch, the rule that picks it, the launch on the shared
+    or the device-memory-bitmap instance and the per-CTA scratch slabs.  `want_ctas` fixes the CTAs per SM; `want_queue` caps the ring entries kept in shared
     memory (tests: force the slab)."""
 
     N_LEVELS = 256                  # levels a search may have on chip (the kernels' level buffers)
@@ -679,6 +679,7 @@ class OnChipSearch:
     CTAS_PER_SM = ""                # the library's occupancy query of the front-end's kernel
     GMEM_CTAS_PER_SM = ""           # ... of its device-memory-bitmap instance
     GMEM_SHAPES = ((7, 4), (8, 4))  # (size, tiles) with device instances: boards a shared bitmap may not hold
+    ARGS = None                     # the argument struct of the front-end's entry points (K9, K10: _args)
 
     def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
         self.t, self.lib, self.device = table, lib(), table.device
@@ -686,6 +687,19 @@ class OnChipSearch:
         self.want_queue = queue_smem
         self._plans: dict = {}
         self._scratch: dict[str, torch.Tensor] = {}
+        self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)   # K9, K10: of the last call, see include/tiler_slider.h
+
+    def _args(self, **kw):
+        """The front-end's argument struct for its table (K9 and K10's fields), with kw set."""
+        t = self.t
+        base = dict(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win), capacity=t.capacity,
+                    d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(), d_pos=t._pos.data_ptr())
+        base.update(kw)
+        return self.ARGS(**base)
+
+    def plan(self, f_max: int) -> dict | None:
+        """The plan for states on up to f_max free cells."""
+        return self._plan(f_max, f_max)
 
     def _plan(self, key, f_max: int) -> dict | None:
         """Shared-memory split and grid for states of T tiles on up to f_max free cells, cached under
@@ -749,6 +763,16 @@ class OnChipSearch:
     def _bitmap(self, plan: dict) -> int:
         """The device-memory bitmaps of a gmem plan (grid x bitmap_words words, contents undefined)."""
         return self._buf("bitmap", plan["grid"] * plan["bitmap_words"], torch.int32).data_ptr()
+
+    def _launch(self, entry: str, a, plan: dict, stream) -> None:
+        """Launch the library's `entry` with arguments a on plan's grid; with a gmem plan its device
+        counterpart `entry`_gmem, on the bitmaps of _bitmap."""
+        if plan.get("gmem"):
+            entry += "_gmem"
+            rc = getattr(self.lib, entry)(C.byref(a), self._bitmap(plan), plan["grid"], stream)
+        else:
+            rc = getattr(self.lib, entry)(C.byref(a), plan["grid"], stream)
+        check(rc, entry)
 
     def fitting_free_cells(self, f_max: int) -> int:
         """The largest F <= f_max whose plan fits (down to F = n_tiles): the free-cell count a launch
@@ -854,10 +878,7 @@ class CudaLocalKernels(OnChipSearch):
                        d_lengths=out["lengths"].data_ptr() if with_paths else None, max_moves=self.MAX_MOVES)
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
-            if plan.get("gmem"):
-                check(self.lib.ts_bfs_local_gmem(C.byref(a), self._bitmap(plan), plan["grid"], stream), "ts_bfs_local_gmem")
-            else:
-                check(self.lib.ts_bfs_local(C.byref(a), plan["grid"], stream), "ts_bfs_local")
+            self._launch("ts_bfs_local", a, plan, stream)
 
 
 def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int, what: str = "optimal_moves") -> None:
@@ -883,21 +904,7 @@ class CudaOptimalMoves(OnChipSearch):
 
     CTAS_PER_SM = "ts_optimal_moves_ctas_per_sm"
     GMEM_CTAS_PER_SM = "ts_optimal_moves_gmem_ctas_per_sm"
-
-    def __init__(self, env: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
-        super().__init__(env, ctas_per_sm, queue_smem)
-        self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)   # of the last call: see include/tiler_slider.h
-
-    def _args(self, **kw) -> OptimalMovesArgs:
-        t = self.t
-        base = dict(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win), capacity=t.capacity,
-                    d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(), d_pos=t._pos.data_ptr())
-        base.update(kw)
-        return OptimalMovesArgs(**base)
-
-    def plan(self, f_max: int) -> dict | None:
-        """The plan for states on up to f_max free cells."""
-        return self._plan(f_max, f_max)
+    ARGS = OptimalMovesArgs
 
     def query(self, ids: torch.Tensor | None, max_depth: int, pos: torch.Tensor | None = None,
               plan: torch.Tensor | None = None, device_bitmap: bool = False) -> tuple[torch.Tensor, torch.Tensor]:
@@ -930,10 +937,7 @@ class CudaOptimalMoves(OnChipSearch):
                            d_counters=self.counters.data_ptr(), d_distance=distance.data_ptr(), d_mask=mask.data_ptr(),
                            d_item_pos=None if pos is None else pos.data_ptr(),
                            d_plan=None if plan is None else plan.data_ptr())
-            if sp.get("gmem"):
-                check(self.lib.ts_optimal_moves_gmem(C.byref(a), self._bitmap(sp), sp["grid"], stream), "ts_optimal_moves_gmem")
-            else:
-                check(self.lib.ts_optimal_moves(C.byref(a), sp["grid"], stream), "ts_optimal_moves")
+            self._launch("ts_optimal_moves", a, sp, stream)
         return distance, mask
 
 
@@ -945,21 +949,7 @@ class CudaStateTable(OnChipSearch):
 
     CTAS_PER_SM = "ts_state_table_ctas_per_sm"
     GMEM_CTAS_PER_SM = "ts_state_table_gmem_ctas_per_sm"
-
-    def __init__(self, env: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
-        super().__init__(env, ctas_per_sm, queue_smem)
-        self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)   # of the last call: see include/tiler_slider.h
-
-    def _args(self, **kw) -> StateTableArgs:
-        t = self.t
-        base = dict(size=t.size, n_tiles=t.n_tiles, goal_mode=t.goal_mode, never_win=int(t.never_win), capacity=t.capacity,
-                    d_walls=t._walls.data_ptr(), d_targets_packed=t._targets.data_ptr(), d_pos=t._pos.data_ptr())
-        base.update(kw)
-        return StateTableArgs(**base)
-
-    def plan(self, f_max: int) -> dict | None:
-        """The plan for states on up to f_max free cells."""
-        return self._plan(f_max, f_max)
+    ARGS = StateTableArgs
 
     def build(self, ids: torch.Tensor | None, pos: torch.Tensor | None = None,
               device_bitmap: bool = False) -> tuple[torch.Tensor, ...]:
@@ -987,13 +977,8 @@ class CudaStateTable(OnChipSearch):
                        queue_smem=sp["queue_smem"], spill_per_cta=sp["spill_per_cta"],
                        d_spill=spill.data_ptr(), d_counters=self.counters.data_ptr(), d_count=count.data_ptr(),
                        d_status=status.data_ptr())
-        # both passes: the same plan and, with a gmem plan, the same bitmaps
-        bitmap = self._bitmap(sp) if sp.get("gmem") else None
         with torch.cuda.device(dev):
-            if bitmap is None:
-                check(self.lib.ts_state_table_count(C.byref(a), sp["grid"], stream), "ts_state_table_count")
-            else:
-                check(self.lib.ts_state_table_count_gmem(C.byref(a), bitmap, sp["grid"], stream), "ts_state_table_count_gmem")
+            self._launch("ts_state_table_count", a, sp, stream)
             torch.cumsum(count, 0, out=offsets[1:])
             total = int(offsets[-1].item())
             rows = torch.empty((total, t.pos_bytes), dtype=torch.uint8, device=dev)
@@ -1001,10 +986,7 @@ class CudaStateTable(OnChipSearch):
             mask = torch.empty(total, dtype=torch.uint8, device=dev)
             if total:
                 a.d_offsets, a.d_rows, a.d_distance, a.d_mask = offsets.data_ptr(), rows.data_ptr(), distance.data_ptr(), mask.data_ptr()
-                if bitmap is None:
-                    check(self.lib.ts_state_table_fill(C.byref(a), sp["grid"], stream), "ts_state_table_fill")
-                else:
-                    check(self.lib.ts_state_table_fill_gmem(C.byref(a), bitmap, sp["grid"], stream), "ts_state_table_fill_gmem")
+                self._launch("ts_state_table_fill", a, sp, stream)
         return offsets, status, rows, distance, mask
 
 

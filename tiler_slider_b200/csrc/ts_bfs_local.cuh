@@ -1,8 +1,9 @@
 // ts_bfs_local.cuh -- what the on-chip searches, K6 (ts_bfs_local.cu, the batched BFS), K9
 // (ts_optimal.cu, the optimal-move query) and K10 (ts_state_table.cu, the state tables), share: the
 // CTA shape, canonical set-goal states, position byte -> bitboard bit, the perfect hash of a state over the free cells of its puzzle that keys the
-// shared-memory bitmap, and on the host the plan check, the shared-memory size and the launch, of
-// the shared instances and of the device-memory-bitmap instances of 7x7 and 8x8 boards with four tiles.
+// shared-memory bitmap, and on the host the plan check, the shared-memory size, the launch and the
+// occupancy query, one each for the shared instances and the device-memory-bitmap instances (GMEM) of
+// 7x7 and 8x8 boards with four tiles.
 #pragma once
 #include "ts_common.cuh"
 #include "../../include/tiler_slider.h"
@@ -78,40 +79,12 @@ template <class A> int check_search_plan(const A& a) {
 
 template <class A> size_t search_smem_bytes(const A& a) { return ((size_t)a.bitmap_words + (size_t)a.queue_smem) * sizeof(uint32_t); }
 
-// Instance <a.size, a.n_tiles> of a search kernel (kernel_of(IC<S>, IC<T>) returns it) with a's
-// dynamic shared memory: launched on `grid` CTAs, or, when ctas_per_sm is given, asked how many of
-// its CTAs fit an SM.
-template <class KernelOf, class A>
-cudaError_t search_kernel(KernelOf&& kernel_of, const A& a, int grid, int* ctas_per_sm, cudaStream_t st) {
-    const size_t smem = search_smem_bytes(a);
-    return dispatch_small(a.size, a.n_tiles, [&](auto S, auto T) {
-        const auto kernel = kernel_of(S, T);
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        if (ctas_per_sm) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kernel, SEARCH_THREADS, smem);
-        kernel<<<grid, SEARCH_THREADS, smem, st>>>(a);
-        return cudaGetLastError();
-    });
-}
-
-// resident CTAs per SM of a's search kernel and the SM count of the current device
-template <class KernelOf, class A>
-int search_ctas_per_sm(KernelOf&& kernel_of, const A& a, int* ctas_per_sm, int* n_sm) {
-    if (!ctas_per_sm || !n_sm) return TS_E_NULL_POINTER;
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (e == cudaSuccess) e = search_kernel(kernel_of, a, 0, ctas_per_sm, nullptr);
-    if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
-    return 0;
-}
-
 // ---- device-memory bitmaps -------------------------------------------------------------------------
 // With four tiles, a board of more than 38 free cells has a state space whose bitmap does not fit
-// one CTA's shared memory; only 7x7 and 8x8 boards have that many.  Their device instances keep the
-// bitmap in device memory instead, CTA b's at d_bitmap + b * bitmap_words, and dynamic shared
-// memory holds the ring alone.  Every other shape fits shared memory at every wall count, so no
-// other device instance is built.
+// one CTA's shared memory; only 7x7 and 8x8 boards have that many.  Their device instances (GMEM)
+// keep the bitmap in device memory instead, CTA b's at d_bitmap + b * bitmap_words, and dynamic
+// shared memory holds the ring alone.  Every other shape fits shared memory at every wall count, so
+// no other device instance is built.
 __host__ __device__ constexpr bool gmem_shape(int size, int n_tiles) { return n_tiles == 4 && (size == 7 || size == 8); }
 
 // the checks the device entry points add after their shared counterpart's: the shape, then the buffer
@@ -122,32 +95,35 @@ template <class A> int check_gmem(const A& a, const uint32_t* d_bitmap) {
     return 0;
 }
 
-// search_kernel for a device instance (gkernel_of(IC<S>, IC<T>) returns it; it takes a and the
-// bitmap buffer d_bitmap[grid][bitmap_words]): the ring is the only dynamic shared memory
-template <class KernelOf, class A>
-cudaError_t search_gmem_kernel(KernelOf&& gkernel_of, const A& a, uint32_t* d_bitmap, int grid, int* ctas_per_sm, cudaStream_t st) {
-    const size_t smem = (size_t)a.queue_smem * sizeof(uint32_t);
+// Instance <a.size, a.n_tiles, GMEM> of a search kernel (kernel_of(IC<S>, IC<T>, bool_constant<GMEM>)
+// returns it; it takes a and the bitmap buffer d_bitmap[grid][bitmap_words], unused by the shared
+// instances) with a's dynamic shared memory, the ring and, shared instances only, the bitmap:
+// launched on `grid` CTAs, or, when ctas_per_sm is given, asked how many of its CTAs fit an SM.
+// GMEM: a.size is 7 or 8 and a.n_tiles 4, checked by the caller.
+template <bool GMEM, class KernelOf, class A>
+cudaError_t search_kernel(KernelOf&& kernel_of, const A& a, uint32_t* d_bitmap, int grid, int* ctas_per_sm, cudaStream_t st) {
+    const size_t smem = GMEM ? (size_t)a.queue_smem * sizeof(uint32_t) : search_smem_bytes(a);
     auto go = [&](auto S, auto T) {
-        const auto kernel = gkernel_of(S, T);
+        const auto kernel = kernel_of(S, T, std::bool_constant<GMEM>{});
         cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         if (ctas_per_sm) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kernel, SEARCH_THREADS, smem);
         kernel<<<grid, SEARCH_THREADS, smem, st>>>(a, d_bitmap);
         return cudaGetLastError();
     };
-    if (a.size == 7) return go(IC<7>{}, IC<4>{});
-    return go(IC<8>{}, IC<4>{});                  // gmem_shape: checked by the caller
+    if constexpr (GMEM) return a.size == 7 ? go(IC<7>{}, IC<4>{}) : go(IC<8>{}, IC<4>{});
+    else return dispatch_small(a.size, a.n_tiles, go);
 }
 
-// search_ctas_per_sm of a device instance
-template <class KernelOf, class A>
-int search_gmem_ctas_per_sm(KernelOf&& gkernel_of, const A& a, int* ctas_per_sm, int* n_sm) {
+// resident CTAs per SM of a's search kernel and the SM count of the current device
+template <bool GMEM, class KernelOf, class A>
+int search_ctas_per_sm(KernelOf&& kernel_of, const A& a, int* ctas_per_sm, int* n_sm) {
     if (!ctas_per_sm || !n_sm) return TS_E_NULL_POINTER;
-    if (!gmem_shape(a.size, a.n_tiles)) return TS_E_UNSUPPORTED;
+    if (GMEM && !gmem_shape(a.size, a.n_tiles)) return TS_E_UNSUPPORTED;
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (e == cudaSuccess) e = search_gmem_kernel(gkernel_of, a, nullptr, 0, ctas_per_sm, nullptr);
+    if (e == cudaSuccess) e = search_kernel<GMEM>(kernel_of, a, nullptr, 0, ctas_per_sm, nullptr);
     if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
     return 0;
 }
