@@ -1,7 +1,8 @@
 """GPU tests of the on-chip searches at their capacity limits: K9 (optimal_moves) next to the largest
-bitmap one CTA can hold, K9 and K6 (LocalBfs) with a slab too small for some of their envs, and K9 on
-the smallest and fullest boards.  Every expectation comes from the CPU oracle's BFS; where a slab
-runs out, the answer is predicted from the oracle's level counts and the kernel's append rule."""
+bitmap one CTA can hold, K9, K10 (state_table) and K6 (LocalBfs) with a slab too small for some of
+their envs, and K9 on the smallest and fullest boards.  Every expectation comes from the CPU
+oracle's BFS; where a slab runs out, the answer is predicted from the oracle's state or level counts
+and the kernel's append rule."""
 import numpy as np
 import pytest
 import torch
@@ -149,6 +150,45 @@ def test_optimal_moves_slab_overflow_is_predicted_exactly(ts, multi):
                 seen.add(("win" if 1 <= dd <= m else "none", want[0] if want[0] < 0 else "exact"))
     # every branch of the prediction was taken
     assert seen >= {("win", "exact"), ("win", NOT_SEARCHED), ("none", NOT_SEARCHED), ("none", -1), ("none", -2)}, seen
+
+
+@pytest.mark.parametrize("multi", [True, False], ids=["ordered", "set"])
+def test_state_table_slab_overflow_is_predicted_exactly(ts, multi):
+    """K10's count pass gives an item up (-3, no rows) as soon as a discovery index reaches the q
+    entries of its slab, even when the ring would hold the entry: exactly the items of more than q
+    states.  Every other item gets the rows and labels of the default plan."""
+    from tiler_slider_b200.bfs import CudaStateTable
+
+    class SmallSlab(CudaStateTable):
+        def __init__(self, env, q, queue_smem=None):
+            super().__init__(env, queue_smem=queue_smem)
+            self.q = q
+
+        def plan(self, f_max):
+            p = super().plan(f_max)
+            return None if p is None else {**p, "spill_per_cta": self.q}
+
+    solvable = puzzles(6, 4, [8], 48, multi, seed=int(multi) + 70)
+    uniform = puzzles(6, 4, [8], 16, multi, seed=int(multi) + 72, walk=None)
+    env = ts.BatchedTilerSliderEnv.from_arrays(6, *(np.concatenate(p) for p in zip(solvable, uniform)), multi)
+    random_steps(env, 3, seed=11)
+    count = np.array([st.bfs(max_states=1 << 22)[0] for st, _ in oracle_states(env)])
+    full = env.state_table()
+    assert (full.status == 0).all()
+    rows_per_item = full.offsets.diff().cpu().numpy()
+    assert np.array_equal(rows_per_item, count)
+    seen = set()
+    for q in (48, 2000, 4000):
+        for ring in (None, 32):
+            offsets, status, pos, distance, mask = SmallSlab(env, q, ring).build(None)
+            big = count > q
+            assert np.array_equal(status.cpu().numpy(), np.where(big, NOT_SEARCHED, 0)), (q, ring)
+            assert np.array_equal(offsets.diff().cpu().numpy(), np.where(big, 0, count)), (q, ring)
+            kept = torch.from_numpy(np.repeat(~big, rows_per_item)).cuda()
+            assert torch.equal(pos, full.pos[kept]) and torch.equal(distance, full.distance[kept]) \
+                and torch.equal(mask, full.mask[kept]), (q, ring)
+            seen.update(big.tolist())
+    assert seen == {True, False}
 
 
 # ---- (d) K6 with a slab too small for some puzzles: the hash-partitioned fallback ----------------

@@ -20,9 +20,9 @@
 // are appended with one shared-memory atomic per warp; one __syncthreads per level (three rotating
 // per-level counters).  Successor function = GameState.move (explainrl/environment/state.py:
 // 120-170) through slide_env<S,T>, goal test = is_won (state.py:172-186): the same device code as
-// the step kernel.  Semantics identical to the hash-partitioned search: set-goal states are
-// canonicalised by sorting, the solve depth is the first depth at which ANY successor (new or not)
-// meets the goal.  BFS itself has no counterpart in the reference (parity unpinned; results pinned
+// the step kernel, in the successor function K9 and K10 share (ts_bfs_local.cuh).  Semantics
+// identical to the hash-partitioned search: set-goal states are canonicalised by sorting, the solve
+// depth is the first depth at which ANY successor (new or not) meets the goal.  BFS itself has no counterpart in the reference (parity unpinned; results pinned
 // to a plain BFS over the reference's move, tests/golden/).
 //
 // A puzzle that does not fit (F^T bits above the bitmap the launch was given, queue spill
@@ -86,10 +86,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) bfs_local_kernel(const ts_bfs_
         if (a.goal_mode == TS_GOAL_SET) sort_bytes4<T>(q_init);
         const uint64_t free_cells = ~walls & cell_mask<S>();
         const uint32_t F = (uint32_t)__popcll(free_cells);
-        if (tid < 128) {
-            const uint32_t bit = pos_to_bit<S>(tid);
-            lut[tid] = bit < 64 ? (uint8_t)__popcll(free_cells & ((1ull << bit) - 1ull)) : 0;
-        }
+        fill_lut<S>(tid, free_cells, lut);
         // states = arrangements of T distinct tiles on F cells: F (F-1) ... (F-T+1) bits
         unsigned long long bits = 1;
 #pragma unroll
@@ -99,7 +96,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) bfs_local_kernel(const ts_bfs_
             if (tid == 0) a.d_status[pid] = 1;
             continue;
         }
-        for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+        clear_bitmap(bitmap, words, tid);
         if (tid == 0) { cnt[0] = cnt[1] = cnt[2] = 0; s_solve = 0xFFFFFFFFu; s_over = 0; s_goal = ~0ull; }
         __syncthreads();
 
@@ -131,16 +128,9 @@ __global__ void __launch_bounds__(SEARCH_THREADS) bfs_local_kernel(const ts_bfs_
                 uint32_t qn = 0;
                 if (live) {
                     const uint32_t q0 = (src - prev_lo) < R ? queue[src & RMASK] : spill[src];
-                    uint32_t q[1] = {q0};
-                    slide_env<S, T>(q, walls, d >> 1, (d & 1u) ^ 1u);
-                    bool won = a.never_win == 0;
-                    if (a.goal_mode == TS_GOAL_SET) {
-                        won &= occupancy<S, T>(q) == tboard;
-                        sort_bytes4<T>(q[0]);     // canonical form: tiles are interchangeable (state.py:185-186)
-                    } else {
-                        won &= q[0] == tq;
-                    }
-                    qn = q[0];
+                    bool won;
+                    qn = successor<S, T>(q0, d, walls, a.goal_mode == TS_GOAL_SET, tboard, tq, won);
+                    won &= a.never_win == 0;
                     if (won) {
                         const uint32_t before = atomicMin(&s_solve, depth + 1u);
                         if (parents && before > depth + 1u) atomicMin(&s_goal, ((unsigned long long)(depth + 1u) << 32) | ((unsigned long long)src << 2) | d);

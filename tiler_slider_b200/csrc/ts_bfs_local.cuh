@@ -1,9 +1,10 @@
 // ts_bfs_local.cuh -- what the on-chip searches, K6 (ts_bfs_local.cu, the batched BFS), K9
 // (ts_optimal.cu, the optimal-move query) and K10 (ts_state_table.cu, the state tables), share: the
-// CTA shape, canonical set-goal states, position byte -> bitboard bit, the perfect hash of a state over the free cells of its puzzle that keys the
-// shared-memory bitmap, and on the host the plan check, the shared-memory size, the launch and the
-// occupancy query, one each for the shared instances and the device-memory-bitmap instances (GMEM) of
-// 7x7 and 8x8 boards with four tiles.
+// CTA shape, canonical set-goal states, position byte -> bitboard bit, the perfect hash of a state
+// over the free cells of its puzzle that keys the visited bitmap, the successor function, the lut
+// fill, the bitmap clear and K9 and K10's root read; on the host the plan and env-table checks of K9 and K10, the plan check, the
+// shared-memory size, the launch and the occupancy query, one each for the shared instances and the
+// device-memory-bitmap instances (GMEM) of 7x7 and 8x8 boards with four tiles.
 #pragma once
 #include "ts_common.cuh"
 #include "../../include/tiler_slider.h"
@@ -67,6 +68,60 @@ template <int T> __device__ __forceinline__ uint32_t state_index(const uint8_t (
     return idx;
 }
 
+// The successor function of the three searches: the state after move m from q0 on a board of these
+// walls, through the step's slide_env (GameState.move, explainrl/environment/state.py:120-170); won =
+// it meets the goal (is_won, state.py:172-186: set goal, occupancy tboard; ordered, word tq).  A
+// set-goal state comes back canonical, its bytes sorted: tiles are interchangeable (state.py:185-186).
+template <int S, int T>
+__device__ __forceinline__ uint32_t successor(uint32_t q0, uint32_t m, uint64_t walls, bool set_goal, uint64_t tboard, uint32_t tq, bool& won) {
+    uint32_t q[1] = {q0};
+    slide_env<S, T>(q, walls, m >> 1, (m & 1u) ^ 1u);
+    if (set_goal) {
+        won = occupancy<S, T>(q) == tboard;
+        sort_bytes4<T>(q[0]);
+    } else {
+        won = q[0] == tq;
+    }
+    return q[0];
+}
+
+// position byte -> rank among the free cells (lut, 128 entries) and, given rank_byte, rank -> position
+// byte, filled by the block; read after the caller's next __syncthreads.  tid as in clear_bitmap.
+template <int S>
+__device__ __forceinline__ void fill_lut(uint32_t tid, uint64_t free_cells, uint8_t* lut, uint8_t* rank_byte = nullptr) {
+    if (tid < 128) {
+        const uint32_t bit = pos_to_bit<S>(tid);
+        const uint32_t rank = bit < 64 ? (uint32_t)__popcll(free_cells & ((1ull << bit) - 1ull)) : 0u;
+        lut[tid] = (uint8_t)rank;
+        if (rank_byte && (cell_bit<S>(tid) & free_cells)) rank_byte[rank] = (uint8_t)tid;
+    }
+}
+
+// The root word of an item (K9, K10): row `ticket` of a.d_item_pos, else env pid's positions.  False
+// when it is no state: each tile must stand on its own free cell (an off-board byte adds no bit, two
+// tiles on one cell one), the states the hash is defined for.
+template <int S, int T, class A>
+__device__ __forceinline__ bool read_root(const A& a, long long ticket, size_t pid, uint64_t free_cells, uint32_t& root) {
+    constexpr int PW = pos_bytes(T);
+    const uint8_t* const root_pos = a.d_item_pos ? a.d_item_pos + (size_t)ticket * PW : a.d_pos + pid * PW;
+    uint64_t occ = 0;
+    root = 0;
+    static_for<0, T>([&](auto I) {
+        constexpr int t = decltype(I)::value;
+        const uint32_t p = root_pos[t];
+        root |= p << (8 * t);
+        occ |= cell_bit<S>(p);
+    });
+    return __popcll(occ) == T && !(occ & ~free_cells);
+}
+
+// the first `words` words of a bitmap, rounded up to whole 16-byte units, cleared by the block.  tid
+// is the kernel's thread index: a read of threadIdx.x outside the kernel's own body loses what
+// __launch_bounds__ tells the compiler about it (tid < SEARCH_THREADS), and registers with it.
+__device__ __forceinline__ void clear_bitmap(uint32_t* bitmap, uint32_t words, uint32_t tid) {
+    for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+}
+
 // ---- host side -------------------------------------------------------------------------------------
 // tile count, goal mode and shared-memory plan of a search launch: a bitmap of whole 16-byte units,
 // a power-of-two ring of at least 32 entries
@@ -74,6 +129,22 @@ template <class A> int check_search_plan(const A& a) {
     if (a.n_tiles < 1 || a.n_tiles > 4) return TS_E_UNSUPPORTED;            // 32-bit states
     if (a.goal_mode != TS_GOAL_ORDERED && a.goal_mode != TS_GOAL_SET) return TS_E_BAD_ARGUMENT;
     if (a.bitmap_words < 4 || a.bitmap_words % 4 || a.queue_smem < 32 || (a.queue_smem & (a.queue_smem - 1))) return TS_E_BAD_ARGUMENT;
+    return 0;
+}
+
+// K9 and K10: shape and shared-memory plan
+template <class A> int check_item_plan(const A* a) {
+    if (!a) return TS_E_NULL_POINTER;
+    if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
+    if (a->size > 8) return TS_E_UNSUPPORTED;                                 // wide boards: no 64-bit board word
+    return check_search_plan(*a);
+}
+
+// K9 and K10: the env table the items are read from
+template <class A> int check_item_table(const A* a) {
+    if (a->capacity <= 0 || a->capacity % TS_CAP_ALIGN) return TS_E_BAD_CAPACITY;
+    if (a->n_items < 0 || (!a->d_env_ids && a->n_items > a->capacity)) return TS_E_BAD_RANGE;
+    if (!a->d_walls || !a->d_targets_packed || !a->d_pos) return TS_E_NULL_POINTER;
     return 0;
 }
 

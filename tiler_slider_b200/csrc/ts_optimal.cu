@@ -1,11 +1,11 @@
 // ts_optimal.cu -- K9: exact distance to the goal and the set of optimal first moves of many items
 // (env id, positions: the env's current ones or a caller's word), one CTA per item, on chip, and
 // optionally a shortest solution per item.  Built on K6's machinery (ts_bfs_local.cu; the CTA
-// shape, hash, plan check and launch are in ts_bfs_local.cuh): persistent CTAs drawing items from a
-// ticket counter, the visited set a shared-memory bitmap over the perfect hash of a state among the
-// free cells of its puzzle (or, in the device instances of 7x7 and 8x8 boards with four tiles, a
-// device-memory one), the frontier ring with a per-CTA HBM slab, the successor function
-// slide_env<S,T> and goal test of the step.
+// shape, hash, successor function, bitmap clear, plan and table checks and launch are in
+// ts_bfs_local.cuh): persistent CTAs drawing items from a ticket counter, the visited set a
+// shared-memory bitmap over the perfect hash of a state among the free cells of its puzzle (or, in
+// the device instances of 7x7 and 8x8 boards with four tiles, a device-memory one), the frontier ring
+// with a per-CTA HBM slab, the successor function slide_env<S,T> and goal test of the step.
 //
 //   0. Root: the item's word must be a well-formed state (every tile on an in-board free cell, no
 //      two on one cell), else TS_OPT_BAD_STATE -- the hash below is only defined for those.
@@ -93,17 +93,8 @@ __global__ void __launch_bounds__(SEARCH_THREADS, GMEM ? 5 : 0) optimal_moves_ke
         // ---- the item: walls, goal, root state, free-cell ranks ---------------------------------
         const uint64_t walls = load_board_elem<NB>(a.d_walls, cap, pid);
         const uint64_t free_cells = ~walls & cell_mask<S>();
-        const uint8_t* const root_pos = a.d_item_pos ? a.d_item_pos + (size_t)ticket * PW : a.d_pos + pid * PW;
-        uint32_t root = 0;
-        uint64_t occ = 0;
-        static_for<0, T>([&](auto I) {
-            constexpr int t = decltype(I)::value;
-            const uint32_t p = root_pos[t];
-            root |= p << (8 * t);
-            occ |= cell_bit<S>(p);
-        });
-        // each tile on its own free cell: an off-board byte adds no bit, two tiles on one cell one
-        if (__popcll(occ) != T || (occ & ~free_cells)) { no_solution(TS_OPT_BAD_STATE); continue; }
+        uint32_t root;
+        if (!read_root<S, T>(a, ticket, pid, free_cells, root)) { no_solution(TS_OPT_BAD_STATE); continue; }
         if (a.never_win) { no_solution(TS_OPT_UNSOLVABLE); continue; }   // no state meets the goal
         uint64_t tboard = 0;
         uint32_t tq = 0;
@@ -111,31 +102,18 @@ __global__ void __launch_bounds__(SEARCH_THREADS, GMEM ? 5 : 0) optimal_moves_ke
         else static_for<0, T>([&](auto I) { constexpr int t = decltype(I)::value; tq |= (uint32_t)a.d_targets_packed[pid * PW + t] << (8 * t); });
         if (a.goal_mode == TS_GOAL_SET) sort_bytes4<T>(root);
         const uint32_t F = (uint32_t)__popcll(free_cells);
-        if (tid < 128) {
-            const uint32_t bit = pos_to_bit<S>(tid);
-            lut[tid] = bit < 64 ? (uint8_t)__popcll(free_cells & ((1ull << bit) - 1ull)) : 0;
-        }
+        fill_lut<S>(tid, free_cells, lut);
         unsigned long long bits = 1;
 #pragma unroll
         for (int t = 0; t < T; ++t) bits *= (F > (uint32_t)t ? F - (uint32_t)t : 1u);
         const uint32_t words = (uint32_t)((bits + 31) / 32);
         if (words > (uint32_t)a.bitmap_words) { no_solution(TS_OPT_NOT_SEARCHED); continue; }
-        for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+        clear_bitmap(bitmap, words, tid);
         if (tid == 0) { cnt[0] = cnt[1] = cnt[2] = 0; lflag[0] = lflag[1] = lflag[2] = 0; }
         __syncthreads();
 
-        // state after move m (set goal: canonical); *won = it meets the goal
-        auto successor = [&](uint32_t q0, uint32_t m, bool& won) {
-            uint32_t q[1] = {q0};
-            slide_env<S, T>(q, walls, m >> 1, (m & 1u) ^ 1u);
-            if (a.goal_mode == TS_GOAL_SET) {
-                won = occupancy<S, T>(q) == tboard;
-                sort_bytes4<T>(q[0]);
-            } else {
-                won = q[0] == tq;
-            }
-            return q[0];
-        };
+        // state after move m (set goal: canonical); won = it meets the goal (ts_bfs_local.cuh)
+        auto successor = [&](uint32_t q0, uint32_t m, bool& won) { return ts::successor<S, T>(q0, m, walls, a.goal_mode == TS_GOAL_SET, tboard, tq, won); };
         auto marked = [&](uint32_t q) {
             const uint32_t idx = state_index<T>(lut, F, q);
             return (bitmap[idx >> 5] >> (idx & 31u)) & 1u;
@@ -207,7 +185,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS, GMEM ? 5 : 0) optimal_moves_ke
         // ---- 2. backward: mark the states of levels d-1 .. 1 that start a shortest solution ------
         const uint32_t D = (uint32_t)dist;
         if (D >= 2) {
-            for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+            clear_bitmap(bitmap, words, tid);
             __syncthreads();                      // bitmap clear, lstart complete
             for (uint32_t k = D - 1u; k >= 1u; --k) {
                 const uint32_t l0 = lstart[k], l1 = lstart[k + 1u];
@@ -310,26 +288,10 @@ static constexpr auto K9_PLAN = [](auto S, auto T, auto G) { return optimal_move
 
 using namespace ts;
 
-// shape and shared-memory plan
-static int optimal_check_plan(const ts_optimal_moves_args* a) {
-    if (!a) return TS_E_NULL_POINTER;
-    if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
-    if (a->size > 8) return TS_E_UNSUPPORTED;                                 // wide boards: no 64-bit board word
-    return check_search_plan(*a);
-}
-
-// the env table the listed envs are read from
-static int optimal_check_table(const ts_optimal_moves_args* a) {
-    if (a->capacity <= 0 || a->capacity % TS_CAP_ALIGN) return TS_E_BAD_CAPACITY;
-    if (a->n_items < 0 || (!a->d_env_ids && a->n_items > a->capacity)) return TS_E_BAD_RANGE;
-    if (!a->d_walls || !a->d_targets_packed || !a->d_pos) return TS_E_NULL_POINTER;
-    return 0;
-}
-
 // the checks of a launch before its empty-query return
 static int optimal_check_launch(const ts_optimal_moves_args* a) {
-    if (int rc = optimal_check_plan(a)) return rc;
-    if (int rc = optimal_check_table(a)) return rc;
+    if (int rc = check_item_plan(a)) return rc;
+    if (int rc = check_item_table(a)) return rc;
     if (a->max_depth < 1 || a->max_depth > TS_OPT_MAX_DEPTH || a->spill_per_cta < 1 || a->spill_per_cta > 0xFFFFFFFFll)
         return TS_E_BAD_ARGUMENT;
     if (!a->d_spill || !a->d_counters || !a->d_distance || !a->d_mask) return TS_E_NULL_POINTER;
@@ -337,7 +299,7 @@ static int optimal_check_launch(const ts_optimal_moves_args* a) {
 }
 
 template <bool GMEM> static int optimal_ctas_per_sm(const ts_optimal_moves_args* a, int* ctas_per_sm, int* n_sm) {
-    if (int rc = optimal_check_plan(a)) return rc;
+    if (int rc = check_item_plan(a)) return rc;
     return a->d_plan ? search_ctas_per_sm<GMEM>(K9_PLAN, *a, ctas_per_sm, n_sm) : search_ctas_per_sm<GMEM>(K9, *a, ctas_per_sm, n_sm);
 }
 
@@ -355,7 +317,7 @@ template <bool GMEM> static int optimal_launch(const ts_optimal_moves_args* a, u
 extern "C" {
 
 int ts_optimal_moves_smem_bytes(const ts_optimal_moves_args* a) {
-    if (int rc = optimal_check_plan(a)) return rc;
+    if (int rc = check_item_plan(a)) return rc;
     return (int)search_smem_bytes(*a);
 }
 
@@ -365,7 +327,7 @@ int ts_optimal_max_free_cells(const ts_optimal_moves_args* a, int32_t* d_max_fre
     if (!a) return TS_E_NULL_POINTER;
     if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
     if (a->size > 8) return TS_E_UNSUPPORTED;
-    if (int rc = optimal_check_table(a)) return rc;
+    if (int rc = check_item_table(a)) return rc;
     if (!d_max_free) return TS_E_NULL_POINTER;
     if (a->n_items == 0) return 0;
     const long long blocks = (a->n_items + 255) / 256;

@@ -3,7 +3,8 @@
 // definitions), one CTA per item, on chip.  K6/K9's machinery (ts_bfs_local.cuh): persistent CTAs
 // drawing items from a ticket counter, the visited set a shared-memory bitmap over the perfect hash
 // of a state among the free cells of its puzzle (or, in the device instances of 7x7 and 8x8 boards
-// with four tiles, a device-memory one), the frontier ring, slide_env<S,T> and the goal test.
+// with four tiles, a device-memory one), the frontier ring, and the successor function, bitmap clear
+// and plan and table checks written once there.
 // Two launches with one plan:
 //
 //   count  root check (TS_OPT_BAD_STATE, K9's rule), then a BFS to exhaustion; the ring spills to a
@@ -95,34 +96,21 @@ __global__ void __launch_bounds__(SEARCH_THREADS) state_table_kernel(const ts_st
         // ---- the item: walls, goal, root state, free-cell ranks (as K9) --------------------------
         const uint64_t walls = load_board_elem<NB>(a.d_walls, cap, pid);
         const uint64_t free_cells = ~walls & cell_mask<S>();
-        const uint8_t* const root_pos = a.d_item_pos ? a.d_item_pos + (size_t)ticket * PW : a.d_pos + pid * PW;
-        uint32_t root = 0;
-        uint64_t occ = 0;
-        static_for<0, T>([&](auto I) {
-            constexpr int t = decltype(I)::value;
-            const uint32_t p = root_pos[t];
-            root |= p << (8 * t);
-            occ |= cell_bit<S>(p);
-        });
-        if (__popcll(occ) != T || (occ & ~free_cells)) { if constexpr (!FILL) no_table(TS_OPT_BAD_STATE); continue; }
+        uint32_t root;
+        if (!read_root<S, T>(a, ticket, pid, free_cells, root)) { if constexpr (!FILL) no_table(TS_OPT_BAD_STATE); continue; }
         uint64_t tboard = 0;
         uint32_t tq = 0;
         if (a.goal_mode == TS_GOAL_SET) tboard = load_board_elem<NB>(a.d_targets_packed, cap, pid);
         else static_for<0, T>([&](auto I) { constexpr int t = decltype(I)::value; tq |= (uint32_t)a.d_targets_packed[pid * PW + t] << (8 * t); });
         if (a.goal_mode == TS_GOAL_SET) sort_bytes4<T>(root);
         const uint32_t F = (uint32_t)__popcll(free_cells);
-        if (tid < 128) {
-            const uint32_t bit = pos_to_bit<S>(tid);
-            const uint32_t rank = bit < 64 ? (uint32_t)__popcll(free_cells & ((1ull << bit) - 1ull)) : 0u;
-            lut[tid] = (uint8_t)rank;
-            if (FILL && (cell_bit<S>(tid) & free_cells)) rank_byte[rank] = (uint8_t)tid;
-        }
+        fill_lut<S>(tid, free_cells, lut, FILL ? rank_byte : nullptr);
         unsigned long long bits = 1;
 #pragma unroll
         for (int t = 0; t < T; ++t) bits *= (F > (uint32_t)t ? F - (uint32_t)t : 1u);
         const uint32_t words = (uint32_t)((bits + 31) / 32);
         if (words > (uint32_t)a.bitmap_words) { if constexpr (!FILL) no_table(TS_OPT_NOT_SEARCHED); continue; }
-        for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+        clear_bitmap(bitmap, words, tid);
         if (tid == 0) { cnt[0] = cnt[1] = cnt[2] = 0; lflag[0] = lflag[1] = lflag[2] = 0; s_won = 0; }
         __syncthreads();
 
@@ -134,18 +122,8 @@ __global__ void __launch_bounds__(SEARCH_THREADS) state_table_kernel(const ts_st
         auto stored = [&](uint32_t p) { if constexpr (FILL) return load_row<PW>(rows + (size_t)p * PW); else return slab[p]; };
         auto store = [&](uint32_t p, uint32_t q) { if constexpr (FILL) store_row<PW>(rows + (size_t)p * PW, q); else slab[p] = q; };
 
-        // state after move m (set goal: canonical); *won = it meets the goal
-        auto successor = [&](uint32_t q0, uint32_t m, bool& won) {
-            uint32_t q[1] = {q0};
-            slide_env<S, T>(q, walls, m >> 1, (m & 1u) ^ 1u);
-            if (a.goal_mode == TS_GOAL_SET) {
-                won = occupancy<S, T>(q) == tboard;
-                sort_bytes4<T>(q[0]);
-            } else {
-                won = q[0] == tq;
-            }
-            return q[0];
-        };
+        // state after move m (set goal: canonical); won = it meets the goal (ts_bfs_local.cuh)
+        auto successor = [&](uint32_t q0, uint32_t m, bool& won) { return ts::successor<S, T>(q0, m, walls, a.goal_mode == TS_GOAL_SET, tboard, tq, won); };
 
         if (tid == 0) {
             const uint32_t idx = state_index<T>(lut, F, root);
@@ -262,7 +240,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) state_table_kernel(const ts_st
 
             // ---- sweep: retrograde rounds over the rows ----------------------------------------------
             if (s_won && !a.never_win) {
-                for (uint32_t k = tid; k < (words + 3) / 4; k += SEARCH_THREADS) reinterpret_cast<uint4*>(bitmap)[k] = make_uint4(0u, 0u, 0u, 0u);
+                clear_bitmap(bitmap, words, tid);
                 if (tid == 0) s_progress[0] = s_progress[1] = 0;
                 for (int32_t round = 1;; ++round) {
                     __syncthreads();             // bitmap clear / previous round marked; rows and dist visible
@@ -321,13 +299,9 @@ using namespace ts;
 
 // shape, shared-memory plan and the env table (the checks of ts_optimal_moves)
 static int state_table_check(const ts_state_table_args* a, int grid) {
-    if (!a) return TS_E_NULL_POINTER;
-    if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
-    if (a->size > 8) return TS_E_UNSUPPORTED;                                 // wide boards: no 64-bit board word
-    if (int rc = check_search_plan(*a)) return rc;
-    if (a->capacity <= 0 || a->capacity % TS_CAP_ALIGN) return TS_E_BAD_CAPACITY;
-    if (a->n_items < 0 || (!a->d_env_ids && a->n_items > a->capacity)) return TS_E_BAD_RANGE;
-    if (!a->d_walls || !a->d_targets_packed || !a->d_pos || !a->d_counters || !a->d_status) return TS_E_NULL_POINTER;
+    if (int rc = check_item_plan(a)) return rc;
+    if (int rc = check_item_table(a)) return rc;
+    if (!a->d_counters || !a->d_status) return TS_E_NULL_POINTER;
     if (a->n_items > 0 && grid < 1) return TS_E_BAD_ARGUMENT;
     return 0;
 }
@@ -344,16 +318,8 @@ static int fill_check(const ts_state_table_args* a, int grid) {
     if (!a->d_offsets || !a->d_rows || !a->d_distance || !a->d_mask) return TS_E_NULL_POINTER;
     return 0;
 }
-// shape and shared-memory plan (the occupancy queries)
-static int occupancy_check(const ts_state_table_args* a) {
-    if (!a) return TS_E_NULL_POINTER;
-    if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
-    if (a->size > 8) return TS_E_UNSUPPORTED;
-    return check_search_plan(*a);
-}
-
 template <bool GMEM> static int table_ctas_per_sm(const ts_state_table_args* a, int* ctas_per_sm, int* n_sm) {
-    if (int rc = occupancy_check(a)) return rc;
+    if (int rc = check_item_plan(a)) return rc;
     if (!ctas_per_sm || !n_sm) return TS_E_NULL_POINTER;
     int count = 0, fill = 0;
     if (int rc = search_ctas_per_sm<GMEM>(K10<false>, *a, &count, n_sm)) return rc;
