@@ -561,6 +561,8 @@ int ts_bfs_local_gmem(const ts_bfs_local_args *a, uint32_t *d_bitmap, int grid, 
  *          when no move changes the state.  Targets = the final positions (ordered goal: tile i's;
  *          set goal: the cells).  Every such puzzle is solvable.
  * Domain: size <= 8, 1 <= n_tiles <= 4 (what K6 grades).
+ * ts_synth_candidates_t8: the same candidates, checks and stream rule for 5 <= n_tiles <= 8 (what
+ * K11 grades); ts_synth_candidates returns TS_E_UNSUPPORTED for those tile counts.
  * ------------------------------------------------------------------------------------- */
 #define TS_RECIPE_UNIFORM 0
 #define TS_RECIPE_WALK 1
@@ -574,6 +576,7 @@ typedef struct ts_synth_candidates_args {
     uint8_t *d_walls, *d_targets_packed, *d_init, *d_pos;
 } ts_synth_candidates_args;
 int ts_synth_candidates(const ts_synth_candidates_args *a, void *stream);
+int ts_synth_candidates_t8(const ts_synth_candidates_args *a, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * K8 ts_pool_reset: auto-reset into a pool of puzzles (csrc/ts_generate.cu; no reference
@@ -669,6 +672,27 @@ int ts_optimal_moves(const ts_optimal_moves_args *a, int grid, void *stream);
 /* device-memory bitmap (see ts_bfs_local_gmem): the instance with plans when d_plan is set */
 int ts_optimal_moves_gmem_ctas_per_sm(const ts_optimal_moves_args *a, int *ctas_per_sm, int *n_sm);
 int ts_optimal_moves_gmem(const ts_optimal_moves_args *a, uint32_t *d_bitmap, int grid, void *stream);
+
+/* ---------------------------------------------------------------------------------------
+ * K11 ts_optimal_moves_table: K9 for boards of size 3..8 with 5..8 tiles (csrc/ts_table_search.cu),
+ * the same struct, items, result definitions (d_distance, d_mask, d_plan) and counters, with the
+ * visited set a per-CTA hash table in device memory instead of the perfect-hash bitmap: CTA b owns
+ * d_table[b * table_slots ..] (uint64; contents on entry do not matter and are left undefined),
+ * table_slots a power of two >= 2 * spill_per_cta.  States are 64-bit words (pos_bytes 8).
+ *   d_spill        [grid][spill_per_cta] 64-bit entries (8-byte aligned); an item that discovers
+ *                  more than spill_per_cta states gets TS_OPT_NOT_SEARCHED (-3): the bound depends
+ *                  on the plan only, never on the other items of the launch.
+ *   bitmap_words   unused, must be 0; queue_smem: ring entries (64-bit) in shared memory, a power
+ *                  of two >= 32.
+ * Argument checks: ts_optimal_moves' checks in the same order with the same codes, with n_tiles
+ * outside 5..8 TS_E_UNSUPPORTED and bitmap_words != 0 TS_E_BAD_ARGUMENT; then table_slots not a
+ * power of two >= 2 * spill_per_cta (TS_E_BAD_ARGUMENT), a NULL d_table (TS_E_NULL_POINTER), a
+ * d_table or d_spill not 8-byte aligned (TS_E_MISALIGNED); all before the empty-query return.
+ * ts_optimal_moves_table_ctas_per_sm: resident CTAs per SM with the ring alone in shared memory
+ * (the instance with plans when d_plan is set) and the SM count.
+ * ------------------------------------------------------------------------------------- */
+int ts_optimal_moves_table_ctas_per_sm(const ts_optimal_moves_args *a, int *ctas_per_sm, int *n_sm);
+int ts_optimal_moves_table(const ts_optimal_moves_args *a, uint64_t *d_table, int64_t table_slots, int grid, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * K10 ts_state_table: every state reachable from items (env id, positions), each with K9's

@@ -192,6 +192,7 @@ SYMBOLS = {
     "ts_bfs_local_gmem_ctas_per_sm": (C.c_int, [C.POINTER(BfsLocalArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_bfs_local_gmem": (C.c_int, [C.POINTER(BfsLocalArgs), _vp, C.c_int, _vp]),
     "ts_synth_candidates": (C.c_int, [C.POINTER(SynthCandidatesArgs), _vp]),
+    "ts_synth_candidates_t8": (C.c_int, [C.POINTER(SynthCandidatesArgs), _vp]),
     "ts_pool_reset": (C.c_int, [C.POINTER(PoolResetArgs), _vp]),
     "ts_optimal_moves_smem_bytes": (C.c_int, [C.POINTER(OptimalMovesArgs)]),
     "ts_optimal_moves_ctas_per_sm": (C.c_int, [C.POINTER(OptimalMovesArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
@@ -199,6 +200,8 @@ SYMBOLS = {
     "ts_optimal_moves": (C.c_int, [C.POINTER(OptimalMovesArgs), C.c_int, _vp]),
     "ts_optimal_moves_gmem_ctas_per_sm": (C.c_int, [C.POINTER(OptimalMovesArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_optimal_moves_gmem": (C.c_int, [C.POINTER(OptimalMovesArgs), _vp, C.c_int, _vp]),
+    "ts_optimal_moves_table_ctas_per_sm": (C.c_int, [C.POINTER(OptimalMovesArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ts_optimal_moves_table": (C.c_int, [C.POINTER(OptimalMovesArgs), _vp, C.c_int64, C.c_int, _vp]),
     "ts_state_table_ctas_per_sm": (C.c_int, [C.POINTER(StateTableArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_state_table_count": (C.c_int, [C.POINTER(StateTableArgs), C.c_int, _vp]),
     "ts_state_table_fill": (C.c_int, [C.POINTER(StateTableArgs), C.c_int, _vp]),

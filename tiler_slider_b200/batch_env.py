@@ -174,7 +174,7 @@ class BatchedTilerSliderEnv:
     def solvable(cls, n_envs: int, size: int, n_tiles: int, n_walls: int, multi_color: bool = False, *,
                  min_depth: int = 1, max_depth: int = 30, recipe: str = "walk", walk_len: int | None = None,
                  seed: int = 0, env_index_base: int = 0, max_attempts: int | None = None, device_bitmap: bool = False,
-                 **kw) -> "BatchedTilerSliderEnv":
+                 hash_table: bool = False, **kw) -> "BatchedTilerSliderEnv":
         """Solvable puzzles whose shortest solution takes between `min_depth` and `max_depth` steps,
         generated and graded on the device (K7 candidates, K6 search; tiler_slider_b200/generate.py).
         `solve_depth` holds each env's shortest-solution length.  recipe "walk": targets where a
@@ -183,12 +183,15 @@ class BatchedTilerSliderEnv:
         depends on (seed, recipe, walk_len, band, env_index_base + i) only.  Sizes up to 8, 1..4 tiles.
         A 7x7 board with four tiles and fewer than 11 walls, or an 8x8 one with fewer than 26, has a
         state space too large for the shared-memory bitmap of the grading search: ValueError, unless
-        device_bitmap=True, which grades such boards with the bitmap in device memory."""
+        device_bitmap=True, which grades such boards with the bitmap in device memory.
+        hash_table=True also takes 5..8 tiles (sizes 3..8): K7 candidates graded by K11's distance of
+        their initial positions (optimal_moves(hash_table=True), bounded at max_depth <= 254); a
+        candidate whose search outgrows the plan's bound (-3) is rejected like one outside the band."""
         from .generate import DEFAULT_MAX_ATTEMPTS, solvable
         return solvable(cls, n_envs, size, n_tiles, n_walls, multi_color, min_depth=min_depth, max_depth=max_depth,
                         recipe=recipe, walk_len=walk_len, seed=seed, env_index_base=env_index_base,
                         max_attempts=DEFAULT_MAX_ATTEMPTS if max_attempts is None else max_attempts,
-                        device_bitmap=device_bitmap, **kw)
+                        device_bitmap=device_bitmap, hash_table=hash_table, **kw)
 
     def encode(self, blocked: torch.Tensor, tiles: torch.Tensor, targets: torch.Tensor) -> None:
         """K1: dense description -> packed planes (GameState.__init__, state.py:61-73)."""
@@ -814,7 +817,7 @@ class BatchedTilerSliderEnv:
         return mask[: self.n_envs]
 
     def optimal_moves(self, ids=None, pos: torch.Tensor | None = None, *, max_depth: int = 254,
-                      paths: bool = False, device_bitmap: bool = False) -> tuple[torch.Tensor, ...]:
+                      paths: bool = False, device_bitmap: bool = False, hash_table: bool = False) -> tuple[torch.Tensor, ...]:
         """Exact solver answers for items (K9, ts_optimal_moves), as supervision for imitation
         learning, value targets, optimality gaps, reward shaping or an exact expert policy.  Items as
         expand() takes them: ids (default every env) give the puzzles, pos (default each listed
@@ -828,7 +831,9 @@ class BatchedTilerSliderEnv:
                     one CTA can hold in shared memory (4 tiles on a 7x7 board with fewer than 11
                     walls or an 8x8 one with fewer than 26; with device_bitmap=True such boards
                     are searched with the bitmap in device memory instead), or than the slab of
-                    the launch (it does not depend on the other items of the query), -4 the
+                    the launch (it does not depend on the other items of the query; with
+                    hash_table=True and 5 to 8 tiles: the item discovered more states than the
+                    plan's bound, see below), -4 the
                     position word is not a well-formed state of
                     its env (a tile on a wall or off the board, two tiles on one cell; e.g. the
                     zero rows playout(record=True) writes past an item's end);
@@ -842,18 +847,22 @@ class BatchedTilerSliderEnv:
                     distance moves.  distance and mask are the same with and without paths.
         Ids are range-checked against [0, n_envs) (IndexError), host and device ids alike.  Runs on
         the current stream after the steps queued before it, reads one scalar back, and changes no
-        env state.  Sizes up to 8, 1..4 tiles, device-memory batches (not host_io)."""
+        env state.  Sizes up to 8, 1..4 tiles, device-memory batches (not host_io).
+        hash_table=True also takes 5..8 tiles (K11, ts_optimal_moves_table): the same answers from a
+        search whose visited set is a per-CTA hash table in device memory, bounded by the plan's
+        spill_per_cta discovered states per item (-3 beyond); it reads nothing back.  With 1..4 tiles
+        it changes nothing."""
         from .bfs import CudaOptimalMoves, check_optimal_moves
-        check_optimal_moves(self.size, self.n_tiles, self.host_io, int(max_depth))
+        check_optimal_moves(self.size, self.n_tiles, self.host_io, int(max_depth), hash_table=bool(hash_table))
         self._require_loaded()
         ids = self._search_items("optimal_moves", ids, pos)
         if self._optimal is None:
             self._optimal = CudaOptimalMoves(self)
         if not paths:
-            return self._optimal.query(ids, int(max_depth), pos, device_bitmap=bool(device_bitmap))
+            return self._optimal.query(ids, int(max_depth), pos, device_bitmap=bool(device_bitmap), hash_table=bool(hash_table))
         n = self.n_envs if ids is None else ids.numel()
         plan = torch.empty((int(max_depth), n), dtype=torch.uint8, device=self.device)
-        return (*self._optimal.query(ids, int(max_depth), pos, plan, bool(device_bitmap)), plan)
+        return (*self._optimal.query(ids, int(max_depth), pos, plan, bool(device_bitmap), bool(hash_table)), plan)
 
     def state_table(self, ids=None, pos: torch.Tensor | None = None, *, device_bitmap: bool = False) -> StateTable:
         """Every state reachable from items, each with its exact distance to a win and its optimal

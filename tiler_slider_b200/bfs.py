@@ -678,13 +678,16 @@ class OnChipSearch:
     MAX_SCRATCH_BYTES = 4 << 30
     CTAS_PER_SM = ""                # the library's occupancy query of the front-end's kernel
     GMEM_CTAS_PER_SM = ""           # ... of its device-memory-bitmap instance
+    TABLE_CTAS_PER_SM = ""          # ... of its hash-table instance (5 to 8 tiles)
     GMEM_SHAPES = ((7, 4), (8, 4))  # (size, tiles) with device instances: boards a shared bitmap may not hold
     ARGS = None                     # the argument struct of the front-end's entry points (K9, K10: _args)
 
-    def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None):
+    def __init__(self, table: BatchedTilerSliderEnv, ctas_per_sm: int | None = None, queue_smem: int | None = None,
+                 table_slots: int | None = None):
         self.t, self.lib, self.device = table, lib(), table.device
         self.want_ctas = ctas_per_sm
         self.want_queue = queue_smem
+        self.want_slots = table_slots   # tests: force a small hash table (and so a small bound)
         self._plans: dict = {}
         self._scratch: dict[str, torch.Tensor] = {}
         self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)   # K9, K10: of the last call, see include/tiler_slider.h
@@ -748,6 +751,33 @@ class OnChipSearch:
                 return {**plan, "gmem": True} if gmem else plan
         return None
 
+    def _plan_table(self) -> dict | None:
+        """The plan of the hash-table instance (5 to 8 tiles, marked table=True): the same CTA-per-SM
+        loop as _plan with a ring of 8-byte entries alone in shared memory; per CTA a table of
+        table_slots 8-byte slots (the largest power of two with grid x 12 x table_slots <=
+        MAX_SCRATCH_BYTES, or the constructor's table_slots) and a slab of spill_per_cta =
+        table_slots / 2 entries, the states an item may discover.  It does not depend on the envs'
+        walls, so it needs no free-cell read-back."""
+        if "table" not in self._plans:
+            self._plans["table"] = {}
+            query = getattr(self.lib, self.TABLE_CTAS_PER_SM)
+            for k in ([self.want_ctas] if self.want_ctas else [8, 6, 5, 4, 3, 2, 1]):
+                budget = self.SMEM_PER_SM // k - self.STATIC_SMEM
+                queue = 1 << (min(budget, 64 * 1024) // 8).bit_length() - 1                    # ring entries: a power of two
+                if self.want_queue is not None:
+                    queue = max(32, 1 << (min(queue, self.want_queue).bit_length() - 1))
+                a = self._args(bitmap_words=0, queue_smem=queue)
+                got, n_sm = C.c_int(0), C.c_int(0)
+                with torch.cuda.device(self.device):
+                    rc = query(C.byref(a), C.byref(got), C.byref(n_sm))
+                if rc == 0 and got.value >= (k if self.want_ctas is None else 1):
+                    grid = got.value * n_sm.value
+                    slots = self.want_slots or 1 << (self.MAX_SCRATCH_BYTES // (12 * grid)).bit_length() - 1
+                    self._plans["table"] = dict(bitmap_words=0, queue_smem=queue, grid=grid, ctas_per_sm=got.value,
+                                                table_slots=slots, spill_per_cta=slots // 2, table=True)
+                    break
+        return self._plans["table"] or None
+
     def search_plan(self, f_max: int, device_bitmap: bool = False) -> dict | None:
         """The plan of a query whose envs have up to f_max free cells, one rule for K9 and K10: the
         shared plan for f_max when it exists; else, with device_bitmap on a shape that has device
@@ -766,8 +796,13 @@ class OnChipSearch:
 
     def _launch(self, entry: str, a, plan: dict, stream) -> None:
         """Launch the library's `entry` with arguments a on plan's grid; with a gmem plan its device
-        counterpart `entry`_gmem, on the bitmaps of _bitmap."""
-        if plan.get("gmem"):
+        counterpart `entry`_gmem, on the bitmaps of _bitmap; with a table plan `entry`_table, on
+        grid x table_slots cached 8-byte slots (contents undefined)."""
+        if plan.get("table"):
+            entry += "_table"
+            tab = self._buf("table", plan["grid"] * plan["table_slots"], torch.int64).data_ptr()
+            rc = getattr(self.lib, entry)(C.byref(a), tab, plan["table_slots"], plan["grid"], stream)
+        elif plan.get("gmem"):
             entry += "_gmem"
             rc = getattr(self.lib, entry)(C.byref(a), self._bitmap(plan), plan["grid"], stream)
         else:
@@ -881,13 +916,14 @@ class CudaLocalKernels(OnChipSearch):
             self._launch("ts_bfs_local", a, plan, stream)
 
 
-def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int, what: str = "optimal_moves") -> None:
-    """The shapes ts_optimal_moves (and ts_state_table, `what`) covers; raised before anything
-    touches the device."""
+def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int, what: str = "optimal_moves",
+                        hash_table: bool = False) -> None:
+    """The shapes ts_optimal_moves (and ts_state_table, `what`) covers, with hash_table also those
+    of ts_optimal_moves_table (5 to 8 tiles); raised before anything touches the device."""
     if size > 8:
         raise ValueError(f"{what} covers board sizes up to 8 (got {size})")
-    if not 1 <= n_tiles <= 4:
-        raise ValueError(f"{what} covers 1 to 4 tiles (got {n_tiles})")
+    if not 1 <= n_tiles <= (8 if hash_table else 4):
+        raise ValueError(f"{what} covers 1 to {8 if hash_table else 4} tiles (got {n_tiles})")
     if host_io:
         raise ValueError(f"{what} is not available for host_io batches")
     if not 1 <= max_depth <= OPT_MAX_DEPTH:
@@ -904,16 +940,19 @@ class CudaOptimalMoves(OnChipSearch):
 
     CTAS_PER_SM = "ts_optimal_moves_ctas_per_sm"
     GMEM_CTAS_PER_SM = "ts_optimal_moves_gmem_ctas_per_sm"
+    TABLE_CTAS_PER_SM = "ts_optimal_moves_table_ctas_per_sm"
     ARGS = OptimalMovesArgs
 
     def query(self, ids: torch.Tensor | None, max_depth: int, pos: torch.Tensor | None = None,
-              plan: torch.Tensor | None = None, device_bitmap: bool = False) -> tuple[torch.Tensor, torch.Tensor]:
+              plan: torch.Tensor | None = None, device_bitmap: bool = False,
+              hash_table: bool = False) -> tuple[torch.Tensor, torch.Tensor]:
         """(distance int32[n], mask uint8[n]) of items (env `ids[i]`, positions `pos[i]`) on the
         current stream.  ids: int32 on the device, each in [0, n_envs) (None: every env); pos:
         contiguous uint8 [n, pos_bytes] on the device (None: the envs' current positions); plan:
         uint8 [max_depth, n] on the device that receives a shortest solution per item (every entry
         is written); device_bitmap: envs too large for a shared-memory bitmap are searched with one
-        in device memory (search_plan)."""
+        in device memory (search_plan); hash_table: 5 to 8 tiles are searched by K11
+        (ts_optimal_moves_table, _plan_table); it changes nothing for 1 to 4 tiles."""
         t, dev = self.t, self.device
         n = t.n_envs if ids is None else ids.numel()
         distance = torch.full((n,), OPT_NOT_SEARCHED, dtype=torch.int32, device=dev)
@@ -926,14 +965,15 @@ class CudaOptimalMoves(OnChipSearch):
         with torch.cuda.device(dev):
             # one plan with and without paths: the same grid and slab, so the same answers (the plan
             # kernel instance may fit fewer CTAs per SM; the surplus CTAs find no ticket left)
-            sp = self.search_plan(self._max_free_cells(ids, n), device_bitmap)
+            table = hash_table and t.n_tiles >= 5
+            sp = self._plan_table() if table else self.search_plan(self._max_free_cells(ids, n), device_bitmap)
             if sp is None:                       # not even T free cells fit on chip
                 if plan is not None:
                     plan.fill_(255)
                 return distance, mask
             a = self._args(n_items=n, d_env_ids=ids_ptr, max_depth=int(max_depth), bitmap_words=sp["bitmap_words"],
                            queue_smem=sp["queue_smem"], spill_per_cta=sp["spill_per_cta"],
-                           d_spill=self._buf("spill", sp["grid"] * sp["spill_per_cta"], torch.int32).data_ptr(),
+                           d_spill=self._buf("spill", sp["grid"] * sp["spill_per_cta"], torch.int64 if table else torch.int32).data_ptr(),
                            d_counters=self.counters.data_ptr(), d_distance=distance.data_ptr(), d_mask=mask.data_ptr(),
                            d_item_pos=None if pos is None else pos.data_ptr(),
                            d_plan=None if plan is None else plan.data_ptr())

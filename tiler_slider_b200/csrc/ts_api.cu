@@ -142,11 +142,12 @@ int ts_synth(const ts_synth_args* a, void* stream) {
     return cuda_result(cudaGetLastError(), "ts_synth launch");
 }
 
-int ts_synth_candidates(const ts_synth_candidates_args* a, void* stream) {
+// K7's checks and launch for the tile counts t_lo..t_hi of one entry point
+static int synth_candidates(const ts_synth_candidates_args* a, void* stream, int t_lo, int t_hi) {
     if (!a) return fail(TS_E_NULL_POINTER, "null args");
     if (int rc = check_shape(a->size, a->n_tiles, 0, 0, a->capacity)) return rc;
-    if (a->size > 8 || a->n_tiles < 1 || a->n_tiles > 4)
-        return fail(TS_E_UNSUPPORTED, "candidates cover sizes up to 8 with 1 to 4 tiles (size %d, n_tiles %d)", a->size, a->n_tiles);
+    if (a->size > 8 || a->n_tiles < t_lo || a->n_tiles > t_hi)
+        return fail(TS_E_UNSUPPORTED, "candidates cover sizes up to 8 with %d to %d tiles (size %d, n_tiles %d)", t_lo, t_hi, a->size, a->n_tiles);
     if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return fail(TS_E_BAD_ARGUMENT, "goal_mode %d", a->goal_mode);
     if (a->recipe != TS_RECIPE_UNIFORM && a->recipe != TS_RECIPE_WALK) return fail(TS_E_BAD_ARGUMENT, "recipe %d", a->recipe);
     if (a->walk_len < 0 || a->walk_len > TS_MAX_WALK) return fail(TS_E_BAD_ARGUMENT, "walk_len %d outside 0..%d", a->walk_len, TS_MAX_WALK);
@@ -161,6 +162,8 @@ int ts_synth_candidates(const ts_synth_candidates_args* a, void* stream) {
     if (a->n_items == 0) return 0;
     return cuda_result(candidates_dispatch(*a, (cudaStream_t)stream), "ts_synth_candidates launch");
 }
+int ts_synth_candidates(const ts_synth_candidates_args* a, void* stream) { return synth_candidates(a, stream, 1, 4); }
+int ts_synth_candidates_t8(const ts_synth_candidates_args* a, void* stream) { return synth_candidates(a, stream, 5, 8); }
 
 int ts_pool_reset(const ts_pool_reset_args* a, void* stream) {
     if (!a) return fail(TS_E_NULL_POINTER, "null args");

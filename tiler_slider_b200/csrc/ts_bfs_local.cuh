@@ -2,7 +2,8 @@
 // (ts_optimal.cu, the optimal-move query) and K10 (ts_state_table.cu, the state tables), share: the
 // CTA shape, canonical set-goal states, position byte -> bitboard bit, the perfect hash of a state
 // over the free cells of its puzzle that keys the visited bitmap, the successor function, the lut
-// fill, the bitmap clear and K9 and K10's root read; on the host the plan and env-table checks of K9 and K10, the plan check, the
+// fill, the bitmap clear and K9 and K10's root read (and their 64-bit siblings for K11's 5..8 tiles,
+// ts_table_search.cu); on the host the plan and env-table checks of K9 and K10, the plan check, the
 // shared-memory size, the launch and the occupancy query, one each for the shared instances and the
 // device-memory-bitmap instances (GMEM) of 7x7 and 8x8 boards with four tiles.
 #pragma once
@@ -83,6 +84,54 @@ __device__ __forceinline__ uint32_t successor(uint32_t q0, uint32_t m, uint64_t 
         won = q[0] == tq;
     }
     return q[0];
+}
+
+// ---- 64-bit states (K11, 5..8 tiles): the 8 position bytes of a state as one word ----------------
+// canonical form of a set-goal state of T <= 8 tiles: its T position bytes sorted ascending
+template <int T> __device__ __forceinline__ void sort_bytes8(uint64_t& q) {
+    uint32_t b[T];
+    static_for<0, T>([&](auto I) { constexpr int i = decltype(I)::value; b[i] = (uint32_t)(q >> (8 * i)) & 0xFFu; });
+#pragma unroll
+    for (int round = 0; round < T; ++round)
+#pragma unroll
+        for (int i = round & 1; i + 1 < T; i += 2) {
+            const uint32_t lo = min(b[i], b[i + 1]), hi = max(b[i], b[i + 1]);
+            b[i] = lo; b[i + 1] = hi;
+        }
+    q = 0;
+    static_for<0, T>([&](auto I) { constexpr int i = decltype(I)::value; q |= (uint64_t)b[i] << (8 * i); });
+}
+
+// successor<S,T> for 5..8 tiles: the same slide, goal test and canonicalisation on a 64-bit word
+template <int S, int T>
+__device__ __forceinline__ uint64_t successor64(uint64_t q0, uint32_t m, uint64_t walls, bool set_goal, uint64_t tboard, uint64_t tq, bool& won) {
+    static_assert(T >= 5 && T <= 8, "two 32-bit position words");
+    uint32_t q[2] = {(uint32_t)q0, (uint32_t)(q0 >> 32)};
+    slide_env<S, T>(q, walls, m >> 1, (m & 1u) ^ 1u);
+    uint64_t qn = (uint64_t)q[1] << 32 | q[0];
+    if (set_goal) {
+        won = occupancy<S, T>(q) == tboard;
+        sort_bytes8<T>(qn);
+    } else {
+        won = qn == tq;
+    }
+    return qn;
+}
+
+// read_root<S,T> for 5..8 tiles: the root word of an item and whether it is a well-formed state
+template <int S, int T, class A>
+__device__ __forceinline__ bool read_root64(const A& a, long long ticket, size_t pid, uint64_t free_cells, uint64_t& root) {
+    constexpr int PW = pos_bytes(T);
+    const uint8_t* const root_pos = a.d_item_pos ? a.d_item_pos + (size_t)ticket * PW : a.d_pos + pid * PW;
+    uint64_t occ = 0;
+    root = 0;
+    static_for<0, T>([&](auto I) {
+        constexpr int t = decltype(I)::value;
+        const uint32_t p = root_pos[t];
+        root |= (uint64_t)p << (8 * t);
+        occ |= cell_bit<S>(p);
+    });
+    return __popcll(occ) == T && !(occ & ~free_cells);
 }
 
 // position byte -> rank among the free cells (lut, 128 entries) and, given rank_byte, rank -> position

@@ -6,7 +6,8 @@
 // (explainrl/environment/environment.py:221-226, K0 here), of which about 1 % are solvable for the
 // benchmark shape, and its reset (environment.py:89-97) restarts the same puzzle.
 //
-// K7: one thread per listed env slot.  The uniform recipe IS K0's draw (synth_env, ts_synth.cuh),
+// K7: one thread per listed env slot, positions in (T+3)/4 32-bit words (1..4 tiles: K6 grades the
+// candidates; 5..8 tiles, ts_synth_candidates_t8: K11 does).  The uniform recipe IS K0's draw (synth_env, ts_synth.cuh),
 // with a fresh seed per attempt after the first.  The walk recipe keeps K0's walls and tiles and
 // slides the tiles with slide_env<S,T> -- the step's own device code -- along a random walk of
 // state-changing moves; the targets are where the tiles end up, so every candidate is solvable.
@@ -32,7 +33,7 @@ __device__ __forceinline__ uint64_t attempt_seed(uint64_t seed, uint32_t attempt
 template <int S, int T>
 __global__ void __launch_bounds__(GEN_THREADS) synth_candidates_kernel(const ts_synth_candidates_args a) {
     constexpr int CELLS = S * S, PW = pos_bytes(T), PS = pos_stride(S), BS = board_stride(S), NB = board_bytes(S);
-    static_assert(T >= 1 && T <= 4 && S <= 8, "K6's domain: one 32-bit position word, one 64-bit board");
+    static_assert(T >= 1 && T <= 8 && S <= 8, "1..8 tiles, one 64-bit board");
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n_items) return;
     const int64_t slot = a.d_env_ids ? (int64_t)a.d_env_ids[i] : i;
@@ -52,18 +53,26 @@ __global__ void __launch_bounds__(GEN_THREADS) synth_candidates_kernel(const ts_
     uint64_t walls = 0;
     if constexpr (padded_board(S)) walls = Padded<S>::SENT;         // the stored sentinels (ts_common.cuh)
     for (int d = 0; d < W; ++d) walls |= 1ull << ((perm[d] / S) * BS + perm[d] % S);
-    uint32_t q[1] = {0u};
+    constexpr int PR = (T + 3) / 4;                                  // 32-bit position words
+    uint32_t q[PR] = {};
 #pragma unroll
-    for (int t = 0; t < T; ++t) q[0] |= (uint32_t)((perm[W + t] / S) * PS + perm[W + t] % S) << (8 * t);
-    const uint32_t init = q[0];
+    for (int t = 0; t < T; ++t) q[t / 4] |= (uint32_t)((perm[W + t] / S) * PS + perm[W + t] % S) << (8 * (t % 4));
+    const uint32_t init = q[0], init_hi = q[PR - 1];           // init_hi: tiles 4..7 (5..8 tiles)
     for (int s = 0; s < a.walk_len; ++s) {
-        uint32_t nxt[4], mask = 0;
+        uint32_t nxt[4][PR], mask = 0;
 #pragma unroll
         for (int d = 0; d < 4; ++d) {
-            uint32_t x[1] = {q[0]};
+            uint32_t x[PR];
+#pragma unroll
+            for (int w = 0; w < PR; ++w) x[w] = q[w];
             slide_env<S, T>(x, walls, (uint32_t)d >> 1, ((uint32_t)d & 1u) ^ 1u);
-            nxt[d] = x[0];
-            mask |= (uint32_t)(x[0] != q[0]) << d;
+            uint32_t changed = 0;
+#pragma unroll
+            for (int w = 0; w < PR; ++w) {
+                nxt[d][w] = x[w];
+                changed |= x[w] ^ q[w];
+            }
+            mask |= (uint32_t)(changed != 0u) << d;
         }
         const int n = __popc(mask);
         if (n == 0) break;                                           // nothing can move: the walk ends here
@@ -71,22 +80,23 @@ __global__ void __launch_bounds__(GEN_THREADS) synth_candidates_kernel(const ts_
         uint32_t m = mask;
         for (int k = (int)(((uint64_t)r * (uint32_t)n) >> 32); k > 0; --k) m &= m - 1u;   // k-th state-changing move
         const int d = __ffs(m) - 1;
-        q[0] = d == 0 ? nxt[0] : d == 1 ? nxt[1] : d == 2 ? nxt[2] : nxt[3];
+#pragma unroll
+        for (int w = 0; w < PR; ++w) q[w] = d == 0 ? nxt[0][w] : d == 1 ? nxt[1][w] : d == 2 ? nxt[2][w] : nxt[3][w];
     }
     for (int b = 0; b < NB; ++b) a.d_walls[board_byte_addr(NB, cap, env, b)] = (uint8_t)(walls >> (8 * b));
 #pragma unroll
     for (int t = 0; t < PW; ++t) {
-        a.d_init[env * PW + t] = (uint8_t)(init >> (8 * t));
-        a.d_pos[env * PW + t] = (uint8_t)(init >> (8 * t));
+        a.d_init[env * PW + t] = (uint8_t)((t < 4 ? init : init_hi) >> (8 * (t % 4)));
+        a.d_pos[env * PW + t] = (uint8_t)((t < 4 ? init : init_hi) >> (8 * (t % 4)));
     }
     if (a.goal_mode == TS_GOAL_ORDERED) {
 #pragma unroll
-        for (int t = 0; t < PW; ++t) a.d_targets_packed[env * PW + t] = (uint8_t)(q[0] >> (8 * t));
+        for (int t = 0; t < PW; ++t) a.d_targets_packed[env * PW + t] = (uint8_t)(q[t / 4] >> (8 * (t % 4)));
     } else {
         uint64_t tb = 0;                                             // target board: no sentinels
 #pragma unroll
         for (int t = 0; t < T; ++t) {
-            const uint32_t p = (q[0] >> (8 * t)) & 0xFFu;
+            const uint32_t p = (q[t / 4] >> (8 * (t % 4))) & 0xFFu;
             tb |= 1ull << (padded_board(S) ? p : (p >> 4) * (uint32_t)S + (p & 15u));
         }
         for (int b = 0; b < NB; ++b) a.d_targets_packed[board_byte_addr(NB, cap, env, b)] = (uint8_t)(tb >> (8 * b));
@@ -95,9 +105,16 @@ __global__ void __launch_bounds__(GEN_THREADS) synth_candidates_kernel(const ts_
 
 cudaError_t candidates_dispatch(const ts_synth_candidates_args& a, cudaStream_t st) {
     const unsigned blocks = (unsigned)((a.n_items + GEN_THREADS - 1) / GEN_THREADS);
-    return dispatch_small(a.size, a.n_tiles, [&](auto S, auto T) {
+    auto go = [&](auto S, auto T) {
         synth_candidates_kernel<decltype(S)::value, decltype(T)::value><<<blocks, GEN_THREADS, 0, st>>>(a);
         return cudaGetLastError();
+    };
+    if (a.n_tiles <= 4) return dispatch_small(a.size, a.n_tiles, go);
+    // 5..8 tiles (ts_synth_candidates_t8): boards of size 3..8, the ones that hold them
+    return dispatch_size(a.size, [&](auto S) {
+        constexpr int SV = decltype(S)::value;
+        if constexpr (SV < 3) return cudaErrorInvalidValue;
+        else return dispatch_tiles<5, 8>(a.n_tiles, [&](auto T) { return go(S, T); });
     });
 }
 
