@@ -746,6 +746,47 @@ int ts_state_table_count_gmem(const ts_state_table_args *a, uint32_t *d_bitmap, 
 int ts_state_table_fill_gmem(const ts_state_table_args *a, uint32_t *d_bitmap, int grid, void *stream);
 
 /* ---------------------------------------------------------------------------------------
+ * K12 ts_state_table_*_table: K10 for boards of size 3..8 with 5..8 tiles
+ * (csrc/ts_table_state_table.cu), the same struct, items, passes and result definitions, with
+ * K11's visited set: CTA b owns d_table[b * table_slots ..] (uint64; contents on entry do not
+ * matter and are left undefined), table_slots a power of two >= 2 * spill_per_cta.  States are
+ * 64-bit words (pos_bytes 8).  Both passes take the same arguments, grid, d_spill and d_table.
+ *   d_spill        [grid][spill_per_cta] 64-bit entries (8-byte aligned), used by BOTH passes: the
+ *                  count pass's queue, and the fill pass's queue and sort buffer.
+ *   bitmap_words   unused, must be 0; queue_smem: ring entries (64-bit) in shared memory, a power
+ *                  of two >= 32.
+ *   ts_state_table_count_table  forward BFS from each root to exhaustion (never_win included):
+ *     d_status[i]   0 enumerated; TS_OPT_NOT_SEARCHED (-3) more than spill_per_cta states are
+ *                   reachable, the root included (the bound depends on spill_per_cta alone, never on
+ *                   the grid or the other items), or e is outside [0, capacity); TS_OPT_BAD_STATE
+ *                   (-4) the root is not a well-formed state (K9's rule)
+ *     d_count[i]    int64: the states reachable from the root, the root included (0 if status != 0)
+ *     d_counters    [0] ticket (zero on entry)
+ *   the caller sets d_offsets (int64 [n_items + 1]) to the exclusive cumsum of d_count, then
+ *   ts_state_table_fill_table   for each item with status 0 (the others are skipped), rows
+ *     [d_offsets[i], d_offsets[i+1]) of:
+ *     d_rows        uint8 [rows][8] (8-byte aligned): each reachable state exactly once (set goal:
+ *                   canonical, bytes ascending; padding bytes 0, never flag bits), in strictly
+ *                   ascending order of the row's 8 bytes read as a little-endian 64-bit word
+ *                   (deterministic: independent of the grid, the ring and the atomics)
+ *     d_distance    int32 [rows]: K11's distance of the row's state (>= 1), or -1 if no win is
+ *                   reachable from it (never_win: every row)
+ *     d_mask        uint8 [rows]: K11's mask of the row's state (0 where distance < 0)
+ *     d_counters    [1] ticket (zero on entry), [2] += rows swept by the retrograde rounds
+ * Argument checks, all before the empty-query return: ts_optimal_moves_table's plan checks (size,
+ * 5..8 tiles, goal mode, bitmap_words == 0, the ring), the env table, then K10's checks of the pass
+ * (d_counters, d_status, grid < 1 with n_items > 0; count: spill_per_cta, d_spill, d_count; fill:
+ * d_offsets, d_rows, d_distance, d_mask), then for both passes spill_per_cta outside 1..2^32-1
+ * (TS_E_BAD_ARGUMENT) and a NULL d_spill (TS_E_NULL_POINTER), table_slots not a power of two >=
+ * 2 * spill_per_cta (TS_E_BAD_ARGUMENT), a NULL d_table (TS_E_NULL_POINTER), a d_table, d_spill or
+ * (fill) d_rows not 8-byte aligned (TS_E_MISALIGNED).
+ * ts_state_table_table_ctas_per_sm: resident CTAs per SM of both kernels (the fewer) and the SM count.
+ * ------------------------------------------------------------------------------------- */
+int ts_state_table_table_ctas_per_sm(const ts_state_table_args *a, int *ctas_per_sm, int *n_sm); /* fewer of the two passes */
+int ts_state_table_count_table(const ts_state_table_args *a, uint64_t *d_table, int64_t table_slots, int grid, void *stream);
+int ts_state_table_fill_table(const ts_state_table_args *a, uint64_t *d_table, int64_t table_slots, int grid, void *stream);
+
+/* ---------------------------------------------------------------------------------------
  * ts_step_host: the same step through HOST buffers (the call a host-side driver makes):
  * h_actions (pinned) -> device, ts_step, reward/done -> h_reward/h_done (pinned), pipelined in
  * chunks over the context's streams; returns after everything has landed.

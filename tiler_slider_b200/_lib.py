@@ -208,6 +208,9 @@ SYMBOLS = {
     "ts_state_table_gmem_ctas_per_sm": (C.c_int, [C.POINTER(StateTableArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "ts_state_table_count_gmem": (C.c_int, [C.POINTER(StateTableArgs), _vp, C.c_int, _vp]),
     "ts_state_table_fill_gmem": (C.c_int, [C.POINTER(StateTableArgs), _vp, C.c_int, _vp]),
+    "ts_state_table_table_ctas_per_sm": (C.c_int, [C.POINTER(StateTableArgs), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ts_state_table_count_table": (C.c_int, [C.POINTER(StateTableArgs), _vp, C.c_int64, C.c_int, _vp]),
+    "ts_state_table_fill_table": (C.c_int, [C.POINTER(StateTableArgs), _vp, C.c_int64, C.c_int, _vp]),
     "ts_host_ctx_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "ts_host_ctx_destroy": (C.c_int, [_vp]),
     "ts_step_host": (C.c_int, [_vp, C.POINTER(StepArgs), _vp, _vp, _vp, _vp, _i64]),

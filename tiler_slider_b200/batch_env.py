@@ -864,7 +864,8 @@ class BatchedTilerSliderEnv:
         plan = torch.empty((int(max_depth), n), dtype=torch.uint8, device=self.device)
         return (*self._optimal.query(ids, int(max_depth), pos, plan, bool(device_bitmap), bool(hash_table)), plan)
 
-    def state_table(self, ids=None, pos: torch.Tensor | None = None, *, device_bitmap: bool = False) -> StateTable:
+    def state_table(self, ids=None, pos: torch.Tensor | None = None, *, device_bitmap: bool = False,
+                    hash_table: bool = False, max_states: int | None = None) -> StateTable:
         """Every state reachable from items, each with its exact distance to a win and its optimal
         moves (K10, ts_state_table), for value / policy datasets over whole state spaces, reverse
         curricula (states a chosen distance from the goal) and puzzle statistics (dead states, the
@@ -882,14 +883,30 @@ class BatchedTilerSliderEnv:
         Ids are range-checked as in optimal_moves() (IndexError).  Runs on the current stream,
         changes no env state and reads back two scalars (the free-cell maximum and the row count,
         to allocate), so it cannot be captured in a CUDA graph.  Sizes up to 8, 1..4 tiles,
-        device-memory batches (not host_io)."""
+        device-memory batches (not host_io).
+        hash_table=True also takes 5..8 tiles (K12, ts_state_table_count_table / _fill_table): the
+        same table from a search whose visited set is a per-CTA hash table in device memory (as
+        optimal_moves(hash_table=True)), pos uint8 [M, 8].  Each item's rows are in ascending order
+        of their 8 bytes read as a little-endian 64-bit word (table.pos.view(torch.int64) ascends
+        per item), the same from call to call and whatever the launch plan.  status -3 means the
+        item reaches more than max_states states, the root included: a bound that depends on
+        max_states alone (None: the bound of optimal_moves(hash_table=True)'s plan).  A larger
+        max_states runs on fewer CTAs, as their tables and slabs share 4 GiB (ValueError when not
+        even one fits).  Reads back the row count only.  With 1..4 tiles hash_table changes nothing,
+        and max_states is taken with hash_table=True and 5..8 tiles only (ValueError)."""
         from .bfs import CudaStateTable, check_optimal_moves
-        check_optimal_moves(self.size, self.n_tiles, self.host_io, OPT_MAX_DEPTH, "state_table")
+        check_optimal_moves(self.size, self.n_tiles, self.host_io, OPT_MAX_DEPTH, "state_table", hash_table=bool(hash_table))
+        if max_states is not None:
+            if not (hash_table and self.n_tiles >= 5):
+                raise ValueError("state_table: max_states bounds the hash-table tables (hash_table=True, 5 to 8 tiles)")
+            if int(max_states) < 1:
+                raise ValueError(f"state_table: max_states must be >= 1 (got {max_states})")
         self._require_loaded()
         ids = self._search_items("state_table", ids, pos)
         if self._state_table is None:
             self._state_table = CudaStateTable(self)
-        return StateTable(*self._state_table.build(ids, pos, bool(device_bitmap)))
+        return StateTable(*self._state_table.build(ids, pos, bool(device_bitmap), bool(hash_table),
+                                                   None if max_states is None else int(max_states)))
 
     def _search_items(self, what: str, ids, pos: torch.Tensor | None) -> torch.Tensor | None:
         """The ids of a solver query as int32 on the device (None: every env), range-checked against
@@ -931,8 +948,10 @@ class StateTable:
     """The states reachable from items with their exact labels (BatchedTilerSliderEnv.state_table):
     item i owns rows offsets[i] .. offsets[i+1]-1 of pos / distance / mask.
       offsets   int64 [n+1]
-      status    int32 [n]: 0 enumerated, -3 the state space does not fit one CTA, -4 malformed root
-      pos       uint8 [M, pos_bytes]: the states, ascending by the search's perfect hash per item
+      status    int32 [n]: 0 enumerated, -3 the state space does not fit one CTA (hash_table=True:
+                more than max_states states), -4 malformed root
+      pos       uint8 [M, pos_bytes]: the states, per item ascending by the search's perfect hash (1
+                to 4 tiles) or as little-endian 64-bit words (5 to 8 tiles, hash_table=True)
       distance  int32 [M]: fewest moves that win (>= 1), -1 if no win is reachable
       mask      uint8 [M]: bit a set iff move a starts a shortest solution (0 where distance < 0)"""
     offsets: torch.Tensor

@@ -751,13 +751,29 @@ class OnChipSearch:
                 return {**plan, "gmem": True} if gmem else plan
         return None
 
-    def _plan_table(self) -> dict | None:
+    def _plan_table(self, max_states: int | None = None) -> dict | None:
         """The plan of the hash-table instance (5 to 8 tiles, marked table=True): the same CTA-per-SM
         loop as _plan with a ring of 8-byte entries alone in shared memory; per CTA a table of
         table_slots 8-byte slots (the largest power of two with grid x 12 x table_slots <=
         MAX_SCRATCH_BYTES, or the constructor's table_slots) and a slab of spill_per_cta =
         table_slots / 2 entries, the states an item may discover.  It does not depend on the envs'
-        walls, so it needs no free-cell read-back."""
+        walls, so it needs no free-cell read-back.  max_states (state tables): that bound instead,
+        spill_per_cta = max_states and table_slots the smallest power of two >= 2 x max_states, on
+        that plan's ring and as many of its CTAs as fit MAX_SCRATCH_BYTES (ValueError: not one)."""
+        if max_states is not None:
+            key = ("table", int(max_states))
+            if key not in self._plans:
+                base = self._plan_table()
+                if base is None:
+                    return None
+                spill = int(max_states)
+                slots = 1 << (2 * spill - 1).bit_length()
+                grid = min(base["grid"], self.MAX_SCRATCH_BYTES // (8 * slots + 8 * spill))
+                if grid < 1:
+                    raise ValueError(f"max_states={spill}: the table and slab of one CTA "
+                                     f"({8 * slots + 8 * spill} bytes) exceed {self.MAX_SCRATCH_BYTES} bytes")
+                self._plans[key] = dict(base, grid=grid, table_slots=slots, spill_per_cta=spill)
+            return self._plans[key]
         if "table" not in self._plans:
             self._plans["table"] = {}
             query = getattr(self.lib, self.TABLE_CTAS_PER_SM)
@@ -919,7 +935,8 @@ class CudaLocalKernels(OnChipSearch):
 def check_optimal_moves(size: int, n_tiles: int, host_io: bool, max_depth: int, what: str = "optimal_moves",
                         hash_table: bool = False) -> None:
     """The shapes ts_optimal_moves (and ts_state_table, `what`) covers, with hash_table also those
-    of ts_optimal_moves_table (5 to 8 tiles); raised before anything touches the device."""
+    of ts_optimal_moves_table (and ts_state_table_*_table: 5 to 8 tiles); raised before anything
+    touches the device."""
     if size > 8:
         raise ValueError(f"{what} covers board sizes up to 8 (got {size})")
     if not 1 <= n_tiles <= (8 if hash_table else 4):
@@ -983,34 +1000,45 @@ class CudaOptimalMoves(OnChipSearch):
 
 class CudaStateTable(OnChipSearch):
     """ctypes front-end of ts_state_table_count / ts_state_table_fill (K10, csrc/ts_state_table.cu)
-    for one batch: every state reachable from items (env id, positions), each with K9's distance
-    and mask.  Planned per call as CudaOptimalMoves.query plans (the most free cells among the
-    queried envs); both launches share the plan, so they agree on the items that fit."""
+    and, for 5 to 8 tiles, of their hash-table counterparts (K12, csrc/ts_table_state_table.cu) for
+    one batch: every state reachable from items (env id, positions), each with K9's distance and
+    mask.  Planned per call as CudaOptimalMoves.query plans (the most free cells among the queried
+    envs; K12: the table plan); both launches share the plan, so they agree on the items that fit."""
 
     CTAS_PER_SM = "ts_state_table_ctas_per_sm"
     GMEM_CTAS_PER_SM = "ts_state_table_gmem_ctas_per_sm"
+    TABLE_CTAS_PER_SM = "ts_state_table_table_ctas_per_sm"
     ARGS = StateTableArgs
 
-    def build(self, ids: torch.Tensor | None, pos: torch.Tensor | None = None,
-              device_bitmap: bool = False) -> tuple[torch.Tensor, ...]:
+    def build(self, ids: torch.Tensor | None, pos: torch.Tensor | None = None, device_bitmap: bool = False,
+              hash_table: bool = False, max_states: int | None = None) -> tuple[torch.Tensor, ...]:
         """(offsets int64[n+1], status int32[n], pos uint8[M, pos_bytes], distance int32[M], mask
         uint8[M]) of items (env `ids[i]`, root `pos[i]`) on the current stream; ids: int32 on the
         device, each in [0, n_envs) (None: every env); pos: contiguous uint8 [n, pos_bytes] on the
-        device (None: the envs' current positions); device_bitmap as in CudaOptimalMoves.query.
-        Reads back the free-cell maximum and the row count."""
+        device (None: the envs' current positions); device_bitmap as in CudaOptimalMoves.query;
+        hash_table: 5 to 8 tiles are enumerated by K12 (ts_state_table_*_table) on
+        _plan_table(max_states), whose slab both passes share (the fill sorts through it); it changes
+        nothing for 1 to 4 tiles.  Reads back the row count and, without the hash table, the
+        free-cell maximum."""
         t, dev = self.t, self.device
         n = t.n_envs if ids is None else ids.numel()
         offsets = torch.zeros(n + 1, dtype=torch.int64, device=dev)
         status = torch.full((n,), OPT_NOT_SEARCHED, dtype=torch.int32, device=dev)
         self.counters.zero_()
-        sp = self.search_plan(self._max_free_cells(ids, n), device_bitmap) if n else None
+        table = hash_table and t.n_tiles >= 5
+        if not n:
+            sp = None
+        elif table:
+            sp = self._plan_table(max_states)
+        else:
+            sp = self.search_plan(self._max_free_cells(ids, n), device_bitmap)
         if sp is None:                           # no items, or not even T free cells fit on chip
             return (offsets, status, torch.empty((0, t.pos_bytes), dtype=torch.uint8, device=dev),
                     torch.empty(0, dtype=torch.int32, device=dev), torch.empty(0, dtype=torch.uint8, device=dev))
         count = torch.empty(n, dtype=torch.int64, device=dev)
         # the count pass's slab (grid x spill_per_cta words, ~0.9 GB at the benchmark shape) lives for
         # this call only: it goes back to the allocator's cache on return, for the rows or K9's slab
-        spill = torch.empty(sp["grid"] * sp["spill_per_cta"], dtype=torch.int32, device=dev)
+        spill = torch.empty(sp["grid"] * sp["spill_per_cta"], dtype=torch.int64 if table else torch.int32, device=dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
         a = self._args(n_items=n, d_env_ids=None if ids is None else ids.data_ptr(),
                        d_item_pos=None if pos is None else pos.data_ptr(), bitmap_words=sp["bitmap_words"],

@@ -2,8 +2,8 @@
 // (ts_optimal.cu, the optimal-move query) and K10 (ts_state_table.cu, the state tables), share: the
 // CTA shape, canonical set-goal states, position byte -> bitboard bit, the perfect hash of a state
 // over the free cells of its puzzle that keys the visited bitmap, the successor function, the lut
-// fill, the bitmap clear and K9 and K10's root read (and their 64-bit siblings for K11's 5..8 tiles,
-// ts_table_search.cu); on the host the plan and env-table checks of K9 and K10, the plan check, the
+// fill, the bitmap clear and K9 and K10's root read (and their 64-bit siblings for K11 and K12's 5..8
+// tiles, ts_table_search.cu and ts_table_state_table.cu); on the host the plan and env-table checks of K9 and K10, the plan check, the
 // shared-memory size, the launch and the occupancy query, one each for the shared instances and the
 // device-memory-bitmap instances (GMEM) of 7x7 and 8x8 boards with four tiles.
 #pragma once

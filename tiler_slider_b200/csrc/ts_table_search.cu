@@ -4,15 +4,7 @@
 // counter, the forward level loop, the backward rule and the plan are K9's (ts_optimal.cu); the
 // visited set is a hash table in device memory whose size follows the states an item reaches.
 //
-//   Table: CTA b owns d_table[b * table_slots ..], table_slots a power of two; open addressing with
-//      linear probing from a 64-bit mix of the key.  A key is the state word; every position byte is
-//      < 128, so bit 7 of each byte is free, and those eight bits hold:
-//        bit 7             MARK: the state is good (backward pass)
-//        bits 15, 23       the lowest optimal move of a good state (plan)
-//        bits 31 .. 63     the item epoch of the slot (5 bits, 1 .. 31)
-//      A slot whose epoch is not the current item's is empty, so an item starts on an empty table
-//      without clearing it; the slice is cleared only when the epoch wraps (every 31 items of a CTA,
-//      and before its first item, as the buffer's contents on entry are undefined).
+//   Table: the per-CTA hash table of ts_hash_table.cuh (keys, flag bits, item epochs).
 //   Bound: the slab holds spill_per_cta states; the item stops with TS_OPT_NOT_SEARCHED once it has
 //      discovered more (K9's rule), and table_slots >= 2 * spill_per_cta.  Inserts stop once the
 //      level has met the goal or overflowed, so a table holds at most spill_per_cta + 255 keys of an
@@ -23,60 +15,9 @@
 //   Backward: K9's rule; the flags of level k are written into bit 7 / the move bits of the level's
 //      slab entries, which keep their keys, and after a barrier ORed into the states' slots.
 //   Plan: from the root, the move stored in the slot of each state reached.
-#include "ts_bfs_local.cuh"
+#include "ts_hash_table.cuh"
 
 namespace ts {
-
-constexpr uint64_t TAB_KEY = 0x7F7F7F7F7F7F7F7Full;        // the position bytes of a slot
-constexpr uint64_t TAB_MARK = 1ull << 7;
-constexpr uint64_t TAB_MOVE = 1ull << 15 | 1ull << 23;
-constexpr uint64_t TAB_EPOCH = 0x8080808080000000ull;      // bits 31, 39, 47, 55, 63
-constexpr uint32_t TAB_EPOCHS = 31;
-constexpr uint32_t TAB_WON = 1u, TAB_OVER = 2u;
-
-__device__ __forceinline__ uint64_t epoch_bits(uint32_t e) {
-    uint64_t b = 0;
-#pragma unroll
-    for (int i = 0; i < 5; ++i) b |= (uint64_t)((e >> i) & 1u) << (31 + 8 * i);
-    return b;
-}
-__device__ __forceinline__ uint64_t move_bits(uint32_t m) { return (uint64_t)(m & 1u) << 15 | (uint64_t)(m >> 1) << 23; }
-__device__ __forceinline__ uint32_t move_of(uint64_t e) { return (uint32_t)((e >> 15) & 1u) | (uint32_t)((e >> 22) & 2u); }
-// first slot of key q's probe sequence (the splitmix64 finaliser)
-__device__ __forceinline__ uint64_t slot_of(uint64_t q, uint64_t smask) {
-    q = (q ^ (q >> 30)) * 0xBF58476D1CE4E5B9ull;
-    q = (q ^ (q >> 27)) * 0x94D049BB133111EBull;
-    return (q ^ (q >> 31)) & smask;
-}
-
-// insert q: 1 new (this thread's CAS claimed an empty slot), 0 present, -1 the table is full.  Slots
-// are read through L2 (ld.cg): other threads of the CTA claim them with atomics meanwhile.
-__device__ __forceinline__ int table_insert(uint64_t* table, uint64_t smask, uint64_t ep, uint64_t q) {
-    uint64_t h = slot_of(q, smask);
-#pragma unroll 1
-    for (uint64_t n = 0; n <= smask; ++n, h = (h + 1) & smask) {
-        uint64_t v = __ldcg(table + h);
-        if ((v & TAB_EPOCH) != ep) {
-            const uint64_t old = atomicCAS((unsigned long long*)(table + h), (unsigned long long)v, (unsigned long long)(q | ep));
-            if (old == v) return 1;
-            v = old;                              // claimed meanwhile, in this epoch
-        }
-        if ((v & TAB_KEY) == q) return 0;
-    }
-    return -1;
-}
-
-// the slot holding q, or -1 when q is not in the table
-__device__ __forceinline__ long long table_find(const uint64_t* table, uint64_t smask, uint64_t ep, uint64_t q) {
-    uint64_t h = slot_of(q, smask);
-#pragma unroll 1
-    for (uint64_t n = 0; n <= smask; ++n, h = (h + 1) & smask) {
-        const uint64_t v = __ldcg(table + h);
-        if ((v & TAB_EPOCH) != ep) return -1;
-        if ((v & TAB_KEY) == q) return (long long)h;
-    }
-    return -1;
-}
 
 // PLAN as in K9: the instance that writes d_plan
 template <int S, int T, bool PLAN>
@@ -281,41 +222,12 @@ __global__ void __launch_bounds__(SEARCH_THREADS) table_search_kernel(const ts_o
 
 static constexpr auto K11 = [](auto S, auto T) { return table_search_kernel<decltype(S)::value, decltype(T)::value, false>; };
 static constexpr auto K11_PLAN = [](auto S, auto T) { return table_search_kernel<decltype(S)::value, decltype(T)::value, true>; };
-
-// K11 instance <a.size, a.n_tiles, PLAN> with the ring alone in dynamic shared memory: launched on
-// `grid` CTAs, or, when ctas_per_sm is given, asked how many of its CTAs fit an SM
-template <class KernelOf>
-static cudaError_t table_kernel(KernelOf&& kernel_of, const ts_optimal_moves_args& a, uint64_t* d_table, uint64_t table_slots,
-                                int grid, int* ctas_per_sm, cudaStream_t st) {
-    const size_t smem = (size_t)a.queue_smem * sizeof(uint64_t);
-    return dispatch_size(a.size, [&](auto S) {
-        constexpr int SV = decltype(S)::value;
-        if constexpr (SV < 3) return cudaErrorInvalidValue;                          // no smaller board holds five tiles
-        else return dispatch_tiles<5, 8>(a.n_tiles, [&](auto T) {
-            const auto kernel = kernel_of(S, T);
-            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            if (ctas_per_sm) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kernel, SEARCH_THREADS, smem);
-            kernel<<<grid, SEARCH_THREADS, smem, st>>>(a, d_table, table_slots);
-            return cudaGetLastError();
-        });
-    });
-}
+// dynamic shared memory of K11: the ring alone
+static size_t k11_smem(const ts_optimal_moves_args& a) { return (size_t)a.queue_smem * sizeof(uint64_t); }
 
 }  // namespace ts
 
 using namespace ts;
-
-// K9's plan checks (check_item_plan) for 5..8 tiles with no bitmap: shape, goal mode, ring
-static int table_check_plan(const ts_optimal_moves_args* a) {
-    if (!a) return TS_E_NULL_POINTER;
-    if (a->size < 1 || a->size > TS_MAX_SIZE) return TS_E_BAD_SIZE;
-    if (a->size > 8) return TS_E_UNSUPPORTED;
-    if (a->n_tiles < 5 || a->n_tiles > 8) return TS_E_UNSUPPORTED;             // 64-bit states; 1..4 tiles: K9
-    if (a->goal_mode != TS_GOAL_ORDERED && a->goal_mode != TS_GOAL_SET) return TS_E_BAD_ARGUMENT;
-    if (a->bitmap_words != 0 || a->queue_smem < 32 || (a->queue_smem & (a->queue_smem - 1))) return TS_E_BAD_ARGUMENT;
-    return 0;
-}
 
 extern "C" {
 
@@ -325,8 +237,8 @@ int ts_optimal_moves_table_ctas_per_sm(const ts_optimal_moves_args* a, int* ctas
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (e == cudaSuccess) e = a->d_plan ? table_kernel(K11_PLAN, *a, nullptr, 0, 0, ctas_per_sm, nullptr)
-                                        : table_kernel(K11, *a, nullptr, 0, 0, ctas_per_sm, nullptr);
+    if (e == cudaSuccess) e = a->d_plan ? table_kernel(K11_PLAN, *a, k11_smem(*a), nullptr, 0, 0, ctas_per_sm, nullptr)
+                                        : table_kernel(K11, *a, k11_smem(*a), nullptr, 0, 0, ctas_per_sm, nullptr);
     if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
     return 0;
 }
@@ -337,13 +249,11 @@ int ts_optimal_moves_table(const ts_optimal_moves_args* a, uint64_t* d_table, in
     if (a->max_depth < 1 || a->max_depth > TS_OPT_MAX_DEPTH || a->spill_per_cta < 1 || a->spill_per_cta > 0xFFFFFFFFll)
         return TS_E_BAD_ARGUMENT;
     if (!a->d_spill || !a->d_counters || !a->d_distance || !a->d_mask) return TS_E_NULL_POINTER;
-    if (table_slots < 2 * a->spill_per_cta || (table_slots & (table_slots - 1))) return TS_E_BAD_ARGUMENT;
-    if (!d_table) return TS_E_NULL_POINTER;
-    if (reinterpret_cast<uintptr_t>(d_table) % 8 || reinterpret_cast<uintptr_t>(a->d_spill) % 8) return TS_E_MISALIGNED;
+    if (int rc = table_check_buffer(a, d_table, table_slots)) return rc;
     if (a->n_items == 0) return 0;
     if (grid < 1) return TS_E_BAD_ARGUMENT;
-    return (int)(a->d_plan ? table_kernel(K11_PLAN, *a, d_table, (uint64_t)table_slots, grid, nullptr, (cudaStream_t)stream)
-                           : table_kernel(K11, *a, d_table, (uint64_t)table_slots, grid, nullptr, (cudaStream_t)stream));
+    return (int)(a->d_plan ? table_kernel(K11_PLAN, *a, k11_smem(*a), d_table, (uint64_t)table_slots, grid, nullptr, (cudaStream_t)stream)
+                           : table_kernel(K11, *a, k11_smem(*a), d_table, (uint64_t)table_slots, grid, nullptr, (cudaStream_t)stream));
 }
 
 }  // extern "C"
